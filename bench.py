@@ -5,6 +5,7 @@
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
       bench.py --gpus N --steps K --warmup W
   python bench.py --impl reference ...     # the CPU restatement of the reference on the host cores
+  python bench.py ... --dump-outputs bench_outputs/a   # also writes the last timed step's outputs as <name>.npy (compare two builds)
 
 BASELINE.json's metric has two halves and the line carries both, plus one nested row per remaining GPU config:
   * top level  — scanned bp/s on configs[3], the scan sweep: 500 PWMs (len 8-40) over 10M x 200 bp (2 Gbp), forward +
@@ -41,7 +42,9 @@ FP32_SIMT_TFLOPS = 148 * 128 * 2 * 1.965e9 / 1e12   # 148 SMs x 128 FMA lanes x 
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=3,
+                    help="timed steps of every timed loop: scan passes, bench steps of --train-steps / --c3-steps optimiser steps (10 of the "
+                         "64-group row, 200 of the 16-group row), code-retrieval calls, score > 0 scans, config-5 steps, and their end-to-end legs")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="all", choices=["all", "both", "scan", "train", "config3", "config5"])
@@ -60,7 +63,41 @@ def parse():
     ap.add_argument("--c5-check-bp", type=int, default=10_000_000, help="prefix of the config-5 sequence the oracle re-counts")
     ap.add_argument("--cpu-seconds", type=float, default=15.0, help="target CPU time of each cpu_baseline sample")
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what each timed path returned in its last step as DIR/<name>.npy (float32 or "
+                         "float64, at most 64 MB in all); the inputs depend on the arguments only, so two builds can be compared file by file")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
+    return args
+
+
+OUTPUTS = {}                                      # name -> what a timed path returned in its last step (--dump-outputs), rank 0
+DUMP_MAX_BYTES = 64 << 20
+CODES_MAX_ROWS = 1_900_000                        # 30.4 MB of float32 per code-retrieval path (two paths + the rest < 64 MB)
+
+
+def code_records(recs, n_seqs):
+    """code records as (n, 4) float32 rows (seq, fil, position, magnitude), sorted, so that two builds compare row by row; exact
+    while sequence indices stay below 2^24.  When the library's bound of 64 records per sequence could exceed CODES_MAX_ROWS, only
+    the records of every k-th sequence are kept: a choice by content, so the kept rows stay comparable whatever the record count."""
+    a = np.stack([recs["seq"], recs["fil"], recs["position"], np.ascontiguousarray(recs["mag_f16"]).view(np.float16)], axis=1).astype(np.float32)
+    k = -(-64 * n_seqs // CODES_MAX_ROWS)
+    if k > 1:
+        a = a[np.asarray(recs["seq"]) % k == 0]
+    return a[np.lexsort(a.T[::-1])]
+
+
+def dump_outputs(d):
+    total = sum(a.nbytes for a in OUTPUTS.values())
+    if total > DUMP_MAX_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed {DUMP_MAX_BYTES}")
+    os.makedirs(d, exist_ok=True)
+    for name, a in OUTPUTS.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(d, f"{name}.npy"), a)
 
 
 class ClockSampler:
@@ -286,6 +323,8 @@ def bench_scan(args, ctx, torch, dist, world, rank, local, dev, stream):
     if rank == 0:
         sampler.start()
     ms_step, counts, t_scan, t_cnt, n_scan_launch, n_launch = timed(step_resident, args.steps, args.warmup)
+    if rank == 0:
+        OUTPUTS["scan_counts"] = counts.astype(np.float64)
     t_verify = timed.t_verify
     scan_path = mblib.scan_last_path(ctx)                                     # 1: tcgen05 pre-filter + exact re-scoring, 0: SIMT scan_kernel
     clocks = sampler.stop() if rank == 0 else None
@@ -299,10 +338,11 @@ def bench_scan(args, ctx, torch, dist, world, rank, local, dev, stream):
     barrier()
     g0, g1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     g0.record(stream)
-    ctx.scan(s_gt0, pw, lens, None, want_hits=False, want_counts=True, reduce=True)
+    for _ in range(args.steps):
+        ctx.scan(s_gt0, pw, lens, None, want_hits=False, want_counts=True, reduce=True)
     g1.record(stream)
     barrier()
-    tg = torch.tensor([g0.elapsed_time(g1)], dtype=torch.float64, device=dev)
+    tg = torch.tensor([g0.elapsed_time(g1) / args.steps], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(tg, op=dist.ReduceOp.MAX)
     ms_gt0 = float(tg.item())
@@ -395,7 +435,7 @@ def flops_per_seq(Lb):
     return 3.0 * 2.0 * mac
 
 
-def bench_train(args, ctx, torch, dist, world, rank, local, dev, N, Lb, opt_steps, index, groups=1, e2e_leg=True, extras=True, warm_mult=50):
+def bench_train(args, ctx, torch, dist, world, rank, local, dev, name, N, Lb, opt_steps, index, groups=1, e2e_leg=True, extras=True, warm_mult=50):
     from motifs_jl_b200 import model as mdl, synth
     from motifs_jl_b200._lib import CscModel
     hp = mdl.Hyperparam()
@@ -450,7 +490,7 @@ def bench_train(args, ctx, torch, dist, world, rank, local, dev, N, Lb, opt_step
         torch.cuda.synchronize()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         l0 = ctx.last_timing()[1]["csc"]
-        n_bench = max(1, args.steps)
+        n_bench = args.steps
         e0.record(side)
         t0 = time.perf_counter()
         for _ in range(n_bench * opt_steps):
@@ -461,6 +501,9 @@ def bench_train(args, ctx, torch, dist, world, rank, local, dev, N, Lb, opt_step
         torch.cuda.synchronize()
         wall = time.perf_counter() - t0
         launches = int(ctx.last_timing()[1]["csc"] - l0)
+        if rank == 0:
+            OUTPUTS[f"{name}_loss_l1"] = np.array([state["loss"], state["l1"]], np.float32)
+            OUTPUTS[f"{name}_params"] = model.get_params()
         tt = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=dev)
         if world > 1:
             dist.all_reduce(tt, op=dist.ReduceOp.MAX)
@@ -482,7 +525,7 @@ def bench_train(args, ctx, torch, dist, world, rank, local, dev, N, Lb, opt_step
             torch.cuda.synchronize()
             f0, f1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             f0.record(side)
-            for _ in range(opt_steps):
+            for _ in range(args.steps * opt_steps):
                 opt_step_host()
             f1.record(side)
             if world > 1:
@@ -491,7 +534,7 @@ def bench_train(args, ctx, torch, dist, world, rank, local, dev, N, Lb, opt_step
             t2 = torch.tensor([f0.elapsed_time(f1)], dtype=torch.float64, device=dev)
             if world > 1:
                 dist.all_reduce(t2, op=dist.ReduceOp.MAX)
-            ms_e2e_opt = float(t2.item()) / opt_steps
+            ms_e2e_opt = float(t2.item()) / (args.steps * opt_steps)
         if rank == 0:
             peaks = load_peaks()
             seq_s = nb * world * opt_steps / (ms_bench_step / 1e3)
@@ -529,7 +572,7 @@ def bench_train(args, ctx, torch, dist, world, rank, local, dev, N, Lb, opt_step
             # 6 per launch sequence, fp32 (the parity path) and with the dense contraction on the tcgen05 BF16 kernel (stated tolerance); with a
             # communicator the batches are sharded over the ranks and the records all-gathered
             res = {}
-            for name, tc in (("fp32", False), ("tensor_cores_bf16", True)):
+            for tag, tc in (("fp32", False), ("tensor_cores_bf16", True)):
                 n_dec = n_train - n_train % hp.batch_size
                 G = max(1, min(1024, -(-(n_dec // hp.batch_size) // world)))
                 mc = CscModel(ctx, hp, Lb, n_groups=G, forward_only=True, tensor_cores=tc)
@@ -540,16 +583,18 @@ def bench_train(args, ctx, torch, dist, world, rank, local, dev, N, Lb, opt_step
                 torch.cuda.synchronize()
                 c0, c1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
                 c0.record(side)
-                for _ in range(3):
-                    mc.codes(seqs, shard="comm" if world > 1 else None)
+                for _ in range(args.steps):
+                    last = mc.codes(seqs, shard="comm" if world > 1 else None)
                 c1.record(side)
                 if world > 1:
                     dist.barrier()
                 torch.cuda.synchronize()
-                tc_ms = torch.tensor([c0.elapsed_time(c1) / 3], dtype=torch.float64, device=dev)
+                if rank == 0:
+                    OUTPUTS[f"{name}_codes_{tag}"] = code_records(last, n_dec)
+                tc_ms = torch.tensor([c0.elapsed_time(c1) / args.steps], dtype=torch.float64, device=dev)
                 if world > 1:
                     dist.all_reduce(tc_ms, op=dist.ReduceOp.MAX)
-                res[name] = (recs, float(tc_ms.item()), n_dec)
+                res[tag] = (recs, float(tc_ms.item()), n_dec)
                 mc.free()
             if rank == 0:
                 r32, ms32, n_dec = res["fp32"]
@@ -573,12 +618,14 @@ def bench_train(args, ctx, torch, dist, world, rank, local, dev, N, Lb, opt_step
                 mg.step_begin(seqs, r2.permutation(n_train)[:6 * G]); mg.adabelief_step()
             torch.cuda.synchronize()
             g0, g1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            nst = 200
+            nst = 200 * args.steps                                         # bench steps of 200 optimiser steps
             g0.record(side)
             for _ in range(nst):
-                mg.step_begin(seqs, r2.permutation(n_train)[:6 * G]); mg.adabelief_step()
+                mg.step_begin(seqs, r2.permutation(n_train)[:6 * G]); loss_l1 = mg.adabelief_step()
             g1.record(side)
             torch.cuda.synchronize()
+            OUTPUTS[f"{name}_batched_groups_loss_l1"] = np.array(loss_l1, np.float32)
+            OUTPUTS[f"{name}_batched_groups_params"] = mg.get_params()
             msg = g0.elapsed_time(g1) / nst
             out["batched_groups"] = {"groups_per_step": G, "global_batch": 6 * G, "value": 6 * G / (msg / 1e3), "unit": "seq/s",
                                      "ms_per_optimizer_step": msg,
@@ -632,7 +679,7 @@ def bench_long_scan(args, ctx, torch, dev, stream):
     for _ in range(2):
         step()
     torch.cuda.synchronize()
-    n = max(2, args.steps)
+    n = args.steps
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record(stream)
     for _ in range(n):
@@ -640,6 +687,8 @@ def bench_long_scan(args, ctx, torch, dev, stream):
     e1.record(stream)
     torch.cuda.synchronize()
     ms_step = e0.elapsed_time(e1) / n
+    OUTPUTS["config5_long_scan_fg_counts"] = c.astype(np.float64)
+    OUTPUTS["config5_long_scan_bg_counts"] = cb.astype(np.float64)
     # end to end: both sequences from pinned host ASCII each step
     bg_host = torch.from_numpy(bg.to_ascii().reshape(-1)).pin_memory()
 
@@ -655,10 +704,11 @@ def bench_long_scan(args, ctx, torch, dev, stream):
     torch.cuda.synchronize()
     f0, f1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     f0.record(stream)
-    c1, c2 = step_e2e()
+    for _ in range(n):
+        c1, c2 = step_e2e()
     f1.record(stream)
     torch.cuda.synchronize()
-    ms_e2e = f0.elapsed_time(f1)
+    ms_e2e = f0.elapsed_time(f1) / n
     assert np.array_equal(c1, c) and np.array_equal(c2, cb)
 
     class _D:
@@ -771,15 +821,16 @@ def main():
         out = bench_scan(args, ctx, torch, dist, world, rank, local, dev, stream)
     nested = {}
     if wl in ("all", "both", "train"):
-        nested["training"] = bench_train(args, ctx, torch, dist, world, rank, local, dev, args.train_nseq, args.train_seqlen, args.train_steps, 1)
+        nested["training"] = bench_train(args, ctx, torch, dist, world, rank, local, dev, "training", args.train_nseq, args.train_seqlen,
+                                         args.train_steps, 1)
     if wl in ("all", "config3"):
-        nested["config3_training"] = bench_train(args, ctx, torch, dist, world, rank, local, dev, args.c3_nseq, args.c3_seqlen, args.c3_steps, 2,
-                                                 groups=args.c3_groups, e2e_leg=False, extras=False)
+        nested["config3_training"] = bench_train(args, ctx, torch, dist, world, rank, local, dev, "config3_training", args.c3_nseq, args.c3_seqlen,
+                                                 args.c3_steps, 2, groups=args.c3_groups, e2e_leg=False, extras=False)
     if wl == "all" and args.c3_groups == 1:
         # the same data-parallel run with 64 reference batches per rank and optimiser step (global batch 384 x ranks): what the ranks are
         # worth once a step carries enough work to fill a GPU (the many-group launch path of the library; DESIGN.md section 3.2)
-        nested["config3_training_64groups"] = bench_train(args, ctx, torch, dist, world, rank, local, dev, args.c3_nseq, args.c3_seqlen, 10, 2,
-                                                          groups=64, e2e_leg=False, extras=False, warm_mult=3)
+        nested["config3_training_64groups"] = bench_train(args, ctx, torch, dist, world, rank, local, dev, "config3_training_64groups",
+                                                          args.c3_nseq, args.c3_seqlen, 10, 2, groups=64, e2e_leg=False, extras=False, warm_mult=3)
     if wl in ("all", "config5") and rank == 0:
         nested["config5_long_scan"] = bench_long_scan(args, ctx, torch, dev, stream)
     if world > 1:
@@ -792,6 +843,8 @@ def main():
         for k, v in nested.items():
             out[k] = v
             out["gpu_launches"] = int(out.get("gpu_launches") or 0) + int((v or {}).get("gpu_launches") or 0)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs)
         print(json.dumps(out), flush=True)
     ctx.close()
     if world > 1:

@@ -86,6 +86,8 @@ struct mb200_csc {
     bool fused_bwd_df = false, no_fused_df = false; size_t fzd_smem = 0;      // loss + ADMM_DF reverse pass as one kernel (needs fused_bwd)
     size_t op_xyz_begin = 0, op_xyz_end = 0;                // tape ops of the ADMM_XYZ passes: [begin, end)
     Buf zero_al{}, zero_be{};
+    std::vector<SlotRange> slots; SlotRange* slots_dev = nullptr;      // block partials of the scalar adjoints (k_sum_slots)
+    size_t grad_extra = 0;          // floats of the grad arena past `arena`: the slices and slots above, which the data arena has no use for
 };
 
 namespace {
@@ -147,7 +149,26 @@ static void build_tape(mb200_csc* s, bool xyz_only) {
     }
     s->Deff = B.alloc(nD, "D0"); s->Feff = B.alloc(nF, "F0"); s->Fnrm0 = B.alloc(d.K);
     s->loss = B.alloc((size_t)d.G * 3 + 4 + d.K, "loss");       // per-group {loss, rec, syn}, then the K per-filter terms of l1(F)
+    // The reverse pass adds no shared adjoint with float atomics, whose order (and so the rounding) changes from run to run: the adjoints
+    // of the prepared D and F get one slice per group, the warm-up's adjoint of D one slice per sequence, the scalar adjoints one slot per
+    // block, and the reverse of prep sums them in a fixed order first (k_sum_slices, k_sum_slots).  Only shapes with fl x M > 512 or
+    // M > 64 keep the per-element warm-up adjoint k_warm_zy_bwd, which still adds with atomics.
+    const bool wz_s = d.fl * d.M <= 512 && d.M <= 64;                 // k_warm_zy_bwd_s: one CTA per sequence
+    const int nDs = xyz_only ? 0 : d.G + (wz_s ? d.NS : 0);
+    // they live in the grad arena only, past the `arena` floats both arenas share: offsets below are relative to S->grad + S->arena
+    s->grad_extra = 0;
+    auto galloc = [s](size_t n) -> size_t { const size_t o = s->grad_extra; s->grad_extra += (n + 63) & ~(size_t)63; return o; };
+    const size_t gDs = galloc((size_t)nDs * nD), gFs = galloc(xyz_only ? 0 : (size_t)d.G * nF);
+    s->slots.clear();
+    auto slots = [&](size_t blocks, std::initializer_list<int> idx) -> size_t {      // offset of blocks x |idx| partials
+        if (xyz_only) return 0;
+        const size_t p = galloc(blocks * idx.size());
+        int lane = 0;
+        for (int i : idx) s->slots.push_back({i, (int32_t)blocks, (int32_t)idx.size(), 0, (int64_t)(p + lane++)});
+        return p;
+    };
     mb200_csc* S = s;
+#define GX(o) (S->grad + S->arena + (o))
     auto& T = s->tape;
     T.clear();
 
@@ -163,6 +184,9 @@ static void build_tape(mb200_csc* s, bool xyz_only) {
                          if (S->tensor) lk(k_tc_prep_F3, nblk((int64_t)d.h * TC_CH * d.K * 8, 256), 256, 0, q, S->data + Fe.off, S->tc_F, d.h, d.M2, d.K);
                      },
                      [=](cudaStream_t q) {
+                         lk(k_sum_slices, nblk(nD, 256), 256, 0, q, (const float*)GX(gDs), nDs, nD, S->grad + De.off);
+                         lk(k_sum_slices, nblk(nF, 256), 256, 0, q, (const float*)GX(gFs), d.G, nF, S->grad + Fe.off);
+                         lk(k_sum_slots, n_sc, 256, 0, q, (const float*)GX(0), (const SlotRange*)S->slots_dev, (int)S->slots.size(), S->grad + sc.off);
                          ScalarSegs tr = S->segs; tr.nseg = 7;      // the warm-up scalars (segment 7) are not trained
                          lk(k_prep_scalars_bwd, 1, 256, 0, q, S->p_raw, S->grad + sc.off, S->g_raw, tr);
                          lk(k_prep_D_bwd, nblk(d.fl * d.M, 128), 128, 0, q, S->p_raw + S->off_D, S->data + De.off, S->grad + De.off, S->g_raw + S->off_D, d);
@@ -172,8 +196,13 @@ static void build_tape(mb200_csc* s, bool xyz_only) {
     }
     const Buf sc = s->sc, De = s->Deff, Fe = s->Feff;
     float* const SC = nullptr; (void)SC;
+    // where the reverse pass adds the adjoint of filter f (group stride gs): the shared prepared D and F go to their per-group slices
+    auto gfilt = [=](Buf f, int64_t gs) -> std::pair<float*, int64_t> {
+        if (gs == 0 && f.off == De.off) return {GX(gDs), nD};
+        if (gs == 0 && f.off == Fe.off) return {GX(gFs), nF};
+        return {S->grad + f.off, gs};
+    };
 #define SCP (S->data + sc.off)
-#define DSCP (S->grad + sc.off)
 
     // helpers that append one op each -------------------------------------------------------------
     const bool fastK = (d.K == 24), fastM = (d.M <= 64);
@@ -255,7 +284,7 @@ static void build_tape(mb200_csc* s, bool xyz_only) {
                      [=](cudaStream_t q) {
                          // d ca, d cb: corr_sig form with signal = d out ; d filt: dgrad form with signal = d out
                          par2(q, [=](cudaStream_t r) { run_corr_sig(S->grad + out.off, 0.f, S->data + filt.off, gs, S->grad + ca.off, S->grad + cb.off, 1, r); },
-                                 [=](cudaStream_t r) { run_dgrad(S->data + ca.off, S->data + cb.off, S->grad + out.off, 0.f, S->grad + filt.off, gs, 1, r); });
+                                 [=](cudaStream_t r) { const auto o = gfilt(filt, gs); run_dgrad(S->data + ca.off, S->data + cb.off, S->grad + out.off, 0.f, o.first, o.second, 1, r); });
                      },
                      nm});
     };
@@ -263,7 +292,7 @@ static void build_tape(mb200_csc* s, bool xyz_only) {
         T.push_back({[=](cudaStream_t q) { run_corr_sig(S->data + sig.off, sgn, S->data + filt.off, gs, S->data + oa.off, S->data + ob.off, 0, q); },
                      [=](cudaStream_t q) {
                          par2(q, [=](cudaStream_t r) { run_recon(S->grad + oa.off, S->grad + ob.off, S->data + filt.off, gs, S->grad + sig.off, 1, r); },
-                                 [=](cudaStream_t r) { run_dgrad(S->grad + oa.off, S->grad + ob.off, S->data + sig.off, sgn, S->grad + filt.off, gs, 1, r); });
+                                 [=](cudaStream_t r) { const auto o = gfilt(filt, gs); run_dgrad(S->grad + oa.off, S->grad + ob.off, S->data + sig.off, sgn, o.first, o.second, 1, r); });
                      },
                      nm});
     };
@@ -281,7 +310,7 @@ static void build_tape(mb200_csc* s, bool xyz_only) {
         T.push_back({[=](cudaStream_t q) { run_corr2d(S->data + A.off, S->data + filt.off, gs, S->data + out.off, 0, q); },
                      [=](cudaStream_t q) {
                          par2(q, [=](cudaStream_t r) { run_tconv(S->grad + out.off, glist, S->data + filt.off, gs, S->grad + A.off, 1, r); },
-                                 [=](cudaStream_t r) { run_fgrad(S->data + A.off, S->grad + out.off, glist, S->grad + filt.off, gs, 1, r); });
+                                 [=](cudaStream_t r) { const auto o = gfilt(filt, gs); run_fgrad(S->data + A.off, S->grad + out.off, glist, o.first, o.second, 1, r); });
                      },
                      nm});
     };
@@ -291,7 +320,7 @@ static void build_tape(mb200_csc* s, bool xyz_only) {
         T.push_back({[=](cudaStream_t q) { run_tconv(S->data + x.off, xl, S->data + filt.off, gs, S->data + out.off, 0, q); },
                      [=](cudaStream_t q) {
                          par2(q, [=](cudaStream_t r) { run_corr2d_kept(S->grad + out.off, S->data + filt.off, gs, xb, S->grad + x.off, 1, r); },
-                                 [=](cudaStream_t r) { run_fgrad(S->grad + out.off, S->data + x.off, xl, S->grad + filt.off, gs, 1, r); });
+                                 [=](cudaStream_t r) { const auto o = gfilt(filt, gs); run_fgrad(S->grad + out.off, S->data + x.off, xl, o.first, o.second, 1, r); });
                      },
                      nm});
     };
@@ -331,8 +360,9 @@ static void build_tape(mb200_csc* s, bool xyz_only) {
         xlist[xout.off] = xl; xbits[xout.off] = bo;
         const bool hp_ = xprev != nullptr; const Buf xp = hp_ ? *xprev : Buf{};
         const size_t smem = (size_t)d.l * d.K * 4;
+        const size_t om_sl = om_train ? slots((size_t)d.NS, {i_om}) : 0;
         T.push_back({[=](cudaStream_t q) { lk(k_topq_s, d.NS, 256, smem, q, hp_ ? S->data + xp.off : nullptr, S->data + g.off, SCP, i_om, coef, S->data + xout.off, S->bits + bo, LCNT(xl), LIDX(xl), LVAL(xl), d); },
-                     [=](cudaStream_t q) { lk(k_topq_s_bwd, d.NS, 256, 0, q, S->bits + bo, S->data + g.off, SCP, i_om, coef, S->grad + xout.off, hp_ ? S->grad + xp.off : nullptr, S->grad + g.off, DSCP, om_train, LCNT(glist), LIDX(glist), LVAL(glist), d); },
+                     [=](cudaStream_t q) { lk(k_topq_s_bwd, d.NS, 256, 0, q, S->bits + bo, S->data + g.off, SCP, i_om, coef, S->grad + xout.off, hp_ ? S->grad + xp.off : nullptr, S->grad + g.off, om_train ? GX(om_sl) : nullptr, om_train, LCNT(glist), LIDX(glist), LVAL(glist), d); },
                      nm});
     };
 
@@ -340,7 +370,7 @@ static void build_tape(mb200_csc* s, bool xyz_only) {
     Buf z = B.alloc(nZ), y = B.alloc(nZ);
     T.push_back({[=](cudaStream_t q) { lk(k_warm_zy, nblk(nZ, 256), 256, 0, q, S->bases, S->data + De.off, SCP, S->i_eta_w, S->i_lam_w, S->data + z.off, S->data + y.off, d); },
                  [=](cudaStream_t q) {
-                     if (batched && d.fl * d.M <= 512 && d.M <= 64) lk(k_warm_zy_bwd_s, d.NS, 512, 0, q, S->bases, SCP, S->i_eta_w, S->data + z.off, S->data + y.off, S->grad + z.off, S->grad + y.off, S->grad + De.off, d);
+                     if (wz_s) lk(k_warm_zy_bwd_s, d.NS, 512, 0, q, S->bases, SCP, S->i_eta_w, S->data + z.off, S->data + y.off, S->grad + z.off, S->grad + y.off, GX(gDs + (size_t)d.G * nD), d);
                      else lk(k_warm_zy_bwd, nblk(nZ, 256), 256, 0, q, S->bases, SCP, S->i_eta_w, S->data + z.off, S->data + y.off, S->grad + z.off, S->grad + y.off, S->grad + De.off, d);
                  },
                  "warm_zy"});
@@ -374,8 +404,9 @@ static void build_tape(mb200_csc* s, bool xyz_only) {
                   XP->i_eta = i_eta; XP->i_lam = i_lam; XP->i_rho = i_rho; XP->i_om = i_om; XP->x_in = (int64_t)x.off; XP->xl_in = cur_xl; XP->al_out = -1; XP->be_out = -1; }
         {
             const Buf zc = z, yc = y, fxc = fx, alc = al, bec = be;
+            const size_t zy_sl = slots(nblk(nZ, 256), {i_eta, i_lam, i_rho});
             T.push_back({[=](cudaStream_t q) { lk(k_zy_update, nblk(nZ, 256), 256, 0, q, S->data + zc.off, S->data + yc.off, S->data + gz.off, S->data + gy.off, S->data + fxc.off, S->data + alc.off, S->data + bec.off, SCP, i_eta, i_lam, i_rho, S->data + zn.off, S->data + yn.off, d); },
-                         [=](cudaStream_t q) { lk(k_zy_update_bwd, nblk(nZ, 256), 256, 0, q, S->data + zc.off, S->data + yc.off, S->data + gz.off, S->data + gy.off, S->data + fxc.off, S->data + alc.off, S->data + bec.off, SCP, i_eta, i_lam, i_rho, S->data + zn.off, S->data + yn.off, S->grad + zn.off, S->grad + yn.off, S->grad + zc.off, S->grad + yc.off, S->grad + gz.off, S->grad + gy.off, S->grad + fxc.off, S->grad + alc.off, S->grad + bec.off, DSCP, d); },
+                         [=](cudaStream_t q) { lk(k_zy_update_bwd, nblk(nZ, 256), 256, 0, q, S->data + zc.off, S->data + yc.off, S->data + gz.off, S->data + gy.off, S->data + fxc.off, S->data + alc.off, S->data + bec.off, SCP, i_eta, i_lam, i_rho, S->data + zn.off, S->data + yn.off, S->grad + zn.off, S->grad + yn.off, S->grad + zc.off, S->grad + yc.off, S->grad + gz.off, S->grad + gy.off, S->grad + fxc.off, S->grad + alc.off, S->grad + bec.off, GX(zy_sl), d); },
                          "zy_update"});
         }
         z = zn; y = yn;
@@ -429,8 +460,9 @@ static void build_tape(mb200_csc* s, bool xyz_only) {
         op_dgrad(z, y, rec, +1.f, Gm, "df_dgrad");                      // R = sumZD + sumYRD + S  ('+S': model.jl:282-285)
         {
             const Buf Dcc = Dc; const int64_t gsc = Dgs;
+            const size_t mu_sl = slots(nblk((int64_t)d.G * d.fl * d.M, 128), {i_mu});
             T.push_back({[=](cudaStream_t q) { lk(k_d_update, nblk((int64_t)d.G * d.fl * d.M, 128), 128, 0, q, S->data + Dcc.off, gsc, S->data + Gm.off, SCP, i_mu, S->data + Dn.off, d); },
-                         [=](cudaStream_t q) { lk(k_d_update_bwd, nblk((int64_t)d.G * d.fl * d.M, 128), 128, 0, q, S->data + Dcc.off, gsc, S->data + Gm.off, SCP, i_mu, S->data + Dn.off, S->grad + Dn.off, S->grad + Dcc.off, gsc, S->grad + Gm.off, DSCP, d); },
+                         [=](cudaStream_t q) { const auto o = gfilt(Dcc, gsc); lk(k_d_update_bwd, nblk((int64_t)d.G * d.fl * d.M, 128), 128, 0, q, S->data + Dcc.off, gsc, S->data + Gm.off, SCP, i_mu, S->data + Dn.off, S->grad + Dn.off, o.first, o.second, S->grad + Gm.off, GX(mu_sl), d); },
                          "d_update"});
         }
         Dc = Dn; Dgs = nD;
@@ -448,8 +480,9 @@ static void build_tape(mb200_csc* s, bool xyz_only) {
         op_fgrad(e, x, Fg, "df_fgrad");
         {
             const Buf Fcc = Fc; const int64_t gsc = Fgs;
+            const size_t kap_sl = slots((size_t)d.G * d.K, {i_kap, i_kaps});
             T.push_back({[=](cudaStream_t q) { lk(k_f_update, d.G * d.K, 256, 0, q, S->data + Fcc.off, gsc, S->data + Fg.off, SCP, i_kap, i_kaps, S->data + Fn.off, S->data + nrm.off, d); },
-                         [=](cudaStream_t q) { lk(k_f_update_bwd, d.G * d.K, 256, 0, q, S->data + Fn.off, S->data + nrm.off, S->data + Fg.off, SCP, i_kap, i_kaps, S->grad + Fn.off, S->grad + Fcc.off, gsc, S->grad + Fg.off, DSCP, d); },
+                         [=](cudaStream_t q) { const auto o = gfilt(Fcc, gsc); lk(k_f_update_bwd, d.G * d.K, 256, 0, q, S->data + Fn.off, S->data + nrm.off, S->data + Fg.off, SCP, i_kap, i_kaps, S->grad + Fn.off, o.first, o.second, S->grad + Fg.off, GX(kap_sl), d); },
                          "f_update"});
         }
         Fc = Fn; Fgs = nF;
@@ -494,7 +527,7 @@ static int csc_alloc(mb200_ctx* ctx, mb200_csc* s) {
     MB_CUDA(ctx, cudaMemset(s->st, 0, (size_t)s->n_total * 4));
     MB_CUDA(ctx, cudaMalloc(&s->data, s->arena * 4));
     MB_CUDA(ctx, cudaMemset(s->data, 0, s->arena * 4));
-    if (!s->xyz_only) { MB_CUDA(ctx, cudaMalloc(&s->grad, s->arena * 4)); MB_CUDA(ctx, cudaMemset(s->grad, 0, s->arena * 4)); }
+    if (!s->xyz_only) { MB_CUDA(ctx, cudaMalloc(&s->grad, (s->arena + s->grad_extra) * 4)); MB_CUDA(ctx, cudaMemset(s->grad, 0, (s->arena + s->grad_extra) * 4)); }
     if (s->batched) {
         MB_CUDA(ctx, cudaMalloc(&s->Ft_scratch, (size_t)s->d.G * s->d.h * s->d.M2 * s->d.K * 4));
         MB_CUDA(ctx, cudaMalloc(&s->Ft_eff, (size_t)s->d.h * s->d.M2 * s->d.K * 4));
@@ -509,6 +542,10 @@ static int csc_alloc(mb200_ctx* ctx, mb200_csc* s) {
             MB_CUDA(ctx, cudaFuncSetAttribute(k_corr2d_s<6, 12>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s->c2s.smem));
             MB_CUDA(ctx, cudaFuncSetAttribute(k_corr2d_s<8, 12>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s->c2s.smem));
         }
+    }
+    if (!s->slots.empty()) {
+        MB_CUDA(ctx, cudaMalloc(&s->slots_dev, s->slots.size() * sizeof(SlotRange)));
+        MB_CUDA(ctx, cudaMemcpy(s->slots_dev, s->slots.data(), s->slots.size() * sizeof(SlotRange), cudaMemcpyHostToDevice));
     }
     MB_CUDA(ctx, cudaMalloc(&s->bits, std::max<size_t>(s->bits_n, 16)));
     MB_CUDA(ctx, cudaMalloc(&s->lcnt, (size_t)std::max(1, s->n_lists) * s->d.NS * 4));
@@ -669,7 +706,7 @@ extern "C" int32_t mb200_csc_destroy(mb200_ctx* ctx, mb200_csc* s) {
     if (s->graph) cudaGraphDestroy(s->graph);
     if (s->aux) cudaStreamDestroy(s->aux);
     if (s->ev_fork) { cudaEventDestroy(s->ev_fork); cudaEventDestroy(s->ev_join); cudaEventDestroy(s->ev_fork2); cudaEventDestroy(s->ev_join2); }
-    cudaFree(s->p_raw); cudaFree(s->g_raw); cudaFree(s->mt); cudaFree(s->st); cudaFree(s->data); cudaFree(s->grad); cudaFree(s->bits); cudaFree(s->lcnt); cudaFree(s->lidx); cudaFree(s->lval); cudaFree(s->tc_A); cudaFree(s->tc_F); cudaFree(s->Ft_scratch); cudaFree(s->Ft_scratch2); cudaFree(s->Ft_eff); cudaFree(s->fz_sync); cudaFree(s->fz_bwd_buf); if (s->fz_err_host) cudaFreeHost(s->fz_err_host);
+    cudaFree(s->p_raw); cudaFree(s->g_raw); cudaFree(s->mt); cudaFree(s->st); cudaFree(s->data); cudaFree(s->grad); cudaFree(s->bits); cudaFree(s->lcnt); cudaFree(s->lidx); cudaFree(s->lval); cudaFree(s->tc_A); cudaFree(s->tc_F); cudaFree(s->Ft_scratch); cudaFree(s->Ft_scratch2); cudaFree(s->Ft_eff); cudaFree(s->fz_sync); cudaFree(s->fz_bwd_buf); cudaFree(s->slots_dev); if (s->fz_err_host) cudaFreeHost(s->fz_err_host);
     cudaFree(s->bases); cudaFree(s->idx_dev); cudaFreeHost(s->idx_pinned); cudaFree(s->idx_identity_dev); cudaFree(s->batch_words); cudaFreeHost(s->batch_pinned); cudaFreeHost(s->host_out);
     delete s;
     return MB200_OK;
@@ -790,7 +827,7 @@ static void enqueue_step(mb200_csc* s, const uint32_t* words, int64_t rowwords, 
     }
     if (backward) {
         if (!fused_all) {
-            cudaMemsetAsync(s->grad, 0, s->arena * 4, q);
+            cudaMemsetAsync(s->grad, 0, (s->arena + s->grad_extra) * 4, q);
             cudaMemsetAsync(s->g_raw, 0, (size_t)s->n_total * 4, q);
         }
         for (size_t i = s->tape.size(); i-- > 0;) {
@@ -898,7 +935,7 @@ static int fused_check(mb200_ctx* ctx, mb200_csc* s) {
     const unsigned int e = *s->fz_err_host;
     *s->fz_err_host = 0;
     cudaMemsetAsync(s->fzw.err, 0, 4, ctx->stream);
-    cudaMemsetAsync(s->grad, 0, s->arena * 4, ctx->stream);                 // the clamped lists may have left d x slots uncleared
+    cudaMemsetAsync(s->grad, 0, (s->arena + s->grad_extra) * 4, ctx->stream);                 // the clamped lists may have left d x slots uncleared
     cudaMemsetAsync(s->fz_sync, 0, s->fz_zero_bytes, ctx->stream);
     MB_FAIL(ctx, MB200_E_UNSUPPORTED, "csc: the fused reverse pass met a degenerate top-q support (flag %u: more than %d kept entries or more than %d codes in a sequence); "
             "create the handle with MB200_CSC_NO_FUSED for such inputs", e, FZ_KCAP, LIST_CAP);

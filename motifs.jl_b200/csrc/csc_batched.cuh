@@ -945,8 +945,6 @@ __global__ void __launch_bounds__(512) k_warm_zy_bwd_s(const uint8_t* __restrict
             }
     }
     if (!active) return;
-    if (a0 != 0.f) atomicAdd(&dD[(4 * j + 0) * d.M + m], a0);
-    if (a1 != 0.f) atomicAdd(&dD[(4 * j + 1) * d.M + m], a1);
-    if (a2 != 0.f) atomicAdd(&dD[(4 * j + 2) * d.M + m], a2);
-    if (a3 != 0.f) atomicAdd(&dD[(4 * j + 3) * d.M + m], a3);
+    float* o = dD + n * (int64_t)d.f_len * d.M;                    // this sequence's own slice, summed over sequences in order (k_sum_slices)
+    o[(4 * j + 0) * d.M + m] = a0; o[(4 * j + 1) * d.M + m] = a1; o[(4 * j + 2) * d.M + m] = a2; o[(4 * j + 3) * d.M + m] = a3;
 }

@@ -278,7 +278,7 @@ __global__ void __launch_bounds__(256) k_zy_update_bwd(const float* __restrict__
                                                        const float* __restrict__ dzn, const float* __restrict__ dyn,
                                                        float* __restrict__ dz, float* __restrict__ dy, float* __restrict__ dgz, float* __restrict__ dgy,
                                                        float* __restrict__ dfx, float* __restrict__ dal, float* __restrict__ dbe,
-                                                       float* __restrict__ dsc, CscDims d) { PDL_SYNC();
+                                                       float* __restrict__ part, CscDims d) { PDL_SYNC();
     const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     float s_eta = 0.f, s_lam = 0.f, s_rho = 0.f;
     if (t < (int64_t)d.NS * d.c * d.M) {
@@ -301,11 +301,7 @@ __global__ void __launch_bounds__(256) k_zy_update_bwd(const float* __restrict__
         s_rho = -eta * (tz * ez + ty * ey);
     }
     s_eta = block_sum(s_eta); s_lam = block_sum(s_lam); s_rho = block_sum(s_rho);
-    if (threadIdx.x == 0) {
-        if (s_eta != 0.f) atomicAdd(&dsc[i_eta], s_eta);
-        if (s_lam != 0.f) atomicAdd(&dsc[i_lam], s_lam);
-        if (s_rho != 0.f) atomicAdd(&dsc[i_rho], s_rho);
-    }
+    if (threadIdx.x == 0) { part[3 * blockIdx.x] = s_eta; part[3 * blockIdx.x + 1] = s_lam; part[3 * blockIdx.x + 2] = s_rho; }      // block partials, summed in block order (k_sum_slots)
 }
 
 // A4 (model.jl:194-210): zy' = mf * [zy >= median{zy > 0 over the whole batch}] * zy.  One block per group:
@@ -528,7 +524,7 @@ __global__ void __launch_bounds__(256) k_d_update(const float* __restrict__ D, i
 }
 __global__ void __launch_bounds__(256) k_d_update_bwd(const float* __restrict__ D, int64_t D_gs, const float* __restrict__ G, const float* __restrict__ sc, int i_mu,
                                                       const float* __restrict__ Dn, const float* __restrict__ dDn,
-                                                      float* __restrict__ dD, int64_t dD_gs, float* __restrict__ dG, float* __restrict__ dsc, CscDims d) { PDL_SYNC();
+                                                      float* __restrict__ dD, int64_t dD_gs, float* __restrict__ dG, float* __restrict__ part, CscDims d) { PDL_SYNC();
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     float s_mu = 0.f;
     if (t < d.G * d.fl * d.M) {
@@ -553,7 +549,7 @@ __global__ void __launch_bounds__(256) k_d_update_bwd(const float* __restrict__ 
         }
     }
     s_mu = block_sum(s_mu);
-    if (threadIdx.x == 0 && s_mu != 0.f) atomicAdd(&dsc[i_mu], s_mu);
+    if (threadIdx.x == 0) part[blockIdx.x] = s_mu;
 }
 
 // A11 update (model.jl:304-308): Fu = relu(F - kap*Fg - kap*kaps) ; Fn[:,:,k] = Fu[:,:,k] / ||Fu[:,:,k]||_2.  One block per (g,k).
@@ -581,7 +577,7 @@ __global__ void __launch_bounds__(256) k_f_update(const float* __restrict__ F, i
 }
 __global__ void __launch_bounds__(256) k_f_update_bwd(const float* __restrict__ Fn, const float* __restrict__ nrm, const float* __restrict__ Fg,
                                                       const float* __restrict__ sc, int i_kap, int i_kaps, const float* __restrict__ dFn,
-                                                      float* __restrict__ dF, int64_t dF_gs, float* __restrict__ dFg, float* __restrict__ dsc, CscDims d) { PDL_SYNC();
+                                                      float* __restrict__ dF, int64_t dF_gs, float* __restrict__ dFg, float* __restrict__ part, CscDims d) { PDL_SYNC();
     __shared__ float s_dot;
     const int k = blockIdx.x % d.K, g = blockIdx.x / d.K;
     const float kap = sc[i_kap], kaps = sc[i_kaps];
@@ -607,7 +603,7 @@ __global__ void __launch_bounds__(256) k_f_update_bwd(const float* __restrict__ 
         }
     }
     s_kap = block_sum(s_kap); s_kaps = block_sum(s_kaps);
-    if (threadIdx.x == 0) { if (s_kap != 0.f) atomicAdd(&dsc[i_kap], s_kap); if (s_kaps != 0.f) atomicAdd(&dsc[i_kaps], s_kaps); }
+    if (threadIdx.x == 0) { part[2 * blockIdx.x] = s_kap; part[2 * blockIdx.x + 1] = s_kaps; }
 }
 
 // A12 (model.jl:310-325): loss[g] = (1/B) (sum (recon - S)^2 + sum (fx - zy)^2).  One block per group.
@@ -730,6 +726,29 @@ __global__ void __launch_bounds__(256) k_unpack_bases(const uint32_t* __restrict
 }
 
 // AdaBelief (Flux 0.14.6 Optimise.AdaBelief, restated; see oracle/csc_oracle.py) over the trainable vector, fp32.
+// Deterministic sums of the tape's shared adjoints.  Where many CTAs or groups feed one adjoint, float atomics would add in an order that
+// varies from run to run; instead each group, sequence or block writes its own slice or slot, and these kernels add them in a fixed order.
+// dst[i] += sum over k < ns of src[k * n + i], k ascending.
+__global__ void __launch_bounds__(256) k_sum_slices(const float* __restrict__ src, int ns, int64_t n, float* __restrict__ dst) { PDL_SYNC();
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    float a = 0.f;
+    for (int k = 0; k < ns; ++k) a += src[(int64_t)k * n + i];
+    dst[i] += a;
+}
+struct SlotRange { int32_t idx, n, stride, pad; int64_t off; };   // scalar idx receives src[off + i * stride], i < n
+// one block per scalar: its ranges in table order, each summed by a fixed thread assignment and block_sum
+__global__ void __launch_bounds__(256) k_sum_slots(const float* __restrict__ src, const SlotRange* __restrict__ r, int nr, float* __restrict__ dsc) { PDL_SYNC();
+    float tot = 0.f;
+    for (int k = 0; k < nr; ++k) {
+        if (r[k].idx != (int)blockIdx.x) continue;
+        float a = 0.f;
+        for (int i = threadIdx.x; i < r[k].n; i += blockDim.x) a += src[r[k].off + (int64_t)i * r[k].stride];
+        tot += block_sum(a);
+    }
+    if (threadIdx.x == 0) dsc[blockIdx.x] += tot;
+}
+
 __global__ void __launch_bounds__(256) k_adabelief(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ mt, float* __restrict__ st,
                                                    float eta, float b1, float b2, float eps2, float c1, float c2, int n) { PDL_SYNC();
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
@@ -944,7 +963,7 @@ __global__ void __launch_bounds__(256) k_topq_s(const float* __restrict__ xprev,
 // adjoints of corr2d) and reduces d omega.
 __global__ void __launch_bounds__(256) k_topq_s_bwd(const uint8_t* __restrict__ bit, const float* __restrict__ g, const float* __restrict__ sc, int i_om,
                                                     float coef, const float* __restrict__ dxout, float* __restrict__ dxprev, float* __restrict__ dg,
-                                                    float* __restrict__ dsc, int om_trainable,
+                                                    float* __restrict__ part, int om_trainable,
                                                     int32_t* __restrict__ lcnt, uint16_t* __restrict__ lidx, float* __restrict__ lval, CscDims d) { PDL_SYNC();
     const int64_t n = blockIdx.x;
     const int E = d.l * d.K;
@@ -968,7 +987,7 @@ __global__ void __launch_bounds__(256) k_topq_s_bwd(const uint8_t* __restrict__ 
         if (dgv != 0.f) { if (o < LIST_CAP) { lidx[n * LIST_CAP + o] = (uint16_t)e; lval[n * LIST_CAP + o] = dgv; } ++o; }
     }
     if (threadIdx.x == 0) lcnt[n] = total;
-    if (om_trainable) { s = block_sum(s); if (threadIdx.x == 0 && s != 0.f) atomicAdd(&dsc[i_om], s); }
+    if (om_trainable) { s = block_sum(s); if (threadIdx.x == 0) part[blockIdx.x] = s; }
 }
 
 // U1 with the x operand given as a list: one block per (n, i), threads over j.

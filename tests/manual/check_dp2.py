@@ -2,7 +2,7 @@
 gradients, and both ranks hold identical parameters after a data-parallel optimiser step."""
 import os, sys
 import numpy as np, torch, torch.distributed as dist
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))))
 import motifs_jl_b200 as mb
 from motifs_jl_b200 import model as mdl, parallel, synth
 

@@ -404,3 +404,24 @@ def test_fused_step_leaves_its_scratch_clean(ctx):
     l1, g1 = m.loss_grad(seqs, idx)
     assert np.array_equal(l0, l1) and np.array_equal(g0, g1)
     m.free(); seqs.free()
+
+
+@pytest.mark.parametrize("groups,fused", [(1, False), (3, False), (64, True)])
+def test_kernel_per_op_step_is_bit_identical_run_to_run(ctx, groups, fused):
+    """The kernel-per-op reverse pass (one group without the fused kernels, a few groups, the many-group launch path) adds the adjoints of
+    the shared D, F and scalars in a fixed order: two handles fed the same batches return the same gradient bits, and the same parameters
+    after several optimiser steps (float atomics would reorder those sums from run to run and the optimiser would amplify the difference)."""
+    hp, ohp, a, seqs, flat = _setup(ctx, 6 * groups + 40, 100, 13)
+    out = []
+    for _ in range(2):
+        m = mb._lib.CscModel(ctx, hp, 100, n_groups=groups, fused=fused)
+        m.set_params(flat)
+        rng = np.random.default_rng(8)
+        loss, g = m.loss_grad(seqs, rng.permutation(len(a))[:6 * groups])
+        for _ in range(4):
+            m.step_begin(seqs, rng.permutation(len(a))[:6 * groups]); m.adabelief_step()
+        out.append((loss, g, m.get_params()))
+        m.free()
+    for x, y in zip(out[0], out[1]):
+        assert np.array_equal(x, y)
+    seqs.free()

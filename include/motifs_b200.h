@@ -94,6 +94,15 @@ int32_t mb200_seqs_from_device_ascii(mb200_ctx* ctx, const void* ascii_dev, int6
  * (4*Lb, N) (the singleton middle dimension is a reshape), exactly one 1 per group of 4. */
 int32_t mb200_seqs_from_onehot_f32(mb200_ctx* ctx, const float* onehot, int64_t N, int64_t Lb,
                                    mb200_seqs** out);
+/* rows of different lengths (a peak set, the N-free fragments of a genome): row i = ascii[offsets[i], offsets[i+1]), offsets has
+ * N+1 non-decreasing entries, empty rows are allowed.  Lb = the longest row (at least 1); shorter rows are padded with zero words
+ * and every consumer honours each row's own length: mb200_scan / mb200_scan_hist return exactly what they return for each row
+ * on its own (start positions 0 .. L_n - len_k), gather / shuffle / base_counts / to_ascii / count_matrices work on [0, L_n).
+ * The CSC entry points (training, code retrieval) need one length and return MB200_E_UNSUPPORTED for such a store.        */
+int32_t mb200_seqs_from_ascii_ragged(mb200_ctx* ctx, const uint8_t* ascii, const int64_t* offsets, int64_t N,
+                                     mb200_seqs** out);
+/* the N row lengths; Lb for every row of a fixed-length store */
+int32_t mb200_seqs_lengths(const mb200_seqs* s, int64_t* out);
 int32_t mb200_seqs_free(mb200_ctx* ctx, mb200_seqs* s);
 int32_t mb200_seqs_shape(const mb200_seqs* s, int64_t* N, int64_t* Lb, int64_t* words_per_seq);
 /* copy the packed words back (N * words_per_seq uint32) — used by tests. */
@@ -109,6 +118,19 @@ typedef struct mb200_fasta mb200_fasta;
 int32_t mb200_fasta_read(const char* path, int64_t max_entries, mb200_fasta** out, int64_t* N, int64_t* L);
 int32_t mb200_fasta_rows(const mb200_fasta* f, uint8_t* out_rows /* N*L bytes */);
 int32_t mb200_fasta_free(mb200_fasta* f);
+/* parse a FASTA file keeping everything: no cap, no length or N filter.  '>' at the start of a line opens a record, its name is
+ * the header up to the first blank; '\r', blanks and tabs in sequence lines are ignored.  A record's coordinates count every
+ * other byte.  A,C,G,T in either case (upper-cased, so soft-masked bases are scanned) form the N-free FRAGMENTS of a record;
+ * any other byte (N, IUPAC codes, '-') ends a fragment and is not scanned.                                                   */
+typedef struct mb200_records mb200_records;
+int32_t mb200_records_read(const char* path, mb200_records** out);
+int32_t mb200_records_counts(const mb200_records* r, int64_t* n_records, int64_t* n_fragments, int64_t* n_bases, int64_t* name_bytes);
+/* names: name_bytes bytes, the record names in order, each NUL-terminated; lengths: n_records record lengths (either may be NULL) */
+int32_t mb200_records_names(const mb200_records* r, char* names, int64_t* lengths);
+/* per fragment (n_fragments entries each, 0-based): its record, start inside the record and length; bases: n_bases bytes, the
+ * fragments' bases concatenated in fragment order (ready for mb200_seqs_from_ascii_ragged).  Any pointer may be NULL.        */
+int32_t mb200_records_fragments(const mb200_records* r, int64_t* record, int64_t* start, int64_t* length, uint8_t* bases);
+int32_t mb200_records_free(mb200_records* r);
 /* 0-based train / test indices: n_test = floor((1 - ratio) * n); shuffle != 0: randperm, test = sample without replacement,
  * train = the remaining indices in randperm order; shuffle == 0: test = the last n_test indices.  train_idx / test_idx: room for n. */
 int32_t mb200_fasta_split(int64_t n, double train_test_split_ratio, int32_t shuffle, uint64_t seed,

@@ -52,6 +52,48 @@ function upload_ascii(ctx, ascii::Matrix{UInt8}; async=false)          # size(as
 end
 wait_seqs(ctx, s) = check(ctx, ccall((:mb200_seqs_wait, lib), Int32, (Ptr{Cvoid}, Ptr{Cvoid}), ctx, s))
 
+# FASTA files as they are (not in the reference, which keeps only equal-length N-free reads): every record, its N-free fragments.
+# Like the rest of this file it is untested here (no Julia in the build image); the Python mirror is records.py.
+function read_records(path::AbstractString)
+    h = Ref{Ptr{Cvoid}}(C_NULL)
+    ccall((:mb200_records_read, lib), Int32, (Cstring, Ref{Ptr{Cvoid}}), path, h) == 0 || error("mb200_records_read($path) failed")
+    nr, nf, nb, nn = Ref{Int64}(0), Ref{Int64}(0), Ref{Int64}(0), Ref{Int64}(0)
+    ccall((:mb200_records_counts, lib), Int32, (Ptr{Cvoid}, Ref{Int64}, Ref{Int64}, Ref{Int64}, Ref{Int64}), h[], nr, nf, nb, nn)
+    names = Vector{UInt8}(undef, nn[]); lengths = Vector{Int64}(undef, nr[])
+    ccall((:mb200_records_names, lib), Int32, (Ptr{Cvoid}, Ptr{UInt8}, Ptr{Int64}), h[], names, lengths)
+    rec, start, len = Vector{Int64}(undef, nf[]), Vector{Int64}(undef, nf[]), Vector{Int64}(undef, nf[])
+    bases = Vector{UInt8}(undef, nb[])
+    ccall((:mb200_records_fragments, lib), Int32, (Ptr{Cvoid}, Ptr{Int64}, Ptr{Int64}, Ptr{Int64}, Ptr{UInt8}), h[], rec, start, len, bases)
+    ccall((:mb200_records_free, lib), Int32, (Ptr{Cvoid},), h[])
+    name_list = String.(split(String(names), '\0'; keepempty=true))[1:nr[]]
+    (names=name_list, lengths=lengths, frag_record=rec, frag_start=start, frag_len=len, bases=bases)   # 0-based record / start
+end
+# the bucketing rule of INTEGRATION.md: fragments >= minlen, longest first, padding <= 1/8 of the positions of each store
+function bucket_fragments(frag_len::Vector{Int64}, minlen::Integer)
+    order = sort(findall(>=(minlen), frag_len); by=i -> (-frag_len[i], i))
+    buckets = Vector{Vector{Int}}(); i = 1
+    while i <= length(order)
+        lmax = frag_len[order[i]]; tot = lmax; j = i + 1
+        while j <= length(order) && 8 * (tot + frag_len[order[j]]) >= 7 * (j - i + 1) * lmax
+            tot += frag_len[order[j]]; j += 1
+        end
+        push!(buckets, order[i:j-1]); i = j
+    end
+    buckets
+end
+# rows of different lengths: offsets (N+1, 0-based, non-decreasing) into the concatenated bytes
+function upload_ragged(ctx, ascii::Vector{UInt8}, offsets::Vector{Int64})
+    h = Ref{Ptr{Cvoid}}(C_NULL)
+    check(ctx, ccall((:mb200_seqs_from_ascii_ragged, lib), Int32, (Ptr{Cvoid}, Ptr{UInt8}, Ptr{Int64}, Int64, Ref{Ptr{Cvoid}}),
+                     ctx, ascii, offsets, length(offsets) - 1, h))
+    h[]
+end
+function seqs_lengths(s, N::Integer)
+    out = Vector{Int64}(undef, N)
+    ccall((:mb200_seqs_lengths, lib), Int32, (Ptr{Cvoid}, Ptr{Int64}), s, out) == 0 || error("mb200_seqs_lengths failed")
+    out
+end
+
 # replaces get_pos_scores_arr + gpu_scan (inference/_h3_1_alignment.jl:57-99).  `pwms` is the (K,4,maxlen) Float16 array the
 # reference builds at :65-69 with rc=false; thresh === nothing gives the reference's "score > 0" scan.
 function gpu_scan(ctx, seqs, pwms::Array{Float16,3}, lens::Vector{Int64}; thresh::Union{Nothing,Vector{Float16}}=nothing,

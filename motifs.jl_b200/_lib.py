@@ -80,12 +80,19 @@ def load():
         "mb200_seqs_wait": (i32, [p, p]),
         "mb200_seqs_from_device_ascii": (i32, [p, p, i64, i64, C.POINTER(p)]),
         "mb200_seqs_from_onehot_f32": (i32, [p, p, i64, i64, C.POINTER(p)]),
+        "mb200_seqs_from_ascii_ragged": (i32, [p, p, p, i64, C.POINTER(p)]),
+        "mb200_seqs_lengths": (i32, [p, p]),
         "mb200_seqs_free": (i32, [p, p]),
         "mb200_seqs_shape": (i32, [p, C.POINTER(i64), C.POINTER(i64), C.POINTER(i64)]),
         "mb200_seqs_download": (i32, [p, p, p, i64]),
         "mb200_fasta_read": (i32, [C.c_char_p, i64, C.POINTER(p), C.POINTER(i64), C.POINTER(i64)]),
         "mb200_fasta_rows": (i32, [p, p]),
         "mb200_fasta_free": (i32, [p]),
+        "mb200_records_read": (i32, [C.c_char_p, C.POINTER(p)]),
+        "mb200_records_counts": (i32, [p, C.POINTER(i64), C.POINTER(i64), C.POINTER(i64), C.POINTER(i64)]),
+        "mb200_records_names": (i32, [p, p, p]),
+        "mb200_records_fragments": (i32, [p, p, p, p, p]),
+        "mb200_records_free": (i32, [p]),
         "mb200_fasta_split": (i32, [i64, C.c_double, i32, C.c_uint64, p, p, C.POINTER(i64), C.POINTER(i64)]),
         "mb200_seqs_gather": (i32, [p, p, p, i64, C.POINTER(p)]),
         "mb200_seqs_shuffle": (i32, [p, p, i32, C.c_uint64, i64, C.POINTER(p)]),
@@ -225,6 +232,21 @@ class Context:
         h = C.c_void_p()
         self._check(self._lib.mb200_seqs_from_ascii(self._h, _ptr(a), a.shape[0], a.shape[1], C.byref(h)))
         return Sequences(self, h, a.shape[0], a.shape[1])
+
+    def seqs_from_ragged(self, ascii: np.ndarray, offsets) -> "Sequences":
+        """Rows of different lengths: row i = ascii[offsets[i]:offsets[i+1]] (mb200_seqs_from_ascii_ragged).  `ascii` is the
+        concatenated uint8 bases (or a bytes object), offsets N+1 non-decreasing int64.  Lb of the store = the longest row."""
+        a = np.frombuffer(ascii, np.uint8) if isinstance(ascii, (bytes, bytearray)) else np.ascontiguousarray(ascii, np.uint8).reshape(-1)
+        off = np.ascontiguousarray(offsets, np.int64)
+        if off.ndim != 1 or len(off) < 1:
+            raise ValueError("offsets must be N+1 int64 values")
+        if len(off) > 1 and (off[0] < 0 or off[-1] > a.size):
+            raise ValueError("offsets must lie inside ascii")
+        h = C.c_void_p()
+        self._check(self._lib.mb200_seqs_from_ascii_ragged(self._h, _ptr(a), _ptr(off), len(off) - 1, C.byref(h)))
+        N, Lb = C.c_int64(), C.c_int64()
+        self._lib.mb200_seqs_shape(h, C.byref(N), C.byref(Lb), None)
+        return Sequences(self, h, N.value, Lb.value)
 
     def seqs_from_host_ptr(self, ptr: int, N: int, Lb: int, wait: bool = True) -> "Sequences":
         """ASCII rows at a raw host address (e.g. a pinned torch tensor's data_ptr()).  wait=False: the upload is queued on the
@@ -371,6 +393,15 @@ class Sequences:
         self.ctx._check(self.ctx._lib.mb200_seqs_download(self.ctx._h, self._h, _ptr(out), out.size))
         return out
 
+    @property
+    def lengths(self) -> np.ndarray:
+        """(N,) int64 row lengths (all Lb for a fixed-length store)."""
+        out = np.zeros(self.N, np.int64)
+        rc = self.ctx._lib.mb200_seqs_lengths(self._h, _ptr(out))
+        if rc != OK:
+            raise MB200Error(rc, "mb200_seqs_lengths failed")
+        return out
+
     def gather(self, idx) -> "Sequences":
         """rows idx of this store as a new store (device gather)."""
         i = np.ascontiguousarray(idx, np.int64)
@@ -379,7 +410,8 @@ class Sequences:
         return Sequences(self.ctx, h, len(i), self.Lb)
 
     def shuffle(self, k: int, seed: int, first_stream: int = 0) -> "Sequences":
-        """seq_shuffle.(reads; k): k-mer-count-preserving shuffle of every sequence on the device, from a host seed."""
+        """seq_shuffle.(reads; k): k-mer-count-preserving shuffle of every sequence on the device, from a host seed.  Row i draws
+        from random stream first_stream + i; rows of a ragged store keep their lengths and zero padding."""
         h = C.c_void_p()
         self.ctx._check(self.ctx._lib.mb200_seqs_shuffle(self.ctx._h, self._h, int(k), C.c_uint64(int(seed) & (2 ** 64 - 1)), int(first_stream), C.byref(h)))
         return Sequences(self.ctx, h, self.N, self.Lb)
@@ -391,6 +423,7 @@ class Sequences:
         return c, t
 
     def to_ascii(self) -> np.ndarray:
+        """(N, Lb) uint8 "ACGT" rows; bytes past a row's length (ragged stores) are 0."""
         out = np.zeros((self.N, self.Lb), np.uint8)
         self.ctx._check(self.ctx._lib.mb200_seqs_to_ascii(self.ctx._h, self._h, _ptr(out)))
         return out

@@ -49,10 +49,18 @@ struct mb200_seqs {
     std::vector<cudaEvent_t> ready; std::vector<int64_t> ready_end;
     uint8_t* stage = nullptr;    // own staging buffers + bad-symbol counter, freed by mb_seqs_finish
     cudaStream_t copy_stream = nullptr;
+    // ragged store (mb200_seqs_from_ascii_ragged): row n holds hlens[n] <= Lb bases, the rest of the row is zero words.
+    // A fixed-length store has ragged == false, lens == nullptr and every kernel takes its fixed-length path.
+    bool ragged = false;
+    int64_t* lens = nullptr;     // device, N row lengths (nullptr for a fixed store or N == 0)
+    size_t lens_bytes = 0;
+    std::vector<int64_t> hlens;  // host copy
 };
 int mb_seqs_finish(mb200_ctx* ctx, mb200_seqs* s);      // waits for a pending upload, frees its staging; MB200_E_BAD_SEQUENCE if a symbol was not A,C,G,T
 static const int64_t SEQ_PAD_WORDS = 64;
 int mb_seqs_alloc(mb200_ctx* ctx, int64_t N, int64_t Lb, mb200_seqs** out);   // empty store (tail pad zeroed on ctx->stream)
+int mb_seqs_set_lens(mb200_ctx* ctx, mb200_seqs* s, std::vector<int64_t> hlens);   // makes s ragged: uploads the row lengths (synchronous)
+static inline int64_t mb_row_len(const mb200_seqs* s, int64_t n) { return s->ragged ? s->hlens[(size_t)n] : s->Lb; }
 
 #define MB_FAIL(ctx, code, ...) do { char _b[512]; snprintf(_b, sizeof _b, __VA_ARGS__); \
     if (ctx) (ctx)->err = _b; return (code); } while (0)

@@ -42,6 +42,12 @@ extern "C" int32_t mb200_count_matrices(mb200_ctx* ctx, const mb200_seqs* seqs, 
     }
     for (int64_t i = 0; i < n_sites; ++i)
         if (sites[i].motif >= (uint32_t)K) MB_FAIL(ctx, MB200_E_INVALID, "count_matrices: site %lld names motif %u (K=%d)", (long long)i, sites[i].motif, K);
+    if (seqs->ragged) {                  // the kernel checks against Lb; a row of a ragged store ends at its own length
+        int64_t bad = 0;
+        for (int64_t i = 0; i < n_sites; ++i)
+            bad += sites[i].seq < (uint64_t)seqs->N && (int64_t)sites[i].pos + lens[sites[i].motif] > seqs->hlens[sites[i].seq];
+        if (bad) MB_FAIL(ctx, MB200_E_INVALID, "count_matrices: %lld sites fall outside their sequence", (long long)bad);
+    }
     const size_t cbytes = (size_t)K * maxlen * 4 * 4;
     const size_t off_cnt = 0, off_bad = (cbytes + 255) & ~(size_t)255, off_lens = off_bad + 256;
     const size_t off_sites = off_lens + (((size_t)K * 4 + 255) & ~(size_t)255);

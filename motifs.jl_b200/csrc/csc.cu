@@ -894,6 +894,7 @@ static int launch_step(mb200_ctx* ctx, mb200_csc* s, const uint32_t* words, int6
 
 static int run_step(mb200_ctx* ctx, mb200_csc* s, const mb200_seqs* seqs, const int64_t* seq_idx, bool backward) {
     const CscDims d = s->d;
+    if (seqs->ragged) MB_FAIL(ctx, MB200_E_UNSUPPORTED, "csc: the network needs sequences of one length; this store has rows of different lengths (a ragged store serves the scan only)");
     if (seqs->Lb != d.Lb) MB_FAIL(ctx, MB200_E_INVALID, "csc: model built for Lb=%d, sequences have Lb=%lld", d.Lb, (long long)seqs->Lb);
     if (seqs->pending) { const int rc = mb_seqs_finish(ctx, const_cast<mb200_seqs*>(seqs)); if (rc) return rc; }
     int64_t* slot = s->idx_pinned + (size_t)(s->ring++ % IDX_RING) * d.NS;
@@ -1083,6 +1084,7 @@ static int32_t codes_impl(mb200_ctx* ctx, mb200_csc* s, const mb200_seqs* seqs, 
                           mb200_code* out, int64_t cap, int64_t* n_out, std::vector<mb200_code>* vec) {
     if (!ctx || !s || !seqs || !n_out) return MB200_E_INVALID;
     const CscDims d = s->d;
+    if (seqs->ragged) MB_FAIL(ctx, MB200_E_UNSUPPORTED, "csc_codes: code retrieval needs sequences of one length; this store has rows of different lengths (a ragged store serves the scan only)");
     if (seqs->Lb != d.Lb) MB_FAIL(ctx, MB200_E_INVALID, "csc: model built for Lb=%d, sequences have Lb=%lld", d.Lb, (long long)seqs->Lb);
     if (seqs->pending) { const int rc = mb_seqs_finish(ctx, const_cast<mb200_seqs*>(seqs)); if (rc) return rc; }
     if (first_seq < 0 || n_seqs < 0 || first_seq + n_seqs > seqs->N || n_seqs % d.B) MB_FAIL(ctx, MB200_E_INVALID, "csc_codes: range must be whole batches inside the data");

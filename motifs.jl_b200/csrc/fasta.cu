@@ -78,6 +78,91 @@ extern "C" int32_t mb200_fasta_rows(const mb200_fasta* f, uint8_t* out_rows) {
 }
 extern "C" int32_t mb200_fasta_free(mb200_fasta* f) { if (!f) return MB200_E_INVALID; delete f; return MB200_OK; }
 
+// ---- host: FASTA records as they are (peak sets, genomes) ---------------------------------------------------------------------
+// Every record is kept, whatever its length.  A record's coordinates count every sequence byte (N and IUPAC codes included);
+// the maximal runs of A/C/G/T (either case, upper-cased here) are its fragments, the unit the ragged stores hold.
+struct mb200_records {
+    std::string names;                                   // NUL-terminated names, record order
+    std::vector<int64_t> rec_len;
+    std::vector<int64_t> frag_rec, frag_start, frag_len;
+    std::vector<uint8_t> bases;                          // fragments concatenated
+};
+
+extern "C" int32_t mb200_records_read(const char* path, mb200_records** out) {
+    if (!path || !out) return MB200_E_INVALID;
+    *out = nullptr;
+    FILE* fh = fopen(path, "rb");
+    if (!fh) return MB200_E_INVALID;
+    mb200_records* R = new mb200_records();
+    static const uint8_t kUpper[4] = {'A', 'C', 'G', 'T'};
+    int64_t pos = 0;                                     // position inside the current record
+    bool in_rec = false, header = false, line_start = true, name_done = false, in_frag = false;
+    auto close_frag = [&]() { if (in_frag) { R->frag_len.back() = pos - R->frag_start.back(); in_frag = false; } };
+    char buf[1 << 16]; size_t got;
+    while ((got = fread(buf, 1, sizeof buf, fh)) > 0) {
+        for (size_t i = 0; i < got; ++i) {
+            const uint8_t c = (uint8_t)buf[i];
+            if (c == '\n') { line_start = true; if (header) { header = false; R->names.push_back('\0'); } continue; }
+            if (c == '\r') continue;
+            if (line_start && c == '>') {                // a new record
+                close_frag();
+                if (in_rec) R->rec_len.back() = pos;
+                R->rec_len.push_back(0); pos = 0;
+                in_rec = true; header = true; name_done = false; line_start = false;
+                continue;
+            }
+            line_start = false;
+            if (header) {
+                if (c == ' ' || c == '\t' || c == '\v' || c == '\f') name_done = true;
+                else if (!name_done) R->names.push_back((char)c);
+                continue;
+            }
+            if (!in_rec || c == ' ' || c == '\t') continue;   // text before the first header, blanks inside sequence lines
+            const uint8_t u = (c >= 'a' && c <= 'z') ? (uint8_t)(c - 32) : c;
+            const int code = u == 'A' ? 0 : u == 'C' ? 1 : u == 'G' ? 2 : u == 'T' ? 3 : -1;
+            if (code >= 0) {
+                if (!in_frag) { R->frag_rec.push_back((int64_t)R->rec_len.size() - 1); R->frag_start.push_back(pos); R->frag_len.push_back(0); in_frag = true; }
+                R->bases.push_back(kUpper[code]);
+            } else {
+                close_frag();                            // N, IUPAC codes, '-', ...: not scanned
+            }
+            ++pos;
+        }
+    }
+    const bool err = ferror(fh) != 0;
+    fclose(fh);
+    if (header) R->names.push_back('\0');
+    close_frag();
+    if (in_rec) R->rec_len.back() = pos;
+    if (err) { delete R; return MB200_E_INVALID; }
+    *out = R;
+    return MB200_OK;
+}
+extern "C" int32_t mb200_records_counts(const mb200_records* r, int64_t* n_records, int64_t* n_fragments, int64_t* n_bases, int64_t* name_bytes) {
+    if (!r) return MB200_E_INVALID;
+    if (n_records) *n_records = (int64_t)r->rec_len.size();
+    if (n_fragments) *n_fragments = (int64_t)r->frag_len.size();
+    if (n_bases) *n_bases = (int64_t)r->bases.size();
+    if (name_bytes) *name_bytes = (int64_t)r->names.size();
+    return MB200_OK;
+}
+extern "C" int32_t mb200_records_names(const mb200_records* r, char* names, int64_t* lengths) {
+    if (!r) return MB200_E_INVALID;
+    if (names && !r->names.empty()) memcpy(names, r->names.data(), r->names.size());
+    if (lengths && !r->rec_len.empty()) memcpy(lengths, r->rec_len.data(), r->rec_len.size() * 8);
+    return MB200_OK;
+}
+extern "C" int32_t mb200_records_fragments(const mb200_records* r, int64_t* record, int64_t* start, int64_t* length, uint8_t* bases) {
+    if (!r) return MB200_E_INVALID;
+    const size_t nf = r->frag_len.size();
+    if (record && nf) memcpy(record, r->frag_rec.data(), nf * 8);
+    if (start && nf) memcpy(start, r->frag_start.data(), nf * 8);
+    if (length && nf) memcpy(length, r->frag_len.data(), nf * 8);
+    if (bases && !r->bases.empty()) memcpy(bases, r->bases.data(), r->bases.size());
+    return MB200_OK;
+}
+extern "C" int32_t mb200_records_free(mb200_records* r) { if (!r) return MB200_E_INVALID; delete r; return MB200_OK; }
+
 // ---- host: train / test indices (get_train_test_inds, helpers.jl:141-159); 0-based --------------------------------------------------
 extern "C" int32_t mb200_fasta_split(int64_t n, double train_test_split_ratio, int32_t shuffle, uint64_t seed,
                                      int64_t* train_idx, int64_t* test_idx, int64_t* n_train, int64_t* n_test) {
@@ -116,13 +201,14 @@ __global__ void __launch_bounds__(256) gather_rows_kernel(const uint32_t* __rest
     const int64_t r = t / rowwords, w = t - r * rowwords;
     dst[t] = src[idx[r] * rowwords + w];
 }
+// lens (ragged stores, may be NULL): ASCII output is 0 past a row's length (codes past it are the padding's zeros anyway)
 __global__ void __launch_bounds__(256) unpack_codes_kernel(const uint32_t* __restrict__ words, int64_t rowwords, int64_t n, int64_t Lb, int ascii,
-                                                           uint8_t* __restrict__ out) {
+                                                           uint8_t* __restrict__ out, const int64_t* __restrict__ lens) {
     const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= n * Lb) return;
     const int64_t r = t / Lb, p = t - r * Lb;
     const uint32_t c = (words[r * rowwords + (p >> 4)] >> ((p & 15) * 2)) & 3u;
-    out[t] = ascii ? (uint8_t)"ACGT"[c] : (uint8_t)c;
+    out[t] = ascii ? (lens && p >= lens[r] ? (uint8_t)0 : (uint8_t)"ACGT"[c]) : (uint8_t)c;
 }
 __global__ void __launch_bounds__(256) pack_codes_kernel(const uint8_t* __restrict__ codes, int64_t n, int64_t Lb, int64_t rowwords, uint32_t* __restrict__ out) {
     const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -138,13 +224,19 @@ __global__ void __launch_bounds__(256) pack_codes_kernel(const uint8_t* __restri
 // Eulerian walk that uses every (k-1)-mer -> base transition of the sequence exactly once (k-mer counts, first and last (k-1)-mer kept).
 #define SHUF_MAXV 64
 __global__ void __launch_bounds__(128) shuffle_rows_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, uint8_t* __restrict__ edges,
-                                                           int64_t n, int Lb, int k, uint64_t seed, int64_t seq0) {
+                                                           int64_t n, int Lb, int k, uint64_t seed, int64_t seq0, const int64_t* __restrict__ lens) {
     const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (r >= n) return;
-    const uint8_t* s = in + r * Lb;
-    uint8_t* o = out + r * Lb;
+    const int64_t stride = Lb;
+    const uint8_t* s = in + r * stride;
+    uint8_t* o = out + r * stride;
     const uint64_t stream = (uint64_t)(seq0 + r);
     uint64_t ctr = 0;
+    if (lens) {                                         // ragged store: shuffle this row's own bases; the padding stays zero
+        const int Ln = (int)lens[r];
+        for (int i = Ln; i < Lb; ++i) o[i] = 0;
+        Lb = Ln;
+    }
     if (k <= 1 || Lb <= k) {
         for (int i = 0; i < Lb; ++i) o[i] = s[i];
         if (k <= 1)
@@ -152,7 +244,7 @@ __global__ void __launch_bounds__(128) shuffle_rows_kernel(const uint8_t* __rest
         return;
     }
     const int V = 1 << (2 * (k - 1)), E = Lb - k + 1;
-    uint8_t* el = edges + r * Lb;                       // out-edge lists (the base an edge appends), grouped by source vertex
+    uint8_t* el = edges + r * stride;                     // out-edge lists (the base an edge appends), grouped by source vertex
     int cnt[SHUF_MAXV], off[SHUF_MAXV], nxt[SHUF_MAXV];
     for (int v = 0; v < V; ++v) cnt[v] = 0;
     int v0 = 0;
@@ -191,7 +283,7 @@ __global__ void __launch_bounds__(256) shuffle_keys_kernel(uint64_t* __restrict_
     if (t < Lb) keys[t] = rnd64(seed, stream, (uint64_t)t);
 }
 __global__ void __launch_bounds__(256) base_counts_kernel(const uint32_t* __restrict__ words, int64_t rowwords, int64_t n, int64_t Lb,
-                                                          unsigned long long* __restrict__ out /* 4 + 16 */) {
+                                                          unsigned long long* __restrict__ out /* 4 + 16 */, const int64_t* __restrict__ lens) {
     __shared__ unsigned long long s_c[20];
     if (threadIdx.x < 20) s_c[threadIdx.x] = 0;
     __syncthreads();
@@ -200,9 +292,11 @@ __global__ void __launch_bounds__(256) base_counts_kernel(const uint32_t* __rest
     for (int i = 0; i < 20; ++i) c[i] = 0;
     for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < n * Lb; t += (int64_t)gridDim.x * blockDim.x) {
         const int64_t r = t / Lb, p = t - r * Lb;
+        const int64_t Ln = lens ? lens[r] : Lb;                 // ragged store: only the row's own bases
+        if (p >= Ln) continue;
         const uint32_t a = (words[r * rowwords + (p >> 4)] >> ((p & 15) * 2)) & 3u;
         ++c[a];
-        if (p + 1 < Lb) { const uint32_t b = (words[r * rowwords + ((p + 1) >> 4)] >> (((p + 1) & 15) * 2)) & 3u; ++c[4 + a * 4 + b]; }
+        if (p + 1 < Ln) { const uint32_t b = (words[r * rowwords + ((p + 1) >> 4)] >> (((p + 1) & 15) * 2)) & 3u; ++c[4 + a * 4 + b]; }
     }
     #pragma unroll
     for (int i = 0; i < 20; ++i) if (c[i]) atomicAdd(&s_c[i], (unsigned long long)c[i]);
@@ -217,6 +311,12 @@ extern "C" int32_t mb200_seqs_gather(mb200_ctx* ctx, const mb200_seqs* src, cons
     if (src->pending) { const int rc = mb_seqs_finish(ctx, const_cast<mb200_seqs*>(src)); if (rc) return rc; }
     for (int64_t i = 0; i < n; ++i) if (idx[i] < 0 || idx[i] >= src->N) MB_FAIL(ctx, MB200_E_INVALID, "seqs_gather: index %lld out of range", (long long)idx[i]);
     int rc = mb_seqs_alloc(ctx, n, src->Lb, out); if (rc) return rc;
+    if (src->ragged) {                                                // the rows keep their lengths (and their zero padding)
+        std::vector<int64_t> hl((size_t)n);
+        for (int64_t i = 0; i < n; ++i) hl[(size_t)i] = src->hlens[(size_t)idx[i]];
+        rc = mb_seqs_set_lens(ctx, *out, std::move(hl));
+        if (rc) { mb200_seqs_free(ctx, *out); *out = nullptr; return rc; }
+    }
     if (n == 0) return MB200_OK;
     rc = mb_ensure_scratch(ctx, (size_t)n * 8);
     cudaError_t e = cudaSuccess;
@@ -239,9 +339,16 @@ extern "C" int32_t mb200_seqs_shuffle(mb200_ctx* ctx, const mb200_seqs* src, int
     if (k < 1 || k > 4) MB_FAIL(ctx, MB200_E_UNSUPPORTED, "seqs_shuffle: k = %d (1..4 supported)", k);
     if (src->pending) { const int rc = mb_seqs_finish(ctx, const_cast<mb200_seqs*>(src)); if (rc) return rc; }
     const int64_t n = src->N, Lb = src->Lb;
-    const bool longseq = Lb > 65536;
-    if (longseq && k != 1) MB_FAIL(ctx, MB200_E_UNSUPPORTED, "seqs_shuffle: sequences longer than 65536 support k = 1 only");
+    const int64_t kShortMax = 65536;
+    const bool longseq = Lb > kShortMax;
+    bool long_rows = longseq;                                        // some row is longer than kShortMax
+    if (src->ragged) { long_rows = false; for (int64_t r = 0; r < n; ++r) long_rows |= src->hlens[(size_t)r] > kShortMax; }
+    if (long_rows && k != 1) MB_FAIL(ctx, MB200_E_UNSUPPORTED, "seqs_shuffle: sequences longer than 65536 support k = 1 only");
     int rc = mb_seqs_alloc(ctx, n, Lb, out); if (rc) return rc;
+    if (src->ragged) {
+        rc = mb_seqs_set_lens(ctx, *out, src->hlens);
+        if (rc) { mb200_seqs_free(ctx, *out); *out = nullptr; return rc; }
+    }
     if (n == 0) return MB200_OK;
     cudaError_t e = cudaSuccess;
     if (!longseq) {
@@ -249,25 +356,39 @@ extern "C" int32_t mb200_seqs_shuffle(mb200_ctx* ctx, const mb200_seqs* src, int
         rc = mb_ensure_scratch(ctx, 3 * plane + 256);
         if (!rc) {
             uint8_t* d_in = (uint8_t*)ctx->scratch; uint8_t* d_out = d_in + plane; uint8_t* d_ed = d_out + plane;
-            unpack_codes_kernel<<<(unsigned)((plane + 255) / 256), 256, 0, ctx->stream>>>(src->words, src->rowwords, n, Lb, 0, d_in);
-            shuffle_rows_kernel<<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>(d_in, d_out, d_ed, n, (int)Lb, k, seed, first_stream);
+            unpack_codes_kernel<<<(unsigned)((plane + 255) / 256), 256, 0, ctx->stream>>>(src->words, src->rowwords, n, Lb, 0, d_in, nullptr);
+            shuffle_rows_kernel<<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>(d_in, d_out, d_ed, n, (int)Lb, k, seed, first_stream, src->lens);
             pack_codes_kernel<<<(unsigned)((n * src->rowwords + 255) / 256), 256, 0, ctx->stream>>>(d_out, n, Lb, src->rowwords, (*out)->words);
             e = cudaGetLastError();
         }
     } else {
+        // one row at a time.  Rows longer than kShortMax: k = 1 as a sort by random keys.  The short rows of a ragged store take the
+        // kernel above (one row per launch), so that a row is shuffled the same way whichever store holds it.
         size_t tmp_bytes = 0;
         cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, (const uint64_t*)nullptr, (uint64_t*)nullptr, (const uint8_t*)nullptr, (uint8_t*)nullptr, (int64_t)Lb, 0, 64, ctx->stream);
         const size_t kb = ((size_t)Lb * 8 + 255) & ~(size_t)255, vb = ((size_t)Lb + 255) & ~(size_t)255;
-        rc = mb_ensure_scratch(ctx, 2 * kb + 2 * vb + tmp_bytes + 256);
+        const size_t sb = src->ragged ? 3 * (size_t)kShortMax : 0;
+        rc = mb_ensure_scratch(ctx, 2 * kb + 2 * vb + tmp_bytes + sb + 512);
         if (!rc) {
             uint8_t* base = (uint8_t*)ctx->scratch;
             uint64_t* k_in = (uint64_t*)base; uint64_t* k_out = (uint64_t*)(base + kb);
             uint8_t* v_in = base + 2 * kb; uint8_t* v_out = v_in + vb; void* tmp = v_out + vb;
+            uint8_t* s_in = (uint8_t*)(((uintptr_t)tmp + tmp_bytes + 255) & ~(uintptr_t)255); uint8_t* s_out = s_in + kShortMax; uint8_t* s_ed = s_out + kShortMax;
             for (int64_t r = 0; r < n && e == cudaSuccess; ++r) {
-                unpack_codes_kernel<<<(unsigned)((Lb + 255) / 256), 256, 0, ctx->stream>>>(src->words + r * src->rowwords, src->rowwords, 1, Lb, 0, v_in);
-                shuffle_keys_kernel<<<(unsigned)((Lb + 255) / 256), 256, 0, ctx->stream>>>(k_in, Lb, seed, (uint64_t)(first_stream + r));
-                e = cub::DeviceRadixSort::SortPairs(tmp, tmp_bytes, k_in, k_out, v_in, v_out, (int64_t)Lb, 0, 64, ctx->stream);
-                pack_codes_kernel<<<(unsigned)((src->rowwords + 255) / 256), 256, 0, ctx->stream>>>(v_out, 1, Lb, src->rowwords, (*out)->words + r * src->rowwords);
+                const int64_t Ln = mb_row_len(src, r);
+                uint32_t* dst = (*out)->words + r * src->rowwords;
+                if (Ln > kShortMax) {
+                    unpack_codes_kernel<<<(unsigned)((Ln + 255) / 256), 256, 0, ctx->stream>>>(src->words + r * src->rowwords, src->rowwords, 1, Ln, 0, v_in, nullptr);
+                    shuffle_keys_kernel<<<(unsigned)((Ln + 255) / 256), 256, 0, ctx->stream>>>(k_in, Ln, seed, (uint64_t)(first_stream + r));
+                    e = cub::DeviceRadixSort::SortPairs(tmp, tmp_bytes, k_in, k_out, v_in, v_out, (int64_t)Ln, 0, 64, ctx->stream);
+                    pack_codes_kernel<<<(unsigned)((src->rowwords + 255) / 256), 256, 0, ctx->stream>>>(v_out, 1, Ln, src->rowwords, dst);
+                } else {
+                    if (Ln > 0) {
+                        unpack_codes_kernel<<<(unsigned)((Ln + 255) / 256), 256, 0, ctx->stream>>>(src->words + r * src->rowwords, src->rowwords, 1, Ln, 0, s_in, nullptr);
+                        shuffle_rows_kernel<<<1, 128, 0, ctx->stream>>>(s_in, s_out, s_ed, 1, (int)Ln, k, seed, first_stream + r, nullptr);
+                    }
+                    pack_codes_kernel<<<(unsigned)((src->rowwords + 255) / 256), 256, 0, ctx->stream>>>(s_out, 1, Ln, src->rowwords, dst);   // zero words past Ln
+                }
             }
             if (e == cudaSuccess) e = cudaGetLastError();
         }
@@ -289,7 +410,7 @@ extern "C" int32_t mb200_seqs_base_counts(mb200_ctx* ctx, const mb200_seqs* seqs
     const int64_t total = seqs->N * seqs->Lb;
     if (total > 0) {
         const unsigned grid = (unsigned)std::min<int64_t>((total + 255) / 256, (int64_t)ctx->sm_count * 8);
-        base_counts_kernel<<<grid, 256, 0, ctx->stream>>>(seqs->words, seqs->rowwords, seqs->N, seqs->Lb, d);
+        base_counts_kernel<<<grid, 256, 0, ctx->stream>>>(seqs->words, seqs->rowwords, seqs->N, seqs->Lb, d, seqs->lens);
         MB_CUDA(ctx, cudaGetLastError());
     }
     unsigned long long h[20];
@@ -311,7 +432,8 @@ extern "C" int32_t mb200_seqs_to_ascii(mb200_ctx* ctx, const mb200_seqs* seqs, u
     int rc = mb_ensure_scratch(ctx, (size_t)std::min(chunk_rows, seqs->N) * (size_t)seqs->Lb); if (rc) return rc;
     for (int64_t r0 = 0; r0 < seqs->N; r0 += chunk_rows) {
         const int64_t nr = std::min(chunk_rows, seqs->N - r0);
-        unpack_codes_kernel<<<(unsigned)((nr * seqs->Lb + 255) / 256), 256, 0, ctx->stream>>>(seqs->words + r0 * seqs->rowwords, seqs->rowwords, nr, seqs->Lb, 1, (uint8_t*)ctx->scratch);
+        unpack_codes_kernel<<<(unsigned)((nr * seqs->Lb + 255) / 256), 256, 0, ctx->stream>>>(seqs->words + r0 * seqs->rowwords, seqs->rowwords, nr, seqs->Lb, 1, (uint8_t*)ctx->scratch,
+                                                                                             seqs->lens ? seqs->lens + r0 : nullptr);
         MB_CUDA(ctx, cudaGetLastError());
         MB_CUDA(ctx, cudaMemcpyAsync(out_rows + r0 * seqs->Lb, ctx->scratch, (size_t)nr * (size_t)seqs->Lb, cudaMemcpyDeviceToHost, ctx->stream));
         MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));

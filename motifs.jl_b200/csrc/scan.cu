@@ -64,6 +64,7 @@ struct ScanArgs {
     const uint8_t* blob; const MBlock* mblocks; int32_t n_mblocks;
     int32_t tile_chunks; int64_t ntiles; int32_t tile_cap_words; int32_t blob_cap_bytes;
     const int64_t* cta_range;          // [gridDim.x + 1] pair ranges (pair = mblock * ntiles + tile)
+    const int64_t* lens; int64_t Lb;   // ragged stores: row lengths (scan_kernel<true> only)
 };
 
 // ---------------------------------------------------------------------------------------------
@@ -109,6 +110,8 @@ __device__ __forceinline__ int64_t block_word(int64_t gq, int32_t W16, int64_t r
     return n * rowwords + (int64_t)pb;
 }
 
+// RAGGED: row n has lens[n] <= Lb bases; its start positions end Lb - lens[n] earlier than the group metas say (the "deficit").
+template <bool RAGGED>
 __global__ void __launch_bounds__(SCAN_THREADS, 1) scan_kernel(const ScanArgs a) {
     extern __shared__ __align__(128) uint8_t smem[];
     uint8_t* s_blob = smem;                                                        // tables + metas of one motif block
@@ -180,6 +183,8 @@ __global__ void __launch_bounds__(SCAN_THREADS, 1) scan_kernel(const ScanArgs a)
             const int64_t lq = first + i;
             const int64_t w0i = block_word(a.chunk0 + lq, a.W, a.rowwords, &n, &pb) - lo4;
             const int32_t p0 = pb * POS_BLOCK;
+            int32_t deficit = 0;                              // warp-uniform: one row per position block
+            if (RAGGED) deficit = (int32_t)(a.Lb - __ldg(a.lens + n));
             // PRMT selectors of this position block: sel[u] picks, from a column's 8 bytes {A,C,G,T}, the entries of
             // base[p0+u] (low half) and base[p0+u+1] (high half).  Same value in every lane (broadcast loads).
             uint32_t sel[NSEL];
@@ -205,7 +210,7 @@ __global__ void __launch_bounds__(SCAN_THREADS, 1) scan_kernel(const ScanArgs a)
 
             for (int32_t g = 0; g < mbk.ng; ++g) {
                 const GroupMeta* gm = s_meta + g;
-                if (p0 >= gm->npos_max) {                     // warp-uniform: no valid start position in this block
+                if (p0 >= gm->npos_max - deficit) {           // warp-uniform: no valid start position in this block
                     mrow[(g * GROUP_SLOTS + lane) * 2] = 0;
                     continue;
                 }
@@ -234,7 +239,7 @@ __global__ void __launch_bounds__(SCAN_THREADS, 1) scan_kernel(const ScanArgs a)
                     const uint32_t m = __hgt2_mask(acc[k], thr);
                     bits |= ((m & 1u) | ((m >> 15) & 2u)) << (2 * k);
                 }
-                const int32_t nvalid = min(max(gm->npos[lane >> 1] - p0, 0), POS_BLOCK);
+                const int32_t nvalid = min(max(gm->npos[lane >> 1] - deficit - p0, 0), POS_BLOCK);
                 bits &= (1u << nvalid) - 1u;
                 mrow[(g * GROUP_SLOTS + lane) * 2] = (uint16_t)bits;
             }
@@ -250,7 +255,8 @@ __global__ void __launch_bounds__(SCAN_THREADS, 1) scan_kernel(const ScanArgs a)
 // sequential Float16 adds, same mask layout.
 __global__ void __launch_bounds__(256) scan_long_kernel(const uint32_t* __restrict__ seqw, int64_t rowwords, int64_t seq0, int64_t nseq,
                                                         int32_t W, int32_t K2pad, const uint8_t* __restrict__ blob,
-                                                        const MBlock* __restrict__ lblocks, int32_t n_lblocks, uint32_t* __restrict__ mask) {
+                                                        const MBlock* __restrict__ lblocks, int32_t n_lblocks, uint32_t* __restrict__ mask,
+                                                        const int64_t* __restrict__ lens, int64_t Lb) {
     const int64_t wid = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int lane = threadIdx.x & 31;
     const int64_t per_seq = (int64_t)n_lblocks * GROUP_SLOTS;
@@ -261,7 +267,9 @@ __global__ void __launch_bounds__(256) scan_long_kernel(const uint32_t* __restri
     const int slot = rem % GROUP_SLOTS;
     const GroupMeta* gm = reinterpret_cast<const GroupMeta*>(blob + mb.blob_off + mb.tab_bytes);
     const uint8_t* tab = blob + mb.blob_off + slot * 8;
-    const int len = gm->len, npos = gm->npos[slot >> 1];
+    const int len = gm->len;
+    int npos = gm->npos[slot >> 1];
+    if (lens) npos = max(0, npos - (int)(Lb - lens[seq0 + n]));          // ragged store: this row's own start positions
     const __half thr = __ushort_as_half(gm->thr[slot]);
     const uint32_t* srow = seqw + (seq0 + n) * rowwords;
     for (int w = 0; w < W; ++w) {
@@ -1093,7 +1101,8 @@ static int32_t scan_impl(mb200_ctx* ctx, const mb200_seqs* seqs, const uint16_t*
     const int32_t blob_cap = (P.max_blob_bytes + 127) & ~127;
     const size_t smem_bytes = (size_t)blob_cap + (size_t)tile_cap_words * 8 + 64;
     if (smem_bytes > ctx->smem_optin) MB_FAIL(ctx, MB200_E_UNSUPPORTED, "scan needs %zu B shared memory (> %zu)", smem_bytes, ctx->smem_optin);
-    MB_CUDA(ctx, cudaFuncSetAttribute(scan_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
+    const bool ragged = seqs->lens != nullptr;
+    MB_CUDA(ctx, cudaFuncSetAttribute(ragged ? scan_kernel<true> : scan_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
 
     MbTimers tm(ctx);
     const int t_total = tm.begin(T_TOTAL);
@@ -1175,7 +1184,7 @@ static int32_t scan_impl(mb200_ctx* ctx, const mb200_seqs* seqs, const uint16_t*
             }
             MB_CUDA(ctx, cudaMemsetAsync(ctr_b, 0, 64, ctx->stream));
             TcArgs ta;
-            ta.seqw = seqs->words; ta.rowwords = rowwords; ta.seq0 = s0;
+            ta.seqw = seqs->words; ta.rowwords = rowwords; ta.seq0 = s0; ta.lens = seqs->lens;
             ta.Lb = (uint32_t)Lb; ta.vtotal = (uint32_t)(ns * Lb);
             ta.blob = d_tc; ta.nblocks = (int32_t)TP.blocks.size();
             memset(ta.blocks, 0, sizeof ta.blocks); memcpy(ta.blocks, TP.blocks.data(), TP.blocks.size() * sizeof(TcBlock));
@@ -1201,7 +1210,7 @@ static int32_t scan_impl(mb200_ctx* ctx, const mb200_seqs* seqs, const uint16_t*
             const int t_vf = tm.begin_on(T_EMIT, aux);
             // 128-thread blocks: next to a k_scan_tc CTA (608 threads x 96 registers) an SM has ~7 K registers left
             k_scan_tc_verify<<<grid * 16, 128, 0, aux>>>(list_b, ctr_b, tc_cap, ta.slots, (const EmitMotif*)(d_plan + off_em), d_plan + off_blob,
-                                                        seqs->words, rowwords, s0, (uint32_t)Lb, W, P.K2pad, d_mask, ctr_b + 2, ubits_b, ulist_b, ctr_b + 4);
+                                                        seqs->words, rowwords, s0, (uint32_t)Lb, W, P.K2pad, d_mask, ctr_b + 2, ubits_b, ulist_b, ctr_b + 4, seqs->lens);
             tm.end_on(t_vf, aux);
             const int t_ct = tm.begin_on(T_COUNT, aux);
             count_listed_kernel<<<grid * 16, 128, 0, aux>>>(d_mask, ulist_b, ctr_b + 4, W, P.K2pad, (const int32_t*)(d_plan + off_p2m),
@@ -1277,6 +1286,7 @@ static int32_t scan_impl(mb200_ctx* ctx, const mb200_seqs* seqs, const uint16_t*
         a.blob = d_plan + off_blob; a.mblocks = (const MBlock*)(d_plan + off_mb); a.n_mblocks = (int32_t)P.mblocks.size();
         a.tile_chunks = tile_chunks; a.ntiles = ntiles; a.tile_cap_words = tile_cap_words; a.blob_cap_bytes = blob_cap;
         a.cta_range = d_rng;
+        a.lens = seqs->lens; a.Lb = Lb;
         bool tc_done = false;
         if (use_tc) {
             const size_t need = (size_t)ns * mask_bytes_per_seq;
@@ -1287,7 +1297,7 @@ static int32_t scan_impl(mb200_ctx* ctx, const mb200_seqs* seqs, const uint16_t*
             MB_CUDA(ctx, cudaMemsetAsync(d_tc_ctr, 0, 64, ctx->stream));
             if (tc_units) MB_CUDA(ctx, cudaMemsetAsync(d_tc_ubits, 0, (((size_t)ns * (size_t)(P.K2pad / 2) + 31) / 32) * 4, ctx->stream));
             TcArgs ta;
-            ta.seqw = seqs->words; ta.rowwords = rowwords; ta.seq0 = s0;
+            ta.seqw = seqs->words; ta.rowwords = rowwords; ta.seq0 = s0; ta.lens = seqs->lens;
             ta.Lb = (uint32_t)Lb; ta.vtotal = (uint32_t)(ns * Lb);
             ta.blob = d_tc; ta.nblocks = (int32_t)TP.blocks.size();
             memset(ta.blocks, 0, sizeof ta.blocks); memcpy(ta.blocks, TP.blocks.data(), TP.blocks.size() * sizeof(TcBlock));
@@ -1306,7 +1316,7 @@ static int32_t scan_impl(mb200_ctx* ctx, const mb200_seqs* seqs, const uint16_t*
             const int t_vf = tm.begin(T_EMIT);
             k_scan_tc_verify<<<grid * 8, 256, 0, ctx->stream>>>(d_tc_list, d_tc_ctr, tc_cap, ta.slots, (const EmitMotif*)(d_plan + off_em), d_plan + off_blob,
                                                                  seqs->words, rowwords, s0, (uint32_t)Lb, W, P.K2pad, d_mask, d_tc_ctr + 2,
-                                                                 tc_units ? d_tc_ubits : nullptr, d_tc_ulist, d_tc_ctr + 4);
+                                                                 tc_units ? d_tc_ubits : nullptr, d_tc_ulist, d_tc_ctr + 4, seqs->lens);
             tm.end(t_vf);
             ctx->launches[T_SCAN] += 1; ctx->launches[T_EMIT] += 1;
             MB_CUDA(ctx, cudaGetLastError());
@@ -1345,11 +1355,16 @@ static int32_t scan_impl(mb200_ctx* ctx, const mb200_seqs* seqs, const uint16_t*
         else {
         int t1 = tm.begin(T_SCAN);
         ctx->mask_clean_bytes = 0;
-        if (!P.mblocks.empty()) { scan_kernel<<<grid, SCAN_THREADS, smem_bytes, ctx->stream>>>(a); ctx->launches[T_SCAN] += 1; }
+        if (!P.mblocks.empty()) {
+            if (ragged) scan_kernel<true><<<grid, SCAN_THREADS, smem_bytes, ctx->stream>>>(a);
+            else scan_kernel<false><<<grid, SCAN_THREADS, smem_bytes, ctx->stream>>>(a);
+            ctx->launches[T_SCAN] += 1;
+        }
         if (!P.lblocks.empty()) {
             const int64_t warps = ns * (int64_t)P.lblocks.size() * GROUP_SLOTS;
             scan_long_kernel<<<(unsigned)((warps * 32 + 255) / 256), 256, 0, ctx->stream>>>(seqs->words, rowwords, s0, ns, W, P.K2pad, d_plan + off_blob,
-                                                                                        (const MBlock*)(d_plan + off_lb), (int32_t)P.lblocks.size(), d_mask);
+                                                                                        (const MBlock*)(d_plan + off_lb), (int32_t)P.lblocks.size(), d_mask,
+                                                                                        seqs->lens, Lb);
             ctx->launches[T_SCAN] += 1;
         }
         tm.end(t1);

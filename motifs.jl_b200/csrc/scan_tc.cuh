@@ -62,6 +62,7 @@ struct TcSlot {                            // per global slot, for the epilogue 
 };
 struct TcArgs {
     const uint32_t* seqw; int64_t rowwords; int64_t seq0;
+    const int64_t* lens;                   // ragged stores: row lengths (nullptr: every row has Lb bases)
     uint32_t Lb; uint32_t vtotal;          // virtual positions of the batch: v = n_local * Lb + p
     const uint8_t* blob; int32_t nblocks;
     TcBlock blocks[TCS_MAX_ENTRIES];       // by value: kernel parameters live in the constant bank, so everything derived from an entry (trip
@@ -399,12 +400,22 @@ __global__ void __launch_bounds__(TCS_THREADS, 1) k_scan_tc(const TcArgs a) {
             __syncwarp();
             if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" :: "r"(bar(2 * TCS_STAGES + 2 + ac)) : "memory");    // the values are in registers: the accumulator may be overwritten
             const float ma = tcs_max32(ua), mb = tcs_max32(ub);
-            const bool pos = inb && fmaxf(ma, mb) > 0.f;
+            bool pos = inb && fmaxf(ma, mb) > 0.f;
             if (__any_sync(0xffffffffu, pos)) {          /* about one use in ten at the usual thresholds */
-                uint32_t cb0 = 0u, cb1 = 0u;             // bit masks of the positive columns, only for the chunk(s) that have any
-                if (__any_sync(0xffffffffu, inb && ma > 0.f)) cb0 = pos ? tcs_posbits(ua) : 0u;
-                if (__any_sync(0xffffffffu, inb && mb > 0.f)) cb1 = pos ? tcs_posbits(ub) : 0u;
-                tcs_append(a.list, a.gcount, a.cap, a.overflow, lane, cb0, cb1, (uint32_t)(blk.slot0[sub] + cg * 64), v, cur_end, &dead);
+                // ragged store: a start position in the row's zero padding (poly-A) is no candidate, or an A-rich PWM would fill the
+                // list with padding.  Windows that start inside the row and run into the padding are left to the verifier.
+                bool live = inb;
+                if (a.lens) {
+                    const uint32_t n = v / a.Lb;
+                    live = inb && (int64_t)(v - n * a.Lb) < __ldg(a.lens + a.seq0 + n);
+                    pos = pos && live;
+                }
+                if (!a.lens || __any_sync(0xffffffffu, pos)) {
+                    uint32_t cb0 = 0u, cb1 = 0u;             // bit masks of the positive columns, only for the chunk(s) that have any
+                    if (__any_sync(0xffffffffu, live && ma > 0.f)) cb0 = pos ? tcs_posbits(ua) : 0u;
+                    if (__any_sync(0xffffffffu, live && mb > 0.f)) cb1 = pos ? tcs_posbits(ub) : 0u;
+                    tcs_append(a.list, a.gcount, a.cap, a.overflow, lane, cb0, cb1, (uint32_t)(blk.slot0[sub] + cg * 64), v, cur_end, &dead);
+                }
             }
         }
         for (unsigned long long i = cur_end[0] + lane; i < cur_end[1]; i += 32) a.list[i] = ~0ull;
@@ -420,7 +431,8 @@ __global__ void __launch_bounds__(256) k_scan_tc_verify(const unsigned long long
                                                         unsigned long long cap, const TcSlot* __restrict__ slots, const EmitMotif* __restrict__ em,
                                                         const uint8_t* __restrict__ blob, const uint32_t* __restrict__ seqw, int64_t rowwords, int64_t seq0,
                                                         uint32_t Lb, int32_t W, int32_t K2pad, uint32_t* __restrict__ mask, unsigned long long* __restrict__ stats,
-                                                        uint32_t* __restrict__ unit_bits, uint32_t* __restrict__ unit_list, unsigned long long* __restrict__ n_units) {
+                                                        uint32_t* __restrict__ unit_bits, uint32_t* __restrict__ unit_list, unsigned long long* __restrict__ n_units,
+                                                        const int64_t* __restrict__ lens) {
     if (gcount[1]) return;                                                                // the list overflowed: this batch is re-run on scan_kernel
     const unsigned long long total = min(*gcount, cap);
     unsigned int n_cand = 0, n_hit = 0;
@@ -431,6 +443,7 @@ __global__ void __launch_bounds__(256) k_scan_tc_verify(const unsigned long long
         const uint32_t n = v / Lb, p = v - n * Lb;
         const TcSlot sl = slots[slot];
         if ((int32_t)p >= sl.npos) continue;                                              // the window runs past the end of its sequence (or the slot is disabled)
+        if (lens && (int64_t)p + sl.len > lens[seq0 + n]) continue;                       // ragged store: ... past the end of its own row
         const EmitMotif m = em[sl.motif];
         const uint8_t* tab = blob + m.tab_off + sl.strand * m.strand_stride;
         const uint32_t* srow = seqw + (seq0 + n) * rowwords;

@@ -58,6 +58,30 @@ __global__ void __launch_bounds__(256) pack_ascii_kernel(const uint8_t* __restri
     if (bad) atomicAdd(bad_count, 1u);
 }
 
+// Concatenated rows of different lengths -> padded 2-bit rows.  One thread per output word; row r's bytes start at
+// off[r] - off0 in the staged chunk.  Words past the row's end are written as zero (the padding every consumer relies on).
+__global__ void __launch_bounds__(256) pack_ascii_ragged_kernel(const uint8_t* __restrict__ ascii, const int64_t* __restrict__ off, int64_t off0,
+                                                                int64_t n0, int64_t nrows, int64_t rowwords, uint32_t* __restrict__ out,
+                                                                unsigned int* __restrict__ bad_count) {
+    int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= nrows * rowwords) return;
+    int64_t r = t / rowwords;
+    int w = (int)(t - r * rowwords);
+    const int64_t a = off[n0 + r], len = off[n0 + r + 1] - a;
+    const uint8_t* src = ascii + (a - off0) + (int64_t)w * 16;
+    const int nb = (int)max((int64_t)0, min((int64_t)16, len - (int64_t)w * 16));
+    uint32_t word = 0, bad = 0;
+    for (int i = 0; i < nb; ++i) {
+        uint32_t c = src[i];
+        uint32_t up = c & 0xDFu;
+        bad |= !(up == 0x41u || up == 0x43u || up == 0x47u || up == 0x54u);
+        uint32_t x = (c >> 1) & 3u; x ^= (x >> 1);
+        word |= x << (2 * i);
+    }
+    out[(n0 + r) * rowwords + w] = word;
+    if (bad) atomicAdd(bad_count, 1u);
+}
+
 // ---------------------------------------------------------------------------------------------
 // one-hot Float32 (4*Lb, N) column-major -> 2 bit.  One lane per base (coalesced float4 loads),
 // 16 lanes OR-reduce into one word with shuffles.
@@ -174,6 +198,89 @@ extern "C" int32_t mb200_seqs_from_onehot_f32(mb200_ctx* ctx, const float* oneho
     return pack_common(ctx, onehot, true, true, N, Lb, out);
 }
 
+int mb_seqs_set_lens(mb200_ctx* ctx, mb200_seqs* s, std::vector<int64_t> hlens) {
+    s->ragged = true;
+    s->hlens = std::move(hlens);
+    if (s->N == 0) return MB200_OK;
+    const size_t bytes = (size_t)s->N * 8;
+    s->lens = (int64_t*)mb_pool_alloc(ctx, bytes, &s->lens_bytes);
+    if (!s->lens) MB_FAIL(ctx, MB200_E_NOMEM, "cudaMalloc(%zu) for row lengths failed", bytes);
+    MB_CUDA(ctx, cudaMemcpyAsync(s->lens, s->hlens.data(), bytes, cudaMemcpyHostToDevice, ctx->stream));
+    MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    return MB200_OK;
+}
+
+// Rows of different lengths: row i = ascii[offsets[i], offsets[i+1]).  Lb = the longest row (at least 1), rows padded with zero words.
+// Staged like pack_common: whole rows per chunk of at most 256 MB (a longer row is a chunk of its own).
+extern "C" int32_t mb200_seqs_from_ascii_ragged(mb200_ctx* ctx, const uint8_t* ascii, const int64_t* offsets, int64_t N, mb200_seqs** out) {
+    if (!ctx) return MB200_E_INVALID;
+    if (!out || N < 0 || !offsets) MB_FAIL(ctx, MB200_E_INVALID, "seqs_ragged: bad arguments (N=%lld)", (long long)N);
+    *out = nullptr;
+    std::vector<int64_t> hl((size_t)N);
+    int64_t Lb = 1;
+    for (int64_t i = 0; i < N; ++i) {
+        hl[(size_t)i] = offsets[i + 1] - offsets[i];
+        if (offsets[i] < 0 || hl[(size_t)i] < 0) MB_FAIL(ctx, MB200_E_INVALID, "seqs_ragged: offsets must be non-negative and non-decreasing (row %lld)", (long long)i);
+        Lb = std::max(Lb, hl[(size_t)i]);
+    }
+    if (!ascii && N > 0 && offsets[N] > offsets[0]) MB_FAIL(ctx, MB200_E_INVALID, "seqs_ragged: null input");
+    mb_reset_timing(ctx);
+    int rc = mb_seqs_alloc(ctx, N, Lb, out);
+    if (rc) return rc;
+    mb200_seqs* s = *out;
+    auto fail = [&](int code) { mb200_seqs_free(ctx, s); *out = nullptr; return code; };
+    rc = mb_seqs_set_lens(ctx, s, hl);
+    if (rc) return fail(rc);
+    if (N == 0) return MB200_OK;
+    MbTimers tm(ctx);
+    int t_total = tm.begin(T_TOTAL);
+    const size_t stage_cap = (size_t)256 << 20;
+    const size_t off_bytes = ((size_t)(N + 1) * 8 + 255) & ~(size_t)255;
+    size_t stage_need = 0;                                   // the largest chunk the loop below stages
+    for (int64_t n0 = 0; n0 < N;) {
+        int64_t n1 = n0 + 1;
+        while (n1 < N && (size_t)(offsets[n1 + 1] - offsets[n0]) <= stage_cap) ++n1;
+        stage_need = std::max(stage_need, (size_t)(offsets[n1] - offsets[n0]));
+        n0 = n1;
+    }
+    rc = mb_ensure_scratch(ctx, 256 + off_bytes + stage_need);
+    if (rc) return fail(rc);
+    unsigned int* d_bad = (unsigned int*)ctx->scratch;
+    int64_t* d_off = (int64_t*)((uint8_t*)ctx->scratch + 256);
+    uint8_t* d_stage = (uint8_t*)ctx->scratch + 256 + off_bytes;
+    cudaError_t e = cudaMemsetAsync(d_bad, 0, 4, ctx->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(d_off, offsets, (size_t)(N + 1) * 8, cudaMemcpyHostToDevice, ctx->stream);
+    for (int64_t n0 = 0; n0 < N && e == cudaSuccess;) {
+        int64_t n1 = n0 + 1;
+        while (n1 < N && (size_t)(offsets[n1 + 1] - offsets[n0]) <= stage_cap) ++n1;
+        const size_t bytes = (size_t)(offsets[n1] - offsets[n0]);
+        int th = tm.begin(T_H2D);
+        if (bytes) e = cudaMemcpyAsync(d_stage, ascii + offsets[n0], bytes, cudaMemcpyHostToDevice, ctx->stream);
+        tm.end(th);
+        int tp = tm.begin(T_PACK);
+        const int64_t threads = (n1 - n0) * s->rowwords;
+        pack_ascii_ragged_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, ctx->stream>>>(d_stage, d_off, offsets[n0], n0, n1 - n0, s->rowwords, s->words, d_bad);
+        tm.end(tp);
+        ctx->launches[T_PACK] += 1;
+        if (e == cudaSuccess) e = cudaGetLastError();
+        n0 = n1;
+    }
+    unsigned int h_bad = 0;
+    if (e == cudaSuccess) e = cudaMemcpyAsync(&h_bad, d_bad, 4, cudaMemcpyDeviceToHost, ctx->stream);
+    tm.end(t_total);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+    if (e != cudaSuccess) { fail(0); MB_FAIL(ctx, MB200_E_CUDA, "seqs_ragged: %s", cudaGetErrorString(e)); }
+    tm.collect();
+    if (h_bad) { fail(0); MB_FAIL(ctx, MB200_E_BAD_SEQUENCE, "%u words contain a symbol that is not A,C,G,T", h_bad); }
+    return MB200_OK;
+}
+
+extern "C" int32_t mb200_seqs_lengths(const mb200_seqs* s, int64_t* out) {
+    if (!s || (!out && s->N > 0)) return MB200_E_INVALID;
+    for (int64_t n = 0; n < s->N; ++n) out[n] = mb_row_len(s, n);
+    return MB200_OK;
+}
+
 // Asynchronous upload: H2D copies (64 MB chunks, two staging buffers) and pack kernels are queued on the ctx's copy stream and the
 // call returns; an event per chunk tells mb200_scan which sequences are ready, so the scan of the first batch starts while later
 // chunks are still crossing PCIe.  The host buffer must stay valid (and should be pinned) until the first scan of these sequences
@@ -238,6 +345,7 @@ extern "C" int32_t mb200_seqs_free(mb200_ctx* ctx, mb200_seqs* s) {
     if (ctx) cudaSetDevice(ctx->device);
     if (s->pending) { cudaStreamSynchronize(s->copy_stream); for (auto ev : s->ready) cudaEventDestroy(ev); mb_pool_free(ctx, s->stage, s->stage_bytes); s->pending = false; }
     if (s->words) mb_pool_free(ctx, s->words, s->words_bytes);
+    if (s->lens) mb_pool_free(ctx, s->lens, s->lens_bytes);
     delete s;
     return MB200_OK;
 }

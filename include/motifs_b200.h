@@ -207,6 +207,22 @@ int32_t mb200_scan_hist(mb200_ctx* ctx, const mb200_seqs* seqs,
                         const uint16_t* pwms_f16, const int64_t* lens, int32_t K, int32_t maxlen,
                         uint32_t flags, uint32_t* hist);
 
+/* Best site per (sequence, motif): the highest score of every window greedy_search! scores (inference/_h3_1_alignment.jl:18-36),
+ * the per-sequence motif feature behind AUC and central-enrichment statistics.  Windows of row n (length L_n) and motif k
+ * (length m_k) start at 0 .. L_n - m_k, on the requested strands (MB200_SCAN_FWD: pwm, MB200_SCAN_RC: reverse(pwm)); a window's
+ * score has the bits mb200_scan reports for it.  NaN windows are ignored, -Inf is a score.  Ties go to the smaller position, then
+ * to the forward strand.  The SIMT scan kernel computes it (no tensor-core path: a best site has no threshold to pre-filter with). */
+typedef struct {
+    uint32_t pos;        /* 0-based start on the forward strand; UINT32_MAX when found == 0          */
+    uint16_t score_f16;  /* Float16 bits, identical to mb200_scan's score of that window            */
+    uint8_t  comp;       /* 0 = pwm, 1 = reverse(pwm)                                               */
+    uint8_t  found;      /* 0: no window of this motif in the row, or every window is NaN           */
+} mb200_best;            /* 8 bytes */
+/* best[n*K + k] for every row n of seqs and motif k; flags: MB200_SCAN_FWD | MB200_SCAN_RC only (any other bit, a null best or
+ * no strand: MB200_E_INVALID).  Rows are per rank: there is nothing to reduce over a communicator.                          */
+int32_t mb200_scan_best(mb200_ctx* ctx, const mb200_seqs* seqs, const uint16_t* pwms_f16, const int64_t* lens,
+                        int32_t K, int32_t maxlen, uint32_t flags, mb200_best* best);
+
 /* ---- unrolled convolutional-sparse-coding network: replaces the GPU work inside
  *      forward_pass_return_loss (model.jl:375-395) + gradient(ps) + Flux.Optimise.update!
  *      (train.jl:42-46) and code_retrieval (inference/_1_code_retrieval.jl:33-56).            */

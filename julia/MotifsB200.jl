@@ -9,6 +9,9 @@ const lib = get(ENV, "MOTIFS_B200_LIB", "libmotifs_b200.so")
 struct Hit            # mb200_hit (16 bytes)
     seq::UInt32; pos::UInt32; motif::UInt16; score::Float16; comp::UInt8; p1::UInt8; p2::UInt8; p3::UInt8
 end
+struct Best           # mb200_best (8 bytes)
+    pos::UInt32; score::Float16; comp::UInt8; found::UInt8
+end
 struct Code           # mb200_code (12 bytes)
     position::UInt16; fil::UInt16; seq::UInt32; mag::Float16; pad::UInt16
 end
@@ -285,6 +288,18 @@ function scan_hist(ctx, seqs, pwms::Array{Float16,3}, lens::Vector{Int64}; reduc
         ctx, seqs, pwms, lens, K, maxlen, SCAN_FWD | SCAN_RC | (reduce ? SCAN_REDUCE : UInt32(0)), hist))
     hist
 end
+# best site per (sequence, motif) over every window greedy_search! scores (_h3_1_alignment.jl:18-36), both strands by default:
+# (K, N) NamedTuples with 1-based `pos` (0 when not found), `comp` (true = reverse(pwm)), `score`, `found`.  Ties: smaller
+# position, then the forward strand.  The per-sequence feature behind AUC / central-enrichment statistics.
+function scan_best(ctx, seqs, N::Integer, pwms::Array{Float16,3}, lens::Vector{Int64}; fwd=true, rc=true)
+    K, _, maxlen = size(pwms)
+    out = Matrix{Best}(undef, K, N)                                    # row-major (N, K) in C = (K, N) in Julia
+    GC.@preserve pwms lens out check(ctx, ccall((:mb200_scan_best, lib), Int32,
+        (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Float16}, Ptr{Int64}, Int32, Int32, UInt32, Ptr{Best}),
+        ctx, seqs, pwms, lens, K, maxlen, (fwd ? SCAN_FWD : UInt32(0)) | (rc ? SCAN_RC : UInt32(0)), out))
+    [(pos = b.found != 0 ? Int(b.pos) + 1 : 0, comp = b.comp != 0, score = b.score, found = b.found != 0) for b in out]
+end
+
 # fused scan + filter_position_by_best_thresh! + get_uniq_counts + union_ranges coverage: (4, K) Int64, rows = hits, unique starts,
 # coverage as the reference computes it (_h4_overlap_ratio.jl:48-56), true coverage
 scan_counts(ctx, seqs, pwms, lens, thresh::Vector{Float16}; reduce=false) =

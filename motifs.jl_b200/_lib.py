@@ -33,6 +33,9 @@ HIT_DTYPE = np.dtype([("seq", "<u4"), ("pos", "<u4"), ("motif", "<u2"), ("score_
                       ("comp", "u1"), ("_pad", "u1", (3,))])
 assert HIT_DTYPE.itemsize == 16
 
+BEST_DTYPE = np.dtype([("pos", "<u4"), ("score_f16", "<u2"), ("comp", "u1"), ("found", "u1")])
+assert BEST_DTYPE.itemsize == 8
+
 SITE_DTYPE = np.dtype([("motif", "<u4"), ("seq", "<u4"), ("pos", "<u4"), ("comp", "<u4")])
 CODE_DTYPE = np.dtype([("position", "<u2"), ("fil", "<u2"), ("seq", "<u4"), ("mag_f16", "<u2"), ("_pad", "<u2")])
 assert CODE_DTYPE.itemsize == 12
@@ -103,6 +106,7 @@ def load():
         "mb200_scan_last_path": (i32, [p]),
         "mb200_scan_prefilter_bound": (i32, [p, i32, C.c_uint16, p, p, p, p]),
         "mb200_scan_hist": (i32, [p, p, p, p, i32, i32, C.c_uint32, p]),
+        "mb200_scan_best": (i32, [p, p, p, p, i32, i32, C.c_uint32, p]),
         "mb200_csc_create": (i32, [p, C.POINTER(HParams), i64, i32, i32, C.POINTER(p)]),
         "mb200_csc_destroy": (i32, [p, p]),
         "mb200_csc_n_params": (i32, [p, C.POINTER(i64), C.POINTER(i64)]),
@@ -274,21 +278,26 @@ class Context:
         return Sequences(self, h, a.shape[0], a.shape[1] // 4)
 
     # ---- scan --------------------------------------------------------------------------------
+    @staticmethod
+    def _pwm_arrays(pwms_f16, lens):
+        pw = np.ascontiguousarray(pwms_f16)
+        if pw.dtype == np.float16:
+            pw = pw.view(np.uint16)
+        if pw.dtype != np.uint16 or pw.ndim != 3 or pw.shape[1] != 4:
+            raise ValueError("pwms_f16 must be float16/uint16 of numpy shape (maxlen, 4, K)")
+        ln = np.ascontiguousarray(lens, dtype=np.int64)
+        if ln.shape != (pw.shape[2],):
+            raise ValueError("lens must have K entries")
+        return pw, ln
+
     def scan(self, seqs: "Sequences", pwms_f16: np.ndarray, lens, thresh_f16=None, *, fwd=True, rc=True,
              want_hits=True, want_counts=True, hits_cap=None, tensor=True, reduce=False):
         """pwms_f16: (K, 4, maxlen) array in Julia memory order, i.e. numpy shape (maxlen, 4, K) C-order
         holding float16 (or uint16 bits).  Returns (hits structured array | None, counts (K,4) int64 | None).
         tensor=False keeps a thresholded scan on the SIMT kernel (MB200_SCAN_NO_TENSOR); results are identical either way.
         reduce=True: counts are summed over the ranks of the ctx's communicator inside the call (MB200_SCAN_REDUCE)."""
-        pw = np.ascontiguousarray(pwms_f16)
-        if pw.dtype == np.float16:
-            pw = pw.view(np.uint16)
-        if pw.dtype != np.uint16 or pw.ndim != 3 or pw.shape[1] != 4:
-            raise ValueError("pwms_f16 must be float16/uint16 of numpy shape (maxlen, 4, K)")
+        pw, ln = self._pwm_arrays(pwms_f16, lens)
         maxlen, _, K = pw.shape
-        ln = np.ascontiguousarray(lens, dtype=np.int64)
-        if ln.shape != (K,):
-            raise ValueError("lens must have K entries")
         th = None
         if thresh_f16 is not None:
             th = np.ascontiguousarray(thresh_f16)
@@ -311,6 +320,17 @@ class Context:
             rc_ = self._lib.mb200_scan_take_hits(self._h, _ptr(hits), len(hits), C.byref(n_hits))
         self._check(rc_)
         return (hits[: n_hits.value] if want_hits else None), counts
+
+    def scan_best(self, seqs: "Sequences", pwms_f16: np.ndarray, lens, *, fwd=True, rc=True) -> np.ndarray:
+        """Best site of every (row, motif) (mb200_scan_best): (N, K) BEST_DTYPE array {pos, score_f16, comp, found}.  pwms_f16 and
+        lens as for scan.  Highest score, then lowest position, then the forward strand; found = 0 (pos = 2**32 - 1) when the row
+        has no window of the motif on the requested strands or every window is NaN."""
+        pw, ln = self._pwm_arrays(pwms_f16, lens)
+        maxlen, _, K = pw.shape
+        out = np.empty((seqs.N, K), BEST_DTYPE)                   # every record is written
+        flags = (SCAN_FWD if fwd else 0) | (SCAN_RC if rc else 0)
+        self._check(self._lib.mb200_scan_best(self._h, seqs._h, _ptr(pw), _ptr(ln), K, maxlen, flags, _ptr(out)))
+        return out
 
 
 def fasta_read(path: str, max_entries: int = 100000) -> np.ndarray:

@@ -48,6 +48,7 @@ struct __align__(16) GroupMeta {
     uint16_t thr[GROUP_SLOTS];         // Float16 bits per slot: max(thresh, 0), +Inf for a disabled strand / padding
 };                                     // 144 bytes
 static_assert(sizeof(GroupMeta) == 144, "GroupMeta must be 144 bytes");
+static_assert(sizeof(mb200_best) == 8, "mb200_best must be 8 bytes");
 
 struct MBlock {
     int64_t blob_off;                  // byte offset of this motif block's blob (tables then metas)
@@ -110,8 +111,13 @@ __device__ __forceinline__ int64_t block_word(int64_t gq, int32_t W16, int64_t r
     return n * rowwords + (int64_t)pb;
 }
 
+// Best-site keys (mb200_scan_best): ord() orders Float16 bit patterns like their values; only a NaN maps to 0.  A block key is
+// ord(score) << 4 | (15 - u) for the best valid start u of a 16-position block (the lowest u among equal scores), 0 for none.
+__device__ __forceinline__ uint32_t h16_ord(uint32_t h) { return (h & 0x8000u) ? (~h & 0xFFFFu) : (h | 0x8000u); }
+
 // RAGGED: row n has lens[n] <= Lb bases; its start positions end Lb - lens[n] earlier than the group metas say (the "deficit").
-template <bool RAGGED>
+// BEST: instead of hit-mask half-words, write one best-site key per (position block, slot) to a.mask[lq * K2pad + slot].
+template <bool RAGGED, bool BEST = false>
 __global__ void __launch_bounds__(SCAN_THREADS, 1) scan_kernel(const ScanArgs a) {
     extern __shared__ __align__(128) uint8_t smem[];
     uint8_t* s_blob = smem;                                                        // tables + metas of one motif block
@@ -207,11 +213,13 @@ __global__ void __launch_bounds__(SCAN_THREADS, 1) scan_kernel(const ScanArgs a)
             }
             // this block is the low (pb even) or high (pb odd) half of mask word (n, pb/2)
             uint16_t* mrow = reinterpret_cast<uint16_t*>(a.mask + (lq >> 1) * (int64_t)a.K2pad + (int64_t)mbk.g0 * GROUP_SLOTS) + (pb & 1);
+            uint32_t* krow = a.mask + lq * (int64_t)a.K2pad + (int64_t)mbk.g0 * GROUP_SLOTS;
 
             for (int32_t g = 0; g < mbk.ng; ++g) {
                 const GroupMeta* gm = s_meta + g;
                 if (p0 >= gm->npos_max - deficit) {           // warp-uniform: no valid start position in this block
-                    mrow[(g * GROUP_SLOTS + lane) * 2] = 0;
+                    if constexpr (BEST) krow[g * GROUP_SLOTS + lane] = 0u;
+                    else mrow[(g * GROUP_SLOTS + lane) * 2] = 0;
                     continue;
                 }
                 const int32_t len = gm->len;
@@ -231,17 +239,41 @@ __global__ void __launch_bounds__(SCAN_THREADS, 1) scan_kernel(const ScanArgs a)
                     #pragma unroll
                     for (int k = 0; k < POS_BLOCK / 2; ++k) acc[k] = __hadd2(acc[k], as_h2(__byte_perm(e1.x, e1.y, sel[2 * k + j + 1])));
                 }
-                const uint32_t t16 = gm->thr[lane];
-                const __half2 thr = as_h2(t16 | (t16 << 16));
-                uint32_t bits = 0;
-                #pragma unroll
-                for (int k = 0; k < POS_BLOCK / 2; ++k) {
-                    const uint32_t m = __hgt2_mask(acc[k], thr);
-                    bits |= ((m & 1u) | ((m >> 15) & 2u)) << (2 * k);
+                if constexpr (BEST) {
+                    // start positions past the row's last window and disabled slots (+Inf threshold: strand not requested, padding)
+                    // become NaN, which __hmax2 ignores; the lowest position holding the maximum wins
+                    const int32_t nvalid = gm->thr[lane] == 0x7C00u ? 0 : min(max(gm->npos[lane >> 1] - deficit - p0, 0), POS_BLOCK);
+                    const uint32_t inv = ~((1u << nvalid) - 1u);
+                    __half2 mx = as_h2(0x7E007E00u);
+                    #pragma unroll
+                    for (int k = 0; k < POS_BLOCK / 2; ++k) {
+                        const uint32_t nan = ((inv >> (2 * k)) & 1u) * 0x7E00u | ((inv >> (2 * k + 1)) & 1u) * 0x7E000000u;
+                        acc[k] = as_h2(*reinterpret_cast<uint32_t*>(&acc[k]) | nan);
+                        mx = __hmax2(mx, acc[k]);
+                    }
+                    const __half m1 = __hmax(__low2half(mx), __high2half(mx));
+                    const __half2 mm = __half2half2(m1);
+                    uint32_t eq = 0;
+                    #pragma unroll
+                    for (int k = 0; k < POS_BLOCK / 2; ++k) {
+                        const uint32_t m = __heq2_mask(acc[k], mm);
+                        eq |= ((m & 1u) | ((m >> 15) & 2u)) << (2 * k);
+                    }
+                    const uint32_t u = (uint32_t)__ffs(eq) - 1u;             // eq == 0 (every position NaN): key 0
+                    krow[g * GROUP_SLOTS + lane] = eq ? (h16_ord(__half_as_ushort(m1)) << 4 | (15u - u)) : 0u;
+                } else {
+                    const uint32_t t16 = gm->thr[lane];
+                    const __half2 thr = as_h2(t16 | (t16 << 16));
+                    uint32_t bits = 0;
+                    #pragma unroll
+                    for (int k = 0; k < POS_BLOCK / 2; ++k) {
+                        const uint32_t m = __hgt2_mask(acc[k], thr);
+                        bits |= ((m & 1u) | ((m >> 15) & 2u)) << (2 * k);
+                    }
+                    const int32_t nvalid = min(max(gm->npos[lane >> 1] - deficit - p0, 0), POS_BLOCK);
+                    bits &= (1u << nvalid) - 1u;
+                    mrow[(g * GROUP_SLOTS + lane) * 2] = (uint16_t)bits;
                 }
-                const int32_t nvalid = min(max(gm->npos[lane >> 1] - deficit - p0, 0), POS_BLOCK);
-                bits &= (1u << nvalid) - 1u;
-                mrow[(g * GROUP_SLOTS + lane) * 2] = (uint16_t)bits;
             }
         }
         __syncthreads();      // tile buffer `buf` and (possibly) the blob may be overwritten next
@@ -252,7 +284,9 @@ __global__ void __launch_bounds__(SCAN_THREADS, 1) scan_kernel(const ScanArgs a)
 
 // Motifs longer than MB200_MAX_MOTIF_LEN columns (rare: the reference trims PWMs to their informative span) are scored by a
 // plain kernel: one warp per (sequence, slot), lanes over 32 start positions, table read from global memory.  Same
-// sequential Float16 adds, same mask layout.
+// sequential Float16 adds, same mask layout.  BEST: lanes 0-15 and 16-31 reduce their starts to the best-site keys of position
+// blocks 2w and 2w+1, in the key layout of scan_kernel<RAGGED, true>.
+template <bool BEST = false>
 __global__ void __launch_bounds__(256) scan_long_kernel(const uint32_t* __restrict__ seqw, int64_t rowwords, int64_t seq0, int64_t nseq,
                                                         int32_t W, int32_t K2pad, const uint8_t* __restrict__ blob,
                                                         const MBlock* __restrict__ lblocks, int32_t n_lblocks, uint32_t* __restrict__ mask,
@@ -272,9 +306,11 @@ __global__ void __launch_bounds__(256) scan_long_kernel(const uint32_t* __restri
     if (lens) npos = max(0, npos - (int)(Lb - lens[seq0 + n]));          // ragged store: this row's own start positions
     const __half thr = __ushort_as_half(gm->thr[slot]);
     const uint32_t* srow = seqw + (seq0 + n) * rowwords;
+    if (BEST && gm->thr[slot] == 0x7C00u) npos = 0;                     // strand not requested
     for (int w = 0; w < W; ++w) {
         const int pos = w * 32 + lane;
         bool hit = false;
+        uint32_t key = 0;
         if (pos < npos) {
             __half s = __ushort_as_half((unsigned short)0);
             for (int j = 0; j < len; ++j) {
@@ -283,10 +319,65 @@ __global__ void __launch_bounds__(256) scan_long_kernel(const uint32_t* __restri
                 s = __hadd(s, *reinterpret_cast<const __half*>(tab + (int64_t)j * COL_BYTES + base * 2));
             }
             hit = __hgt(s, thr);
+            if (BEST && !__hisnan(s)) key = h16_ord(__half_as_ushort(s)) << 4 | (15u - (uint32_t)(lane & 15));
         }
-        const uint32_t word = __ballot_sync(0xffffffffu, hit);
-        if (lane == 0) mask[(n * W + w) * (int64_t)K2pad + (int64_t)mb.g0 * GROUP_SLOTS + slot] = word;
+        if constexpr (BEST) {
+            #pragma unroll
+            for (int o = 8; o >= 1; o >>= 1) key = max(key, __shfl_xor_sync(0xffffffffu, key, o));
+            if ((lane & 15) == 0) mask[(n * 2 * W + 2 * w + (lane >> 4)) * (int64_t)K2pad + (int64_t)mb.g0 * GROUP_SLOTS + slot] = key;
+        } else {
+            const uint32_t word = __ballot_sync(0xffffffffu, hit);
+            if (lane == 0) mask[(n * W + w) * (int64_t)K2pad + (int64_t)mb.g0 * GROUP_SLOTS + slot] = word;
+        }
     }
+}
+
+// ---------------------------------------------------------------------------------------------
+// Best site per (row, motif) from the block keys of scan_kernel<RAGGED, true> / scan_long_kernel<true>: one thread per (row,
+// motif, chunk of <= BEST_CHUNK position blocks); adjacent threads take adjacent motifs, so the (fwd, rc) key pairs load
+// coalesced.  A thread's best goes into best64[row * K + motif] by atomicMax on
+//   ord(score) << 48 | (0xFFFFFFFF - pos) << 1 | (1 - comp)
+// (higher score, then lower position, then the forward strand), a total order: the result does not depend on the order of
+// arrival.  0 = no window.
+// ---------------------------------------------------------------------------------------------
+#define BEST_CHUNK 1024
+__global__ void __launch_bounds__(256) best_reduce_kernel(const uint32_t* __restrict__ keys, int64_t nseq, int32_t W16, int32_t K2pad, int32_t nch,
+                                                          const int32_t* __restrict__ pair2motif, int32_t K, unsigned long long* __restrict__ best64) {
+    const int32_t P = K2pad / 2;
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= nseq * nch * P) return;
+    const int32_t m2 = (int32_t)(t % P);
+    const int64_t nc = t / P;
+    const int32_t c = (int32_t)(nc % nch);
+    const int64_t n = nc / nch;
+    const int32_t k = pair2motif[m2];
+    if (k < 0) return;
+    const uint2* kp = reinterpret_cast<const uint2*>(keys) + (n * W16) * (int64_t)P + m2;
+    const int32_t b0 = c * BEST_CHUNK, b1 = min(W16, b0 + BEST_CHUNK);
+    unsigned long long best = 0;
+    for (int32_t b = b0; b < b1; ++b) {
+        const uint2 fr = __ldg(kp + (int64_t)b * P);
+        if (fr.x) best = max(best, (unsigned long long)(fr.x >> 4) << 48 | (unsigned long long)(0xFFFFFFFFu - (uint32_t)(b * POS_BLOCK + 15 - (fr.x & 15u))) << 1 | 1ull);
+        if (fr.y) best = max(best, (unsigned long long)(fr.y >> 4) << 48 | (unsigned long long)(0xFFFFFFFFu - (uint32_t)(b * POS_BLOCK + 15 - (fr.y & 15u))) << 1);
+    }
+    if (best) atomicMax(best64 + n * K + k, best);
+}
+
+__global__ void __launch_bounds__(256) best_finalize_kernel(const unsigned long long* __restrict__ best64, int64_t n, mb200_best* __restrict__ out) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const unsigned long long v = best64[i];
+    mb200_best r;
+    if (v) {
+        const uint32_t o = (uint32_t)(v >> 48);
+        r.pos = 0xFFFFFFFFu - (uint32_t)(v >> 1);
+        r.score_f16 = (uint16_t)((o & 0x8000u) ? (o & 0x7FFFu) : (~o & 0xFFFFu));
+        r.comp = (uint8_t)(1u - (uint32_t)(v & 1u));
+        r.found = 1;
+    } else {
+        r.pos = 0xFFFFFFFFu; r.score_f16 = 0; r.comp = 0; r.found = 0;
+    }
+    out[i] = r;
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -955,7 +1046,7 @@ static int build_plan(mb200_ctx* ctx, const uint16_t* pwms, const int64_t* lens,
 
 static int32_t scan_impl(mb200_ctx* ctx, const mb200_seqs* seqs, const uint16_t* pwms_f16, const int64_t* lens, int32_t K,
                          int32_t maxlen, const uint16_t* thresh_f16, uint32_t flags, mb200_hit* hits, int64_t hits_cap,
-                         int64_t* n_hits, int64_t* counts, uint32_t* hist) {
+                         int64_t* n_hits, int64_t* counts, uint32_t* hist, mb200_best* best) {
     if (!ctx) return MB200_E_INVALID;
     if (!seqs || !pwms_f16 || !lens || K <= 0 || K > 65535 || maxlen <= 0)
         MB_FAIL(ctx, MB200_E_INVALID, "scan: bad arguments (K=%d maxlen=%d)", K, maxlen);
@@ -980,7 +1071,7 @@ static int32_t scan_impl(mb200_ctx* ctx, const mb200_seqs* seqs, const uint16_t*
     // Thresholded scans take the tensor-core pre-filter + exact verification (scan_tc.cuh) unless the caller or the inputs rule
     // it out; the hit masks, and everything derived from them, are identical either way.
     TcPlan TP;
-    bool use_tc = !(flags & MB200_SCAN_NO_TENSOR) && !hist && Lb < (1ll << 31);
+    bool use_tc = !(flags & MB200_SCAN_NO_TENSOR) && !hist && !best && Lb < (1ll << 31);
     if (use_tc) use_tc = build_tc_plan(P, pwms_f16, lens, K, thresh_f16, flags, Lb, ctx->sm_count, TP);
     ctx->last_scan_path = 0;
     if (use_tc) {
@@ -993,6 +1084,10 @@ static int32_t scan_impl(mb200_ctx* ctx, const mb200_seqs* seqs, const uint16_t*
     const int64_t npos_max = Lb - P.minlen + 1;
     const bool reduce = (flags & MB200_SCAN_REDUCE) != 0 && ctx->world > 1;
     if (N == 0 || npos_max <= 0) {                      // nothing can be scored on this rank; it still takes part in the reduction
+        if (best) {                                     // no row holds a window (otherwise every batch writes all its records)
+            const mb200_best none = {0xFFFFFFFFu, 0, 0, 0};
+            std::fill(best, best + (size_t)N * K, none);
+        }
         if (reduce && (want_counts || hist)) {
             const size_t nb = hist ? (size_t)K * HIST_BINS * 4 : (size_t)K * 4 * 8;
             rc = mb_ensure_scratch(ctx, nb); if (rc) return rc;
@@ -1035,7 +1130,7 @@ static int32_t scan_impl(mb200_ctx* ctx, const mb200_seqs* seqs, const uint16_t*
 
     // ---- batching: masks of one batch stay under a budget -----------------------------------
     const size_t mask_budget = (size_t)8 << 30;
-    const size_t mask_bytes_per_seq = (size_t)W * P.K2pad * 4;
+    const size_t mask_bytes_per_seq = (size_t)W * P.K2pad * 4 * (best ? 2 : 1);      // best sites: one 32-bit key per 16-position block
     int64_t seqs_per_batch = std::max<int64_t>(1, (int64_t)(mask_budget / mask_bytes_per_seq));
     if (seqs_per_batch > N) seqs_per_batch = N;
     if ((double)seqs_per_batch * W > 2.0e9) seqs_per_batch = std::max<int64_t>(1, (int64_t)(2.0e9 / W));
@@ -1082,6 +1177,13 @@ static int32_t scan_impl(mb200_ctx* ctx, const mb200_seqs* seqs, const uint16_t*
     uint32_t* d_unit_cnt = nullptr; unsigned long long* d_unit_off = nullptr; unsigned long long* d_bsum = nullptr;
     int64_t units_per_batch = seqs_per_batch * K * 2;
     int64_t ps_blocks = (units_per_batch + PS_TILE - 1) / PS_TILE;
+    unsigned long long* d_best64 = nullptr; mb200_best* d_best = nullptr;
+    const int32_t best_nch = (W16 + BEST_CHUNK - 1) / BEST_CHUNK;
+    if (best) {                                         // per batch: 64-bit best keys, then the records
+        rc = mb_ensure_buf(ctx, 3, (size_t)seqs_per_batch * K * 16); if (rc) return rc;
+        d_best64 = (unsigned long long*)ctx->bufs[3];
+        d_best = (mb200_best*)(d_best64 + (size_t)seqs_per_batch * K);
+    }
     if (want_hits) {
         size_t b = (((size_t)units_per_batch * 4 + 255) & ~(size_t)255) + (((size_t)units_per_batch * 8 + 255) & ~(size_t)255) +
                    (size_t)ps_blocks * 8 + 256;
@@ -1102,7 +1204,8 @@ static int32_t scan_impl(mb200_ctx* ctx, const mb200_seqs* seqs, const uint16_t*
     const size_t smem_bytes = (size_t)blob_cap + (size_t)tile_cap_words * 8 + 64;
     if (smem_bytes > ctx->smem_optin) MB_FAIL(ctx, MB200_E_UNSUPPORTED, "scan needs %zu B shared memory (> %zu)", smem_bytes, ctx->smem_optin);
     const bool ragged = seqs->lens != nullptr;
-    MB_CUDA(ctx, cudaFuncSetAttribute(ragged ? scan_kernel<true> : scan_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
+    if (best) MB_CUDA(ctx, cudaFuncSetAttribute(ragged ? scan_kernel<true, true> : scan_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
+    else MB_CUDA(ctx, cudaFuncSetAttribute(ragged ? scan_kernel<true> : scan_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
 
     MbTimers tm(ctx);
     const int t_total = tm.begin(T_TOTAL);
@@ -1356,20 +1459,42 @@ static int32_t scan_impl(mb200_ctx* ctx, const mb200_seqs* seqs, const uint16_t*
         int t1 = tm.begin(T_SCAN);
         ctx->mask_clean_bytes = 0;
         if (!P.mblocks.empty()) {
-            if (ragged) scan_kernel<true><<<grid, SCAN_THREADS, smem_bytes, ctx->stream>>>(a);
-            else scan_kernel<false><<<grid, SCAN_THREADS, smem_bytes, ctx->stream>>>(a);
+            if (best) {
+                if (ragged) scan_kernel<true, true><<<grid, SCAN_THREADS, smem_bytes, ctx->stream>>>(a);
+                else scan_kernel<false, true><<<grid, SCAN_THREADS, smem_bytes, ctx->stream>>>(a);
+            } else {
+                if (ragged) scan_kernel<true><<<grid, SCAN_THREADS, smem_bytes, ctx->stream>>>(a);
+                else scan_kernel<false><<<grid, SCAN_THREADS, smem_bytes, ctx->stream>>>(a);
+            }
             ctx->launches[T_SCAN] += 1;
         }
         if (!P.lblocks.empty()) {
             const int64_t warps = ns * (int64_t)P.lblocks.size() * GROUP_SLOTS;
-            scan_long_kernel<<<(unsigned)((warps * 32 + 255) / 256), 256, 0, ctx->stream>>>(seqs->words, rowwords, s0, ns, W, P.K2pad, d_plan + off_blob,
-                                                                                        (const MBlock*)(d_plan + off_lb), (int32_t)P.lblocks.size(), d_mask,
-                                                                                        seqs->lens, Lb);
+            auto long_kernel = best ? scan_long_kernel<true> : scan_long_kernel<false>;
+            long_kernel<<<(unsigned)((warps * 32 + 255) / 256), 256, 0, ctx->stream>>>(seqs->words, rowwords, s0, ns, W, P.K2pad, d_plan + off_blob,
+                                                                                   (const MBlock*)(d_plan + off_lb), (int32_t)P.lblocks.size(), d_mask,
+                                                                                   seqs->lens, Lb);
             ctx->launches[T_SCAN] += 1;
         }
         tm.end(t1);
         }
         MB_CUDA(ctx, cudaGetLastError());
+
+        if (best) {
+            const int t2 = tm.begin(T_COUNT);
+            MB_CUDA(ctx, cudaMemsetAsync(d_best64, 0, (size_t)ns * K * 8, ctx->stream));
+            const int64_t rthreads = ns * (int64_t)best_nch * (P.K2pad / 2);
+            best_reduce_kernel<<<(unsigned)((rthreads + 255) / 256), 256, 0, ctx->stream>>>(d_mask, ns, W16, P.K2pad, best_nch,
+                                                                                          (const int32_t*)(d_plan + off_p2m), K, d_best64);
+            best_finalize_kernel<<<(unsigned)((ns * K + 255) / 256), 256, 0, ctx->stream>>>(d_best64, ns * K, d_best);
+            tm.end(t2);
+            ctx->launches[T_COUNT] += 2;
+            MB_CUDA(ctx, cudaGetLastError());
+            const int t6 = tm.begin(T_D2H);
+            MB_CUDA(ctx, cudaMemcpyAsync(best + (size_t)s0 * K, d_best, (size_t)ns * K * sizeof(mb200_best), cudaMemcpyDeviceToHost, ctx->stream));
+            tm.end(t6);
+            continue;
+        }
 
         int t2 = tm.begin(T_COUNT);
         const int32_t Pp = P.K2pad / 2;
@@ -1488,7 +1613,7 @@ static int32_t scan_impl(mb200_ctx* ctx, const mb200_seqs* seqs, const uint16_t*
 extern "C" int32_t mb200_scan(mb200_ctx* ctx, const mb200_seqs* seqs, const uint16_t* pwms_f16, const int64_t* lens, int32_t K,
                               int32_t maxlen, const uint16_t* thresh_f16, uint32_t flags, mb200_hit* hits, int64_t hits_cap,
                               int64_t* n_hits, int64_t* counts) {
-    return scan_impl(ctx, seqs, pwms_f16, lens, K, maxlen, thresh_f16, flags, hits, hits_cap, n_hits, counts, nullptr);
+    return scan_impl(ctx, seqs, pwms_f16, lens, K, maxlen, thresh_f16, flags, hits, hits_cap, n_hits, counts, nullptr, nullptr);
 }
 
 // Diagnostic (host arithmetic only, ctx-free): the tensor-core pre-filter's error bound and threshold for one (motif, strand) slot.
@@ -1534,5 +1659,13 @@ extern "C" int32_t mb200_scan_hist(mb200_ctx* ctx, const mb200_seqs* seqs, const
     if (!ctx) return MB200_E_INVALID;
     if (!hist) MB_FAIL(ctx, MB200_E_INVALID, "scan_hist: null histogram");
     const uint32_t f = (flags & (MB200_SCAN_FWD | MB200_SCAN_RC | MB200_SCAN_REDUCE));
-    return scan_impl(ctx, seqs, pwms_f16, lens, K, maxlen, nullptr, f, nullptr, 0, nullptr, nullptr, hist);
+    return scan_impl(ctx, seqs, pwms_f16, lens, K, maxlen, nullptr, f, nullptr, 0, nullptr, nullptr, hist, nullptr);
+}
+
+extern "C" int32_t mb200_scan_best(mb200_ctx* ctx, const mb200_seqs* seqs, const uint16_t* pwms_f16, const int64_t* lens, int32_t K,
+                                   int32_t maxlen, uint32_t flags, mb200_best* best) {
+    if (!ctx) return MB200_E_INVALID;
+    if (!best) MB_FAIL(ctx, MB200_E_INVALID, "scan_best: null output");
+    if (flags & ~(MB200_SCAN_FWD | MB200_SCAN_RC)) MB_FAIL(ctx, MB200_E_INVALID, "scan_best: flags 0x%x: only MB200_SCAN_FWD | MB200_SCAN_RC", flags);
+    return scan_impl(ctx, seqs, pwms_f16, lens, K, maxlen, nullptr, flags, nullptr, 0, nullptr, nullptr, nullptr, best);
 }

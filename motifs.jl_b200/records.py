@@ -190,3 +190,138 @@ def scan_fasta(ctx, path_or_records, motifs_or_pwms, thresh=None, *, want_hits=T
     res.pvalues = np.array([1.0 if (a == 0 and b == 0) else inference.fisher_right(a, res.S - a, b, bg.S - b)
                             for a, b in zip(a_.tolist(), b_.tolist())], np.float64)
     return res
+
+
+# ---- best site per (record, motif), and the statistics built on it ------------------------------------------------------
+@dataclass
+class BestSites:
+    """The best site of every (record, motif): the highest score over every window of the record's N-free fragments on both
+    strands, ties to the lowest record position, then to the forward strand (comp = 0).  score: Float16, exactly mb200_scan's
+    score of that window; pos: 0-based start in record coordinates, -1 when found is False (no fragment holds a window of the
+    motif, or every window is NaN; score and comp are 0 then)."""
+    names: List[str]
+    lengths: np.ndarray          # (R,) int64 record lengths
+    score: np.ndarray            # (R, K) float16
+    pos: np.ndarray              # (R, K) int64
+    comp: np.ndarray             # (R, K) uint8
+    found: np.ndarray            # (R, K) bool
+
+
+def _h16_ord(bits):
+    """Float16 bit patterns -> integers in the order of their values (-0 ties +0)."""
+    b = np.asarray(bits, np.uint16).astype(np.int64)
+    b = np.where(b == 0x8000, 0, b)
+    return np.where(b & 0x8000, ~b & 0xFFFF, b | 0x8000)
+
+
+def reduce_fragment_best(frag_record, frag_start, fbest, n_records):
+    """Fragment best sites (F, K) _lib.BEST_DTYPE -> record best sites: (score (R,K) float16, pos (R,K) int64, comp, found).
+    Same rule as the kernel's, in record coordinates: highest score, then lowest record position, then forward."""
+    F, K = fbest.shape
+    R = int(n_records)
+    found = fbest["found"].astype(bool)
+    rec = np.broadcast_to(np.asarray(frag_record, np.int64)[:, None], (F, K))[found]
+    mot = np.broadcast_to(np.arange(K, dtype=np.int64)[None, :], (F, K))[found]
+    pos = (np.asarray(frag_start, np.int64)[:, None] + fbest["pos"].astype(np.int64))[found]
+    key = (_h16_ord(fbest["score_f16"][found]).astype(np.uint64) << np.uint64(48)) | \
+          (((np.uint64(1 << 47) - np.uint64(1) - pos.astype(np.uint64)) << np.uint64(1))) | \
+          (np.uint64(1) - fbest["comp"][found].astype(np.uint64))
+    best = np.zeros(R * K, np.uint64)
+    np.maximum.at(best, rec * K + mot, key)
+    best = best.reshape(R, K)
+    f = best != 0
+    o = (best >> np.uint64(48)).astype(np.int64)
+    bits = np.where(o & 0x8000, o & 0x7FFF, ~o & 0xFFFF).astype(np.uint16)
+    score = np.where(f, bits, 0).astype(np.uint16).view(np.float16)
+    p = np.where(f, np.int64((1 << 47) - 1) - ((best >> np.uint64(1)) & np.uint64((1 << 47) - 1)).astype(np.int64), -1)
+    comp = np.where(f, 1 - (best & np.uint64(1)).astype(np.int64), 0).astype(np.uint8)
+    return score, p, comp, f
+
+
+def best_sites(ctx, path_or_records, motifs_or_pwms, *, max_padding: float = 1.0 / 8) -> BestSites:
+    """Best site of every (record, motif) of a FASTA file (a path or a Records): the fragments are scanned in the buckets of
+    scan_fasta (mb200_scan_best on both strands) and reduced to records on the host.  motifs_or_pwms: an inference.Motifs or a
+    list of (4, len) PWMs (thresholds play no part)."""
+    rec = path_or_records if isinstance(path_or_records, Records) else read_records(path_or_records)
+    pw, lens, _ = _pwm_args(motifs_or_pwms, None)
+    K = len(lens)
+    fbest = np.zeros((len(rec.frag_len), K), _lib.BEST_DTYPE)
+    off = rec.frag_offsets
+    for b in bucket_fragments(rec.frag_len, int(lens.min()), max_padding):
+        ls = rec.frag_len[b]
+        seqs = ctx.seqs_from_ragged(np.concatenate([rec.bases[off[f]: off[f + 1]] for f in b]), np.concatenate([[0], np.cumsum(ls)]))
+        try:
+            fbest[b] = ctx.scan_best(seqs, pw, lens)
+        finally:
+            seqs.free()
+    score, pos, comp, found = reduce_fragment_best(rec.frag_record, rec.frag_start, fbest, len(rec.names))
+    return BestSites(list(rec.names), rec.lengths.copy(), score, pos, comp, found)
+
+
+def best_site_auc(fg: BestSites, bg: BestSites) -> np.ndarray:
+    """(K,) float64: the probability that a foreground record's best score beats a background record's, ties counted 1/2
+    (Mann-Whitney U / (n1 n2)), from average ranks.  Records without a site rank below every found score and tie with each
+    other.  NaN for a motif when either side has no records."""
+    n1, n2 = fg.found.shape[0], bg.found.shape[0]
+    K = fg.found.shape[1]
+    out = np.full(K, np.nan)
+    if n1 == 0 or n2 == 0:
+        return out
+    for k in range(K):
+        key = np.concatenate([np.where(fg.found[:, k], _h16_ord(fg.score[:, k].view(np.uint16)), 0),
+                              np.where(bg.found[:, k], _h16_ord(bg.score[:, k].view(np.uint16)), 0)])
+        u, inv, cnt = np.unique(key, return_inverse=True, return_counts=True)
+        first = np.concatenate([[0], np.cumsum(cnt)[:-1]])
+        avg = first + (cnt + 1) / 2.0                       # 1-based average rank of each distinct key
+        r1 = avg[inv[:n1]].sum()
+        out[k] = (r1 - n1 * (n1 + 1) / 2.0) / (n1 * n2)
+    return out
+
+
+@dataclass
+class CentralEnrichment:
+    """Per motif, the central window with the smallest binomial p-value (CentriMo): it holds `window` start positions and `k` of
+    the `n` found best sites, `expected` = n * window / (L - m + 1); p = P[Binom(n, window / (L - m + 1)) >= k], p_adj = min(1,
+    p * number of windows tried).  window = 0, p = p_adj = 1 when there is no window (L - m <= 1) or no site."""
+    window: np.ndarray           # (K,) int64
+    k: np.ndarray                # (K,) int64
+    n: np.ndarray                # (K,) int64
+    expected: np.ndarray         # (K,) float64
+    p: np.ndarray                # (K,) float64
+    p_adj: np.ndarray            # (K,) float64
+
+
+def central_enrichment(best: BestSites, lens) -> CentralEnrichment:
+    """CentriMo's central enrichment test on summit-centred peaks of one length L.  A start p of a motif of length m lies at
+    doubled offset d = 2p + m - L from the centre; for every r in {|d|} below L - m the window {p : |d| <= r} holds r + 1 starts
+    and is tested against the uniform null over all L - m + 1 starts (N runs included).  lens: the K motif lengths."""
+    L_all = np.unique(np.asarray(best.lengths, np.int64))
+    if len(L_all) > 1:
+        raise ValueError(f"central_enrichment needs records of one length (summit-centred peaks); found lengths {L_all.tolist()}")
+    lens = np.asarray(lens, np.int64)
+    K = len(lens)
+    res = CentralEnrichment(np.zeros(K, np.int64), np.zeros(K, np.int64), np.zeros(K, np.int64), np.zeros(K), np.ones(K), np.ones(K))
+    if len(L_all) == 0:
+        return res
+    L = int(L_all[0])
+    for k in range(K):
+        m = int(lens[k])
+        f = best.found[:, k]
+        N = int(f.sum())
+        res.n[k] = N
+        if L - m <= 1 or N == 0:
+            continue
+        npos = L - m + 1
+        d = np.abs(2 * best.pos[f, k] + m - L)
+        radii = np.arange((L - m) % 2, L - m, 2)        # every |d| below L - m (all of one parity)
+        cum = np.cumsum(np.bincount(d, minlength=L - m + 1))
+        best_p, best_i = 2.0, 0
+        for i, r in enumerate(radii.tolist()):
+            p = inference.binom_right(int(cum[r]), N, (r + 1) / npos)
+            if p < best_p:
+                best_p, best_i = p, i
+        r = int(radii[best_i])
+        res.window[k], res.k[k] = r + 1, int(cum[r])
+        res.expected[k] = N * (r + 1) / npos
+        res.p[k], res.p_adj[k] = best_p, min(1.0, best_p * len(radii))
+    return res

@@ -573,15 +573,20 @@ class CscModel:
         if n_seqs is None:
             n_seqs = (seqs.N - first_seq) - (seqs.N - first_seq) % B          # DataLoader(partial=false)
         cap = max(1024, 64 * int(n_seqs))
-        out = np.zeros(cap, CODE_DTYPE)
         n = C.c_int64()
-        if shard is None:
-            self.ctx._check(self.ctx._lib.mb200_csc_codes(self.ctx._h, self._h, seqs._h, int(first_seq), int(n_seqs), _ptr(out), cap, C.byref(n)))
-        else:
-            r, w = (-1, -1) if shard == "comm" else shard
-            self.ctx._check(self.ctx._lib.mb200_csc_codes_sharded(self.ctx._h, self._h, seqs._h, int(first_seq), int(n_seqs), int(r), int(w),
-                                                                   _ptr(out), cap, C.byref(n)))
-        return out[: n.value]
+        while True:
+            out = np.zeros(cap, CODE_DTYPE)
+            if shard is None:
+                rc = self.ctx._lib.mb200_csc_codes(self.ctx._h, self._h, seqs._h, int(first_seq), int(n_seqs), _ptr(out), cap, C.byref(n))
+            else:
+                r, w = (-1, -1) if shard == "comm" else shard
+                rc = self.ctx._lib.mb200_csc_codes_sharded(self.ctx._h, self._h, seqs._h, int(first_seq), int(n_seqs), int(r), int(w),
+                                                           _ptr(out), cap, C.byref(n))
+            if rc == E_HITS_OVERFLOW and n.value > cap:      # more codes than the guess (large q, ties): decode again into the reported size
+                cap = int(n.value)
+                continue
+            self.ctx._check(rc)
+            return out[: n.value]
 
 
 def pvalue2score(ctx: "Context", pwm, pval, eps, bg):

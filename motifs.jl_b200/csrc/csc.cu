@@ -79,6 +79,7 @@ struct mb200_csc {
     bool batched = false; float* Ft_scratch = nullptr; float* Ft_scratch2 = nullptr; float* Ft_eff = nullptr;      // one-CTA-per-sequence kernels (csc_batched.cuh) for many-group shapes      // tap-grouped kernel (k_corr2d_tc3)
     cudaGraph_t graph = nullptr; cudaGraphExec_t gexec = nullptr; bool graph_ok = false;
     const uint32_t* graph_words = nullptr; int64_t graph_rowwords = 0;
+    const uint32_t* last_words = nullptr; int64_t last_rowwords = 0; const int64_t* last_idx = nullptr;      // batch of the last training step (fused_fallback)
     // fused persistent forward kernel (csc_fused.cuh): plan = arena offsets of the tape's buffers, sync area, eligibility
     FzPlan fz{}; bool fused = false, no_fused = false; size_t fz_smem = 0; int fz_nmed = 0;
     uint8_t* fz_sync = nullptr; size_t fz_sync_bytes = 0, fz_zero_bytes = 0; FzBufs fzb{};
@@ -577,8 +578,10 @@ static int csc_alloc(mb200_ctx* ctx, mb200_csc* s) {
         s->fused = false;
         s->fz_smem = fz::fz_smem_bytes(d.Lb);
         s->fz_nmed = d.npx + 2;
+        // a training step with q > LIST_CAP always has code lists the fused reverse pass cannot hold: such handles keep the tape
         const bool shape_ok = d.M == FZ_M && d.K == FZ_K && d.h == FZ_H && d.fl == FZ_FL && d.npx <= FZ_MAXPX && d.npd <= FZ_MAXPD &&
-                              d.B * LIST_CAP <= FZ_THREADS && d.B * FZ_CL >= FZ_K && d.c >= FZ_CL && d.l >= 1 && fz::fz_rows(d.c) <= 32 && d.G <= FZ_BAR_DF;
+                              d.B * LIST_CAP <= FZ_THREADS && d.B * FZ_CL >= FZ_K && d.c >= FZ_CL && d.l >= 1 && fz::fz_rows(d.c) <= 32 && d.G <= FZ_BAR_DF &&
+                              (s->xyz_only || d.q <= LIST_CAP);
         if (!s->no_fused && !s->tensor && shape_ok && s->fz_smem <= ctx->smem_optin) {
             cudaError_t e = cudaFuncSetAttribute(k_csc_fused_fwd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s->fz_smem);
 #if FZ_CL > 8
@@ -812,10 +815,12 @@ static void launch_fused(mb200_csc* s, int which, cudaStream_t q) {
     ++g_lk_count;
 }
 
-static void enqueue_step(mb200_csc* s, const uint32_t* words, int64_t rowwords, const int64_t* idx_dev, bool backward, cudaStream_t q) {
+// tape = true runs the kernel-per-op tape on a handle built for the fused kernels (fused_fallback)
+static void enqueue_step(mb200_csc* s, const uint32_t* words, int64_t rowwords, const int64_t* idx_dev, bool backward, cudaStream_t q, bool tape = false) {
     const CscDims d = s->d;
-    const bool fused_all = backward && s->fused && s->fused_bwd && s->fused_bwd_df;
-    if (s->fused) {
+    const bool fused = s->fused && !tape, fused_bwd = fused && s->fused_bwd, fused_bwd_df = fused_bwd && s->fused_bwd_df;
+    const bool fused_all = backward && fused_bwd_df;
+    if (fused) {
         // prep_params + unpacking of the batch in one kernel, then the whole forward pass as ONE persistent cooperative kernel
         lk(k_csc_fused_head, d.K + 2 + (unsigned)std::min<int64_t>(8, ((int64_t)d.NS * d.Lb + 255) / 256), 256, 0, q, (const float*)s->p_raw, s->off_D, s->off_F,
            s->data + s->Feff.off, s->data + s->Fnrm0.off, s->data + s->Deff.off, s->data + s->sc.off, s->segs, words, rowwords, idx_dev, s->bases, d);
@@ -831,18 +836,18 @@ static void enqueue_step(mb200_csc* s, const uint32_t* words, int64_t rowwords, 
             cudaMemsetAsync(s->g_raw, 0, (size_t)s->n_total * 4, q);
         }
         for (size_t i = s->tape.size(); i-- > 0;) {
-            if (s->fused_bwd_df && i >= s->op_xyz_end) {
+            if (fused_bwd_df && i >= s->op_xyz_end) {
                 // loss, ADMM_DF passes and the final mask in reverse as ONE persistent kernel: leaves d z, d y, d x (kept support) of the
                 // final codes for the XYZ kernel below and its share of dD, dF, d scalars in the second half of gsum
                 if (i + 1 == s->tape.size()) launch_fused(s, 1, q);
                 continue;
             }
-            if (s->fused_bwd && i >= s->op_xyz_begin && i < s->op_xyz_end) {
+            if (fused_bwd && i >= s->op_xyz_begin && i < s->op_xyz_end) {
                 if (i + 1 == s->op_xyz_end) {
                     // the reverse pass of all ADMM_XYZ passes and of the warm-up as ONE persistent kernel: reads the adjoints left for the final
                     // z, y, x and adds its share of dD, dF, d scalars to gsum
                     launch_fused(s, 2, q);
-                    if (!s->fused_bwd_df) {              // A/B mode with the DF reverse pass on the tape: add the group sums to the tape's adjoints
+                    if (!fused_bwd_df) {            // A/B mode with the DF reverse pass on the tape: add the group sums to the tape's adjoints
                         const int nF = d.h * d.M2 * d.K, nD = d.f_len * d.M, nsc = 3 * d.npx + d.npx + 3 * d.npd + 3;
                         lk(k_csc_fused_finish, nblk(nF + nD + 64, 256), 256, 0, q, (const float*)s->fzw.gsum, d.G, nF, nD, nsc,
                            s->grad + s->Feff.off, s->grad + s->Deff.off, s->grad + s->sc.off);
@@ -851,7 +856,7 @@ static void enqueue_step(mb200_csc* s, const uint32_t* words, int64_t rowwords, 
                 }
                 continue;
             }
-            if (s->fused_bwd && i >= 1 && i < s->op_xyz_begin) continue;       // the reverse pass of the warm-up is the tail of k_csc_fused_bwd_xyz
+            if (fused_bwd && i >= 1 && i < s->op_xyz_begin) continue;      // the reverse pass of the warm-up is the tail of k_csc_fused_bwd_xyz
             if (fused_all && i == 0) {
                 // group sums of both reverse kernels -> adjoint of prep_params -> raw gradient vector; also clears the sync area
                 ScalarSegs tr = s->segs; tr.nseg = 7;      // the warm-up scalars (segment 7) are not trained
@@ -869,6 +874,7 @@ static void enqueue_step(mb200_csc* s, const uint32_t* words, int64_t rowwords, 
 // launches one step on `words` (resident sequence store, or the handle's own buffer holding a host-supplied batch)
 static int launch_step(mb200_ctx* ctx, mb200_csc* s, const uint32_t* words, int64_t rowwords, const int64_t* idx_dev, bool backward) {
     if (backward) {                        // the training step is replayed thousands of times: capture it once per source
+        s->last_words = words; s->last_rowwords = rowwords; s->last_idx = idx_dev;
         if (!s->graph_ok || s->graph_words != words || s->graph_rowwords != rowwords) {
             if (s->gexec) { cudaGraphExecDestroy(s->gexec); s->gexec = nullptr; }
             if (s->graph) { cudaGraphDestroy(s->graph); s->graph = nullptr; }
@@ -929,17 +935,24 @@ static int run_step_host(mb200_ctx* ctx, mb200_csc* s, const uint8_t* ascii, int
 }
 
 
-// the fused reverse pass handles top-q supports of up to FZ_KCAP entries per sequence (q = 32 plus exact ties) and code lists of up to
-// LIST_CAP entries; a degenerate step (e.g. an all-zero code tensor, where every entry ties at the threshold) is reported, not approximated
-static int fused_check(mb200_ctx* ctx, mb200_csc* s) {
-    if (!s->fused_bwd || !s->fz_err_host || *s->fz_err_host == 0) return MB200_OK;
-    const unsigned int e = *s->fz_err_host;
+// The fused reverse pass handles top-q supports of up to FZ_KCAP entries per sequence (q = 32 plus exact ties) and code lists of up to
+// LIST_CAP entries.  A step beyond that (ties at the q-th value: an all-zero top-q input, or equal values at many positions of a
+// repetitive sequence) raises the error word.  That step is then run again on the same batch, which is still in
+// idx_dev or batch_words, through the kernel-per-op tape: its consumers take their dense paths for such lists, so the step returns the
+// gradient the reference computes instead of an error.  k_adabelief and k_l1_F read the same word and skip a flagged gradient.
+static bool fused_flagged(const mb200_csc* s) { return s->fused_bwd && s->fz_err_host && *s->fz_err_host != 0; }
+
+static int fused_fallback(mb200_ctx* ctx, mb200_csc* s) {
     *s->fz_err_host = 0;
-    cudaMemsetAsync(s->fzw.err, 0, 4, ctx->stream);
-    cudaMemsetAsync(s->grad, 0, (s->arena + s->grad_extra) * 4, ctx->stream);                 // the clamped lists may have left d x slots uncleared
-    cudaMemsetAsync(s->fz_sync, 0, s->fz_zero_bytes, ctx->stream);
-    MB_FAIL(ctx, MB200_E_UNSUPPORTED, "csc: the fused reverse pass met a degenerate top-q support (flag %u: more than %d kept entries or more than %d codes in a sequence); "
-            "create the handle with MB200_CSC_NO_FUSED for such inputs", e, FZ_KCAP, LIST_CAP);
+    MB_CUDA(ctx, cudaMemsetAsync(s->fzw.err, 0, 4, ctx->stream));
+    MB_CUDA(ctx, cudaMemsetAsync(s->fz_sync, 0, s->fz_zero_bytes, ctx->stream));
+    const int64_t c0 = g_lk_count;
+    enqueue_step(s, s->last_words, s->last_rowwords, s->last_idx, true, ctx->stream, true);
+    ctx->launches[T_CSC] += g_lk_count - c0;
+    // the fully fused step expects its d x slots zero when it begins (their reader clears them); the tape leaves the whole arena written
+    MB_CUDA(ctx, cudaMemsetAsync(s->grad, 0, (s->arena + s->grad_extra) * 4, ctx->stream));
+    MB_CUDA(ctx, cudaGetLastError());
+    return MB200_OK;
 }
 
 // loss (and gradient) of n_groups batches.  seq_idx: n_groups*batch_size indices into seqs.
@@ -961,7 +974,13 @@ extern "C" int32_t mb200_csc_loss_grad(mb200_ctx* ctx, mb200_csc* s, const mb200
     tm.end(td); tm.end(tt);
     MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     tm.collect();
-    return fused_check(ctx, s);
+    if (fused_flagged(s)) {
+        rc = fused_fallback(ctx, s); if (rc) return rc;
+        if (loss_out) MB_CUDA(ctx, cudaMemcpyAsync(loss_out, s->data + s->loss.off, (size_t)s->d.G * 3 * 4, cudaMemcpyDeviceToHost, ctx->stream));
+        if (grads) MB_CUDA(ctx, cudaMemcpyAsync(grads, s->g_raw, (size_t)s->n_train * 4, cudaMemcpyDeviceToHost, ctx->stream));
+        MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    }
+    return MB200_OK;
 }
 
 // forward + reverse pass only; gradients stay on the device (mb200_csc_device_ptrs) so that the host framework can
@@ -988,20 +1007,32 @@ extern "C" int32_t mb200_csc_adabelief_step(mb200_ctx* ctx, mb200_csc* s, float 
                                             float* loss_out, float* l1_F_out) {
     if (!ctx || !s) return MB200_E_INVALID;
     MB_CUDA(ctx, cudaSetDevice(ctx->device));
+    const unsigned int* err = s->fused_bwd ? s->fzw.err : nullptr;
+    // with a communicator the flag is read before the gradient leaves the rank: a flagged step is re-run on the tape first, so every rank
+    // still makes exactly one all-reduce per step
+    if (err && ctx->comm && ctx->world > 1) {
+        MB_CUDA(ctx, cudaMemcpyAsync(s->fz_err_host, err, 4, cudaMemcpyDeviceToHost, ctx->stream));
+        MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+        if (fused_flagged(s)) { const int rc = fused_fallback(ctx, s); if (rc) return rc; }
+    }
     // data parallel (SURVEY §8e): ONE all-reduce (average) of the n_train gradients per step, on the stream the reverse pass ran on
     { const int rc = mb_comm_allreduce_f32(ctx, s->g_raw, (size_t)s->n_train, true); if (rc) return rc; }
-    s->step_count += 1;
-    const float c1 = 1.f - powf(beta1, (float)s->step_count), c2 = 1.f - powf(beta2, (float)s->step_count);
-    lk(k_adabelief, nblk(s->n_train, 256), 256, 0, ctx->stream, s->p_raw, s->g_raw, s->mt, s->st, eta, beta1, beta2, eps * eps, c1, c2, (int)s->n_train);
-    // l1(F): one term per syntax filter, summed on the host in a fixed order — bit-identical on every rank, so that all ranks of a
-    // data-parallel run take the early-stop branch (train.jl:47-52) on the same step
+    const float c1 = 1.f - powf(beta1, (float)(s->step_count + 1)), c2 = 1.f - powf(beta2, (float)(s->step_count + 1));
     float* d_l1 = s->data + s->loss.off + (size_t)s->d.G * 3;       // K slots right after the per-group losses
-    lk(k_l1_F, s->d.K, 256, 0, ctx->stream, s->p_raw + s->off_F, d_l1, s->d);
-    ctx->launches[T_CSC] += 2;
-    MB_CUDA(ctx, cudaMemcpyAsync(s->host_out, s->data + s->loss.off, ((size_t)s->d.G * 3 + s->d.K) * 4, cudaMemcpyDeviceToHost, ctx->stream));
-    if (s->fused_bwd) MB_CUDA(ctx, cudaMemcpyAsync(s->fz_err_host, s->fzw.err, 4, cudaMemcpyDeviceToHost, ctx->stream));
-    MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    { const int rc = fused_check(ctx, s); if (rc) return rc; }
+    for (int attempt = 0; attempt < 2; ++attempt) {
+        lk(k_adabelief, nblk(s->n_train, 256), 256, 0, ctx->stream, s->p_raw, (const float*)s->g_raw, s->mt, s->st, eta, beta1, beta2, eps * eps, c1, c2, (int)s->n_train, err);
+        // l1(F): one term per syntax filter, summed on the host in a fixed order — bit-identical on every rank, so that all ranks of a
+        // data-parallel run take the early-stop branch (train.jl:47-52) on the same step
+        lk(k_l1_F, s->d.K, 256, 0, ctx->stream, (const float*)(s->p_raw + s->off_F), d_l1, s->d, err);
+        ctx->launches[T_CSC] += 2;
+        MB_CUDA(ctx, cudaMemcpyAsync(s->host_out, s->data + s->loss.off, ((size_t)s->d.G * 3 + s->d.K) * 4, cudaMemcpyDeviceToHost, ctx->stream));
+        if (err) MB_CUDA(ctx, cudaMemcpyAsync(s->fz_err_host, err, 4, cudaMemcpyDeviceToHost, ctx->stream));
+        MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+        if (!fused_flagged(s)) break;
+        // one GPU, flagged step: nothing was updated; take the tape's gradient and update once more
+        const int rc = fused_fallback(ctx, s); if (rc) return rc;
+    }
+    s->step_count += 1;
     if (loss_out) { float m = 0.f; for (int g = 0; g < s->d.G; ++g) m += s->host_out[g * 3]; *loss_out = m / (float)s->d.G; }
     if (l1_F_out) { float l1 = 0.f; for (int k = 0; k < s->d.K; ++k) l1 += s->host_out[(size_t)s->d.G * 3 + k]; *l1_F_out = l1; }
     return MB200_OK;
@@ -1051,8 +1082,8 @@ extern "C" int32_t mb200_csc_median_mask(mb200_ctx* ctx, mb200_csc* s, const flo
 // code retrieval (inference/_1_code_retrieval.jl:33-56): forward-only ADMM_XYZ over consecutive groups of batch_size
 // sequences; non-zeros of X as (position, fil, seq, Float16 mag), ordered by seq, fil, position.
 // ---------------------------------------------------------------------------------------------
-#define CODE_SLOTS 96
-__global__ void __launch_bounds__(128) k_emit_codes(const float* __restrict__ x, int64_t seq0, mb200_code* __restrict__ slots, int32_t* __restrict__ counts, CscDims d) {
+#define CODE_SLOTS 96          // records per sequence of the first emission; a batch with a longer sequence is emitted again with a wider stride
+__global__ void __launch_bounds__(128) k_emit_codes(const float* __restrict__ x, int64_t seq0, mb200_code* __restrict__ slots, int32_t* __restrict__ counts, int stride, CscDims d) {
     PDL_SYNC();
     // one warp per sequence walks (fil, position) in order and compacts entries > 0 with ballots
     const int64_t n = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -1068,10 +1099,10 @@ __global__ void __launch_bounds__(128) k_emit_codes(const float* __restrict__ x,
         const unsigned m = __ballot_sync(FULLMASK, hit);
         if (hit) {
             const int o = cnt + __popc(m & ((1u << lane) - 1u));
-            if (o < CODE_SLOTS) {
+            if (o < stride) {
                 mb200_code c; c.position = (uint16_t)i; c.fil = (uint16_t)k; c.seq = (uint32_t)(seq0 + n);
                 c.mag_f16 = __half_as_ushort(__float2half_rn(v)); c._pad = 0;
-                slots[n * CODE_SLOTS + o] = c;
+                slots[n * stride + o] = c;
             }
         }
         cnt += __popc(m);
@@ -1092,11 +1123,24 @@ static int32_t codes_impl(mb200_ctx* ctx, mb200_csc* s, const mb200_seqs* seqs, 
     mb_reset_timing(ctx);
     MbTimers tm(ctx);
     const int tt = tm.begin(T_TOTAL);
-    int rc = mb_ensure_buf(ctx, 5, (size_t)d.NS * CODE_SLOTS * sizeof(mb200_code) + (size_t)d.NS * 4 + 256); if (rc) return rc;
-    mb200_code* d_slots = (mb200_code*)ctx->bufs[5];
-    int32_t* d_cnt = (int32_t*)((uint8_t*)ctx->bufs[5] + (size_t)d.NS * CODE_SLOTS * sizeof(mb200_code));
-    std::vector<mb200_code> h_slots((size_t)d.NS * CODE_SLOTS);
+    std::vector<mb200_code> h_slots;
     std::vector<int32_t> h_cnt(d.NS);
+    // k_emit_codes on the x of the last forward pass: `stride` records per sequence, then counts and records to the host
+    auto emit = [&](int64_t seq0, int stride) -> int {
+        const int rc = mb_ensure_buf(ctx, 5, (size_t)d.NS * stride * sizeof(mb200_code) + (size_t)d.NS * 4 + 256); if (rc) return rc;
+        mb200_code* d_slots = (mb200_code*)ctx->bufs[5];
+        int32_t* d_cnt = (int32_t*)(d_slots + (size_t)d.NS * stride);
+        lk(k_emit_codes, nblk((int64_t)d.NS * 32, 128), 128, 0, ctx->stream, s->data + s->named["x"].off, seq0, d_slots, d_cnt, stride, d);
+        ctx->launches[T_CSC] += 1;
+        MB_CUDA(ctx, cudaGetLastError());
+        const int td = tm.begin(T_D2H);
+        h_slots.resize((size_t)d.NS * stride);
+        MB_CUDA(ctx, cudaMemcpyAsync(h_cnt.data(), d_cnt, (size_t)d.NS * 4, cudaMemcpyDeviceToHost, ctx->stream));
+        MB_CUDA(ctx, cudaMemcpyAsync(h_slots.data(), d_slots, (size_t)d.NS * stride * sizeof(mb200_code), cudaMemcpyDeviceToHost, ctx->stream));
+        tm.end(td);
+        MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+        return MB200_OK;
+    };
     int64_t total = 0; bool overflow = false;
     for (int64_t s0 = 0; s0 < n_seqs; s0 += d.NS) {
         const int64_t ns = std::min<int64_t>(d.NS, n_seqs - s0);
@@ -1107,20 +1151,16 @@ static int32_t codes_impl(mb200_ctx* ctx, mb200_csc* s, const mb200_seqs* seqs, 
         const int64_t c0 = g_lk_count;
         lk(k_unpack_bases, nblk((int64_t)d.NS * d.Lb, 256), 256, 0, ctx->stream, seqs->words, seqs->rowwords, s->idx_dev, s->bases, d);
         for (auto& op : s->tape) { if (op.kind) break; op.fwd(ctx->stream); if (std::string(op.name) == "df_mask") break; }
-        lk(k_emit_codes, nblk((int64_t)d.NS * 32, 128), 128, 0, ctx->stream, s->data + s->named["x"].off, first_seq + s0, d_slots, d_cnt, d);
         ctx->launches[T_CSC] += g_lk_count - c0;
         tm.end(tc);
-        MB_CUDA(ctx, cudaGetLastError());
-        const int td = tm.begin(T_D2H);
-        MB_CUDA(ctx, cudaMemcpyAsync(h_cnt.data(), d_cnt, (size_t)d.NS * 4, cudaMemcpyDeviceToHost, ctx->stream));
-        MB_CUDA(ctx, cudaMemcpyAsync(h_slots.data(), d_slots, (size_t)d.NS * CODE_SLOTS * sizeof(mb200_code), cudaMemcpyDeviceToHost, ctx->stream));
-        tm.end(td);
-        MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+        int stride = CODE_SLOTS;
+        int rc = emit(first_seq + s0, stride); if (rc) return rc;
+        const int mx = *std::max_element(h_cnt.begin(), h_cnt.end());      // the tail's repeated sequences count too: they share the stride
+        if (mx > stride) { stride = mx; rc = emit(first_seq + s0, stride); if (rc) return rc; }      // x is still in the arena
         for (int64_t i = 0; i < ns; ++i) {
-            if (h_cnt[i] > CODE_SLOTS) MB_FAIL(ctx, MB200_E_UNSUPPORTED, "csc_codes: sequence %lld has %d non-zero codes (> %d slots)", (long long)(first_seq + s0 + i), h_cnt[i], CODE_SLOTS);
             for (int j = 0; j < h_cnt[i]; ++j) {
-                if (vec) vec->push_back(h_slots[(size_t)i * CODE_SLOTS + j]);
-                else if (total < cap && out) out[total] = h_slots[(size_t)i * CODE_SLOTS + j]; else overflow = overflow || (total >= cap);
+                if (vec) vec->push_back(h_slots[(size_t)i * stride + j]);
+                else if (total < cap && out) out[total] = h_slots[(size_t)i * stride + j]; else overflow = overflow || (total >= cap);
                 ++total;
             }
         }

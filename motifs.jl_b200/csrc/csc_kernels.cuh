@@ -749,10 +749,11 @@ __global__ void __launch_bounds__(256) k_sum_slots(const float* __restrict__ src
     if (threadIdx.x == 0) dsc[blockIdx.x] += tot;
 }
 
+// err: the fused reverse pass's error word (null for handles without it); a step it flagged is not applied (csc.cu: fused_fallback)
 __global__ void __launch_bounds__(256) k_adabelief(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ mt, float* __restrict__ st,
-                                                   float eta, float b1, float b2, float eps2, float c1, float c2, int n) { PDL_SYNC();
+                                                   float eta, float b1, float b2, float eps2, float c1, float c2, int n, const unsigned int* __restrict__ err) { PDL_SYNC();
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= n) return;
+    if (t >= n || (err && *err)) return;
     const float gr = g[t];
     const float m = b1 * mt[t] + (1.f - b1) * gr;
     const float dv = gr - m;
@@ -762,7 +763,8 @@ __global__ void __launch_bounds__(256) k_adabelief(float* __restrict__ p, const 
 }
 // l1 = sum |prep_syntax_filters(F)| (train.jl:47): per k sum(r^2)/sqrt(sum r^4).  One block per k writes its term to out[k]; the host
 // adds the K terms in index order (no atomics: the statistic is bit-identical across data-parallel ranks).
-__global__ void __launch_bounds__(256) k_l1_F(const float* __restrict__ raw, float* __restrict__ out, CscDims d) { PDL_SYNC();
+__global__ void __launch_bounds__(256) k_l1_F(const float* __restrict__ raw, float* __restrict__ out, CscDims d, const unsigned int* __restrict__ err) { PDL_SYNC();
+    if (err && *err) return;                      // block-uniform: no update was applied (k_adabelief)
     const int k = blockIdx.x;
     const int HJ = d.h * d.M2;
     float s2 = 0.f, s4 = 0.f;

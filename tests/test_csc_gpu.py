@@ -339,17 +339,32 @@ def test_per_step_parity_on_training_steps_1_2_3_1000(ctx):
     m.free(); seqs.free()
 
 
-@pytest.mark.parametrize("Lb,groups", [(100, 1), (200, 1), (64, 2), (100, 2)])
-def test_fused_forward_kernel_matches_the_tape(ctx, Lb, groups):
+@pytest.mark.parametrize("Lb,groups,batch,fused", [
+    pytest.param(100, 1, 6, True, id="100-1"),
+    pytest.param(200, 1, 6, True, id="200-1"),
+    pytest.param(64, 2, 6, False, id="64-2"),            # 12 clusters of 16 CTAs are not co-resident: the default handle takes the tape
+    pytest.param(100, 2, 6, False, id="100-2"),
+    pytest.param(100, 2, 3, True, id="100-2-batch3"),    # 6 clusters, as many as the default step: per-group barriers, histograms, sums
+    pytest.param(64, 3, 2, True, id="64-3-batch2"),
+])
+def test_fused_forward_kernel_matches_the_tape(ctx, Lb, groups, batch, fused):
     """csc_fused.cuh (one persistent cluster kernel for the forward pass) against the kernel-per-op tape (MB200_CSC_NO_FUSED): same
-    discrete results (top-q supports, i.e. the same median masks), values and gradients equal within fp32 summation order."""
-    hp, ohp, a, seqs, flat = _setup(ctx, 40, Lb, 21)
+    discrete results (top-q supports, i.e. the same median masks), values and gradients equal within fp32 summation order.  Which path
+    the default handle took is read from the step's kernel count: the fully fused step is a handful of kernels, the tape hundreds."""
+    hp = mdl.Hyperparam(batch_size=batch)
+    hp, ohp, a, seqs, flat = _setup(ctx, 40, Lb, 21, hp=hp)
     mf = mb._lib.CscModel(ctx, hp, Lb, n_groups=groups)
     mt = mb._lib.CscModel(ctx, hp, Lb, n_groups=groups, fused=False)
     mf.set_params(flat); mt.set_params(flat)
-    idx = np.random.default_rng(5).permutation(40)[:6 * groups]
+    idx = np.random.default_rng(5).permutation(40)[:batch * groups]
     lf, gf = mf.loss_grad(seqs, idx)
+    n_f = ctx.last_timing()[1]["csc"]
     lt, gt = mt.loss_grad(seqs, idx)
+    n_t = ctx.last_timing()[1]["csc"]
+    if fused:
+        assert 0 < n_f <= 8 and n_t > 5 * n_f, (n_f, n_t)
+    else:
+        assert n_f == n_t, (n_f, n_t)
     assert np.allclose(lf, lt, rtol=2e-6)
     B, c, l = hp.batch_size * groups, Lb - 7, Lb - 7 - 11
     for name, n in (("x", B * l * hp.K), ("z", B * c * hp.M), ("y", B * c * hp.M), ("zy", B * c * hp.twoM), ("D", groups * 32 * hp.M), ("F", groups * hp.h * hp.twoM * hp.K)):

@@ -137,6 +137,11 @@ int32_t mb200_fasta_split(int64_t n, double train_test_split_ratio, int32_t shuf
                           int64_t* train_idx, int64_t* test_idx, int64_t* n_train, int64_t* n_test);
 /* rows idx[0..n) of src as a new store (device gather) */
 int32_t mb200_seqs_gather(mb200_ctx* ctx, const mb200_seqs* src, const int64_t* idx, int64_t n, mb200_seqs** out);
+/* windows of a store as a new fixed-length store of n rows of len bases (device gather): row i holds bases
+ * [start[i], start[i] + len) of row row[i] of src (fixed or ragged; a ragged row's own length is the limit).  A window that leaves
+ * its row, an index out of range or len < 1: MB200_E_INVALID.                                                              */
+int32_t mb200_seqs_windows(mb200_ctx* ctx, const mb200_seqs* src, const int64_t* row, const int64_t* start, int64_t n, int64_t len,
+                           mb200_seqs** out);
 /* every sequence shuffled with its k-mer counts preserved exactly (k = 1: uniform permutation; k = 2..4: uniform random Eulerian
  * walk through the (k-1)-mer graph, sequences up to 65 536 bp; k = 1 also for chromosome-scale sequences).  Sequence i draws from
  * random stream first_stream + i of `seed`: shards shuffled on different GPUs equal the single-GPU result.          */
@@ -222,6 +227,30 @@ typedef struct {
  * no strand: MB200_E_INVALID).  Rows are per rank: there is nothing to reduce over a communicator.                          */
 int32_t mb200_scan_best(mb200_ctx* ctx, const mb200_seqs* seqs, const uint16_t* pwms_f16, const int64_t* lens,
                         int32_t K, int32_t maxlen, uint32_t flags, mb200_best* best);
+
+/* Secondary-motif spacings around primary sites (SpaMo).  An anchor is a primary motif's site of length len at [start, start + len)
+ * of row `row`, on strand comp; its margins are the W = margin bases on either side, [start - W, start) and [start + len,
+ * start + len + W), both inside the row.  For every (anchor, secondary k) the best window of k (both strands) in the two margins
+ * together is found with the mb200_scan_best rule (ties: lower position, so the left margin, then the forward strand).  It is
+ * counted when its score is > 0 and > thresh_f16[k] (NULL: > 0), exactly when mb200_scan would report it as a hit.  A counted
+ * window at gap g from the primary (g = start - (s + m_k) on the left, s - (start + len) on the right) goes to
+ *   hist[((primary * K + k) * 4 + q) * margin + g],  q = 2 * (comp_k != comp) + downstream,
+ * where downstream means the right margin for comp = 0 and the left margin for comp = 1 (0: same strand upstream, 1: same strand
+ * downstream, 2: opposite upstream, 3: opposite downstream).  sites (n_anchors * K, may be NULL): the best window of each pair, pos
+ * in row coordinates, found = counted (pos = UINT32_MAX when the margins hold no window).  The histogram is summed on the device.
+ * MB200_E_INVALID: margin outside [1, 65536], n_primary outside [1, 65535], an anchor's primary >= n_primary, comp > 1, len < 1 or
+ * a flank leaving its row, a null hist.  MB200_E_NOMEM: the histogram does not fit on the device.                            */
+typedef struct {
+    int64_t  row;        /* row of seqs                                                              */
+    int64_t  start;      /* 0-based start of the primary site in the row                            */
+    int32_t  len;        /* primary motif length m_p                                                 */
+    uint16_t primary;    /* 0-based primary motif index (< n_primary)                                */
+    uint8_t  comp;       /* strand of the primary site: 0 = pwm, 1 = reverse(pwm)                   */
+    uint8_t  _pad;
+} mb200_anchor;          /* 24 bytes */
+int32_t mb200_scan_spacing(mb200_ctx* ctx, const mb200_seqs* seqs, const mb200_anchor* anchors, int64_t n_anchors,
+                           int32_t n_primary, int32_t margin, const uint16_t* pwms_f16, const int64_t* lens, int32_t K,
+                           int32_t maxlen, const uint16_t* thresh_f16, uint32_t* hist, mb200_best* sites);
 
 /* ---- unrolled convolutional-sparse-coding network: replaces the GPU work inside
  *      forward_pass_return_loss (model.jl:375-395) + gradient(ps) + Flux.Optimise.update!

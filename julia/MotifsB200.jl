@@ -300,6 +300,44 @@ function scan_best(ctx, seqs, N::Integer, pwms::Array{Float16,3}, lens::Vector{I
     [(pos = b.found != 0 ? Int(b.pos) + 1 : 0, comp = b.comp != 0, score = b.score, found = b.found != 0) for b in out]
 end
 
+# windows [start, start + len) of rows `row` (1-based rows and starts) as a new fixed-length store (mb200_seqs_windows)
+function seqs_windows(ctx, seqs, row::Vector{Int64}, start::Vector{Int64}, len::Integer)
+    length(row) == length(start) || error("row and start must have one length")
+    r0, s0 = row .- 1, start .- 1
+    out = Ref{Ptr{Cvoid}}(C_NULL)
+    GC.@preserve r0 s0 check(ctx, ccall((:mb200_seqs_windows, lib), Int32,
+        (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Int64}, Ptr{Int64}, Int64, Int64, Ref{Ptr{Cvoid}}), ctx, seqs, r0, s0, length(r0), len, out))
+    out[]
+end
+
+struct Anchor                      # mb200_anchor (24 bytes), 0-based inside
+    row::Int64
+    start::Int64
+    len::Int32
+    primary::UInt16
+    comp::UInt8
+    _pad::UInt8
+end
+
+# SpaMo spacing histogram (mb200_scan_spacing).  Anchors: (row, start, len, primary, comp) with 1-based row, start and primary;
+# returns hist as an Int array (margin, 4, K, n_primary) in Julia order = hist[g+1, q+1, k, p] with gap g and quadrant q (0 same
+# strand upstream, 1 same downstream, 2 opposite upstream, 3 opposite downstream), and with want_sites the (K, n) best sites of
+# every (anchor, secondary) as NamedTuples (1-based pos in the row, found = counted).
+function scan_spacing(ctx, seqs, anchors::Vector{<:NamedTuple}, n_primary::Integer, pwms::Array{Float16,3}, lens::Vector{Int64};
+                      margin::Integer=150, thresh::Union{Nothing,Vector{Float16}}=nothing, want_sites::Bool=false)
+    K, _, maxlen = size(pwms)
+    an = [Anchor(a.row - 1, a.start - 1, Int32(a.len), UInt16(a.primary - 1), UInt8(a.comp), 0x00) for a in anchors]
+    hist = zeros(UInt32, margin, 4, K, n_primary)
+    sites = want_sites ? Matrix{Best}(undef, K, length(an)) : Matrix{Best}(undef, 0, 0)
+    tp = thresh === nothing ? Ptr{Float16}(C_NULL) : pointer(thresh)
+    sp = want_sites ? pointer(sites) : Ptr{Best}(C_NULL)
+    GC.@preserve an pwms lens thresh hist sites check(ctx, ccall((:mb200_scan_spacing, lib), Int32,
+        (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Anchor}, Int64, Int32, Int32, Ptr{Float16}, Ptr{Int64}, Int32, Int32, Ptr{Float16}, Ptr{UInt32}, Ptr{Best}),
+        ctx, seqs, an, length(an), n_primary, margin, pwms, lens, K, maxlen, tp, hist, sp))
+    st = want_sites ? [(pos = b.pos == typemax(UInt32) ? 0 : Int(b.pos) + 1, comp = b.comp != 0, score = b.score, found = b.found != 0) for b in sites] : nothing
+    Int.(hist), st
+end
+
 # fused scan + filter_position_by_best_thresh! + get_uniq_counts + union_ranges coverage: (4, K) Int64, rows = hits, unique starts,
 # coverage as the reference computes it (_h4_overlap_ratio.jl:48-56), true coverage
 scan_counts(ctx, seqs, pwms, lens, thresh::Vector{Float16}; reduce=false) =

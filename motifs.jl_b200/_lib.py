@@ -36,6 +36,9 @@ assert HIT_DTYPE.itemsize == 16
 BEST_DTYPE = np.dtype([("pos", "<u4"), ("score_f16", "<u2"), ("comp", "u1"), ("found", "u1")])
 assert BEST_DTYPE.itemsize == 8
 
+ANCHOR_DTYPE = np.dtype([("row", "<i8"), ("start", "<i8"), ("len", "<i4"), ("primary", "<u2"), ("comp", "u1"), ("_pad", "u1")])
+assert ANCHOR_DTYPE.itemsize == 24
+
 SITE_DTYPE = np.dtype([("motif", "<u4"), ("seq", "<u4"), ("pos", "<u4"), ("comp", "<u4")])
 CODE_DTYPE = np.dtype([("position", "<u2"), ("fil", "<u2"), ("seq", "<u4"), ("mag_f16", "<u2"), ("_pad", "<u2")])
 assert CODE_DTYPE.itemsize == 12
@@ -98,6 +101,7 @@ def load():
         "mb200_records_free": (i32, [p]),
         "mb200_fasta_split": (i32, [i64, C.c_double, i32, C.c_uint64, p, p, C.POINTER(i64), C.POINTER(i64)]),
         "mb200_seqs_gather": (i32, [p, p, p, i64, C.POINTER(p)]),
+        "mb200_seqs_windows": (i32, [p, p, p, p, i64, i64, C.POINTER(p)]),
         "mb200_seqs_shuffle": (i32, [p, p, i32, C.c_uint64, i64, C.POINTER(p)]),
         "mb200_seqs_base_counts": (i32, [p, p, p, p]),
         "mb200_seqs_to_ascii": (i32, [p, p, p]),
@@ -107,6 +111,7 @@ def load():
         "mb200_scan_prefilter_bound": (i32, [p, i32, C.c_uint16, p, p, p, p]),
         "mb200_scan_hist": (i32, [p, p, p, p, i32, i32, C.c_uint32, p]),
         "mb200_scan_best": (i32, [p, p, p, p, i32, i32, C.c_uint32, p]),
+        "mb200_scan_spacing": (i32, [p, p, p, i64, i32, i32, p, p, i32, i32, p, p, p]),
         "mb200_csc_create": (i32, [p, C.POINTER(HParams), i64, i32, i32, C.POINTER(p)]),
         "mb200_csc_destroy": (i32, [p, p]),
         "mb200_csc_n_params": (i32, [p, C.POINTER(i64), C.POINTER(i64)]),
@@ -331,6 +336,40 @@ class Context:
         flags = (SCAN_FWD if fwd else 0) | (SCAN_RC if rc else 0)
         self._check(self._lib.mb200_scan_best(self._h, seqs._h, _ptr(pw), _ptr(ln), K, maxlen, flags, _ptr(out)))
         return out
+
+    def seqs_windows(self, seqs: "Sequences", rows, starts, length: int) -> "Sequences":
+        """mb200_seqs_windows: a new fixed-length store whose row i holds bases [starts[i], starts[i] + length) of row rows[i] of
+        seqs (fixed or ragged)."""
+        r = np.ascontiguousarray(rows, np.int64)
+        s = np.ascontiguousarray(starts, np.int64)
+        if r.shape != s.shape or r.ndim != 1:
+            raise ValueError("rows and starts must be 1-D arrays of one length")
+        h = C.c_void_p()
+        self._check(self._lib.mb200_seqs_windows(self._h, seqs._h, _ptr(r), _ptr(s), len(r), int(length), C.byref(h)))
+        return Sequences(self, h, len(r), int(length))
+
+    def scan_spacing(self, seqs: "Sequences", anchors, n_primary: int, pwms_f16: np.ndarray, lens, thresh=None, *, margin: int,
+                     want_sites: bool = False):
+        """mb200_scan_spacing: (hist (n_primary, K, 4, margin) uint32, sites (n_anchors, K) BEST_DTYPE or None).  anchors:
+        ANCHOR_DTYPE array (row, start, len, primary, comp) of primary sites in rows of seqs; pwms_f16 and lens: the K secondaries
+        as for scan; thresh: K Float16 thresholds or None (a counted site needs score > 0 and > thresh).  hist[p, k, q, g] counts
+        the anchors of primary p whose best site of k in the two margins is counted and lies at gap g in quadrant q (0: same strand
+        upstream, 1: same strand downstream, 2: opposite upstream, 3: opposite downstream, in the primary's orientation)."""
+        pw, ln = self._pwm_arrays(pwms_f16, lens)
+        maxlen, _, K = pw.shape
+        an = np.ascontiguousarray(anchors, ANCHOR_DTYPE)
+        th = None
+        if thresh is not None:
+            th = np.ascontiguousarray(thresh)
+            if th.dtype != np.uint16:
+                th = np.ascontiguousarray(th, np.float16).view(np.uint16)
+            if th.shape != (K,):
+                raise ValueError("thresh must hold K float16 values")
+        hist = np.zeros((int(n_primary), K, 4, int(margin)), np.uint32) if 0 < n_primary and 0 < margin else np.zeros(1, np.uint32)
+        sites = np.empty((len(an), K), BEST_DTYPE) if want_sites else None
+        self._check(self._lib.mb200_scan_spacing(self._h, seqs._h, _ptr(an), len(an), int(n_primary), int(margin), _ptr(pw), _ptr(ln),
+                                                  K, maxlen, _ptr(th), _ptr(hist), _ptr(sites)))
+        return hist, sites
 
 
 def fasta_read(path: str, max_entries: int = 100000) -> np.ndarray:

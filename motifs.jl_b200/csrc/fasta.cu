@@ -201,6 +201,24 @@ __global__ void __launch_bounds__(256) gather_rows_kernel(const uint32_t* __rest
     const int64_t r = t / rowwords, w = t - r * rowwords;
     dst[t] = src[idx[r] * rowwords + w];
 }
+// output word w of window r holds bases [start[r] + 16w, +16) of source row row[r]: a window may start at any base, so a word is
+// the funnel shift of two source words (the second is read only when the word needs it: it then lies inside the source row).
+// Bits past `len` are zero, as in every store.
+__global__ void __launch_bounds__(256) windows_kernel(const uint32_t* __restrict__ src, int64_t rowwords, const int64_t* __restrict__ row,
+                                                      const int64_t* __restrict__ start, int64_t n, int64_t len, int64_t owords,
+                                                      uint32_t* __restrict__ dst) {
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= n * owords) return;
+    const int64_t r = t / owords, w = t - r * owords;
+    const int64_t b0 = start[r] + 16 * w;
+    const uint32_t* sp = src + row[r] * rowwords + (b0 >> 4);
+    const int o = (int)(b0 & 15);
+    const int64_t nb = min((int64_t)16, len - 16 * w);
+    uint32_t word = sp[0];
+    if (o) word = __funnelshift_r(word, 16 - o < nb ? sp[1] : 0u, 2 * o);
+    if (nb < 16) word &= (1u << (2 * nb)) - 1u;
+    dst[t] = word;
+}
 // lens (ragged stores, may be NULL): ASCII output is 0 past a row's length (codes past it are the padding's zeros anyway)
 __global__ void __launch_bounds__(256) unpack_codes_kernel(const uint32_t* __restrict__ words, int64_t rowwords, int64_t n, int64_t Lb, int ascii,
                                                            uint8_t* __restrict__ out, const int64_t* __restrict__ lens) {
@@ -328,6 +346,39 @@ extern "C" int32_t mb200_seqs_gather(mb200_ctx* ctx, const mb200_seqs* src, cons
         if (e == cudaSuccess) e = cudaGetLastError();
     }
     if (rc || e != cudaSuccess) { mb200_seqs_free(ctx, *out); *out = nullptr; if (rc) return rc; MB_FAIL(ctx, MB200_E_CUDA, "seqs_gather: %s", cudaGetErrorString(e)); }
+    return MB200_OK;
+}
+
+// windows [start[i], start[i] + len) of rows row[i] of `src` (fixed or ragged) as a new fixed-length store of n rows of len bases:
+// the flanks of best sites (mb200_scan_spacing), or any other fixed-width view of a store without a round trip to the host
+extern "C" int32_t mb200_seqs_windows(mb200_ctx* ctx, const mb200_seqs* src, const int64_t* row, const int64_t* start, int64_t n, int64_t len,
+                                      mb200_seqs** out) {
+    if (!ctx || !src || !out) return MB200_E_INVALID;
+    *out = nullptr;
+    if (n < 0 || len < 1 || (n > 0 && (!row || !start))) MB_FAIL(ctx, MB200_E_INVALID, "seqs_windows: bad arguments (n=%lld len=%lld)", (long long)n, (long long)len);
+    if (src->device != ctx->device) MB_FAIL(ctx, MB200_E_INVALID, "seqs_windows: sequences live on device %d, ctx on %d", src->device, ctx->device);
+    for (int64_t i = 0; i < n; ++i) {
+        if (row[i] < 0 || row[i] >= src->N) MB_FAIL(ctx, MB200_E_INVALID, "seqs_windows: window %lld: row %lld out of range", (long long)i, (long long)row[i]);
+        if (start[i] < 0 || start[i] > mb_row_len(src, row[i]) - len)
+            MB_FAIL(ctx, MB200_E_INVALID, "seqs_windows: window %lld: [%lld, %lld) leaves row %lld (%lld bases)", (long long)i, (long long)start[i],
+                    (long long)(start[i] + len), (long long)row[i], (long long)mb_row_len(src, row[i]));
+    }
+    if (src->pending) { const int rc = mb_seqs_finish(ctx, const_cast<mb200_seqs*>(src)); if (rc) return rc; }
+    MB_CUDA(ctx, cudaSetDevice(ctx->device));
+    int rc = mb_seqs_alloc(ctx, n, len, out); if (rc) return rc;
+    if (n == 0) return MB200_OK;
+    rc = mb_ensure_scratch(ctx, (size_t)n * 16);
+    cudaError_t e = cudaSuccess;
+    if (!rc) e = cudaMemcpyAsync(ctx->scratch, row, (size_t)n * 8, cudaMemcpyHostToDevice, ctx->stream);
+    if (!rc && e == cudaSuccess) e = cudaMemcpyAsync((int64_t*)ctx->scratch + n, start, (size_t)n * 8, cudaMemcpyHostToDevice, ctx->stream);
+    if (!rc && e == cudaSuccess) {
+        const int64_t th = n * (*out)->rowwords;
+        windows_kernel<<<(unsigned)((th + 255) / 256), 256, 0, ctx->stream>>>(src->words, src->rowwords, (const int64_t*)ctx->scratch,
+                                                                              (const int64_t*)ctx->scratch + n, n, len, (*out)->rowwords, (*out)->words);
+        e = cudaStreamSynchronize(ctx->stream);                       // row / start are the caller's
+        if (e == cudaSuccess) e = cudaGetLastError();
+    }
+    if (rc || e != cudaSuccess) { mb200_seqs_free(ctx, *out); *out = nullptr; if (rc) return rc; MB_FAIL(ctx, MB200_E_CUDA, "seqs_windows: %s", cudaGetErrorString(e)); }
     return MB200_OK;
 }
 

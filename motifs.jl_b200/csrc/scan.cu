@@ -381,6 +381,55 @@ __global__ void __launch_bounds__(256) best_finalize_kernel(const unsigned long 
 }
 
 // ---------------------------------------------------------------------------------------------
+// Spacing mode (mb200_scan_spacing): rows 2i and 2i + 1 of the scanned store are the left and right margins of anchor i, and
+// best64 holds their best-site keys.  One thread per (anchor, secondary), adjacent threads on adjacent secondaries (the key loads
+// coalesce).  The two margins merge by score alone: on equal scores the left margin's window lies lower in the row.  A counted
+// window (score > thr[k], with thr = max(thresh, 0) and +Inf for a NaN threshold, as build_plan sets them) adds 1 to its
+// (primary, k, quadrant, gap) bin; integer atomics make the histogram independent of the order of arrival.
+// ---------------------------------------------------------------------------------------------
+static_assert(sizeof(mb200_anchor) == 24, "mb200_anchor must be 24 bytes");
+__global__ void __launch_bounds__(256) spacing_kernel(const unsigned long long* __restrict__ best64, int64_t na, int32_t K,
+                                                      const mb200_anchor* __restrict__ anchors, const uint16_t* __restrict__ thr,
+                                                      const int32_t* __restrict__ mlen, int32_t margin, unsigned int* __restrict__ hist,
+                                                      mb200_best* __restrict__ sites) {
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= na * K) return;
+    const int64_t i = t / K;
+    const int32_t k = (int32_t)(t - i * K);
+    const unsigned long long l = best64[2 * i * K + k], r = best64[(2 * i + 1) * K + k];
+    const bool left = l && (l >> 48) >= (r >> 48);
+    const unsigned long long v = left ? l : r;
+    mb200_best out;
+    out.pos = 0xFFFFFFFFu; out.score_f16 = 0; out.comp = 0; out.found = 0;
+    if (v) {
+        const mb200_anchor an = anchors[i];
+        const uint32_t o = (uint32_t)(v >> 48);
+        const uint16_t s = (uint16_t)((o & 0x8000u) ? (o & 0x7FFFu) : (~o & 0xFFFFu));
+        const int32_t u = (int32_t)(0xFFFFFFFFu - (uint32_t)(v >> 1));          // start inside the margin
+        const uint32_t c = 1u - (uint32_t)(v & 1u);
+        const bool counted = __hgt(__ushort_as_half(s), __ushort_as_half(thr[k]));
+        out.pos = (uint32_t)(left ? an.start - margin + u : an.start + an.len + u);
+        out.score_f16 = s; out.comp = (uint8_t)c; out.found = counted;
+        if (counted) {
+            const int32_t g = left ? margin - u - mlen[k] : u;
+            const int32_t down = left == (an.comp != 0);
+            const int32_t q = 2 * (int32_t)(c != an.comp) + down;
+            atomicAdd(hist + (((int64_t)an.primary * K + k) * 4 + q) * margin + g, 1u);
+        }
+    }
+    if (sites) sites[t] = out;
+}
+
+// what mb200_scan_spacing hands to scan_impl: host arrays
+struct SpacingJob {
+    const mb200_anchor* anchors; int64_t n;
+    int32_t n_primary, margin;
+    const uint16_t* thresh;            // K Float16 bits or NULL
+    uint32_t* hist;                    // n_primary * K * 4 * margin
+    mb200_best* sites;                 // n * K or NULL
+};
+
+// ---------------------------------------------------------------------------------------------
 // Counting from the masks: one thread per (sequence, motif).  Mask word layout:
 //   mask[(n*W + w) * K2pad + slotpair*2 + strand]
 // ---------------------------------------------------------------------------------------------
@@ -1046,8 +1095,9 @@ static int build_plan(mb200_ctx* ctx, const uint16_t* pwms, const int64_t* lens,
 
 static int32_t scan_impl(mb200_ctx* ctx, const mb200_seqs* seqs, const uint16_t* pwms_f16, const int64_t* lens, int32_t K,
                          int32_t maxlen, const uint16_t* thresh_f16, uint32_t flags, mb200_hit* hits, int64_t hits_cap,
-                         int64_t* n_hits, int64_t* counts, uint32_t* hist, mb200_best* best) {
+                         int64_t* n_hits, int64_t* counts, uint32_t* hist, mb200_best* best, const SpacingJob* sp = nullptr) {
     if (!ctx) return MB200_E_INVALID;
+    const bool best_mode = best || sp;                 // block keys and best_reduce_kernel; sp: rows are anchor margins in pairs
     if (!seqs || !pwms_f16 || !lens || K <= 0 || K > 65535 || maxlen <= 0)
         MB_FAIL(ctx, MB200_E_INVALID, "scan: bad arguments (K=%d maxlen=%d)", K, maxlen);
     if (!(flags & (MB200_SCAN_FWD | MB200_SCAN_RC))) MB_FAIL(ctx, MB200_E_INVALID, "scan: neither FWD nor RC requested");
@@ -1071,7 +1121,7 @@ static int32_t scan_impl(mb200_ctx* ctx, const mb200_seqs* seqs, const uint16_t*
     // Thresholded scans take the tensor-core pre-filter + exact verification (scan_tc.cuh) unless the caller or the inputs rule
     // it out; the hit masks, and everything derived from them, are identical either way.
     TcPlan TP;
-    bool use_tc = !(flags & MB200_SCAN_NO_TENSOR) && !hist && !best && Lb < (1ll << 31);
+    bool use_tc = !(flags & MB200_SCAN_NO_TENSOR) && !hist && !best_mode && Lb < (1ll << 31);
     if (use_tc) use_tc = build_tc_plan(P, pwms_f16, lens, K, thresh_f16, flags, Lb, ctx->sm_count, TP);
     ctx->last_scan_path = 0;
     if (use_tc) {
@@ -1087,6 +1137,11 @@ static int32_t scan_impl(mb200_ctx* ctx, const mb200_seqs* seqs, const uint16_t*
         if (best) {                                     // no row holds a window (otherwise every batch writes all its records)
             const mb200_best none = {0xFFFFFFFFu, 0, 0, 0};
             std::fill(best, best + (size_t)N * K, none);
+        }
+        if (sp) {                                       // every secondary is longer than the margin
+            const mb200_best none = {0xFFFFFFFFu, 0, 0, 0};
+            memset(sp->hist, 0, (size_t)sp->n_primary * K * 4 * sp->margin * 4);
+            if (sp->sites) std::fill(sp->sites, sp->sites + (size_t)sp->n * K, none);
         }
         if (reduce && (want_counts || hist)) {
             const size_t nb = hist ? (size_t)K * HIST_BINS * 4 : (size_t)K * 4 * 8;
@@ -1130,10 +1185,11 @@ static int32_t scan_impl(mb200_ctx* ctx, const mb200_seqs* seqs, const uint16_t*
 
     // ---- batching: masks of one batch stay under a budget -----------------------------------
     const size_t mask_budget = (size_t)8 << 30;
-    const size_t mask_bytes_per_seq = (size_t)W * P.K2pad * 4 * (best ? 2 : 1);      // best sites: one 32-bit key per 16-position block
+    const size_t mask_bytes_per_seq = (size_t)W * P.K2pad * 4 * (best_mode ? 2 : 1);      // best sites: one 32-bit key per 16-position block
     int64_t seqs_per_batch = std::max<int64_t>(1, (int64_t)(mask_budget / mask_bytes_per_seq));
     if (seqs_per_batch > N) seqs_per_batch = N;
     if ((double)seqs_per_batch * W > 2.0e9) seqs_per_batch = std::max<int64_t>(1, (int64_t)(2.0e9 / W));
+    if (sp) seqs_per_batch = std::max<int64_t>(2, seqs_per_batch & ~(int64_t)1);    // both margins of an anchor in one batch (N is even)
     if (use_tc && (double)seqs_per_batch * (double)Lb > 2.0e9) seqs_per_batch = std::max<int64_t>(1, (int64_t)(2.0e9 / (double)Lb));   // 32-bit virtual positions
     // tensor-core path: plan (B operands, blocks, slots) in buf 8, candidate list + counters in buf 9
     const unsigned long long tc_cap = (unsigned long long)24 << 20;      // candidate records per batch and buffer set
@@ -1179,10 +1235,38 @@ static int32_t scan_impl(mb200_ctx* ctx, const mb200_seqs* seqs, const uint16_t*
     int64_t ps_blocks = (units_per_batch + PS_TILE - 1) / PS_TILE;
     unsigned long long* d_best64 = nullptr; mb200_best* d_best = nullptr;
     const int32_t best_nch = (W16 + BEST_CHUNK - 1) / BEST_CHUNK;
-    if (best) {                                         // per batch: 64-bit best keys, then the records
+    if (best_mode) {                                    // per batch: 64-bit best keys, then the records (spacing: the sites)
         rc = mb_ensure_buf(ctx, 3, (size_t)seqs_per_batch * K * 16); if (rc) return rc;
         d_best64 = (unsigned long long*)ctx->bufs[3];
         d_best = (mb200_best*)(d_best64 + (size_t)seqs_per_batch * K);
+    }
+    // spacing: the histogram (buf 0) and the anchors, thresholds and secondary lengths (buf 11)
+    unsigned int* d_sphist = nullptr; const mb200_anchor* d_anchors = nullptr; const uint16_t* d_spthr = nullptr; const int32_t* d_mlen = nullptr;
+    const size_t sphist_bytes = sp ? (size_t)sp->n_primary * K * 4 * (size_t)sp->margin * 4 : 0;
+    if (sp) {
+        rc = mb_ensure_buf(ctx, 0, sphist_bytes); if (rc) return rc;
+        d_sphist = (unsigned int*)ctx->bufs[0];
+        const size_t off_thr = ((size_t)sp->n * sizeof(mb200_anchor) + 255) & ~(size_t)255;
+        const size_t off_len = off_thr + (((size_t)K * 2 + 255) & ~(size_t)255);
+        const size_t bytes = off_len + (size_t)K * 4;
+        rc = mb_ensure_buf(ctx, 11, bytes); if (rc) return rc;
+        std::vector<uint8_t> h(bytes, 0);
+        memcpy(h.data(), sp->anchors, (size_t)sp->n * sizeof(mb200_anchor));
+        uint16_t* ht = reinterpret_cast<uint16_t*>(h.data() + off_thr);
+        int32_t* hl = reinterpret_cast<int32_t*>(h.data() + off_len);
+        for (int k = 0; k < K; ++k) {                   // the hit rule of build_plan: score > max(thresh, 0), never for a NaN threshold
+            uint16_t t = 0;
+            if (sp->thresh) {
+                const uint16_t raw = sp->thresh[k];
+                t = (h16_nonfinite(raw) && (raw & 0x03FFu)) ? (uint16_t)0x7C00u : h16_to_float(raw) > 0.f ? raw : (uint16_t)0;
+            }
+            ht[k] = t; hl[k] = (int32_t)lens[k];
+        }
+        uint8_t* d = (uint8_t*)ctx->bufs[11];
+        MB_CUDA(ctx, cudaMemcpyAsync(d, h.data(), bytes, cudaMemcpyHostToDevice, ctx->stream));
+        MB_CUDA(ctx, cudaMemsetAsync(d_sphist, 0, sphist_bytes, ctx->stream));
+        MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));         // h goes out of scope
+        d_anchors = (const mb200_anchor*)d; d_spthr = (const uint16_t*)(d + off_thr); d_mlen = (const int32_t*)(d + off_len);
     }
     if (want_hits) {
         size_t b = (((size_t)units_per_batch * 4 + 255) & ~(size_t)255) + (((size_t)units_per_batch * 8 + 255) & ~(size_t)255) +
@@ -1204,7 +1288,7 @@ static int32_t scan_impl(mb200_ctx* ctx, const mb200_seqs* seqs, const uint16_t*
     const size_t smem_bytes = (size_t)blob_cap + (size_t)tile_cap_words * 8 + 64;
     if (smem_bytes > ctx->smem_optin) MB_FAIL(ctx, MB200_E_UNSUPPORTED, "scan needs %zu B shared memory (> %zu)", smem_bytes, ctx->smem_optin);
     const bool ragged = seqs->lens != nullptr;
-    if (best) MB_CUDA(ctx, cudaFuncSetAttribute(ragged ? scan_kernel<true, true> : scan_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
+    if (best_mode) MB_CUDA(ctx, cudaFuncSetAttribute(ragged ? scan_kernel<true, true> : scan_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
     else MB_CUDA(ctx, cudaFuncSetAttribute(ragged ? scan_kernel<true> : scan_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
 
     MbTimers tm(ctx);
@@ -1459,7 +1543,7 @@ static int32_t scan_impl(mb200_ctx* ctx, const mb200_seqs* seqs, const uint16_t*
         int t1 = tm.begin(T_SCAN);
         ctx->mask_clean_bytes = 0;
         if (!P.mblocks.empty()) {
-            if (best) {
+            if (best_mode) {
                 if (ragged) scan_kernel<true, true><<<grid, SCAN_THREADS, smem_bytes, ctx->stream>>>(a);
                 else scan_kernel<false, true><<<grid, SCAN_THREADS, smem_bytes, ctx->stream>>>(a);
             } else {
@@ -1470,7 +1554,7 @@ static int32_t scan_impl(mb200_ctx* ctx, const mb200_seqs* seqs, const uint16_t*
         }
         if (!P.lblocks.empty()) {
             const int64_t warps = ns * (int64_t)P.lblocks.size() * GROUP_SLOTS;
-            auto long_kernel = best ? scan_long_kernel<true> : scan_long_kernel<false>;
+            auto long_kernel = best_mode ? scan_long_kernel<true> : scan_long_kernel<false>;
             long_kernel<<<(unsigned)((warps * 32 + 255) / 256), 256, 0, ctx->stream>>>(seqs->words, rowwords, s0, ns, W, P.K2pad, d_plan + off_blob,
                                                                                    (const MBlock*)(d_plan + off_lb), (int32_t)P.lblocks.size(), d_mask,
                                                                                    seqs->lens, Lb);
@@ -1480,12 +1564,26 @@ static int32_t scan_impl(mb200_ctx* ctx, const mb200_seqs* seqs, const uint16_t*
         }
         MB_CUDA(ctx, cudaGetLastError());
 
-        if (best) {
+        if (best_mode) {
             const int t2 = tm.begin(T_COUNT);
             MB_CUDA(ctx, cudaMemsetAsync(d_best64, 0, (size_t)ns * K * 8, ctx->stream));
             const int64_t rthreads = ns * (int64_t)best_nch * (P.K2pad / 2);
             best_reduce_kernel<<<(unsigned)((rthreads + 255) / 256), 256, 0, ctx->stream>>>(d_mask, ns, W16, P.K2pad, best_nch,
                                                                                           (const int32_t*)(d_plan + off_p2m), K, d_best64);
+            if (sp) {                                   // anchors s0/2 .. (s0 + ns)/2: count into the histogram instead of returning records
+                const int64_t na = ns / 2;
+                spacing_kernel<<<(unsigned)((na * K + 255) / 256), 256, 0, ctx->stream>>>(d_best64, na, K, d_anchors + s0 / 2, d_spthr, d_mlen, sp->margin,
+                                                                                         d_sphist, sp->sites ? d_best : nullptr);
+                tm.end(t2);
+                ctx->launches[T_COUNT] += 2;
+                MB_CUDA(ctx, cudaGetLastError());
+                if (sp->sites) {
+                    const int t6 = tm.begin(T_D2H);
+                    MB_CUDA(ctx, cudaMemcpyAsync(sp->sites + (size_t)(s0 / 2) * K, d_best, (size_t)na * K * sizeof(mb200_best), cudaMemcpyDeviceToHost, ctx->stream));
+                    tm.end(t6);
+                }
+                continue;
+            }
             best_finalize_kernel<<<(unsigned)((ns * K + 255) / 256), 256, 0, ctx->stream>>>(d_best64, ns * K, d_best);
             tm.end(t2);
             ctx->launches[T_COUNT] += 2;
@@ -1596,6 +1694,11 @@ static int32_t scan_impl(mb200_ctx* ctx, const mb200_seqs* seqs, const uint16_t*
         MB_CUDA(ctx, cudaMemcpyAsync(counts, d_counts, (size_t)K * 4 * 8, cudaMemcpyDeviceToHost, ctx->stream));
         tm.end(t6);
     }
+    if (sp) {
+        const int t9 = tm.begin(T_D2H);
+        MB_CUDA(ctx, cudaMemcpyAsync(sp->hist, d_sphist, sphist_bytes, cudaMemcpyDeviceToHost, ctx->stream));
+        tm.end(t9);
+    }
     tm.end(t_total);
     MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     tm.collect();
@@ -1668,4 +1771,48 @@ extern "C" int32_t mb200_scan_best(mb200_ctx* ctx, const mb200_seqs* seqs, const
     if (!best) MB_FAIL(ctx, MB200_E_INVALID, "scan_best: null output");
     if (flags & ~(MB200_SCAN_FWD | MB200_SCAN_RC)) MB_FAIL(ctx, MB200_E_INVALID, "scan_best: flags 0x%x: only MB200_SCAN_FWD | MB200_SCAN_RC", flags);
     return scan_impl(ctx, seqs, pwms_f16, lens, K, maxlen, nullptr, flags, nullptr, 0, nullptr, nullptr, nullptr, best);
+}
+
+// The margins of every anchor become rows 2i (left) and 2i + 1 (right) of a fixed-length store (mb200_seqs_windows); the best-site
+// scan of that store feeds spacing_kernel batch by batch, and only the histogram (and the sites, when asked) comes back.
+extern "C" int32_t mb200_scan_spacing(mb200_ctx* ctx, const mb200_seqs* seqs, const mb200_anchor* anchors, int64_t n_anchors,
+                                      int32_t n_primary, int32_t margin, const uint16_t* pwms_f16, const int64_t* lens, int32_t K,
+                                      int32_t maxlen, const uint16_t* thresh_f16, uint32_t* hist, mb200_best* sites) {
+    if (!ctx) return MB200_E_INVALID;
+    if (!seqs || !hist || !pwms_f16 || !lens || K <= 0 || K > 65535 || n_anchors < 0 || (n_anchors > 0 && !anchors))
+        MB_FAIL(ctx, MB200_E_INVALID, "scan_spacing: bad arguments (K=%d n_anchors=%lld)", K, (long long)n_anchors);
+    if (margin < 1 || margin > 65536) MB_FAIL(ctx, MB200_E_INVALID, "scan_spacing: margin %d outside [1, 65536]", margin);
+    if (n_primary < 1 || n_primary > 65535) MB_FAIL(ctx, MB200_E_INVALID, "scan_spacing: n_primary %d outside [1, 65535]", n_primary);
+    std::vector<int64_t> row((size_t)n_anchors * 2), start((size_t)n_anchors * 2);
+    for (int64_t i = 0; i < n_anchors; ++i) {
+        const mb200_anchor& a = anchors[i];
+        if (a.primary >= n_primary || a.comp > 1 || a.len < 1 || a.row < 0 || a.row >= seqs->N)
+            MB_FAIL(ctx, MB200_E_INVALID, "scan_spacing: anchor %lld: primary %d comp %d len %d row %lld", (long long)i, (int)a.primary, (int)a.comp, a.len, (long long)a.row);
+        if (a.start - margin < 0 || a.start > mb_row_len(seqs, a.row) - a.len - margin)
+            MB_FAIL(ctx, MB200_E_INVALID, "scan_spacing: anchor %lld: flank [%lld, %lld) leaves row %lld (%lld bases)", (long long)i, (long long)(a.start - margin),
+                    (long long)(a.start + a.len + margin), (long long)a.row, (long long)mb_row_len(seqs, a.row));
+        row[2 * i] = row[2 * i + 1] = a.row;
+        start[2 * i] = a.start - margin;
+        start[2 * i + 1] = a.start + a.len;
+    }
+    if (n_anchors == 0) { mb_reset_timing(ctx); memset(hist, 0, (size_t)n_primary * K * 4 * (size_t)margin * 4); return MB200_OK; }
+    MB_CUDA(ctx, cudaSetDevice(ctx->device));
+    struct Guard {                                      // events and the margin store are released on every way out (error returns included)
+        mb200_ctx* ctx; cudaEvent_t e0 = nullptr, e1 = nullptr; mb200_seqs* win = nullptr;
+        ~Guard() { if (e0) cudaEventDestroy(e0); if (e1) cudaEventDestroy(e1); if (win) mb200_seqs_free(ctx, win); }
+    } g{ctx};
+    MB_CUDA(ctx, cudaEventCreate(&g.e0));
+    MB_CUDA(ctx, cudaEventCreate(&g.e1));
+    MB_CUDA(ctx, cudaEventRecord(g.e0, ctx->stream));
+    int rc = mb200_seqs_windows(ctx, seqs, row.data(), start.data(), 2 * n_anchors, margin, &g.win);
+    if (rc) return rc;
+    MB_CUDA(ctx, cudaEventRecord(g.e1, ctx->stream));
+    MB_CUDA(ctx, cudaEventSynchronize(g.e1));
+    float pack_ms = 0;
+    MB_CUDA(ctx, cudaEventElapsedTime(&pack_ms, g.e0, g.e1));
+    const SpacingJob job = {anchors, n_anchors, n_primary, margin, thresh_f16, hist, sites};
+    rc = scan_impl(ctx, g.win, pwms_f16, lens, K, maxlen, nullptr, MB200_SCAN_FWD | MB200_SCAN_RC, nullptr, 0, nullptr, nullptr, nullptr, nullptr, &job);
+    if (rc) return rc;
+    ctx->ms[T_PACK] += pack_ms; ctx->ms[T_TOTAL] += pack_ms; ctx->launches[T_PACK] += 1;       // scan_impl reset the timing
+    return MB200_OK;
 }

@@ -325,3 +325,169 @@ def central_enrichment(best: BestSites, lens) -> CentralEnrichment:
         res.expected[k] = N * (r + 1) / npos
         res.p[k], res.p_adj[k] = best_p, min(1.0, best_p * len(radii))
     return res
+
+
+# ---- secondary-motif spacing around primary sites (SpaMo) ----------------------------------------------------------------
+SPACING_SITE_DTYPE = np.dtype([("pos", "<i8"), ("score", "<f2"), ("comp", "u1"), ("found", "?")])
+
+
+@dataclass
+class Spacing:
+    """Spacings of secondary motifs around the record best sites of primary motifs (`spacing`).  An anchor is a record whose best
+    site of primary p (at pos[r, p] on strand comp[r, p], record coordinates) is a hit (score > 0 and > the primary's threshold)
+    with its whole flank [pos - margin, pos + m_p + margin) inside one N-free fragment.  hist[p, k, q, g] counts the anchors of p
+    whose best site of secondary k in the two margins is a hit at gap g in quadrant q, in the primary's orientation: 0 same strand
+    upstream, 1 same strand downstream, 2 opposite strand upstream, 3 opposite strand downstream.  pos / comp are -1 for records
+    that are not anchors of p.  sites (with want_sites): the best window of every (record, primary, secondary) in record
+    coordinates, found = counted; pos = -1 where there is no anchor or no window."""
+    names: List[str]
+    margin: int
+    hist: np.ndarray             # (P, K, 4, margin) int64
+    n_anchors: np.ndarray        # (P,) int64
+    pos: np.ndarray              # (R, P) int64
+    comp: np.ndarray             # (R, P) int64
+    sites: Optional[np.ndarray] = None      # (R, P, K) SPACING_SITE_DTYPE
+
+
+def spacing_bin(a, m_p, c_p, s, m_k, c_k):
+    """(q, g) of a secondary site at s (length m_k, strand c_k) next to a primary site at a (length m_p, strand c_p), as
+    mb200_scan_spacing bins it (element-wise over arrays).  Left of the primary (s < a): g = a - (s + m_k); right: g = s -
+    (a + m_p).  Downstream is the right side for c_p = 0 and the left side for c_p = 1; q = 2 (c_k != c_p) + downstream."""
+    a, m_p, c_p, s, m_k, c_k = (np.asarray(x, np.int64) for x in (a, m_p, c_p, s, m_k, c_k))
+    left = s < a
+    g = np.where(left, a - (s + m_k), s - (a + m_p))
+    down = (left == (c_p != 0)).astype(np.int64)
+    return 2 * (c_k != c_p).astype(np.int64) + down, g
+
+
+def _hit_mask(score, thresh):
+    """score > 0 and > thresh (float16, NaN threshold: never), the hit rule of mb200_scan, per column."""
+    s = np.asarray(score, np.float16)
+    ok = s > np.float16(0)
+    if thresh is not None:
+        t = np.asarray(thresh, np.float16)
+        ok &= ~np.isnan(t)[None, :] & (s > np.where(np.isnan(t), np.float16(0), t)[None, :])
+    return ok
+
+
+def spacing_anchors(rec: Records, score, pos, comp, found, primary_lens, primary_thresh, margin: int):
+    """Record best sites of the primaries -> anchors.  Returns (frag (R, P) int64 fragment holding the flank, -1 for no anchor,
+    and the (R, P) bool anchor mask).  A best site counts when it is a hit and [pos - margin, pos + m_p + margin) lies inside
+    one fragment (no N run, no record end)."""
+    R, P = np.shape(pos)
+    m = np.asarray(primary_lens, np.int64)[None, :]
+    ok = np.asarray(found, bool) & _hit_mask(score, primary_thresh)
+    lo = np.asarray(pos, np.int64) - margin
+    hi = np.asarray(pos, np.int64) + m + margin
+    frag = np.full((R, P), -1, np.int64)
+    if len(rec.frag_len) and R:
+        coff = np.concatenate([[0], np.cumsum(rec.lengths)]).astype(np.int64)
+        gstart = coff[rec.frag_record] + rec.frag_start             # increasing: fragments come in record order
+        rr = np.broadcast_to(np.arange(R, dtype=np.int64)[:, None], (R, P))
+        f = np.searchsorted(gstart, coff[rr] + lo, side="right") - 1
+        fc = np.clip(f, 0, len(gstart) - 1)
+        inside = (f >= 0) & (lo >= 0) & (rec.frag_record[fc] == rr) & (rec.frag_start[fc] <= lo) & \
+                 (hi <= rec.frag_start[fc] + rec.frag_len[fc])
+        ok &= inside
+        frag = np.where(ok, fc, -1)
+    else:
+        ok[:] = False
+    return frag, ok
+
+
+def spacing(ctx, path_or_records, primary, secondary, *, primary_thresh=None, secondary_thresh=None, margin: int = 150,
+            want_sites: bool = False, max_padding: float = 1.0 / 8) -> Spacing:
+    """SpaMo-style spacing analysis of a FASTA peak set (a path or a Records).  The primaries' record best sites (best_sites)
+    that are hits with a whole flank become anchors; the fragments holding them are bucketed as in scan_fasta (only those
+    fragments), and one mb200_scan_spacing call per bucket finds the best site of every secondary in both margins of each
+    anchor and adds it to the device histogram.  primary / secondary: an inference.Motifs (its score_thresh is the threshold
+    when none is given) or a list of (4, len) PWMs.  spacing_enrichment tests the histogram."""
+    rec = path_or_records if isinstance(path_or_records, Records) else read_records(path_or_records)
+    ppw, plens, pthr = _pwm_args(primary, primary_thresh)
+    spw, slens, sthr = _pwm_args(secondary, secondary_thresh)
+    margin = int(margin)
+    if margin < 1:
+        raise ValueError("margin must be >= 1")
+    P, K, R = len(plens), len(slens), len(rec.names)
+    bs = best_sites(ctx, rec, primary, max_padding=max_padding)
+    frag, ok = spacing_anchors(rec, bs.score, bs.pos, bs.comp, bs.found, plens, None if pthr is None else pthr.view(np.float16),
+                               margin)
+    hist = np.zeros((P, K, 4, margin), np.int64)
+    sites = None
+    if want_sites:
+        sites = np.zeros((R, P, K), SPACING_SITE_DTYPE)
+        sites["pos"] = -1
+    has = np.zeros(len(rec.frag_len), bool)
+    has[frag[ok]] = True
+    off = rec.frag_offsets
+    for b in bucket_fragments(np.where(has, rec.frag_len, 0), 1, max_padding):
+        row_of = np.full(len(rec.frag_len), -1, np.int64)
+        row_of[b] = np.arange(len(b))
+        sel = ok & (row_of[np.maximum(frag, 0)] >= 0)
+        rr, pp = np.nonzero(sel)
+        f = frag[rr, pp]
+        an = np.zeros(len(rr), _lib.ANCHOR_DTYPE)
+        an["row"] = row_of[f]
+        an["start"] = bs.pos[rr, pp] - rec.frag_start[f]
+        an["len"] = plens[pp]
+        an["primary"] = pp
+        an["comp"] = bs.comp[rr, pp]
+        ls = rec.frag_len[b]
+        seqs = ctx.seqs_from_ragged(np.concatenate([rec.bases[off[g]: off[g + 1]] for g in b]), np.concatenate([[0], np.cumsum(ls)]))
+        try:
+            h, st = ctx.scan_spacing(seqs, an, P, spw, slens, sthr, margin=margin, want_sites=want_sites)
+        finally:
+            seqs.free()
+        hist += h
+        if want_sites:
+            w = st["pos"] != np.uint32(0xFFFFFFFF)
+            out = sites[rr, pp]
+            out["pos"] = np.where(w, rec.frag_start[f][:, None] + st["pos"].astype(np.int64), -1)
+            out["score"] = st["score_f16"].view(np.float16)
+            out["comp"] = st["comp"]
+            out["found"] = st["found"].astype(bool)
+            sites[rr, pp] = out
+    pos = np.where(ok, bs.pos, -1)
+    comp = np.where(ok, bs.comp.astype(np.int64), -1)
+    return Spacing(list(rec.names), margin, hist, ok.sum(axis=0).astype(np.int64), pos, comp, sites)
+
+
+@dataclass
+class SpacingEnrichment:
+    """Per (primary, secondary): the most populated (quadrant, gap) bin among the B = 4 (margin - m_k + 1) bins where a
+    secondary of length m_k fits (ties: lowest q, then lowest gap), its count of the n counted sites, p = P[Binom(n, 1/B) >=
+    count] (SpaMo's uniform null) and p_adj = min(1, p * B * K), Bonferroni over bins and secondaries.  q = gap = -1, p = p_adj =
+    1 where n = 0 or the secondary does not fit in the margin."""
+    n: np.ndarray                # (P, K) int64
+    q: np.ndarray                # (P, K) int64
+    gap: np.ndarray              # (P, K) int64
+    count: np.ndarray            # (P, K) int64
+    p: np.ndarray                # (P, K) float64
+    p_adj: np.ndarray            # (P, K) float64
+
+
+def spacing_enrichment(sp: Spacing, secondary_lens) -> SpacingEnrichment:
+    P, K, _, W = sp.hist.shape
+    lens = np.asarray(secondary_lens, np.int64)
+    if lens.shape != (K,):
+        raise ValueError("secondary_lens must hold K lengths")
+    res = SpacingEnrichment(np.zeros((P, K), np.int64), np.full((P, K), -1, np.int64), np.full((P, K), -1, np.int64),
+                            np.zeros((P, K), np.int64), np.ones((P, K)), np.ones((P, K)))
+    for k in range(K):
+        G = W - int(lens[k]) + 1
+        if G < 1:
+            continue
+        B = 4 * G
+        for p in range(P):
+            h = sp.hist[p, k, :, :G]
+            n = int(h.sum())
+            res.n[p, k] = n
+            if n == 0:
+                continue
+            i = int(np.argmax(h.reshape(-1)))               # first maximum in (q, gap) order
+            q, g = divmod(i, G)
+            c = int(h[q, g])
+            pv = inference.binom_right(c, n, 1.0 / B)
+            res.q[p, k], res.gap[p, k], res.count[p, k] = q, g, c
+            res.p[p, k], res.p_adj[p, k] = pv, min(1.0, pv * B * K)
+    return res

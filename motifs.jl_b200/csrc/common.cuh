@@ -11,6 +11,23 @@
 
 enum { T_PACK = 0, T_SCAN = 1, T_COUNT = 2, T_EMIT = 3, T_CSC = 4, T_H2D = 5, T_D2H = 6, T_TOTAL = 7, T_N = 8 };
 
+// Slots of ctx->bufs.  BUF_HIST and BUF_UNITS each serve two scan modes; no single call uses both meanings of one slot.
+enum {
+    BUF_HIST = 0,         // scan: score histogram (mb200_scan_hist) or spacing histogram (mb200_scan_spacing)
+    BUF_PLAN = 1,         // scan: tables, motif blocks, pair and emit tables, CTA ranges, counts
+    BUF_MASK = 2,         // scan: hit masks or best keys of one batch (ctx->mask_clean_bytes)
+    BUF_UNITS = 3,        // scan: per-unit hit counts and offsets (hit lists) or 64-bit best keys and records (best site, spacing)
+    BUF_HITS = 4,         // scan: hit records of one batch
+    BUF_CODES = 5,        // csc_codes: code records and counts
+    BUF_SITES = 6,        // count matrices: counts, sites
+    BUF_LONG_COUNT = 7,   // scan: count_long_* scratch (chromosome-scale rows)
+    BUF_TC_PLAN = 8,      // tensor-core scan: B operands, slot blocks, slots
+    BUF_TC_LIST = 9,      // tensor-core scan: candidate lists and counters (two sets)
+    BUF_TC_UNITS = 10,    // tensor-core scan: listed units and their bitmap (two sets)
+    BUF_SPACING = 11,     // spacing: anchors, thresholds, secondary lengths
+    BUF_N = 12
+};
+
 struct mb200_ctx {
     int device = 0;
     int sm_count = 148;
@@ -24,15 +41,15 @@ struct mb200_ctx {
     float ms[T_N] = {0};
     int64_t launches[T_N] = {0};
     cudaEvent_t ev[2 * T_N] = {nullptr};      // start/stop per slot
-    // grow-only device buffers reused across calls (slot 0 = generic scratch)
+    // grow-only device buffers reused across calls (bufs: one per BUF_* slot)
     void* scratch = nullptr; size_t scratch_bytes = 0;
-    void* bufs[12] = {nullptr}; size_t buf_bytes[12] = {0};
+    void* bufs[BUF_N] = {nullptr}; size_t buf_bytes[BUF_N] = {0};
     void* pinned = nullptr;  size_t pinned_bytes = 0;
     int last_scan_path = 0;                   // mb200_scan_last_path
     // freed sequence stores / staging buffers kept for the next upload (cudaMalloc + cudaFree of 0.5 GB cost 100s of ms per call)
     std::vector<std::pair<void*, size_t>> pool; size_t pool_bytes = 0;
     std::vector<int32_t> tc_cost_sig; std::vector<double> tc_cost;   // tensor-core scan: measured clocks per tile of the last block structure
-    size_t mask_clean_bytes = 0;              // leading bytes of bufs[2] (hit masks) known to be zero (tensor-core scan path)
+    size_t mask_clean_bytes = 0;              // leading bytes of bufs[BUF_MASK] (hit masks) known to be zero (tensor-core scan path)
     // multi-GPU (csrc/comm.cu): one NCCL communicator per ctx, created by mb200_comm_init; world == 1 without one
     void* comm = nullptr; int rank = 0, world = 1;
     std::vector<mb200_hit> held_hits;         // hit list of a scan whose caller buffer was too small (mb200_scan_take_hits)

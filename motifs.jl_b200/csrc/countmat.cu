@@ -51,8 +51,8 @@ extern "C" int32_t mb200_count_matrices(mb200_ctx* ctx, const mb200_seqs* seqs, 
     const size_t cbytes = (size_t)K * maxlen * 4 * 4;
     const size_t off_cnt = 0, off_bad = (cbytes + 255) & ~(size_t)255, off_lens = off_bad + 256;
     const size_t off_sites = off_lens + (((size_t)K * 4 + 255) & ~(size_t)255);
-    int rc = mb_ensure_buf(ctx, 6, off_sites + (size_t)std::max<int64_t>(n_sites, 1) * sizeof(mb200_site)); if (rc) return rc;
-    uint8_t* base = (uint8_t*)ctx->bufs[6];
+    int rc = mb_ensure_buf(ctx, BUF_SITES, off_sites + (size_t)std::max<int64_t>(n_sites, 1) * sizeof(mb200_site)); if (rc) return rc;
+    uint8_t* base = (uint8_t*)ctx->bufs[BUF_SITES];
     MbTimers tm(ctx);
     const int tt = tm.begin(T_TOTAL);
     MB_CUDA(ctx, cudaMemsetAsync(base, 0, off_lens, ctx->stream));

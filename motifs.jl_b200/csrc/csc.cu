@@ -1127,8 +1127,8 @@ static int32_t codes_impl(mb200_ctx* ctx, mb200_csc* s, const mb200_seqs* seqs, 
     std::vector<int32_t> h_cnt(d.NS);
     // k_emit_codes on the x of the last forward pass: `stride` records per sequence, then counts and records to the host
     auto emit = [&](int64_t seq0, int stride) -> int {
-        const int rc = mb_ensure_buf(ctx, 5, (size_t)d.NS * stride * sizeof(mb200_code) + (size_t)d.NS * 4 + 256); if (rc) return rc;
-        mb200_code* d_slots = (mb200_code*)ctx->bufs[5];
+        const int rc = mb_ensure_buf(ctx, BUF_CODES, (size_t)d.NS * stride * sizeof(mb200_code) + (size_t)d.NS * 4 + 256); if (rc) return rc;
+        mb200_code* d_slots = (mb200_code*)ctx->bufs[BUF_CODES];
         int32_t* d_cnt = (int32_t*)(d_slots + (size_t)d.NS * stride);
         lk(k_emit_codes, nblk((int64_t)d.NS * 32, 128), 128, 0, ctx->stream, s->data + s->named["x"].off, seq0, d_slots, d_cnt, stride, d);
         ctx->launches[T_CSC] += 1;

@@ -33,7 +33,7 @@ extern "C" int32_t mb200_destroy(mb200_ctx* ctx) {
     cudaSetDevice(ctx->device);
     mb200_comm_destroy(ctx);
     if (ctx->scratch) cudaFree(ctx->scratch);
-    for (int i = 0; i < 12; ++i) if (ctx->bufs[i]) cudaFree(ctx->bufs[i]);
+    for (int i = 0; i < BUF_N; ++i) if (ctx->bufs[i]) cudaFree(ctx->bufs[i]);
     if (ctx->pinned) cudaFreeHost(ctx->pinned);
     for (auto& b : ctx->pool) cudaFree(b.first);
     if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
@@ -87,7 +87,7 @@ int mb_ensure_pinned(mb200_ctx* ctx, size_t bytes) {
 int mb_ensure_buf(mb200_ctx* ctx, int slot, size_t bytes) {
     if (ctx->buf_bytes[slot] >= bytes) return MB200_OK;
     if (ctx->bufs[slot]) { cudaFree(ctx->bufs[slot]); ctx->bufs[slot] = nullptr; ctx->buf_bytes[slot] = 0; }
-    if (slot == 2) ctx->mask_clean_bytes = 0;
+    if (slot == BUF_MASK) ctx->mask_clean_bytes = 0;
     if (cudaMalloc(&ctx->bufs[slot], bytes) != cudaSuccess) {
         cudaGetLastError();
         MB_FAIL(ctx, MB200_E_NOMEM, "cudaMalloc(%zu) for buffer %d failed", bytes, slot);

@@ -765,6 +765,14 @@ __global__ void __launch_bounds__(256) hist_kernel(const uint32_t* __restrict__ 
 // ---------------------------------------------------------------------------------------------
 static inline bool h16_nonfinite(uint16_t h) { return (h & 0x7C00u) == 0x7C00u; }
 static inline float h16_to_float(uint16_t h) { __half_raw r; r.x = h; return __half2float(__half(r)); }
+// The hit rule: a window hits when its Float16 score > max(thresh[k], 0), and never for a NaN threshold.  Returns the Float16 bits
+// of that effective threshold: 0x7C00 (+Inf) for a NaN threshold, 0 without thresholds.
+static uint16_t hit_threshold(const uint16_t* thresh, int k) {
+    if (!thresh) return 0;
+    const uint16_t raw = thresh[k];
+    if (h16_nonfinite(raw) && (raw & 0x03FFu)) return 0x7C00u;
+    return h16_to_float(raw) > 0.f ? raw : (uint16_t)0;
+}
 
 struct ScanPlan {
     int K = 0, ngroups = 0, K2pad = 0;
@@ -875,10 +883,8 @@ static bool build_tc_plan(const ScanPlan& P, const uint16_t* pwms, const int64_t
                 const uint16_t v = pw(k, b, j);
                 if (h16_nonfinite(v)) { if (v == 0xFC00u) neg_inf = true; else return false; }     // +Inf / NaN entries: leave it to scan_kernel
             }
-        const uint16_t raw = thresh[k];
-        if (h16_nonfinite(raw) && (raw & 0x03FFu)) continue;       // NaN threshold: never a hit
-        if (raw == 0x7C00u) continue;                              // +Inf threshold: never a hit
-        const uint16_t tb = h16_to_float(raw) > 0.f ? raw : (uint16_t)0;
+        const uint16_t tb = hit_threshold(thresh, k);
+        if (tb == 0x7C00u) continue;                               // NaN or +Inf threshold: never a hit
         const double t = (double)h16_to_float(tb);
         if (neg_inf) continue;                                     // a -Inf entry makes every window -Inf or NaN (0 * -Inf): never a hit
         for (int strand = 0; strand < 2; ++strand) {
@@ -1049,13 +1055,7 @@ static int build_plan(mb200_ctx* ctx, const uint16_t* pwms, const int64_t* lens,
                     const int len = (int)lens[k];
                     gm.npos[i] = (int32_t)std::max<int64_t>(0, Lb - len + 1);
                     gm.npos_max = std::max(gm.npos_max, gm.npos[i]);
-                    uint16_t t = 0;
-                    if (thresh) {
-                        const uint16_t raw = thresh[k];
-                        const bool isnan = h16_nonfinite(raw) && (raw & 0x03FFu);
-                        if (isnan) t = 0x7C00u;
-                        else t = h16_to_float(raw) > 0.f ? raw : (uint16_t)0;
-                    }
+                    const uint16_t t = hit_threshold(thresh, k);
                     if (flags & MB200_SCAN_FWD) thr_f = t;
                     if (flags & MB200_SCAN_RC) thr_r = t;
                     P.pair2motif[gg * GROUP_MOTIFS + i] = k;
@@ -1093,630 +1093,672 @@ static int build_plan(mb200_ctx* ctx, const uint16_t* pwms, const int64_t* lens,
     return MB200_OK;
 }
 
-static int32_t scan_impl(mb200_ctx* ctx, const mb200_seqs* seqs, const uint16_t* pwms_f16, const int64_t* lens, int32_t K,
-                         int32_t maxlen, const uint16_t* thresh_f16, uint32_t flags, mb200_hit* hits, int64_t hits_cap,
-                         int64_t* n_hits, int64_t* counts, uint32_t* hist, mb200_best* best, const SpacingJob* sp = nullptr) {
-    if (!ctx) return MB200_E_INVALID;
-    const bool best_mode = best || sp;                 // block keys and best_reduce_kernel; sp: rows are anchor margins in pairs
-    if (!seqs || !pwms_f16 || !lens || K <= 0 || K > 65535 || maxlen <= 0)
-        MB_FAIL(ctx, MB200_E_INVALID, "scan: bad arguments (K=%d maxlen=%d)", K, maxlen);
-    if (!(flags & (MB200_SCAN_FWD | MB200_SCAN_RC))) MB_FAIL(ctx, MB200_E_INVALID, "scan: neither FWD nor RC requested");
-    const bool want_hits = (flags & MB200_SCAN_WANT_HITS) != 0;
-    const bool want_counts = (flags & MB200_SCAN_WANT_COUNTS) != 0;
-    if (want_hits && (!n_hits || (hits_cap > 0 && !hits))) MB_FAIL(ctx, MB200_E_INVALID, "scan: WANT_HITS needs hits/n_hits");
-    if (want_counts && !counts) MB_FAIL(ctx, MB200_E_INVALID, "scan: WANT_COUNTS needs counts");
-    if (seqs->device != ctx->device) MB_FAIL(ctx, MB200_E_INVALID, "scan: sequences live on device %d, ctx on %d", seqs->device, ctx->device);
+// ---- the scan driver: scan_impl runs the stages below; ScanCall holds what they share ----------------------------------------
+
+// What a scan call returns.  Each extern "C" entry point fills one kind; every choice that depends on the mode is made from it.
+struct ScanOut {
+    enum Kind { HITS, HIST, BEST, SPACING };
+    Kind kind = HITS;
+    mb200_hit* hits = nullptr; int64_t hits_cap = 0; int64_t* n_hits = nullptr; int64_t* counts = nullptr;   // HITS: as the flags ask
+    uint32_t* hist = nullptr;              // HIST: K x HIST_BINS
+    mb200_best* best = nullptr;            // BEST: N x K records
+    const SpacingJob* sp = nullptr;        // SPACING
+};
+
+// Appends n bytes (zeros without src) to a host staging image, padded to `align`; returns their offset.
+static size_t put(std::vector<uint8_t>& h, const void* src, size_t n, size_t align = 256) {
+    const size_t off = h.size();
+    h.resize(off + (n + align - 1) / align * align, 0);
+    if (src && n) memcpy(h.data() + off, src, n);
+    return off;
+}
+
+static const unsigned long long TC_CAP = (unsigned long long)24 << 20;     // candidate records per batch and buffer set
+static const int32_t TILE_CHUNKS = 16 * 26;                                  // scan_kernel: position blocks per tile
+
+struct ScanCall {
+    mb200_ctx* ctx; const mb200_seqs* seqs; const ScanOut out; const int K; const uint32_t flags;
+    const bool keys = out.kind == ScanOut::BEST || out.kind == ScanOut::SPACING;     // best keys and best_reduce_kernel, no hit masks
+    const bool want_hits = out.kind == ScanOut::HITS && (flags & MB200_SCAN_WANT_HITS);
+    const bool want_counts = out.kind == ScanOut::HITS && (flags & MB200_SCAN_WANT_COUNTS);
+    const bool reduce = (flags & MB200_SCAN_REDUCE) && ctx->world > 1;                 // sum the totals across ranks
+    int64_t N = 0, Lb = 0, rowwords = 0;
+    int grid = 0;
+    ScanPlan P;
+    TcPlan TP;
+    bool use_tc = false;                   // this and later batches take the tensor-core pre-filter + exact verification (scan_tc.cuh)
+    bool tc_units = false;                 // the verifier lists the (sequence, motif) units that received a hit
+    int32_t W = 0, W16 = 0;                // 32-position mask words and 16-position blocks per sequence
+    size_t mask_bytes_per_seq = 0;
+    int64_t seqs_per_batch = 0;
+    uint32_t* d_mask = nullptr;
+    std::vector<uint8_t> h_plan;           // BUF_PLAN's host copy, alive until the final synchronise
+    const uint8_t* d_blob = nullptr; const MBlock* d_mblocks = nullptr; const MBlock* d_lblocks = nullptr;
+    const int32_t* d_p2m = nullptr; const int32_t* d_plen = nullptr; const EmitMotif* d_em = nullptr;
+    int64_t* d_rng = nullptr; unsigned long long* d_counts = nullptr; unsigned long long* d_total = nullptr;
+    void (*scan_fn)(const ScanArgs) = nullptr;                     // scan_kernel<RAGGED, BEST> of this call
+    int32_t tile_cap_words = 0, blob_cap = 0; size_t smem_bytes = 0;
+    int64_t last_nchunks = -1;
+    // tensor-core path; counters: [0] reserved, [1] overflow, [2] candidates, [3] hits, [4] listed units, [8 + 2c] clocks and
+    // [9 + 2c] tiles of CTA c
+    uint8_t* d_tc = nullptr; const TcSlot* d_tc_slots = nullptr; size_t tc_smem = 0, tc_set_stride = 0, tc_uset_stride = 0;
+    unsigned long long* d_tc_list = nullptr; unsigned long long* d_tc_ctr = nullptr; uint32_t* d_tc_ulist = nullptr; uint32_t* d_tc_ubits = nullptr;
+    unsigned long long tc_stat_cand = 0, tc_stat_hits = 0;
+    uint32_t* d_unit_cnt = nullptr; unsigned long long* d_unit_off = nullptr; unsigned long long* d_bsum = nullptr;   // hit lists
+    int64_t hits_written = 0, hits_needed = 0;
+    unsigned int* d_hist = nullptr;                                                                                   // HIST
+    unsigned long long* d_best64 = nullptr; mb200_best* d_best = nullptr; int32_t best_nch = 0;                       // BEST, SPACING
+    unsigned int* d_sphist = nullptr; const size_t sphist_bytes = out.sp ? (size_t)out.sp->n_primary * K * 4 * (size_t)out.sp->margin * 4 : 0;   // SPACING
+    const mb200_anchor* d_anchors = nullptr; const uint16_t* d_spthr = nullptr; const int32_t* d_mlen = nullptr;
+    size_t next_ready = 0;                 // chunks of a pending asynchronous upload this call has waited for
+    MbTimers tm{ctx}; int t_total = -1;
+    size_t tc_nctr() const { return 8 + 2 * (size_t)grid; }
+    size_t tc_ubits_bytes(int64_t ns) const { return (((size_t)ns * (size_t)(P.K2pad / 2) + 31) / 32) * 4; }
+};
+
+static int scan_validate(ScanCall& S, const uint16_t* pwms, const int64_t* lens, int maxlen) {
+    mb200_ctx* ctx = S.ctx; const ScanOut& o = S.out;
+    if (!S.seqs || !pwms || !lens || S.K <= 0 || S.K > 65535 || maxlen <= 0)
+        MB_FAIL(ctx, MB200_E_INVALID, "scan: bad arguments (K=%d maxlen=%d)", S.K, maxlen);
+    if (!(S.flags & (MB200_SCAN_FWD | MB200_SCAN_RC))) MB_FAIL(ctx, MB200_E_INVALID, "scan: neither FWD nor RC requested");
+    if (S.want_hits && (!o.n_hits || (o.hits_cap > 0 && !o.hits))) MB_FAIL(ctx, MB200_E_INVALID, "scan: WANT_HITS needs hits/n_hits");
+    if (S.want_counts && !o.counts) MB_FAIL(ctx, MB200_E_INVALID, "scan: WANT_COUNTS needs counts");
+    if (S.seqs->device != ctx->device) MB_FAIL(ctx, MB200_E_INVALID, "scan: sequences live on device %d, ctx on %d", S.seqs->device, ctx->device);
     MB_CUDA(ctx, cudaSetDevice(ctx->device));
     mb_reset_timing(ctx);
-    if (n_hits) *n_hits = 0;
+    if (o.n_hits) *o.n_hits = 0;
     ctx->held_hits.clear(); ctx->held_hits.shrink_to_fit();
-    if (counts) memset(counts, 0, sizeof(int64_t) * 4 * (size_t)K);
-    if (hist) memset(hist, 0, (size_t)K * HIST_BINS * 4);
+    if (o.counts) memset(o.counts, 0, sizeof(int64_t) * 4 * (size_t)S.K);
+    if (o.hist) memset(o.hist, 0, (size_t)S.K * HIST_BINS * 4);
+    return MB200_OK;
+}
 
-    const int64_t N = seqs->N, Lb = seqs->Lb, rowwords = seqs->rowwords;
-    const size_t table_budget = 160 * 1024;
-    ScanPlan P;
-    int rc = build_plan(ctx, pwms_f16, lens, K, maxlen, thresh_f16, flags, Lb, table_budget, P);
+static int scan_plan(ScanCall& S, const uint16_t* pwms, const int64_t* lens, int maxlen, const uint16_t* thresh) {
+    mb200_ctx* ctx = S.ctx;
+    S.N = S.seqs->N; S.Lb = S.seqs->Lb; S.rowwords = S.seqs->rowwords; S.grid = ctx->sm_count;
+    int rc = build_plan(ctx, pwms, lens, S.K, maxlen, thresh, S.flags, S.Lb, 160 * 1024, S.P);
     if (rc) return rc;
-    // Thresholded scans take the tensor-core pre-filter + exact verification (scan_tc.cuh) unless the caller or the inputs rule
-    // it out; the hit masks, and everything derived from them, are identical either way.
-    TcPlan TP;
-    bool use_tc = !(flags & MB200_SCAN_NO_TENSOR) && !hist && !best_mode && Lb < (1ll << 31);
-    if (use_tc) use_tc = build_tc_plan(P, pwms_f16, lens, K, thresh_f16, flags, Lb, ctx->sm_count, TP);
+    // Thresholded hit lists and counts take the tensor-core path unless the caller or the inputs rule it out; the hit masks, and
+    // everything derived from them, are identical either way.
+    S.use_tc = S.out.kind == ScanOut::HITS && !(S.flags & MB200_SCAN_NO_TENSOR) && S.Lb < (1ll << 31) &&
+               build_tc_plan(S.P, pwms, lens, S.K, thresh, S.flags, S.Lb, S.grid, S.TP);
     ctx->last_scan_path = 0;
-    if (use_tc) {
+    if (S.use_tc) {
         // start from the clocks per tile measured by the previous scan of this ctx when it had the same block structure
         std::vector<int32_t> sig;
-        for (auto& e : TP.blocks) { sig.push_back(e.nsub); sig.push_back(e.kchunks[0]); sig.push_back(e.kchunks[1]); }
-        if (sig == ctx->tc_cost_sig && ctx->tc_cost.size() == TP.blocks.size()) { TP.cost = ctx->tc_cost; tc_assign_ctas(TP.blocks, TP.cost, ctx->sm_count); }
+        for (auto& e : S.TP.blocks) { sig.push_back(e.nsub); sig.push_back(e.kchunks[0]); sig.push_back(e.kchunks[1]); }
+        if (sig == ctx->tc_cost_sig && ctx->tc_cost.size() == S.TP.blocks.size()) { S.TP.cost = ctx->tc_cost; tc_assign_ctas(S.TP.blocks, S.TP.cost, S.grid); }
         else { ctx->tc_cost_sig = sig; ctx->tc_cost.clear(); }
     }
-    const int64_t npos_max = Lb - P.minlen + 1;
-    const bool reduce = (flags & MB200_SCAN_REDUCE) != 0 && ctx->world > 1;
-    if (N == 0 || npos_max <= 0) {                      // nothing can be scored on this rank; it still takes part in the reduction
-        if (best) {                                     // no row holds a window (otherwise every batch writes all its records)
-            const mb200_best none = {0xFFFFFFFFu, 0, 0, 0};
-            std::fill(best, best + (size_t)N * K, none);
-        }
-        if (sp) {                                       // every secondary is longer than the margin
-            const mb200_best none = {0xFFFFFFFFu, 0, 0, 0};
-            memset(sp->hist, 0, (size_t)sp->n_primary * K * 4 * sp->margin * 4);
-            if (sp->sites) std::fill(sp->sites, sp->sites + (size_t)sp->n * K, none);
-        }
-        if (reduce && (want_counts || hist)) {
-            const size_t nb = hist ? (size_t)K * HIST_BINS * 4 : (size_t)K * 4 * 8;
-            rc = mb_ensure_scratch(ctx, nb); if (rc) return rc;
-            MB_CUDA(ctx, cudaMemsetAsync(ctx->scratch, 0, nb, ctx->stream));
-            if (want_counts) { rc = mb_comm_allreduce_u64(ctx, (unsigned long long*)ctx->scratch, (size_t)K * 4); if (rc) return rc;
-                               MB_CUDA(ctx, cudaMemcpyAsync(counts, ctx->scratch, (size_t)K * 4 * 8, cudaMemcpyDeviceToHost, ctx->stream)); }
-            if (hist) { rc = mb_comm_allreduce_u32(ctx, (unsigned int*)ctx->scratch, (size_t)K * HIST_BINS); if (rc) return rc;
-                        MB_CUDA(ctx, cudaMemcpyAsync(hist, ctx->scratch, (size_t)K * HIST_BINS * 4, cudaMemcpyDeviceToHost, ctx->stream)); }
-            MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-        }
-        return MB200_OK;
-    }
-    const int64_t W64 = (npos_max + 31) / 32;                      // 32-position mask words per sequence
-    if (W64 > 0x1fffffff) MB_FAIL(ctx, MB200_E_UNSUPPORTED, "sequence too long");
-    const int32_t W = (int32_t)W64;
-    const int32_t W16 = 2 * W;                                     // 16-position blocks per sequence (two per mask word)
-
-    // ---- device buffers -------------------------------------------------------------------
-    // buf 1: plan (blob, mblocks, pair tables, emit table, cta ranges, counts)
-    const size_t off_blob = 0;
-    const size_t off_mb = (P.blob.size() + 255) & ~(size_t)255;
-    const size_t off_lb = off_mb + ((P.mblocks.size() * sizeof(MBlock) + 255) & ~(size_t)255);
-    const size_t off_p2m = off_lb + ((P.lblocks.size() * sizeof(MBlock) + 255) & ~(size_t)255);
-    const size_t off_plen = off_p2m + ((P.pair2motif.size() * 4 + 255) & ~(size_t)255);
-    const size_t off_em = off_plen + ((P.pairlen.size() * 4 + 255) & ~(size_t)255);
-    const size_t off_rng = off_em + ((P.em.size() * sizeof(EmitMotif) + 255) & ~(size_t)255);
-    const int grid = ctx->sm_count;
-    const size_t off_cnt = off_rng + (((size_t)(grid + 1) * 8 + 255) & ~(size_t)255);
-    const size_t off_tot = off_cnt + (((size_t)K * 4 * 8 + 255) & ~(size_t)255);
-    const size_t plan_bytes = off_tot + 256;
-    rc = mb_ensure_buf(ctx, 1, plan_bytes); if (rc) return rc;
-    uint8_t* d_plan = (uint8_t*)ctx->bufs[1];
-    std::vector<uint8_t> h_plan(plan_bytes, 0);
-    memcpy(h_plan.data() + off_blob, P.blob.data(), P.blob.size());
-    memcpy(h_plan.data() + off_mb, P.mblocks.data(), P.mblocks.size() * sizeof(MBlock));
-    memcpy(h_plan.data() + off_lb, P.lblocks.data(), P.lblocks.size() * sizeof(MBlock));
-    memcpy(h_plan.data() + off_p2m, P.pair2motif.data(), P.pair2motif.size() * 4);
-    memcpy(h_plan.data() + off_plen, P.pairlen.data(), P.pairlen.size() * 4);
-    memcpy(h_plan.data() + off_em, P.em.data(), P.em.size() * sizeof(EmitMotif));
-
-    // ---- batching: masks of one batch stay under a budget -----------------------------------
-    const size_t mask_budget = (size_t)8 << 30;
-    const size_t mask_bytes_per_seq = (size_t)W * P.K2pad * 4 * (best_mode ? 2 : 1);      // best sites: one 32-bit key per 16-position block
-    int64_t seqs_per_batch = std::max<int64_t>(1, (int64_t)(mask_budget / mask_bytes_per_seq));
-    if (seqs_per_batch > N) seqs_per_batch = N;
-    if ((double)seqs_per_batch * W > 2.0e9) seqs_per_batch = std::max<int64_t>(1, (int64_t)(2.0e9 / W));
-    if (sp) seqs_per_batch = std::max<int64_t>(2, seqs_per_batch & ~(int64_t)1);    // both margins of an anchor in one batch (N is even)
-    if (use_tc && (double)seqs_per_batch * (double)Lb > 2.0e9) seqs_per_batch = std::max<int64_t>(1, (int64_t)(2.0e9 / (double)Lb));   // 32-bit virtual positions
-    // tensor-core path: plan (B operands, blocks, slots) in buf 8, candidate list + counters in buf 9
-    const unsigned long long tc_cap = (unsigned long long)24 << 20;      // candidate records per batch and buffer set
-    const bool tc_sparse = !want_hits && !hist && W <= 4096;        // counts only: count the units the verifier lists, never walk (or clear) the whole mask
-    const bool tc_units = !hist && W <= 4096;                       // the verifier lists the (sequence, motif) units that received a hit (also for hit lists)
-    size_t tc_off_blocks = 0, tc_off_slots = 0, tc_smem = 0, tc_set_stride = 0, tc_uset_stride = 0;      // strides between the two buffer sets of the pipelined path
-    uint8_t* d_tc = nullptr; unsigned long long* d_tc_list = nullptr; unsigned long long* d_tc_ctr = nullptr;     // ctr: [0] reserved, [1] overflow, [2] candidates, [3] hits, [4] listed units, [8..] clocks per CTA
-    uint32_t* d_tc_ulist = nullptr; uint32_t* d_tc_ubits = nullptr; unsigned long long tc_stat_cand = 0, tc_stat_hits = 0;
-    if (use_tc) {
-        tc_off_blocks = (TP.blob.size() + 255) & ~(size_t)255;
-        tc_off_slots = tc_off_blocks + ((TP.blocks.size() * sizeof(TcBlock) + 255) & ~(size_t)255);
-        const size_t tc_bytes = tc_off_slots + TP.slots.size() * sizeof(TcSlot);
-        rc = mb_ensure_buf(ctx, 8, tc_bytes); if (rc) return rc;
-        const size_t tc_set_bytes = (((size_t)tc_cap * 8 + (size_t)(8 + 2 * ctx->sm_count) * 8) + 255) & ~(size_t)255;     // list + counters
-        rc = mb_ensure_buf(ctx, 9, 2 * tc_set_bytes); if (rc) return rc;
-        d_tc = (uint8_t*)ctx->bufs[8];
-        d_tc_list = (unsigned long long*)ctx->bufs[9];
-        d_tc_ctr = d_tc_list + tc_cap;
-        // (sequence, motif) units with hits: list + bitmap (buf 10), for the sparse counting kernel
-        const size_t ubits_bytes = (((size_t)seqs_per_batch * (size_t)(P.K2pad / 2) + 31) / 32) * 4 + 256;
-        const size_t tc_uset_bytes = (((size_t)tc_cap * 4 + ubits_bytes) + 255) & ~(size_t)255;
-        rc = mb_ensure_buf(ctx, 10, 2 * tc_uset_bytes); if (rc) return rc;
-        d_tc_ulist = (uint32_t*)ctx->bufs[10];
-        d_tc_ubits = d_tc_ulist + tc_cap;
-        tc_set_stride = tc_set_bytes; tc_uset_stride = tc_uset_bytes;
-        std::vector<uint8_t> h_tc(tc_bytes, 0);
-        memcpy(h_tc.data(), TP.blob.data(), TP.blob.size());
-        memcpy(h_tc.data() + tc_off_blocks, TP.blocks.data(), TP.blocks.size() * sizeof(TcBlock));
-        memcpy(h_tc.data() + tc_off_slots, TP.slots.data(), TP.slots.size() * sizeof(TcSlot));
-        MB_CUDA(ctx, cudaMemcpyAsync(d_tc, h_tc.data(), tc_bytes, cudaMemcpyHostToDevice, ctx->stream));
-        MB_CUDA(ctx, cudaMemsetAsync(d_tc_ctr, 0, (size_t)(8 + 2 * ctx->sm_count) * 8, ctx->stream));
-        MB_CUDA(ctx, cudaMemsetAsync((uint8_t*)d_tc_ctr + tc_set_stride, 0, (size_t)(8 + 2 * ctx->sm_count) * 8, ctx->stream));
-        MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));           // h_tc goes out of scope
-        // at least half of the shared memory: one CTA per SM (each CTA allocates all 512 TMEM columns)
-        tc_smem = std::max<size_t>((size_t)TCS_STAGES * TCS_STAGE_BYTES + TP.max_b_bytes, (size_t)120 * 1024);
-        if (tc_smem > ctx->smem_optin) use_tc = false;
-        else MB_CUDA(ctx, cudaFuncSetAttribute(k_scan_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc_smem));
-    }
-    rc = mb_ensure_buf(ctx, 2, (size_t)seqs_per_batch * mask_bytes_per_seq); if (rc) return rc;
-    uint32_t* d_mask = (uint32_t*)ctx->bufs[2];
-    uint32_t* d_unit_cnt = nullptr; unsigned long long* d_unit_off = nullptr; unsigned long long* d_bsum = nullptr;
-    int64_t units_per_batch = seqs_per_batch * K * 2;
-    int64_t ps_blocks = (units_per_batch + PS_TILE - 1) / PS_TILE;
-    unsigned long long* d_best64 = nullptr; mb200_best* d_best = nullptr;
-    const int32_t best_nch = (W16 + BEST_CHUNK - 1) / BEST_CHUNK;
-    if (best_mode) {                                    // per batch: 64-bit best keys, then the records (spacing: the sites)
-        rc = mb_ensure_buf(ctx, 3, (size_t)seqs_per_batch * K * 16); if (rc) return rc;
-        d_best64 = (unsigned long long*)ctx->bufs[3];
-        d_best = (mb200_best*)(d_best64 + (size_t)seqs_per_batch * K);
-    }
-    // spacing: the histogram (buf 0) and the anchors, thresholds and secondary lengths (buf 11)
-    unsigned int* d_sphist = nullptr; const mb200_anchor* d_anchors = nullptr; const uint16_t* d_spthr = nullptr; const int32_t* d_mlen = nullptr;
-    const size_t sphist_bytes = sp ? (size_t)sp->n_primary * K * 4 * (size_t)sp->margin * 4 : 0;
-    if (sp) {
-        rc = mb_ensure_buf(ctx, 0, sphist_bytes); if (rc) return rc;
-        d_sphist = (unsigned int*)ctx->bufs[0];
-        const size_t off_thr = ((size_t)sp->n * sizeof(mb200_anchor) + 255) & ~(size_t)255;
-        const size_t off_len = off_thr + (((size_t)K * 2 + 255) & ~(size_t)255);
-        const size_t bytes = off_len + (size_t)K * 4;
-        rc = mb_ensure_buf(ctx, 11, bytes); if (rc) return rc;
-        std::vector<uint8_t> h(bytes, 0);
-        memcpy(h.data(), sp->anchors, (size_t)sp->n * sizeof(mb200_anchor));
-        uint16_t* ht = reinterpret_cast<uint16_t*>(h.data() + off_thr);
-        int32_t* hl = reinterpret_cast<int32_t*>(h.data() + off_len);
-        for (int k = 0; k < K; ++k) {                   // the hit rule of build_plan: score > max(thresh, 0), never for a NaN threshold
-            uint16_t t = 0;
-            if (sp->thresh) {
-                const uint16_t raw = sp->thresh[k];
-                t = (h16_nonfinite(raw) && (raw & 0x03FFu)) ? (uint16_t)0x7C00u : h16_to_float(raw) > 0.f ? raw : (uint16_t)0;
-            }
-            ht[k] = t; hl[k] = (int32_t)lens[k];
-        }
-        uint8_t* d = (uint8_t*)ctx->bufs[11];
-        MB_CUDA(ctx, cudaMemcpyAsync(d, h.data(), bytes, cudaMemcpyHostToDevice, ctx->stream));
-        MB_CUDA(ctx, cudaMemsetAsync(d_sphist, 0, sphist_bytes, ctx->stream));
-        MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));         // h goes out of scope
-        d_anchors = (const mb200_anchor*)d; d_spthr = (const uint16_t*)(d + off_thr); d_mlen = (const int32_t*)(d + off_len);
-    }
-    if (want_hits) {
-        size_t b = (((size_t)units_per_batch * 4 + 255) & ~(size_t)255) + (((size_t)units_per_batch * 8 + 255) & ~(size_t)255) +
-                   (size_t)ps_blocks * 8 + 256;
-        rc = mb_ensure_buf(ctx, 3, b); if (rc) return rc;
-        d_unit_cnt = (uint32_t*)ctx->bufs[3];
-        d_unit_off = (unsigned long long*)((uint8_t*)ctx->bufs[3] + (((size_t)units_per_batch * 4 + 255) & ~(size_t)255));
-        d_bsum = (unsigned long long*)((uint8_t*)d_unit_off + (((size_t)units_per_batch * 8 + 255) & ~(size_t)255));
-    }
-
-    // ---- tiling and per-CTA pair ranges (balanced by column count of the motif block) --------
-    const int32_t tile_chunks = 16 * 26;                           // position blocks per tile
-    auto tiles_of = [&](int64_t nchunks) { return (nchunks + tile_chunks - 1) / tile_chunks; };
-    // words spanned by a tile: +1 per block inside a sequence, + (rowwords - W16 + 1) when crossing to the next sequence
-    const int64_t crossings = (tile_chunks - 1) / W16 + 1;
-    const int64_t gap = std::max<int64_t>(0, rowwords - (int64_t)W16 + 1);
-    const int32_t tile_cap_words = (int32_t)(((int64_t)tile_chunks + crossings * gap + 6 + 4 + 3) & ~(int64_t)3);
-    const int32_t blob_cap = (P.max_blob_bytes + 127) & ~127;
-    const size_t smem_bytes = (size_t)blob_cap + (size_t)tile_cap_words * 8 + 64;
-    if (smem_bytes > ctx->smem_optin) MB_FAIL(ctx, MB200_E_UNSUPPORTED, "scan needs %zu B shared memory (> %zu)", smem_bytes, ctx->smem_optin);
-    const bool ragged = seqs->lens != nullptr;
-    if (best_mode) MB_CUDA(ctx, cudaFuncSetAttribute(ragged ? scan_kernel<true, true> : scan_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
-    else MB_CUDA(ctx, cudaFuncSetAttribute(ragged ? scan_kernel<true> : scan_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
-
-    MbTimers tm(ctx);
-    const int t_total = tm.begin(T_TOTAL);
-    int th = tm.begin(T_H2D);
-    MB_CUDA(ctx, cudaMemcpyAsync(d_plan, h_plan.data(), plan_bytes, cudaMemcpyHostToDevice, ctx->stream));
-    tm.end(th);
-    unsigned long long* d_counts = (unsigned long long*)(d_plan + off_cnt);
-    unsigned long long* d_total = (unsigned long long*)(d_plan + off_tot);
-    int64_t* d_rng = (int64_t*)(d_plan + off_rng);
-
-    unsigned int* d_hist = nullptr;
-    if (hist) {
-        rc = mb_ensure_buf(ctx, 0, (size_t)K * HIST_BINS * 4); if (rc) return rc;
-        d_hist = (unsigned int*)ctx->bufs[0];
-        MB_CUDA(ctx, cudaMemsetAsync(d_hist, 0, (size_t)K * HIST_BINS * 4, ctx->stream));
-    }
-    int64_t hits_written = 0, hits_needed = 0;
-    std::vector<int64_t> h_rng(grid + 1);
-    int64_t last_nchunks = -1;
-    size_t next_ready = 0;                                         // chunks of a pending asynchronous upload this scan has waited for
-    std::vector<int64_t> todo;                                     // first sequences of the batches the loop below still has to do
-    for (int64_t s0 = 0; s0 < N; s0 += seqs_per_batch) todo.push_back(s0);
-
-    // ---- counts-only thresholded scans: pipelined tensor-core path.  The pre-filter of batch i+1 (ctx->stream) runs while batch i is
-    //      re-scored and counted on ctx->aux_stream; two sets of list / counter / unit buffers alternate.  The host looks at batch i's
-    //      counters (overflow, clocks for the re-balancing) while batch i+1 is already running, so the GPU never waits for it. ----
-    if (use_tc && tc_sparse) {
-        if (!ctx->aux_stream && cudaStreamCreateWithFlags(&ctx->aux_stream, cudaStreamNonBlocking) != cudaSuccess) MB_FAIL(ctx, MB200_E_CUDA, "scan: cannot create the auxiliary stream");
-        cudaStream_t aux = ctx->aux_stream;
-        const size_t nctr = 8 + 2 * (size_t)grid;
-        rc = mb_ensure_pinned(ctx, 2 * nctr * 8); if (rc) return rc;
-        unsigned long long* h_ctr2 = (unsigned long long*)ctx->pinned;
-        struct EvGuard {                                            // the events are destroyed on every way out of this block (error returns included)
-            cudaEvent_t tc[2] = {nullptr, nullptr}, aux[2] = {nullptr, nullptr};
-            ~EvGuard() { for (int b = 0; b < 2; ++b) { if (tc[b]) cudaEventDestroy(tc[b]); if (aux[b]) cudaEventDestroy(aux[b]); } }
-        } evg;
-        cudaEvent_t* ev_tc = evg.tc; cudaEvent_t* ev_aux = evg.aux;
-        for (int b = 0; b < 2; ++b) { MB_CUDA(ctx, cudaEventCreateWithFlags(&ev_tc[b], cudaEventDisableTiming)); MB_CUDA(ctx, cudaEventCreateWithFlags(&ev_aux[b], cudaEventDisableTiming)); }
-        const int nb = (int)todo.size();
-        std::vector<char> launched(nb, 0), failed(nb, 0);
-        bool overflowed = false;
-        // batch j's counters: statistics, overflow, measured clocks per tile -> CTA split of the next launch
-        auto process = [&](int j) -> int {
-            if (cudaEventSynchronize(ev_aux[j & 1]) != cudaSuccess) return MB200_E_CUDA;
-            const unsigned long long* h = h_ctr2 + (size_t)(j & 1) * nctr;
-            if (h[1]) { failed[j] = 1; overflowed = true; return MB200_OK; }
-            tc_stat_cand += h[2]; tc_stat_hits += h[3];
-            std::vector<double> cost(TP.blocks.size(), 0.0);
-            bool ok = true;
-            for (size_t bi = 0; bi < TP.blocks.size(); ++bi) {
-                double clk = 0, tiles = 0;
-                for (int c = TP.blocks[bi].cta0; c < TP.blocks[bi].cta0 + TP.blocks[bi].nctas; ++c) { clk += (double)h[8 + 2 * c]; tiles += (double)h[8 + 2 * c + 1]; }
-                if (tiles <= 0 || clk <= 0) { ok = false; break; }
-                cost[bi] = clk / tiles;
-            }
-            if (ok) ctx->tc_cost = cost;
-            if (ok) tc_assign_ctas(TP.blocks, cost, grid);          // the next launch carries the new split in its parameters
-            return MB200_OK;
-        };
-        int i = 0;
-        for (; i < nb && !overflowed; ++i) {
-            const int64_t s0 = todo[i];
-            const int64_t ns = std::min(seqs_per_batch, N - s0);
-            if (seqs->pending) {
-                while (next_ready < seqs->ready.size() && (next_ready == 0 || seqs->ready_end[next_ready - 1] < s0 + ns)) {
-                    MB_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, seqs->ready[next_ready], 0));
-                    ++next_ready;
-                }
-            }
-            const int b = i & 1;
-            unsigned long long* list_b = (unsigned long long*)((uint8_t*)d_tc_list + (size_t)b * tc_set_stride);
-            unsigned long long* ctr_b = list_b + tc_cap;
-            uint32_t* ulist_b = (uint32_t*)((uint8_t*)d_tc_ulist + (size_t)b * tc_uset_stride);
-            uint32_t* ubits_b = ulist_b + tc_cap;
-            const size_t need = (size_t)ns * mask_bytes_per_seq;
-            if (ctx->mask_clean_bytes < need) {
-                MB_CUDA(ctx, cudaMemsetAsync(d_mask, 0, need, ctx->stream));
-                ctx->mask_clean_bytes = need;
-            }
-            MB_CUDA(ctx, cudaMemsetAsync(ctr_b, 0, 64, ctx->stream));
-            TcArgs ta;
-            ta.seqw = seqs->words; ta.rowwords = rowwords; ta.seq0 = s0; ta.lens = seqs->lens;
-            ta.Lb = (uint32_t)Lb; ta.vtotal = (uint32_t)(ns * Lb);
-            ta.blob = d_tc; ta.nblocks = (int32_t)TP.blocks.size();
-            memset(ta.blocks, 0, sizeof ta.blocks); memcpy(ta.blocks, TP.blocks.data(), TP.blocks.size() * sizeof(TcBlock));
-            ta.slots = (const TcSlot*)(d_tc + tc_off_slots);
-            ta.list = list_b; ta.cap = tc_cap; ta.gcount = ctr_b; ta.overflow = (uint32_t*)(ctr_b + 1);
-            ta.ntiles = (int32_t)((ns * Lb + 255) / 256);
-            ta.clocks = (long long*)(ctr_b + 8);
-            ta.dbg = nullptr;
-#if TCS_PROFILE
-            static long long* d_dbg2 = nullptr;
-            if (getenv("MB200_SCAN_TC_DEBUG") && i == atoi(getenv("MB200_SCAN_TC_DEBUG"))) {
-                if (!d_dbg2) MB_CUDA(ctx, cudaMalloc(&d_dbg2, (size_t)grid * 8 * 8));
-                MB_CUDA(ctx, cudaMemsetAsync(d_dbg2, 0, (size_t)grid * 8 * 8, ctx->stream)); ta.dbg = d_dbg2;
-            }
-#endif
-            const int t_tc = tm.begin(T_SCAN);
-            k_scan_tc<<<grid, TCS_THREADS, tc_smem, ctx->stream>>>(ta);
-            tm.end(t_tc);
-            MB_CUDA(ctx, cudaGetLastError());
-            MB_CUDA(ctx, cudaEventRecord(ev_tc[b], ctx->stream));
-            MB_CUDA(ctx, cudaStreamWaitEvent(aux, ev_tc[b], 0));
-            MB_CUDA(ctx, cudaMemsetAsync(ubits_b, 0, (((size_t)ns * (size_t)(P.K2pad / 2) + 31) / 32) * 4, aux));
-            const int t_vf = tm.begin_on(T_EMIT, aux);
-            // 128-thread blocks: next to a k_scan_tc CTA (608 threads x 96 registers) an SM has ~7 K registers left
-            k_scan_tc_verify<<<grid * 16, 128, 0, aux>>>(list_b, ctr_b, tc_cap, ta.slots, (const EmitMotif*)(d_plan + off_em), d_plan + off_blob,
-                                                        seqs->words, rowwords, s0, (uint32_t)Lb, W, P.K2pad, d_mask, ctr_b + 2, ubits_b, ulist_b, ctr_b + 4, seqs->lens);
-            tm.end_on(t_vf, aux);
-            const int t_ct = tm.begin_on(T_COUNT, aux);
-            count_listed_kernel<<<grid * 16, 128, 0, aux>>>(d_mask, ulist_b, ctr_b + 4, W, P.K2pad, (const int32_t*)(d_plan + off_p2m),
-                                                           (const int32_t*)(d_plan + off_plen), d_counts, ctr_b + 1, nullptr, 0, 1);
-            tm.end_on(t_ct, aux);
-            MB_CUDA(ctx, cudaGetLastError());
-            MB_CUDA(ctx, cudaMemcpyAsync(h_ctr2 + (size_t)b * nctr, ctr_b, nctr * 8, cudaMemcpyDeviceToHost, aux));
-            MB_CUDA(ctx, cudaEventRecord(ev_aux[b], aux));
-            ctx->launches[T_SCAN] += 1; ctx->launches[T_EMIT] += 1; ctx->launches[T_COUNT] += 1;
-            launched[i] = 1;
-#if TCS_PROFILE
-            if (ta.dbg) {
-                std::vector<long long> h((size_t)grid * 8);
-                cudaStreamSynchronize(ctx->stream);
-                cudaMemcpy(h.data(), ta.dbg, (size_t)grid * 8 * 8, cudaMemcpyDeviceToHost);
-                for (int c = 0; c < grid; c += 1)
-                    fprintf(stderr, "[tcdbg] cta %3d blk %lld tiles %lld | mma total %9lld wait_full %9lld wait_acc %9lld | epi total %9lld wait %9lld | prod wait %9lld\n", c, h[c * 8 + 6], h[c * 8 + 7],
-                            h[c * 8 + 0], h[c * 8 + 1], h[c * 8 + 2], h[c * 8 + 4], h[c * 8 + 3], h[c * 8 + 5]);
-            }
-#endif
-            if (i >= 1) { rc = process(i - 1); if (rc) return rc; }
-        }
-        const int n_launched = i;
-        // every batch but the last launched one was looked at inside the loop
-        if (n_launched > 0) { rc = process(n_launched - 1); if (rc) return rc; }
-        MB_CUDA(ctx, cudaStreamSynchronize(aux));
-        std::vector<int64_t> rest;
-        for (int j = 0; j < nb; ++j) if (!launched[j] || failed[j]) rest.push_back(todo[j]);
-        todo.swap(rest);
-        if (overflowed) { use_tc = false; ctx->last_scan_path = 2; ctx->mask_clean_bytes = 0; }     // a failed batch may have left bits behind (its count was skipped)
-        else ctx->last_scan_path = 1;
-    }
-
-    for (size_t ti = 0; ti < todo.size(); ++ti) {
-        const int64_t s0 = todo[ti];
-        const int64_t ns = std::min(seqs_per_batch, N - s0);
-        if (seqs->pending) {
-            // a batch may start as soon as the chunks holding its sequences are packed (the kernel reads a few words past its last
-            // sequence: in bounds, and whatever they hold only reaches positions that are masked out)
-            while (next_ready < seqs->ready.size() && (next_ready == 0 || seqs->ready_end[next_ready - 1] < s0 + ns)) {
-                MB_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, seqs->ready[next_ready], 0));
-                ++next_ready;
-            }
-        }
-        const int64_t nchunks = ns * (int64_t)W16;
-        const int64_t ntiles = tiles_of(nchunks);
-        if (nchunks != last_nchunks) {
-            // weighted contiguous split of pairs (mblock-major) over CTAs
-            double total_cost = 0;
-            for (auto& mb : P.mblocks) total_cost += (double)mb.cost * (double)ntiles;
-            size_t mbi = 0; double acc = 0; int64_t q = 0;
-            h_rng[0] = 0;
-            for (int b = 1; b <= grid; ++b) {
-                const double target = total_cost * b / grid;
-                while (mbi < P.mblocks.size()) {
-                    const double c = (double)P.mblocks[mbi].cost;
-                    const int64_t qend = (int64_t)(mbi + 1) * ntiles;
-                    int64_t take = (int64_t)((target - acc) / c + 0.5);
-                    if (take < 0) take = 0;
-                    if (q + take >= qend) { acc += (double)(qend - q) * c; q = qend; ++mbi; }
-                    else { acc += (double)take * c; q += take; break; }
-                }
-                h_rng[b] = (b == grid) ? (int64_t)P.mblocks.size() * ntiles : q;
-            }
-            MB_CUDA(ctx, cudaMemcpyAsync(d_rng, h_rng.data(), (size_t)(grid + 1) * 8, cudaMemcpyHostToDevice, ctx->stream));
-            MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));   // h_rng is reused by the next batch shape
-            last_nchunks = nchunks;
-        }
-        ScanArgs a;
-        a.seqw = seqs->words; a.rowwords = rowwords; a.W = W16;
-        a.chunk0 = s0 * (int64_t)W16; a.nchunks = nchunks;
-        a.mask = d_mask; a.K2pad = P.K2pad;
-        a.blob = d_plan + off_blob; a.mblocks = (const MBlock*)(d_plan + off_mb); a.n_mblocks = (int32_t)P.mblocks.size();
-        a.tile_chunks = tile_chunks; a.ntiles = ntiles; a.tile_cap_words = tile_cap_words; a.blob_cap_bytes = blob_cap;
-        a.cta_range = d_rng;
-        a.lens = seqs->lens; a.Lb = Lb;
-        bool tc_done = false;
-        if (use_tc) {
-            const size_t need = (size_t)ns * mask_bytes_per_seq;
-            if (ctx->mask_clean_bytes < need) {                      // the buffer is kept all-zero between tensor-core batches (count_listed_kernel clears what it reads)
-                MB_CUDA(ctx, cudaMemsetAsync(d_mask, 0, need, ctx->stream));
-                ctx->mask_clean_bytes = need;
-            }
-            MB_CUDA(ctx, cudaMemsetAsync(d_tc_ctr, 0, 64, ctx->stream));
-            if (tc_units) MB_CUDA(ctx, cudaMemsetAsync(d_tc_ubits, 0, (((size_t)ns * (size_t)(P.K2pad / 2) + 31) / 32) * 4, ctx->stream));
-            TcArgs ta;
-            ta.seqw = seqs->words; ta.rowwords = rowwords; ta.seq0 = s0; ta.lens = seqs->lens;
-            ta.Lb = (uint32_t)Lb; ta.vtotal = (uint32_t)(ns * Lb);
-            ta.blob = d_tc; ta.nblocks = (int32_t)TP.blocks.size();
-            memset(ta.blocks, 0, sizeof ta.blocks); memcpy(ta.blocks, TP.blocks.data(), TP.blocks.size() * sizeof(TcBlock));
-            ta.slots = (const TcSlot*)(d_tc + tc_off_slots);
-            ta.list = d_tc_list; ta.cap = tc_cap; ta.gcount = d_tc_ctr; ta.overflow = (uint32_t*)(d_tc_ctr + 1);
-            ta.ntiles = (int32_t)((ns * Lb + 255) / 256);
-            ta.clocks = (long long*)(d_tc_ctr + 8);
-            ta.dbg = nullptr;
-#if TCS_PROFILE
-            static long long* d_dbg = nullptr;
-            if (getenv("MB200_SCAN_TC_DEBUG")) { if (!d_dbg) MB_CUDA(ctx, cudaMalloc(&d_dbg, (size_t)grid * 8 * 8)); MB_CUDA(ctx, cudaMemset(d_dbg, 0, (size_t)grid * 8 * 8)); ta.dbg = d_dbg; }
-#endif
-            const int t_tc = tm.begin(T_SCAN);
-            k_scan_tc<<<grid, TCS_THREADS, tc_smem, ctx->stream>>>(ta);
-            tm.end(t_tc);
-            const int t_vf = tm.begin(T_EMIT);
-            k_scan_tc_verify<<<grid * 8, 256, 0, ctx->stream>>>(d_tc_list, d_tc_ctr, tc_cap, ta.slots, (const EmitMotif*)(d_plan + off_em), d_plan + off_blob,
-                                                                 seqs->words, rowwords, s0, (uint32_t)Lb, W, P.K2pad, d_mask, d_tc_ctr + 2,
-                                                                 tc_units ? d_tc_ubits : nullptr, d_tc_ulist, d_tc_ctr + 4, seqs->lens);
-            tm.end(t_vf);
-            ctx->launches[T_SCAN] += 1; ctx->launches[T_EMIT] += 1;
-            MB_CUDA(ctx, cudaGetLastError());
-            std::vector<unsigned long long> h_ctr(8 + 2 * (size_t)grid, 0);
-            MB_CUDA(ctx, cudaMemcpyAsync(h_ctr.data(), d_tc_ctr, h_ctr.size() * 8, cudaMemcpyDeviceToHost, ctx->stream));
-            MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-#if TCS_PROFILE
-            if (ta.dbg && s0 / seqs_per_batch == atoi(getenv("MB200_SCAN_TC_DEBUG"))) {
-                std::vector<long long> h((size_t)grid * 8);
-                cudaMemcpy(h.data(), ta.dbg, (size_t)grid * 8 * 8, cudaMemcpyDeviceToHost);
-                for (int c = 0; c < grid; c += 1)
-                    fprintf(stderr, "[tcdbg] cta %3d blk %lld tiles %lld | mma total %9lld wait_full %9lld wait_acc %9lld | epi total %9lld wait %9lld | prod wait %9lld\n", c, h[c * 8 + 6], h[c * 8 + 7],
-                            h[c * 8 + 0], h[c * 8 + 1], h[c * 8 + 2], h[c * 8 + 4], h[c * 8 + 3], h[c * 8 + 5]);
-            }
-#endif
-            if (!h_ctr[1]) {
-                // re-balance the CTAs over the slot blocks with the clocks per tile this batch measured (the epilogue's share depends on
-                // the candidate density of the block, which no static model knows)
-                std::vector<double> cost(TP.blocks.size(), 0.0);
-                bool ok = true;
-                for (size_t bi = 0; bi < TP.blocks.size(); ++bi) {
-                    double clk = 0, tiles = 0;
-                    for (int c = TP.blocks[bi].cta0; c < TP.blocks[bi].cta0 + TP.blocks[bi].nctas; ++c) { clk += (double)h_ctr[8 + 2 * c]; tiles += (double)h_ctr[8 + 2 * c + 1]; }
-                    if (tiles <= 0 || clk <= 0) { ok = false; break; }
-                    cost[bi] = clk / tiles;
-                }
-                if (ok) ctx->tc_cost = cost;
-                if (ok) tc_assign_ctas(TP.blocks, cost, grid);
-            }
-            tc_stat_cand += h_ctr[2]; tc_stat_hits += h_ctr[3];
-            ctx->mask_clean_bytes = 0;                               // the verifier has set bits (re-established below when the sparse count clears them)
-            if (h_ctr[1]) { use_tc = false; ctx->last_scan_path = 2; }   // candidate list overflowed (thresholds too permissive): this and later batches take scan_kernel
-            else { tc_done = true; if (ctx->last_scan_path == 0) ctx->last_scan_path = 1; }
-        }
-        if (tc_done) { /* masks are complete */ }
-        else {
-        int t1 = tm.begin(T_SCAN);
-        ctx->mask_clean_bytes = 0;
-        if (!P.mblocks.empty()) {
-            if (best_mode) {
-                if (ragged) scan_kernel<true, true><<<grid, SCAN_THREADS, smem_bytes, ctx->stream>>>(a);
-                else scan_kernel<false, true><<<grid, SCAN_THREADS, smem_bytes, ctx->stream>>>(a);
-            } else {
-                if (ragged) scan_kernel<true><<<grid, SCAN_THREADS, smem_bytes, ctx->stream>>>(a);
-                else scan_kernel<false><<<grid, SCAN_THREADS, smem_bytes, ctx->stream>>>(a);
-            }
-            ctx->launches[T_SCAN] += 1;
-        }
-        if (!P.lblocks.empty()) {
-            const int64_t warps = ns * (int64_t)P.lblocks.size() * GROUP_SLOTS;
-            auto long_kernel = best_mode ? scan_long_kernel<true> : scan_long_kernel<false>;
-            long_kernel<<<(unsigned)((warps * 32 + 255) / 256), 256, 0, ctx->stream>>>(seqs->words, rowwords, s0, ns, W, P.K2pad, d_plan + off_blob,
-                                                                                   (const MBlock*)(d_plan + off_lb), (int32_t)P.lblocks.size(), d_mask,
-                                                                                   seqs->lens, Lb);
-            ctx->launches[T_SCAN] += 1;
-        }
-        tm.end(t1);
-        }
-        MB_CUDA(ctx, cudaGetLastError());
-
-        if (best_mode) {
-            const int t2 = tm.begin(T_COUNT);
-            MB_CUDA(ctx, cudaMemsetAsync(d_best64, 0, (size_t)ns * K * 8, ctx->stream));
-            const int64_t rthreads = ns * (int64_t)best_nch * (P.K2pad / 2);
-            best_reduce_kernel<<<(unsigned)((rthreads + 255) / 256), 256, 0, ctx->stream>>>(d_mask, ns, W16, P.K2pad, best_nch,
-                                                                                          (const int32_t*)(d_plan + off_p2m), K, d_best64);
-            if (sp) {                                   // anchors s0/2 .. (s0 + ns)/2: count into the histogram instead of returning records
-                const int64_t na = ns / 2;
-                spacing_kernel<<<(unsigned)((na * K + 255) / 256), 256, 0, ctx->stream>>>(d_best64, na, K, d_anchors + s0 / 2, d_spthr, d_mlen, sp->margin,
-                                                                                         d_sphist, sp->sites ? d_best : nullptr);
-                tm.end(t2);
-                ctx->launches[T_COUNT] += 2;
-                MB_CUDA(ctx, cudaGetLastError());
-                if (sp->sites) {
-                    const int t6 = tm.begin(T_D2H);
-                    MB_CUDA(ctx, cudaMemcpyAsync(sp->sites + (size_t)(s0 / 2) * K, d_best, (size_t)na * K * sizeof(mb200_best), cudaMemcpyDeviceToHost, ctx->stream));
-                    tm.end(t6);
-                }
-                continue;
-            }
-            best_finalize_kernel<<<(unsigned)((ns * K + 255) / 256), 256, 0, ctx->stream>>>(d_best64, ns * K, d_best);
-            tm.end(t2);
-            ctx->launches[T_COUNT] += 2;
-            MB_CUDA(ctx, cudaGetLastError());
-            const int t6 = tm.begin(T_D2H);
-            MB_CUDA(ctx, cudaMemcpyAsync(best + (size_t)s0 * K, d_best, (size_t)ns * K * sizeof(mb200_best), cudaMemcpyDeviceToHost, ctx->stream));
-            tm.end(t6);
-            continue;
-        }
-
-        int t2 = tm.begin(T_COUNT);
-        const int32_t Pp = P.K2pad / 2;
-        if (!want_hits && W > 4096) {
-            // chromosome-scale sequences: blocked parallel counting
-            const int32_t WB = 512, nblocks = (W + WB - 1) / WB;
-            const int64_t nbt = ns * (int64_t)nblocks * Pp;
-            const size_t o_top1 = 0, o_top2 = o_top1 + (size_t)ns * Pp * 8, o_nh = o_top2 + (size_t)ns * Pp * 8, o_dup = o_nh + (size_t)ns * Pp * 4;
-            const size_t o_cand = (o_dup + (size_t)ns * Pp * 4 + 255) & ~(size_t)255;
-            rc = mb_ensure_buf(ctx, 7, o_cand + (size_t)nbt * sizeof(LongCand)); if (rc) return rc;
-            uint8_t* lb = (uint8_t*)ctx->bufs[7];
-            MB_CUDA(ctx, cudaMemsetAsync(lb, 0, o_cand, ctx->stream));
-            count_long_a<<<(unsigned)((nbt + 255) / 256), 256, 0, ctx->stream>>>(d_mask, ns, W, P.K2pad, WB, nblocks, (const int32_t*)(d_plan + off_p2m),
-                (const int32_t*)(d_plan + off_plen), d_counts, (unsigned long long*)(lb + o_top1), (unsigned int*)(lb + o_nh), (LongCand*)(lb + o_cand));
-            count_long_b<<<(unsigned)((nbt + 255) / 256), 256, 0, ctx->stream>>>(ns, Pp, nblocks, (const LongCand*)(lb + o_cand), (const unsigned long long*)(lb + o_top1),
-                (unsigned long long*)(lb + o_top2), (unsigned int*)(lb + o_dup));
-            count_long_c<<<(unsigned)((ns * Pp + 255) / 256), 256, 0, ctx->stream>>>(ns, Pp, (const int32_t*)(d_plan + off_p2m), (const int32_t*)(d_plan + off_plen),
-                (const unsigned long long*)(lb + o_top1), (const unsigned long long*)(lb + o_top2), (const unsigned int*)(lb + o_dup), (const unsigned int*)(lb + o_nh), d_counts);
-            ctx->launches[T_COUNT] += 3;
-        } else if (tc_done && tc_units) {
-            // only the units the verifier listed have hits.  Counts-only: count and clear them.  With a hit list: the unit counts feed the
-            // prefix sum (zero elsewhere), the words stay until emit_kernel has read them and are cleared after that.
-            if (want_hits) MB_CUDA(ctx, cudaMemsetAsync(d_unit_cnt, 0, (size_t)ns * K * 2 * 4, ctx->stream));
-            count_listed_kernel<<<grid * 8, 256, 0, ctx->stream>>>(d_mask, d_tc_ulist, d_tc_ctr + 4, W, P.K2pad, (const int32_t*)(d_plan + off_p2m),
-                                                                    (const int32_t*)(d_plan + off_plen), d_counts, nullptr, want_hits ? d_unit_cnt : nullptr, K, want_hits ? 0 : 1);
-            ctx->launches[T_COUNT] += 1;
-            if (!want_hits) ctx->mask_clean_bytes = (size_t)ns * mask_bytes_per_seq;   // every word with a bit belongs to a listed unit and was cleared
-        } else {
-            const int64_t cthreads = ns * Pp;
-            count_kernel<<<(unsigned)((cthreads + 255) / 256), 256, 0, ctx->stream>>>(d_mask, ns, W, P.K2pad, (const int32_t*)(d_plan + off_p2m),
-                                                                                  (const int32_t*)(d_plan + off_plen), d_counts, d_unit_cnt, K);
-            ctx->launches[T_COUNT] += 1;
-        }
-        tm.end(t2);
-        MB_CUDA(ctx, cudaGetLastError());
-
-        if (hist) {
-            const int64_t units = ns * K * 2;
-            const int t7 = tm.begin(T_EMIT);
-            hist_kernel<<<(unsigned)((units + 255) / 256), 256, 0, ctx->stream>>>(d_mask, seqs->words, rowwords, s0, ns, W, P.K2pad, K,
-                                                                               (const EmitMotif*)(d_plan + off_em), d_plan + off_blob, d_hist);
-            tm.end(t7);
-            ctx->launches[T_EMIT] += 1;
-            MB_CUDA(ctx, cudaGetLastError());
-        }
-        if (want_hits) {
-            const int64_t units = ns * K * 2;
-            const int64_t nb = (units + PS_TILE - 1) / PS_TILE;
-            int t3 = tm.begin(T_EMIT);
-            ps_block_sums<<<(unsigned)nb, PS_THREADS, 0, ctx->stream>>>(d_unit_cnt, units, d_bsum);
-            ps_scan_sums<<<1, PS_THREADS, 0, ctx->stream>>>(d_bsum, nb, d_total);
-            ps_apply<<<(unsigned)nb, PS_THREADS, 0, ctx->stream>>>(d_unit_cnt, units, d_bsum, d_unit_off);
-            tm.end(t3);
-            ctx->launches[T_EMIT] += 3;
-            unsigned long long h_total = 0;
-            MB_CUDA(ctx, cudaMemcpyAsync(&h_total, d_total, 8, cudaMemcpyDeviceToHost, ctx->stream));
-            MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-            hits_needed += (int64_t)h_total;
-            // a list that outgrows the caller's buffer is kept in the ctx (host memory) and handed over by mb200_scan_take_hits:
-            // the caller's retry does not pay for the scan, count and prefix kernels a second time
-            const bool spill = hits_needed > hits_cap;
-            if (spill && ctx->held_hits.empty() && hits_written) ctx->held_hits.assign(hits, hits + hits_written);
-            if (h_total) {
-                rc = mb_ensure_buf(ctx, 4, (size_t)h_total * sizeof(mb200_hit)); if (rc) return rc;
-                mb200_hit* d_hits = (mb200_hit*)ctx->bufs[4];
-                int t4 = tm.begin(T_EMIT);
-                emit_kernel<<<(unsigned)((units + 255) / 256), 256, 0, ctx->stream>>>(d_mask, seqs->words, rowwords, s0, ns, W, P.K2pad, K,
-                                                                                   (const EmitMotif*)(d_plan + off_em), d_plan + off_blob,
-                                                                                   d_unit_cnt, d_unit_off, d_hits);
-                tm.end(t4);
-                ctx->launches[T_EMIT] += 1;
-                MB_CUDA(ctx, cudaGetLastError());
-                int t5 = tm.begin(T_D2H);
-                mb200_hit* dst = hits + hits_written;
-                if (spill) { ctx->held_hits.resize((size_t)hits_written + (size_t)h_total); dst = ctx->held_hits.data() + hits_written; }
-                MB_CUDA(ctx, cudaMemcpyAsync(dst, d_hits, (size_t)h_total * sizeof(mb200_hit), cudaMemcpyDeviceToHost, ctx->stream));
-                tm.end(t5);
-                MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-                hits_written += (int64_t)h_total;
-            }
-            if (tc_done && tc_units) {
-                clear_listed_kernel<<<grid * 8, 256, 0, ctx->stream>>>(d_mask, d_tc_ulist, d_tc_ctr + 4, W, P.K2pad);
-                ctx->launches[T_EMIT] += 1;
-                ctx->mask_clean_bytes = (size_t)ns * mask_bytes_per_seq;
-            }
-        }
-    }
-    if (reduce) {                                       // one all-reduce per scan (SURVEY §8e): K x 4 counts, or the K x 32768 histogram
-        if (want_counts) { rc = mb_comm_allreduce_u64(ctx, d_counts, (size_t)K * 4); if (rc) return rc; }
-        if (hist) { rc = mb_comm_allreduce_u32(ctx, d_hist, (size_t)K * HIST_BINS); if (rc) return rc; }
-    }
-    if (hist) {
-        int t8 = tm.begin(T_D2H);
-        MB_CUDA(ctx, cudaMemcpyAsync(hist, d_hist, (size_t)K * HIST_BINS * 4, cudaMemcpyDeviceToHost, ctx->stream));
-        tm.end(t8);
-    }
-    if (want_counts) {
-        int t6 = tm.begin(T_D2H);
-        MB_CUDA(ctx, cudaMemcpyAsync(counts, d_counts, (size_t)K * 4 * 8, cudaMemcpyDeviceToHost, ctx->stream));
-        tm.end(t6);
-    }
-    if (sp) {
-        const int t9 = tm.begin(T_D2H);
-        MB_CUDA(ctx, cudaMemcpyAsync(sp->hist, d_sphist, sphist_bytes, cudaMemcpyDeviceToHost, ctx->stream));
-        tm.end(t9);
-    }
-    tm.end(t_total);
-    MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    tm.collect();
-    if (d_tc_ctr && getenv("MB200_SCAN_TC_STATS")) {
-        fprintf(stderr, "[mb200] tensor-core scan: %s, candidates %llu, hits %llu, scan %.3f ms, count %.3f ms\n", use_tc ? "used" : "fell back", tc_stat_cand, tc_stat_hits,
-                ctx->ms[T_SCAN], ctx->ms[T_COUNT]);
-    }
-    if (seqs->pending) { rc = mb_seqs_finish(ctx, const_cast<mb200_seqs*>(seqs)); if (rc) return rc; }      // the upload has completed: report bad symbols
-    if (n_hits) *n_hits = hits_needed;
-    if (want_hits && hits_needed > hits_cap)
-        MB_FAIL(ctx, MB200_E_HITS_OVERFLOW, "scan: %lld hits, capacity %lld", (long long)hits_needed, (long long)hits_cap);
     return MB200_OK;
+}
+
+// The totals of a call, K x 4 uint64 counts (WANT_COUNTS) or the K x HIST_BINS uint32 score histogram (HIST), never both: summed
+// across ranks (one all-reduce per scan, SURVEY §8e) and copied to the caller.  tm == nullptr: the copy is not timed.
+static size_t totals_bytes(const ScanCall& S) { return S.out.hist ? (size_t)S.K * HIST_BINS * 4 : S.want_counts ? (size_t)S.K * 4 * 8 : 0; }
+static int copy_totals(ScanCall& S, void* d_totals, MbTimers* tm) {
+    mb200_ctx* ctx = S.ctx;
+    const size_t bytes = totals_bytes(S);
+    if (!bytes) return MB200_OK;
+    if (S.reduce) {
+        const int rc = S.out.hist ? mb_comm_allreduce_u32(ctx, (unsigned int*)d_totals, bytes / 4) : mb_comm_allreduce_u64(ctx, (unsigned long long*)d_totals, bytes / 8);
+        if (rc) return rc;
+    }
+    const int t = tm ? tm->begin(T_D2H) : -1;
+    MB_CUDA(ctx, cudaMemcpyAsync(S.out.hist ? (void*)S.out.hist : (void*)S.out.counts, d_totals, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    if (tm) tm->end(t);
+    return MB200_OK;
+}
+
+// Nothing can be scored on this rank (no rows, or no PWM fits a row).  It writes its "none" outputs and still takes part in the
+// reduction, with zeroed scratch in place of the counts and the histogram.
+static int scan_empty(ScanCall& S) {
+    mb200_ctx* ctx = S.ctx; const ScanOut& o = S.out;
+    const mb200_best none = {0xFFFFFFFFu, 0, 0, 0};
+    if (o.best) std::fill(o.best, o.best + (size_t)S.N * S.K, none);     // no row holds a window (otherwise every batch writes all its records)
+    if (o.sp) {                                                          // every secondary is longer than the margin
+        memset(o.sp->hist, 0, S.sphist_bytes);
+        if (o.sp->sites) std::fill(o.sp->sites, o.sp->sites + (size_t)o.sp->n * S.K, none);
+    }
+    if (S.reduce && totals_bytes(S)) {
+        int rc = mb_ensure_scratch(ctx, totals_bytes(S)); if (rc) return rc;
+        MB_CUDA(ctx, cudaMemsetAsync(ctx->scratch, 0, totals_bytes(S), ctx->stream));
+        rc = copy_totals(S, ctx->scratch, nullptr); if (rc) return rc;
+        MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    }
+    return MB200_OK;
+}
+
+// BUF_PLAN and the batch size: the masks of a batch stay under 8 GB.
+static int stage_plan(ScanCall& S) {
+    mb200_ctx* ctx = S.ctx; const ScanPlan& P = S.P;
+    const int64_t W64 = (S.Lb - P.minlen + 1 + 31) / 32;
+    if (W64 > 0x1fffffff) MB_FAIL(ctx, MB200_E_UNSUPPORTED, "sequence too long");
+    S.W = (int32_t)W64; S.W16 = 2 * S.W;
+    S.tc_units = S.W <= 4096;
+    const size_t off_blob = put(S.h_plan, P.blob.data(), P.blob.size());
+    const size_t off_mb = put(S.h_plan, P.mblocks.data(), P.mblocks.size() * sizeof(MBlock));
+    const size_t off_lb = put(S.h_plan, P.lblocks.data(), P.lblocks.size() * sizeof(MBlock));
+    const size_t off_p2m = put(S.h_plan, P.pair2motif.data(), P.pair2motif.size() * 4);
+    const size_t off_plen = put(S.h_plan, P.pairlen.data(), P.pairlen.size() * 4);
+    const size_t off_em = put(S.h_plan, P.em.data(), P.em.size() * sizeof(EmitMotif));
+    const size_t off_rng = put(S.h_plan, nullptr, (size_t)(S.grid + 1) * 8);
+    const size_t off_cnt = put(S.h_plan, nullptr, (size_t)S.K * 4 * 8);
+    const size_t off_tot = put(S.h_plan, nullptr, 8);
+    int rc = mb_ensure_buf(ctx, BUF_PLAN, S.h_plan.size()); if (rc) return rc;
+    uint8_t* d_plan = (uint8_t*)ctx->bufs[BUF_PLAN];
+    S.d_blob = d_plan + off_blob; S.d_mblocks = (const MBlock*)(d_plan + off_mb); S.d_lblocks = (const MBlock*)(d_plan + off_lb);
+    S.d_p2m = (const int32_t*)(d_plan + off_p2m); S.d_plen = (const int32_t*)(d_plan + off_plen); S.d_em = (const EmitMotif*)(d_plan + off_em);
+    S.d_rng = (int64_t*)(d_plan + off_rng); S.d_counts = (unsigned long long*)(d_plan + off_cnt); S.d_total = (unsigned long long*)(d_plan + off_tot);
+
+    const size_t mask_budget = (size_t)8 << 30;
+    S.mask_bytes_per_seq = (size_t)S.W * P.K2pad * 4 * (S.keys ? 2 : 1);        // best keys: one 32-bit key per 16-position block
+    int64_t spb = std::max<int64_t>(1, (int64_t)(mask_budget / S.mask_bytes_per_seq));
+    if (spb > S.N) spb = S.N;
+    if ((double)spb * S.W > 2.0e9) spb = std::max<int64_t>(1, (int64_t)(2.0e9 / S.W));
+    if (S.out.kind == ScanOut::SPACING) spb = std::max<int64_t>(2, spb & ~(int64_t)1);   // both margins of an anchor in one batch (N is even)
+    if (S.use_tc && (double)spb * (double)S.Lb > 2.0e9) spb = std::max<int64_t>(1, (int64_t)(2.0e9 / (double)S.Lb));   // 32-bit virtual positions
+    S.seqs_per_batch = spb;
+    return MB200_OK;
+}
+
+// Tensor-core buffers; BUF_TC_LIST and BUF_TC_UNITS hold two sets each, which the pipelined loop alternates.
+static int stage_tc(ScanCall& S) {
+    mb200_ctx* ctx = S.ctx; const TcPlan& TP = S.TP;
+    std::vector<uint8_t> h_tc;
+    put(h_tc, TP.blob.data(), TP.blob.size());
+    put(h_tc, TP.blocks.data(), TP.blocks.size() * sizeof(TcBlock));
+    const size_t off_slots = put(h_tc, TP.slots.data(), TP.slots.size() * sizeof(TcSlot), 1);
+    int rc = mb_ensure_buf(ctx, BUF_TC_PLAN, h_tc.size()); if (rc) return rc;
+    const size_t set_bytes = (((size_t)TC_CAP * 8 + S.tc_nctr() * 8) + 255) & ~(size_t)255;
+    rc = mb_ensure_buf(ctx, BUF_TC_LIST, 2 * set_bytes); if (rc) return rc;
+    S.d_tc = (uint8_t*)ctx->bufs[BUF_TC_PLAN];
+    S.d_tc_slots = (const TcSlot*)(S.d_tc + off_slots);
+    S.d_tc_list = (unsigned long long*)ctx->bufs[BUF_TC_LIST];
+    S.d_tc_ctr = S.d_tc_list + TC_CAP;
+    const size_t ubits_bytes = S.tc_ubits_bytes(S.seqs_per_batch) + 256;
+    const size_t uset_bytes = (((size_t)TC_CAP * 4 + ubits_bytes) + 255) & ~(size_t)255;
+    rc = mb_ensure_buf(ctx, BUF_TC_UNITS, 2 * uset_bytes); if (rc) return rc;
+    S.d_tc_ulist = (uint32_t*)ctx->bufs[BUF_TC_UNITS];
+    S.d_tc_ubits = S.d_tc_ulist + TC_CAP;
+    S.tc_set_stride = set_bytes; S.tc_uset_stride = uset_bytes;
+    MB_CUDA(ctx, cudaMemcpyAsync(S.d_tc, h_tc.data(), h_tc.size(), cudaMemcpyHostToDevice, ctx->stream));
+    MB_CUDA(ctx, cudaMemsetAsync(S.d_tc_ctr, 0, S.tc_nctr() * 8, ctx->stream));
+    MB_CUDA(ctx, cudaMemsetAsync((uint8_t*)S.d_tc_ctr + S.tc_set_stride, 0, S.tc_nctr() * 8, ctx->stream));
+    MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));           // h_tc goes out of scope
+    // at least half of the shared memory: one CTA per SM (each CTA allocates all 512 TMEM columns)
+    S.tc_smem = std::max<size_t>((size_t)TCS_STAGES * TCS_STAGE_BYTES + TP.max_b_bytes, (size_t)120 * 1024);
+    if (S.tc_smem > ctx->smem_optin) S.use_tc = false;
+    else MB_CUDA(ctx, cudaFuncSetAttribute(k_scan_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S.tc_smem));
+    return MB200_OK;
+}
+
+// The device buffers of the call (BUF_* in common.cuh) and the launch set-up of scan_kernel.
+static int stage_buffers(ScanCall& S, const int64_t* lens) {
+    mb200_ctx* ctx = S.ctx; const int K = S.K;
+    int rc = stage_plan(S); if (rc) return rc;
+    if (S.use_tc) { rc = stage_tc(S); if (rc) return rc; }
+    const int64_t spb = S.seqs_per_batch;
+    rc = mb_ensure_buf(ctx, BUF_MASK, (size_t)spb * S.mask_bytes_per_seq); if (rc) return rc;
+    S.d_mask = (uint32_t*)ctx->bufs[BUF_MASK];
+    if (S.keys) {                                       // per batch: 64-bit best keys, then the records (spacing: the sites)
+        rc = mb_ensure_buf(ctx, BUF_UNITS, (size_t)spb * K * 16); if (rc) return rc;
+        S.d_best64 = (unsigned long long*)ctx->bufs[BUF_UNITS];
+        S.d_best = (mb200_best*)(S.d_best64 + (size_t)spb * K);
+        S.best_nch = (S.W16 + BEST_CHUNK - 1) / BEST_CHUNK;
+    }
+    if (const SpacingJob* sp = S.out.sp) {
+        rc = mb_ensure_buf(ctx, BUF_HIST, S.sphist_bytes); if (rc) return rc;
+        S.d_sphist = (unsigned int*)ctx->bufs[BUF_HIST];
+        std::vector<uint8_t> h;
+        std::vector<uint16_t> thr(K); std::vector<int32_t> mlen(K);
+        for (int k = 0; k < K; ++k) { thr[k] = hit_threshold(sp->thresh, k); mlen[k] = (int32_t)lens[k]; }
+        put(h, sp->anchors, (size_t)sp->n * sizeof(mb200_anchor));
+        const size_t off_thr = put(h, thr.data(), (size_t)K * 2), off_len = put(h, mlen.data(), (size_t)K * 4, 1);
+        rc = mb_ensure_buf(ctx, BUF_SPACING, h.size()); if (rc) return rc;
+        uint8_t* d = (uint8_t*)ctx->bufs[BUF_SPACING];
+        MB_CUDA(ctx, cudaMemcpyAsync(d, h.data(), h.size(), cudaMemcpyHostToDevice, ctx->stream));
+        MB_CUDA(ctx, cudaMemsetAsync(S.d_sphist, 0, S.sphist_bytes, ctx->stream));
+        MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));         // h goes out of scope
+        S.d_anchors = (const mb200_anchor*)d; S.d_spthr = (const uint16_t*)(d + off_thr); S.d_mlen = (const int32_t*)(d + off_len);
+    }
+    if (S.want_hits) {
+        const int64_t units = spb * K * 2, ps_blocks = (units + PS_TILE - 1) / PS_TILE;
+        const size_t off_off = ((size_t)units * 4 + 255) & ~(size_t)255;
+        const size_t off_bsum = off_off + (((size_t)units * 8 + 255) & ~(size_t)255);
+        rc = mb_ensure_buf(ctx, BUF_UNITS, off_bsum + (size_t)ps_blocks * 8 + 256); if (rc) return rc;
+        S.d_unit_cnt = (uint32_t*)ctx->bufs[BUF_UNITS];
+        S.d_unit_off = (unsigned long long*)((uint8_t*)ctx->bufs[BUF_UNITS] + off_off);
+        S.d_bsum = (unsigned long long*)((uint8_t*)ctx->bufs[BUF_UNITS] + off_bsum);
+    }
+    // scan_kernel: words spanned by a tile: +1 per block inside a sequence, + (rowwords - W16 + 1) when crossing to the next sequence
+    const int64_t crossings = (TILE_CHUNKS - 1) / S.W16 + 1;
+    const int64_t gap = std::max<int64_t>(0, S.rowwords - (int64_t)S.W16 + 1);
+    S.tile_cap_words = (int32_t)(((int64_t)TILE_CHUNKS + crossings * gap + 6 + 4 + 3) & ~(int64_t)3);
+    S.blob_cap = (S.P.max_blob_bytes + 127) & ~127;
+    S.smem_bytes = (size_t)S.blob_cap + (size_t)S.tile_cap_words * 8 + 64;
+    if (S.smem_bytes > ctx->smem_optin) MB_FAIL(ctx, MB200_E_UNSUPPORTED, "scan needs %zu B shared memory (> %zu)", S.smem_bytes, ctx->smem_optin);
+    const bool ragged = S.seqs->lens != nullptr;
+    S.scan_fn = S.keys ? (ragged ? scan_kernel<true, true> : scan_kernel<false, true>) : (ragged ? scan_kernel<true> : scan_kernel<false>);
+    MB_CUDA(ctx, cudaFuncSetAttribute(S.scan_fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S.smem_bytes));
+
+    S.t_total = S.tm.begin(T_TOTAL);
+    const int th = S.tm.begin(T_H2D);
+    MB_CUDA(ctx, cudaMemcpyAsync(ctx->bufs[BUF_PLAN], S.h_plan.data(), S.h_plan.size(), cudaMemcpyHostToDevice, ctx->stream));
+    S.tm.end(th);
+    if (S.out.hist) {
+        rc = mb_ensure_buf(ctx, BUF_HIST, (size_t)K * HIST_BINS * 4); if (rc) return rc;
+        S.d_hist = (unsigned int*)ctx->bufs[BUF_HIST];
+        MB_CUDA(ctx, cudaMemsetAsync(S.d_hist, 0, (size_t)K * HIST_BINS * 4, ctx->stream));
+    }
+    return MB200_OK;
+}
+
+// A batch may start as soon as the chunks of a pending asynchronous upload that hold rows [0, end) are packed (the kernels read a
+// few words past the batch's last row: in bounds, and whatever they hold only reaches positions that are masked out).
+static int wait_for_rows(ScanCall& S, int64_t end) {
+    const mb200_seqs* seqs = S.seqs;
+    if (!seqs->pending) return MB200_OK;
+    while (S.next_ready < seqs->ready.size() && (S.next_ready == 0 || seqs->ready_end[S.next_ready - 1] < end)) {
+        MB_CUDA(S.ctx, cudaStreamWaitEvent(S.ctx->stream, seqs->ready[S.next_ready], 0));
+        ++S.next_ready;
+    }
+    return MB200_OK;
+}
+
+// ---- one k_scan_tc batch, shared by the pipelined and the serial loop ------------------------------------------------------------
+// make TCS_PROFILE=1, MB200_SCAN_TC_DEBUG=<batch>: the per-role wait clocks of that batch's CTAs (captured by tc_launch)
+static void tc_debug_dump(ScanCall& S, const TcArgs& ta) {
+#if TCS_PROFILE
+    if (!ta.dbg) return;
+    std::vector<long long> h((size_t)S.grid * 8);
+    cudaStreamSynchronize(S.ctx->stream);
+    cudaMemcpy(h.data(), ta.dbg, (size_t)S.grid * 8 * 8, cudaMemcpyDeviceToHost);
+    for (int c = 0; c < S.grid; c += 1)
+        fprintf(stderr, "[tcdbg] cta %3d blk %lld tiles %lld | mma total %9lld wait_full %9lld wait_acc %9lld | epi total %9lld wait %9lld | prod wait %9lld\n", c, h[c * 8 + 6], h[c * 8 + 7],
+                h[c * 8 + 0], h[c * 8 + 1], h[c * 8 + 2], h[c * 8 + 4], h[c * 8 + 3], h[c * 8 + 5]);
+#endif
+}
+
+// Zeroes the counters, the unit bitmap when given and the part of the mask buffer that ctx->mask_clean_bytes does not cover (the
+// buffer is kept all-zero between tensor-core batches), then launches k_scan_tc on ctx->stream.
+static int tc_launch(ScanCall& S, int64_t s0, int64_t ns, unsigned long long* list, unsigned long long* ctr, uint32_t* ubits, TcArgs& ta) {
+    mb200_ctx* ctx = S.ctx;
+    const size_t need = (size_t)ns * S.mask_bytes_per_seq;
+    if (ctx->mask_clean_bytes < need) {
+        MB_CUDA(ctx, cudaMemsetAsync(S.d_mask, 0, need, ctx->stream));
+        ctx->mask_clean_bytes = need;
+    }
+    MB_CUDA(ctx, cudaMemsetAsync(ctr, 0, 64, ctx->stream));
+    if (ubits) MB_CUDA(ctx, cudaMemsetAsync(ubits, 0, S.tc_ubits_bytes(ns), ctx->stream));
+    ta.seqw = S.seqs->words; ta.rowwords = S.rowwords; ta.seq0 = s0; ta.lens = S.seqs->lens;
+    ta.Lb = (uint32_t)S.Lb; ta.vtotal = (uint32_t)(ns * S.Lb);
+    ta.blob = S.d_tc; ta.nblocks = (int32_t)S.TP.blocks.size();
+    memset(ta.blocks, 0, sizeof ta.blocks); memcpy(ta.blocks, S.TP.blocks.data(), S.TP.blocks.size() * sizeof(TcBlock));
+    ta.slots = S.d_tc_slots;
+    ta.list = list; ta.cap = TC_CAP; ta.gcount = ctr; ta.overflow = (uint32_t*)(ctr + 1);
+    ta.ntiles = (int32_t)((ns * S.Lb + 255) / 256);
+    ta.clocks = (long long*)(ctr + 8);
+    ta.dbg = nullptr;
+#if TCS_PROFILE
+    static long long* d_dbg = nullptr;
+    const char* e = getenv("MB200_SCAN_TC_DEBUG");
+    if (e && s0 / S.seqs_per_batch == atoi(e)) {
+        if (!d_dbg) MB_CUDA(ctx, cudaMalloc(&d_dbg, (size_t)S.grid * 8 * 8));
+        MB_CUDA(ctx, cudaMemsetAsync(d_dbg, 0, (size_t)S.grid * 8 * 8, ctx->stream)); ta.dbg = d_dbg;
+    }
+#endif
+    const int t_tc = S.tm.begin(T_SCAN);
+    k_scan_tc<<<S.grid, TCS_THREADS, S.tc_smem, ctx->stream>>>(ta);
+    S.tm.end(t_tc);
+    ctx->launches[T_SCAN] += 1;
+    return MB200_OK;
+}
+
+// The counters h of a finished batch.  false: its candidate list overflowed (thresholds so permissive that most cells pass).
+// Otherwise adds its statistics and re-balances the CTAs over the slot blocks with the clocks per tile it measured (the epilogue's
+// share depends on the candidate density of a block, which no static model knows).
+static bool tc_read_counters(ScanCall& S, const unsigned long long* h) {
+    if (h[1]) return false;
+    S.tc_stat_cand += h[2]; S.tc_stat_hits += h[3];
+    const std::vector<TcBlock>& blocks = S.TP.blocks;
+    std::vector<double> cost(blocks.size(), 0.0);
+    for (size_t bi = 0; bi < blocks.size(); ++bi) {
+        double clk = 0, tiles = 0;
+        for (int c = blocks[bi].cta0; c < blocks[bi].cta0 + blocks[bi].nctas; ++c) { clk += (double)h[8 + 2 * c]; tiles += (double)h[8 + 2 * c + 1]; }
+        if (tiles <= 0 || clk <= 0) return true;
+        cost[bi] = clk / tiles;
+    }
+    S.ctx->tc_cost = cost;
+    tc_assign_ctas(S.TP.blocks, cost, S.grid);
+    return true;
+}
+
+// Counts-only scans: the pipelined tensor-core path.  The pre-filter of batch i+1 (ctx->stream) runs while batch i is re-scored and
+// counted on ctx->aux_stream with the other buffer set, and the host reads batch i's counters while batch i+1 is already running.
+// Leaves in todo the batches still to run: those that overflowed (their count is skipped) and those not launched after that.
+static int tc_pipelined(ScanCall& S, std::vector<int64_t>& todo) {
+    mb200_ctx* ctx = S.ctx; const int grid = S.grid;
+    if (!ctx->aux_stream && cudaStreamCreateWithFlags(&ctx->aux_stream, cudaStreamNonBlocking) != cudaSuccess) MB_FAIL(ctx, MB200_E_CUDA, "scan: cannot create the auxiliary stream");
+    cudaStream_t aux = ctx->aux_stream;
+    const size_t nctr = S.tc_nctr();
+    int rc = mb_ensure_pinned(ctx, 2 * nctr * 8); if (rc) return rc;
+    unsigned long long* h_ctr2 = (unsigned long long*)ctx->pinned;
+    struct EvGuard {                                            // the events are destroyed on every way out (error returns included)
+        cudaEvent_t tc[2] = {nullptr, nullptr}, aux[2] = {nullptr, nullptr};
+        ~EvGuard() { for (int b = 0; b < 2; ++b) { if (tc[b]) cudaEventDestroy(tc[b]); if (aux[b]) cudaEventDestroy(aux[b]); } }
+    } evg;
+    for (int b = 0; b < 2; ++b) { MB_CUDA(ctx, cudaEventCreateWithFlags(&evg.tc[b], cudaEventDisableTiming)); MB_CUDA(ctx, cudaEventCreateWithFlags(&evg.aux[b], cudaEventDisableTiming)); }
+    const int nb = (int)todo.size();
+    std::vector<char> launched(nb, 0), failed(nb, 0);
+    bool overflowed = false;
+    auto process = [&](int j) -> int {
+        if (cudaEventSynchronize(evg.aux[j & 1]) != cudaSuccess) return MB200_E_CUDA;
+        if (!tc_read_counters(S, h_ctr2 + (size_t)(j & 1) * nctr)) { failed[j] = 1; overflowed = true; }
+        return MB200_OK;
+    };
+    int i = 0;
+    for (; i < nb && !overflowed; ++i) {
+        const int64_t s0 = todo[i];
+        const int64_t ns = std::min(S.seqs_per_batch, S.N - s0);
+        rc = wait_for_rows(S, s0 + ns); if (rc) return rc;
+        const int b = i & 1;
+        unsigned long long* list_b = (unsigned long long*)((uint8_t*)S.d_tc_list + (size_t)b * S.tc_set_stride);
+        unsigned long long* ctr_b = list_b + TC_CAP;
+        uint32_t* ulist_b = (uint32_t*)((uint8_t*)S.d_tc_ulist + (size_t)b * S.tc_uset_stride);
+        uint32_t* ubits_b = ulist_b + TC_CAP;
+        TcArgs ta;
+        rc = tc_launch(S, s0, ns, list_b, ctr_b, nullptr, ta); if (rc) return rc;
+        MB_CUDA(ctx, cudaGetLastError());
+        MB_CUDA(ctx, cudaEventRecord(evg.tc[b], ctx->stream));
+        MB_CUDA(ctx, cudaStreamWaitEvent(aux, evg.tc[b], 0));
+        MB_CUDA(ctx, cudaMemsetAsync(ubits_b, 0, S.tc_ubits_bytes(ns), aux));
+        const int t_vf = S.tm.begin_on(T_EMIT, aux);
+        // 128-thread blocks: next to a k_scan_tc CTA (608 threads x 96 registers) an SM has ~7 K registers left
+        k_scan_tc_verify<<<grid * 16, 128, 0, aux>>>(list_b, ctr_b, TC_CAP, ta.slots, S.d_em, S.d_blob, S.seqs->words, S.rowwords, s0, (uint32_t)S.Lb,
+                                                    S.W, S.P.K2pad, S.d_mask, ctr_b + 2, ubits_b, ulist_b, ctr_b + 4, S.seqs->lens);
+        S.tm.end_on(t_vf, aux);
+        const int t_ct = S.tm.begin_on(T_COUNT, aux);
+        count_listed_kernel<<<grid * 16, 128, 0, aux>>>(S.d_mask, ulist_b, ctr_b + 4, S.W, S.P.K2pad, S.d_p2m, S.d_plen, S.d_counts, ctr_b + 1, nullptr, 0, 1);
+        S.tm.end_on(t_ct, aux);
+        MB_CUDA(ctx, cudaGetLastError());
+        MB_CUDA(ctx, cudaMemcpyAsync(h_ctr2 + (size_t)b * nctr, ctr_b, nctr * 8, cudaMemcpyDeviceToHost, aux));
+        MB_CUDA(ctx, cudaEventRecord(evg.aux[b], aux));
+        ctx->launches[T_EMIT] += 1; ctx->launches[T_COUNT] += 1;
+        launched[i] = 1;
+        tc_debug_dump(S, ta);
+        if (i >= 1) { rc = process(i - 1); if (rc) return rc; }
+    }
+    // every batch but the last launched one was looked at inside the loop
+    if (i > 0) { rc = process(i - 1); if (rc) return rc; }
+    MB_CUDA(ctx, cudaStreamSynchronize(aux));
+    std::vector<int64_t> rest;
+    for (int j = 0; j < nb; ++j) if (!launched[j] || failed[j]) rest.push_back(todo[j]);
+    todo.swap(rest);
+    if (overflowed) { S.use_tc = false; ctx->last_scan_path = 2; ctx->mask_clean_bytes = 0; }     // a failed batch may have left bits behind (its count was skipped)
+    else ctx->last_scan_path = 1;
+    return MB200_OK;
+}
+
+// A tensor-core batch outside the pipeline: pre-filter and verifier on ctx->stream, and the host reads the counters before the next
+// batch.  *done: the masks are complete.  After a candidate-list overflow this and every later batch take scan_kernel.
+static int tc_serial_batch(ScanCall& S, int64_t s0, int64_t ns, bool* done) {
+    mb200_ctx* ctx = S.ctx;
+    TcArgs ta;
+    int rc = tc_launch(S, s0, ns, S.d_tc_list, S.d_tc_ctr, S.tc_units ? S.d_tc_ubits : nullptr, ta); if (rc) return rc;
+    const int t_vf = S.tm.begin(T_EMIT);
+    k_scan_tc_verify<<<S.grid * 8, 256, 0, ctx->stream>>>(S.d_tc_list, S.d_tc_ctr, TC_CAP, ta.slots, S.d_em, S.d_blob, S.seqs->words, S.rowwords, s0,
+                                                         (uint32_t)S.Lb, S.W, S.P.K2pad, S.d_mask, S.d_tc_ctr + 2,
+                                                         S.tc_units ? S.d_tc_ubits : nullptr, S.d_tc_ulist, S.d_tc_ctr + 4, S.seqs->lens);
+    S.tm.end(t_vf);
+    ctx->launches[T_EMIT] += 1;
+    MB_CUDA(ctx, cudaGetLastError());
+    std::vector<unsigned long long> h_ctr(S.tc_nctr(), 0);
+    MB_CUDA(ctx, cudaMemcpyAsync(h_ctr.data(), S.d_tc_ctr, h_ctr.size() * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    tc_debug_dump(S, ta);
+    *done = tc_read_counters(S, h_ctr.data());
+    ctx->mask_clean_bytes = 0;                               // the verifier has set bits (re-established when the listed count or clear_listed_kernel clears them)
+    if (!*done) { S.use_tc = false; ctx->last_scan_path = 2; }
+    else if (ctx->last_scan_path == 0) ctx->last_scan_path = 1;
+    return MB200_OK;
+}
+
+// ---- scan_kernel / scan_long_kernel --------------------------------------------------------------------------------------------
+// Per-CTA ranges of (motif block, tile) pairs for each new batch shape: a contiguous split, mblock-major, weighted by column count.
+static int update_cta_ranges(ScanCall& S, int64_t ns) {
+    const int64_t nchunks = ns * (int64_t)S.W16;
+    if (nchunks == S.last_nchunks) return MB200_OK;
+    const std::vector<MBlock>& mblocks = S.P.mblocks;
+    const int grid = S.grid;
+    const int64_t ntiles = (nchunks + TILE_CHUNKS - 1) / TILE_CHUNKS;
+    std::vector<int64_t> h_rng(grid + 1);
+    double total_cost = 0;
+    for (auto& mb : mblocks) total_cost += (double)mb.cost * (double)ntiles;
+    size_t mbi = 0; double acc = 0; int64_t q = 0;
+    h_rng[0] = 0;
+    for (int b = 1; b <= grid; ++b) {
+        const double target = total_cost * b / grid;
+        while (mbi < mblocks.size()) {
+            const double c = (double)mblocks[mbi].cost;
+            const int64_t qend = (int64_t)(mbi + 1) * ntiles;
+            int64_t take = (int64_t)((target - acc) / c + 0.5);
+            if (take < 0) take = 0;
+            if (q + take >= qend) { acc += (double)(qend - q) * c; q = qend; ++mbi; }
+            else { acc += (double)take * c; q += take; break; }
+        }
+        h_rng[b] = (b == grid) ? (int64_t)mblocks.size() * ntiles : q;
+    }
+    MB_CUDA(S.ctx, cudaMemcpyAsync(S.d_rng, h_rng.data(), (size_t)(grid + 1) * 8, cudaMemcpyHostToDevice, S.ctx->stream));
+    MB_CUDA(S.ctx, cudaStreamSynchronize(S.ctx->stream));   // h_rng goes out of scope
+    S.last_nchunks = nchunks;
+    return MB200_OK;
+}
+
+static void simt_batch(ScanCall& S, int64_t s0, int64_t ns) {
+    mb200_ctx* ctx = S.ctx; const ScanPlan& P = S.P;
+    const int t1 = S.tm.begin(T_SCAN);
+    ctx->mask_clean_bytes = 0;
+    if (!P.mblocks.empty()) {
+        ScanArgs a;
+        a.seqw = S.seqs->words; a.rowwords = S.rowwords; a.W = S.W16;
+        a.chunk0 = s0 * (int64_t)S.W16; a.nchunks = ns * (int64_t)S.W16;
+        a.mask = S.d_mask; a.K2pad = P.K2pad;
+        a.blob = S.d_blob; a.mblocks = S.d_mblocks; a.n_mblocks = (int32_t)P.mblocks.size();
+        a.tile_chunks = TILE_CHUNKS; a.ntiles = (a.nchunks + TILE_CHUNKS - 1) / TILE_CHUNKS; a.tile_cap_words = S.tile_cap_words; a.blob_cap_bytes = S.blob_cap;
+        a.cta_range = S.d_rng;
+        a.lens = S.seqs->lens; a.Lb = S.Lb;
+        S.scan_fn<<<S.grid, SCAN_THREADS, S.smem_bytes, ctx->stream>>>(a);
+        ctx->launches[T_SCAN] += 1;
+    }
+    if (!P.lblocks.empty()) {
+        const int64_t warps = ns * (int64_t)P.lblocks.size() * GROUP_SLOTS;
+        auto long_kernel = S.keys ? scan_long_kernel<true> : scan_long_kernel<false>;
+        long_kernel<<<(unsigned)((warps * 32 + 255) / 256), 256, 0, ctx->stream>>>(S.seqs->words, S.rowwords, s0, ns, S.W, P.K2pad, S.d_blob,
+                                                                               S.d_lblocks, (int32_t)P.lblocks.size(), S.d_mask, S.seqs->lens, S.Lb);
+        ctx->launches[T_SCAN] += 1;
+    }
+    S.tm.end(t1);
+}
+
+// ---- per-batch output stages ----------------------------------------------------------------------------------------------------
+// Counts from the masks: chromosome-scale rows without a hit list take the blocked count_long_*; after the tensor-core verifier
+// only the listed units have hits (counts only: counted and cleared; with a hit list: their counts feed the prefix sum, zero
+// elsewhere, and the words stay until emit_kernel has read them); otherwise count_kernel walks every unit.
+static int count_batch(ScanCall& S, int64_t ns, bool tc_done) {
+    mb200_ctx* ctx = S.ctx; const int32_t W = S.W, K2pad = S.P.K2pad, Pp = K2pad / 2;
+    const int t2 = S.tm.begin(T_COUNT);
+    if (!S.want_hits && W > 4096) {
+        const int32_t WB = 512, nblocks = (W + WB - 1) / WB;
+        const int64_t nbt = ns * (int64_t)nblocks * Pp;
+        const size_t o_top1 = 0, o_top2 = o_top1 + (size_t)ns * Pp * 8, o_nh = o_top2 + (size_t)ns * Pp * 8, o_dup = o_nh + (size_t)ns * Pp * 4;
+        const size_t o_cand = (o_dup + (size_t)ns * Pp * 4 + 255) & ~(size_t)255;
+        const int rc = mb_ensure_buf(ctx, BUF_LONG_COUNT, o_cand + (size_t)nbt * sizeof(LongCand)); if (rc) return rc;
+        uint8_t* lb = (uint8_t*)ctx->bufs[BUF_LONG_COUNT];
+        MB_CUDA(ctx, cudaMemsetAsync(lb, 0, o_cand, ctx->stream));
+        count_long_a<<<(unsigned)((nbt + 255) / 256), 256, 0, ctx->stream>>>(S.d_mask, ns, W, K2pad, WB, nblocks, S.d_p2m, S.d_plen, S.d_counts,
+            (unsigned long long*)(lb + o_top1), (unsigned int*)(lb + o_nh), (LongCand*)(lb + o_cand));
+        count_long_b<<<(unsigned)((nbt + 255) / 256), 256, 0, ctx->stream>>>(ns, Pp, nblocks, (const LongCand*)(lb + o_cand), (const unsigned long long*)(lb + o_top1),
+            (unsigned long long*)(lb + o_top2), (unsigned int*)(lb + o_dup));
+        count_long_c<<<(unsigned)((ns * Pp + 255) / 256), 256, 0, ctx->stream>>>(ns, Pp, S.d_p2m, S.d_plen,
+            (const unsigned long long*)(lb + o_top1), (const unsigned long long*)(lb + o_top2), (const unsigned int*)(lb + o_dup), (const unsigned int*)(lb + o_nh), S.d_counts);
+        ctx->launches[T_COUNT] += 3;
+    } else if (tc_done && S.tc_units) {
+        if (S.want_hits) MB_CUDA(ctx, cudaMemsetAsync(S.d_unit_cnt, 0, (size_t)ns * S.K * 2 * 4, ctx->stream));
+        count_listed_kernel<<<S.grid * 8, 256, 0, ctx->stream>>>(S.d_mask, S.d_tc_ulist, S.d_tc_ctr + 4, W, K2pad, S.d_p2m, S.d_plen, S.d_counts, nullptr,
+                                                                  S.want_hits ? S.d_unit_cnt : nullptr, S.K, S.want_hits ? 0 : 1);
+        ctx->launches[T_COUNT] += 1;
+        if (!S.want_hits) ctx->mask_clean_bytes = (size_t)ns * S.mask_bytes_per_seq;   // every word with a bit belongs to a listed unit and was cleared
+    } else {
+        count_kernel<<<(unsigned)((ns * Pp + 255) / 256), 256, 0, ctx->stream>>>(S.d_mask, ns, W, K2pad, S.d_p2m, S.d_plen, S.d_counts, S.d_unit_cnt, S.K);
+        ctx->launches[T_COUNT] += 1;
+    }
+    S.tm.end(t2);
+    MB_CUDA(ctx, cudaGetLastError());
+    return MB200_OK;
+}
+
+// Hit list of a batch: prefix sum over the unit counts, emit_kernel, copy to the caller's array (or, once it is outgrown, to the
+// list held in the ctx), then clear the listed words of the tensor-core path.
+static int emit_batch(ScanCall& S, int64_t s0, int64_t ns, bool tc_done) {
+    mb200_ctx* ctx = S.ctx; const ScanOut& o = S.out;
+    const int64_t units = ns * S.K * 2;
+    const int64_t nb = (units + PS_TILE - 1) / PS_TILE;
+    const int t3 = S.tm.begin(T_EMIT);
+    ps_block_sums<<<(unsigned)nb, PS_THREADS, 0, ctx->stream>>>(S.d_unit_cnt, units, S.d_bsum);
+    ps_scan_sums<<<1, PS_THREADS, 0, ctx->stream>>>(S.d_bsum, nb, S.d_total);
+    ps_apply<<<(unsigned)nb, PS_THREADS, 0, ctx->stream>>>(S.d_unit_cnt, units, S.d_bsum, S.d_unit_off);
+    S.tm.end(t3);
+    ctx->launches[T_EMIT] += 3;
+    unsigned long long h_total = 0;
+    MB_CUDA(ctx, cudaMemcpyAsync(&h_total, S.d_total, 8, cudaMemcpyDeviceToHost, ctx->stream));
+    MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    S.hits_needed += (int64_t)h_total;
+    // a list that outgrows the caller's buffer is kept in the ctx (host memory) and handed over by mb200_scan_take_hits:
+    // the caller's retry does not pay for the scan, count and prefix kernels a second time
+    const bool spill = S.hits_needed > o.hits_cap;
+    if (spill && ctx->held_hits.empty() && S.hits_written) ctx->held_hits.assign(o.hits, o.hits + S.hits_written);
+    if (h_total) {
+        const int rc = mb_ensure_buf(ctx, BUF_HITS, (size_t)h_total * sizeof(mb200_hit)); if (rc) return rc;
+        mb200_hit* d_hits = (mb200_hit*)ctx->bufs[BUF_HITS];
+        const int t4 = S.tm.begin(T_EMIT);
+        emit_kernel<<<(unsigned)((units + 255) / 256), 256, 0, ctx->stream>>>(S.d_mask, S.seqs->words, S.rowwords, s0, ns, S.W, S.P.K2pad, S.K,
+                                                                           S.d_em, S.d_blob, S.d_unit_cnt, S.d_unit_off, d_hits);
+        S.tm.end(t4);
+        ctx->launches[T_EMIT] += 1;
+        MB_CUDA(ctx, cudaGetLastError());
+        const int t5 = S.tm.begin(T_D2H);
+        mb200_hit* dst = o.hits + S.hits_written;
+        if (spill) { ctx->held_hits.resize((size_t)S.hits_written + (size_t)h_total); dst = ctx->held_hits.data() + S.hits_written; }
+        MB_CUDA(ctx, cudaMemcpyAsync(dst, d_hits, (size_t)h_total * sizeof(mb200_hit), cudaMemcpyDeviceToHost, ctx->stream));
+        S.tm.end(t5);
+        MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+        S.hits_written += (int64_t)h_total;
+    }
+    if (tc_done && S.tc_units) {
+        clear_listed_kernel<<<S.grid * 8, 256, 0, ctx->stream>>>(S.d_mask, S.d_tc_ulist, S.d_tc_ctr + 4, S.W, S.P.K2pad);
+        ctx->launches[T_EMIT] += 1;
+        ctx->mask_clean_bytes = (size_t)ns * S.mask_bytes_per_seq;
+    }
+    return MB200_OK;
+}
+
+static int hist_batch(ScanCall& S, int64_t s0, int64_t ns) {
+    mb200_ctx* ctx = S.ctx;
+    const int64_t units = ns * S.K * 2;
+    const int t7 = S.tm.begin(T_EMIT);
+    hist_kernel<<<(unsigned)((units + 255) / 256), 256, 0, ctx->stream>>>(S.d_mask, S.seqs->words, S.rowwords, s0, ns, S.W, S.P.K2pad, S.K, S.d_em, S.d_blob, S.d_hist);
+    S.tm.end(t7);
+    ctx->launches[T_EMIT] += 1;
+    MB_CUDA(ctx, cudaGetLastError());
+    return MB200_OK;
+}
+
+// Best keys of a batch reduced to one 64-bit slot per (row, motif), then records to the caller (BEST) or, for anchors s0/2 ..
+// (s0 + ns)/2, counts into the spacing histogram and the sites when asked (SPACING).
+static int best_batch(ScanCall& S, int64_t s0, int64_t ns) {
+    mb200_ctx* ctx = S.ctx; const SpacingJob* sp = S.out.sp; const int K = S.K;
+    const int t2 = S.tm.begin(T_COUNT);
+    MB_CUDA(ctx, cudaMemsetAsync(S.d_best64, 0, (size_t)ns * K * 8, ctx->stream));
+    const int64_t rthreads = ns * (int64_t)S.best_nch * (S.P.K2pad / 2);
+    best_reduce_kernel<<<(unsigned)((rthreads + 255) / 256), 256, 0, ctx->stream>>>(S.d_mask, ns, S.W16, S.P.K2pad, S.best_nch, S.d_p2m, K, S.d_best64);
+    mb200_best* dst = nullptr; int64_t n = 0;
+    if (sp) {
+        const int64_t na = ns / 2;
+        spacing_kernel<<<(unsigned)((na * K + 255) / 256), 256, 0, ctx->stream>>>(S.d_best64, na, K, S.d_anchors + s0 / 2, S.d_spthr, S.d_mlen, sp->margin,
+                                                                                 S.d_sphist, sp->sites ? S.d_best : nullptr);
+        if (sp->sites) { dst = sp->sites + (size_t)(s0 / 2) * K; n = na * K; }
+    } else {
+        best_finalize_kernel<<<(unsigned)((ns * K + 255) / 256), 256, 0, ctx->stream>>>(S.d_best64, ns * K, S.d_best);
+        dst = S.out.best + (size_t)s0 * K; n = ns * K;
+    }
+    S.tm.end(t2);
+    ctx->launches[T_COUNT] += 2;
+    MB_CUDA(ctx, cudaGetLastError());
+    if (dst) {
+        const int t6 = S.tm.begin(T_D2H);
+        MB_CUDA(ctx, cudaMemcpyAsync(dst, S.d_best, (size_t)n * sizeof(mb200_best), cudaMemcpyDeviceToHost, ctx->stream));
+        S.tm.end(t6);
+    }
+    return MB200_OK;
+}
+
+// One batch outside the pipelined loop: the masks (or best keys), then the output stage of the mode.
+static int run_batch(ScanCall& S, int64_t s0, int64_t ns) {
+    int rc = wait_for_rows(S, s0 + ns); if (rc) return rc;
+    rc = update_cta_ranges(S, ns); if (rc) return rc;
+    bool tc_done = false;
+    if (S.use_tc) { rc = tc_serial_batch(S, s0, ns, &tc_done); if (rc) return rc; }
+    if (!tc_done) simt_batch(S, s0, ns);
+    MB_CUDA(S.ctx, cudaGetLastError());
+    if (S.keys) return best_batch(S, s0, ns);                       // BEST, SPACING
+    rc = count_batch(S, ns, tc_done); if (rc) return rc;            // HITS, HIST
+    if (S.out.hist) return hist_batch(S, s0, ns);
+    return S.want_hits ? emit_batch(S, s0, ns, tc_done) : MB200_OK;
+}
+
+static int scan_finish(ScanCall& S) {
+    mb200_ctx* ctx = S.ctx; const ScanOut& o = S.out;
+    int rc = copy_totals(S, o.hist ? (void*)S.d_hist : (void*)S.d_counts, &S.tm); if (rc) return rc;
+    if (o.sp) {
+        const int t9 = S.tm.begin(T_D2H);
+        MB_CUDA(ctx, cudaMemcpyAsync(o.sp->hist, S.d_sphist, S.sphist_bytes, cudaMemcpyDeviceToHost, ctx->stream));
+        S.tm.end(t9);
+    }
+    S.tm.end(S.t_total);
+    MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    S.tm.collect();
+    if (S.d_tc_ctr && getenv("MB200_SCAN_TC_STATS")) {
+        fprintf(stderr, "[mb200] tensor-core scan: %s, candidates %llu, hits %llu, scan %.3f ms, count %.3f ms\n", S.use_tc ? "used" : "fell back", S.tc_stat_cand,
+                S.tc_stat_hits, ctx->ms[T_SCAN], ctx->ms[T_COUNT]);
+    }
+    if (S.seqs->pending) { rc = mb_seqs_finish(ctx, const_cast<mb200_seqs*>(S.seqs)); if (rc) return rc; }      // the upload has completed: report bad symbols
+    if (o.n_hits) *o.n_hits = S.hits_needed;
+    if (S.want_hits && S.hits_needed > o.hits_cap)
+        MB_FAIL(ctx, MB200_E_HITS_OVERFLOW, "scan: %lld hits, capacity %lld", (long long)S.hits_needed, (long long)o.hits_cap);
+    return MB200_OK;
+}
+
+static int32_t scan_impl(mb200_ctx* ctx, const mb200_seqs* seqs, const uint16_t* pwms_f16, const int64_t* lens, int32_t K,
+                         int32_t maxlen, const uint16_t* thresh_f16, uint32_t flags, const ScanOut& out) {
+    if (!ctx) return MB200_E_INVALID;
+    ScanCall S{ctx, seqs, out, K, flags};
+    int rc = scan_validate(S, pwms_f16, lens, maxlen); if (rc) return rc;
+    rc = scan_plan(S, pwms_f16, lens, maxlen, thresh_f16); if (rc) return rc;
+    if (S.N == 0 || S.Lb - S.P.minlen + 1 <= 0) return scan_empty(S);
+    rc = stage_buffers(S, lens); if (rc) return rc;
+    std::vector<int64_t> todo;                                     // first rows of the batches still to run
+    for (int64_t s0 = 0; s0 < S.N; s0 += S.seqs_per_batch) todo.push_back(s0);
+    if (S.use_tc && !S.want_hits && S.tc_units) { rc = tc_pipelined(S, todo); if (rc) return rc; }
+    for (const int64_t s0 : todo) { rc = run_batch(S, s0, std::min(S.seqs_per_batch, S.N - s0)); if (rc) return rc; }
+    return scan_finish(S);
 }
 
 extern "C" int32_t mb200_scan(mb200_ctx* ctx, const mb200_seqs* seqs, const uint16_t* pwms_f16, const int64_t* lens, int32_t K,
                               int32_t maxlen, const uint16_t* thresh_f16, uint32_t flags, mb200_hit* hits, int64_t hits_cap,
                               int64_t* n_hits, int64_t* counts) {
-    return scan_impl(ctx, seqs, pwms_f16, lens, K, maxlen, thresh_f16, flags, hits, hits_cap, n_hits, counts, nullptr, nullptr);
+    ScanOut out; out.hits = hits; out.hits_cap = hits_cap; out.n_hits = n_hits; out.counts = counts;
+    return scan_impl(ctx, seqs, pwms_f16, lens, K, maxlen, thresh_f16, flags, out);
 }
 
 // Diagnostic (host arithmetic only, ctx-free): the tensor-core pre-filter's error bound and threshold for one (motif, strand) slot.
@@ -1762,7 +1804,8 @@ extern "C" int32_t mb200_scan_hist(mb200_ctx* ctx, const mb200_seqs* seqs, const
     if (!ctx) return MB200_E_INVALID;
     if (!hist) MB_FAIL(ctx, MB200_E_INVALID, "scan_hist: null histogram");
     const uint32_t f = (flags & (MB200_SCAN_FWD | MB200_SCAN_RC | MB200_SCAN_REDUCE));
-    return scan_impl(ctx, seqs, pwms_f16, lens, K, maxlen, nullptr, f, nullptr, 0, nullptr, nullptr, hist, nullptr);
+    ScanOut out; out.kind = ScanOut::HIST; out.hist = hist;
+    return scan_impl(ctx, seqs, pwms_f16, lens, K, maxlen, nullptr, f, out);
 }
 
 extern "C" int32_t mb200_scan_best(mb200_ctx* ctx, const mb200_seqs* seqs, const uint16_t* pwms_f16, const int64_t* lens, int32_t K,
@@ -1770,7 +1813,8 @@ extern "C" int32_t mb200_scan_best(mb200_ctx* ctx, const mb200_seqs* seqs, const
     if (!ctx) return MB200_E_INVALID;
     if (!best) MB_FAIL(ctx, MB200_E_INVALID, "scan_best: null output");
     if (flags & ~(MB200_SCAN_FWD | MB200_SCAN_RC)) MB_FAIL(ctx, MB200_E_INVALID, "scan_best: flags 0x%x: only MB200_SCAN_FWD | MB200_SCAN_RC", flags);
-    return scan_impl(ctx, seqs, pwms_f16, lens, K, maxlen, nullptr, flags, nullptr, 0, nullptr, nullptr, nullptr, best);
+    ScanOut out; out.kind = ScanOut::BEST; out.best = best;
+    return scan_impl(ctx, seqs, pwms_f16, lens, K, maxlen, nullptr, flags, out);
 }
 
 // The margins of every anchor become rows 2i (left) and 2i + 1 (right) of a fixed-length store (mb200_seqs_windows); the best-site
@@ -1811,7 +1855,8 @@ extern "C" int32_t mb200_scan_spacing(mb200_ctx* ctx, const mb200_seqs* seqs, co
     float pack_ms = 0;
     MB_CUDA(ctx, cudaEventElapsedTime(&pack_ms, g.e0, g.e1));
     const SpacingJob job = {anchors, n_anchors, n_primary, margin, thresh_f16, hist, sites};
-    rc = scan_impl(ctx, g.win, pwms_f16, lens, K, maxlen, nullptr, MB200_SCAN_FWD | MB200_SCAN_RC, nullptr, 0, nullptr, nullptr, nullptr, nullptr, &job);
+    ScanOut out; out.kind = ScanOut::SPACING; out.sp = &job;
+    rc = scan_impl(ctx, g.win, pwms_f16, lens, K, maxlen, nullptr, MB200_SCAN_FWD | MB200_SCAN_RC, out);
     if (rc) return rc;
     ctx->ms[T_PACK] += pack_ms; ctx->ms[T_TOTAL] += pack_ms; ctx->launches[T_PACK] += 1;       // scan_impl reset the timing
     return MB200_OK;

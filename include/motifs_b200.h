@@ -344,6 +344,30 @@ int32_t mb200_count_matrices(mb200_ctx* ctx, const mb200_seqs* seqs, const mb200
 int32_t mb200_pvalue2score(mb200_ctx* ctx, const double* pwm, int32_t m, double pval, double eps, const double* bg,
                            double* score, int32_t* found);
 
+/* ---- exact p-values of the scan's score: new; the exact p-value of greedy_search!'s Float16 score (_h3_1_alignment.jl:18-36).
+ *      A window's score is a sequential Float16 sum, so after every column it is one of the 63 489 non-NaN Float16 values (-0 = +0).
+ *      Under a background of independent bases with frequencies bg (A,C,G,T), the survival function S(t) = P(score >= t) of every
+ *      (motif, strand) slot is computed exactly over those values on the device, in float64, column by column (DESIGN.md §3.1c).  The
+ *      table is the scan's own effective table (the Inf * 0 = NaN rule) and, for comp = 1, that of reverse(pwm).  NaN windows carry no
+ *      mass: S(-Inf) is the probability that a window is not NaN.  Two builds of one input are bit-identical.                     */
+typedef struct mb200_pvtab mb200_pvtab;
+/* pwms_f16, lens, K, maxlen: exactly as for mb200_scan.  The tables take 2K x 63 489 float64 (0.5 MB per slot) of device memory
+ * and the build at most 1 GiB more of working space.  MB200_E_INVALID: a null pointer, K < 1, a len outside [1, maxlen], a bg entry
+ * that is negative or non-finite, or a bg whose sum is not within 1e-6 of 1.  MB200_E_NOMEM: the tables do not fit.          */
+int32_t mb200_pvtab_create(mb200_ctx* ctx, const uint16_t* pwms_f16, const int64_t* lens, int32_t K, int32_t maxlen,
+                           const double* bg, mb200_pvtab** out);
+int32_t mb200_pvtab_destroy(mb200_ctx* ctx, mb200_pvtab* t);
+/* per slot and pval[k] in [0, 1]: s* = the smallest non-NaN value with S(s*) <= pval[k], thresh_f16[k*2 + comp] = the Float16 value
+ * just below s*, so that score > thresh <=> S(score) <= pval[k] for every non-NaN score; -Inf when s* = -Inf, +Inf when no value
+ * qualifies (pval[k] < S(+Inf)).  A scan at this threshold still needs score > 0.  MB200_E_INVALID: a p outside [0, 1].      */
+int32_t mb200_pvtab_thresholds(mb200_ctx* ctx, const mb200_pvtab* t, const double* pval, uint16_t* thresh_f16);
+/* p[i] = S(score_f16[i]) of slot (motif[i], comp[i]), gathered on the device; NaN for a NaN score, -0 is looked up as +0.
+ * MB200_E_INVALID: a motif >= K or a comp > 1.                                                                                */
+int32_t mb200_pvtab_lookup(mb200_ctx* ctx, const mb200_pvtab* t, const uint16_t* motif, const uint8_t* comp,
+                           const uint16_t* score_f16, int64_t n, double* p);
+/* the whole table of slot (k, comp): out[65536] indexed by Float16 bit pattern, NaN for the NaN patterns. */
+int32_t mb200_pvtab_survival(mb200_ctx* ctx, const mb200_pvtab* t, int32_t k, int32_t comp, double* out);
+
 /* ---- code components -> triplet dictionary: replaces get_scanning_range_of_filtered_code_components, enumerate_triplets /
  *      insert_H! (inference/_2_enumerate.jl:25-65) and the key counting of get_words / get_enriched_keys
  *      (inference/_3_make_pfms.jl:3-26).  A key is f1 | f2<<8 | f3<<16 | d12<<24 | d13<<40 with 1-based filter ids (the fields of

@@ -388,6 +388,39 @@ function pvec_from_test_data(ctx, ms, seqs_test, seqs_bg_test, pwms, NL_test::In
     pvec, Float64.(c[2, :])
 end
 
+# exact p-values of greedy_search!'s Float16 score (new): survival tables of every (motif, strand) under an independent-base
+# background bg (A, C, G, T), built on the device; the handle owns them until pvtab_destroy.  pwms / lens as for gpu_scan.
+function pvtab_create(ctx, pwms::Array{Float16,3}, lens::Vector{Int64}, bg::Vector{Float64})
+    K, _, maxlen = size(pwms)
+    h = Ref{Ptr{Cvoid}}(C_NULL)
+    GC.@preserve pwms lens bg check(ctx, ccall((:mb200_pvtab_create, lib), Int32,
+        (Ptr{Cvoid}, Ptr{Float16}, Ptr{Int64}, Int32, Int32, Ptr{Float64}, Ref{Ptr{Cvoid}}), ctx, pwms, lens, K, maxlen, bg, h))
+    h[]
+end
+pvtab_destroy(ctx, t) = ccall((:mb200_pvtab_destroy, lib), Int32, (Ptr{Cvoid}, Ptr{Cvoid}), ctx, t)
+# (2, K) Float16 thresholds, column k = (forward, reverse(pwm)): score > thresh <=> p-value <= pval[k]
+function pvtab_thresholds(ctx, t, pval::Vector{Float64})
+    out = zeros(Float16, 2, length(pval))
+    GC.@preserve pval out check(ctx, ccall((:mb200_pvtab_thresholds, lib), Int32,
+        (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Float64}, Ptr{Float16}), ctx, t, pval, out))
+    out
+end
+# p-values of hits (1-based motif, comp = true for reverse(pwm)); NaN for a NaN score
+function pvtab_lookup(ctx, t, motif::Vector{<:Integer}, comp::AbstractVector{Bool}, score::Vector{Float16})
+    m0, c0 = UInt16.(motif .- 1), UInt8.(comp)
+    p = zeros(Float64, length(score))
+    GC.@preserve m0 c0 score p check(ctx, ccall((:mb200_pvtab_lookup, lib), Int32,
+        (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{UInt16}, Ptr{UInt8}, Ptr{Float16}, Int64, Ptr{Float64}), ctx, t, m0, c0, score, length(score), p))
+    p
+end
+# the whole table of (motif k, strand comp): 65536 Float64 indexed by Float16 bit pattern + 1, NaN for the NaN patterns
+function pvtab_survival(ctx, t, k::Integer, comp::Bool)
+    out = zeros(Float64, 65536)
+    GC.@preserve out check(ctx, ccall((:mb200_pvtab_survival, lib), Int32,
+        (Ptr{Cvoid}, Ptr{Cvoid}, Int32, Int32, Ptr{Float64}), ctx, t, k - 1, Int32(comp), out))
+    out
+end
+
 # positions -> count matrices: posdicts2countmats / msa_add! (inference/_h6_positions2countmat.jl:7-54).  sites: 0-based
 # (motif, seq, pos, comp) rows; returns Vector of 4 x len_k UInt32 matrices (add the 0.01 pseudo-count and convert on the host).
 struct Site; motif::UInt32; seq::UInt32; pos::UInt32; comp::UInt32; end

@@ -131,6 +131,11 @@ def load():
         "mb200_csc_codes": (i32, [p, p, p, i64, i64, p, i64, C.POINTER(i64)]),
         "mb200_count_matrices": (i32, [p, p, p, i64, p, i32, i32, p]),
         "mb200_pvalue2score": (i32, [p, p, i32, C.c_double, C.c_double, p, p, p]),
+        "mb200_pvtab_create": (i32, [p, p, p, i32, i32, p, C.POINTER(p)]),
+        "mb200_pvtab_destroy": (i32, [p, p]),
+        "mb200_pvtab_thresholds": (i32, [p, p, p, p]),
+        "mb200_pvtab_lookup": (i32, [p, p, p, p, p, i64, p]),
+        "mb200_pvtab_survival": (i32, [p, p, i32, i32, p]),
         "mb200_triplets_create": (i32, [p, p, p, p, i64, p, p, p]),
         "mb200_triplets_destroy": (i32, [p, p]),
         "mb200_triplets_ranges": (i32, [p, p, p, p]),
@@ -337,6 +342,18 @@ class Context:
         self._check(self._lib.mb200_scan_best(self._h, seqs._h, _ptr(pw), _ptr(ln), K, maxlen, flags, _ptr(out)))
         return out
 
+    def score_null(self, pwms_f16: np.ndarray, lens, bg) -> "ScoreNull":
+        """mb200_pvtab_create: the exact null distribution of every (motif, strand) slot's Float16 window score under a background
+        of independent bases with frequencies bg (A, C, G, T).  pwms_f16 and lens as for scan."""
+        pw, ln = self._pwm_arrays(pwms_f16, lens)
+        maxlen, _, K = pw.shape
+        b = np.ascontiguousarray(bg, np.float64)
+        if b.shape != (4,):
+            raise ValueError("bg must hold 4 frequencies (A, C, G, T)")
+        h = C.c_void_p()
+        self._check(self._lib.mb200_pvtab_create(self._h, _ptr(pw), _ptr(ln), K, maxlen, _ptr(b), C.byref(h)))
+        return ScoreNull(self, h, K)
+
     def seqs_windows(self, seqs: "Sequences", rows, starts, length: int) -> "Sequences":
         """mb200_seqs_windows: a new fixed-length store whose row i holds bases [starts[i], starts[i] + length) of row rows[i] of
         seqs (fixed or ragged)."""
@@ -370,6 +387,50 @@ class Context:
         self._check(self._lib.mb200_scan_spacing(self._h, seqs._h, _ptr(an), len(an), int(n_primary), int(margin), _ptr(pw), _ptr(ln),
                                                   K, maxlen, _ptr(th), _ptr(hist), _ptr(sites)))
         return hist, sites
+
+
+class ScoreNull:
+    """mb200_pvtab: survival tables S(t) = P(score >= t) of the scan's Float16 score for every (motif k, strand comp) slot, held on
+    the device (Context.score_null)."""
+
+    def __init__(self, ctx: Context, handle, K):
+        self.ctx, self._h, self.K = ctx, handle, int(K)
+
+    def thresholds(self, pvals) -> np.ndarray:
+        """(K, 2) float16: per slot the threshold t with score > t <=> S(score) <= p (mb200_pvtab_thresholds); pvals: one p or K."""
+        p = np.ascontiguousarray(np.broadcast_to(np.asarray(pvals, np.float64), (self.K,)))
+        out = np.zeros((self.K, 2), np.uint16)
+        self.ctx._check(self.ctx._lib.mb200_pvtab_thresholds(self.ctx._h, self._h, _ptr(p), _ptr(out)))
+        return out.view(np.float16)
+
+    def pvalues(self, motif, comp, score_f16) -> np.ndarray:
+        """float64 S(score) of each (motif, comp, score) on the device (mb200_pvtab_lookup); NaN for a NaN score."""
+        m = np.ascontiguousarray(motif, np.uint16).reshape(-1)
+        c = np.ascontiguousarray(comp, np.uint8).reshape(-1)
+        s = np.asarray(score_f16)
+        s = np.ascontiguousarray(s.view(np.uint16) if s.dtype == np.float16 else s.astype(np.uint16)).reshape(-1)
+        if not (len(m) == len(c) == len(s)):
+            raise ValueError("motif, comp and score_f16 must have one length")
+        out = np.empty(len(s), np.float64)
+        self.ctx._check(self.ctx._lib.mb200_pvtab_lookup(self.ctx._h, self._h, _ptr(m), _ptr(c), _ptr(s), len(s), _ptr(out)))
+        return out
+
+    def survival(self, k: int, comp: int) -> np.ndarray:
+        """(65536,) float64 S indexed by Float16 bit pattern, NaN for the NaN patterns (mb200_pvtab_survival)."""
+        out = np.empty(65536, np.float64)
+        self.ctx._check(self.ctx._lib.mb200_pvtab_survival(self.ctx._h, self._h, int(k), int(comp), _ptr(out)))
+        return out
+
+    def free(self):
+        if self._h and self.ctx._h:
+            self.ctx._lib.mb200_pvtab_destroy(self.ctx._h, self._h)
+        self._h = None
+
+    def __del__(self):
+        try:
+            self.free()
+        except Exception:
+            pass
 
 
 def fasta_read(path: str, max_entries: int = 100000) -> np.ndarray:

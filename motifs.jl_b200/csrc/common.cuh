@@ -25,7 +25,8 @@ enum {
     BUF_TC_LIST = 9,      // tensor-core scan: candidate lists and counters (two sets)
     BUF_TC_UNITS = 10,    // tensor-core scan: listed units and their bitmap (two sets)
     BUF_SPACING = 11,     // spacing: anchors, thresholds, secondary lengths
-    BUF_N = 12
+    BUF_PVALUE = 12,      // p-value lookups (mb200_pvtab_lookup): keys and results of one chunk
+    BUF_N = 13
 };
 
 struct mb200_ctx {
@@ -78,6 +79,17 @@ static const int64_t SEQ_PAD_WORDS = 64;
 int mb_seqs_alloc(mb200_ctx* ctx, int64_t N, int64_t Lb, mb200_seqs** out);   // empty store (tail pad zeroed on ctx->stream)
 int mb_seqs_set_lens(mb200_ctx* ctx, mb200_seqs* s, std::vector<int64_t> hlens);   // makes s ragged: uploads the row lengths (synchronous)
 static inline int64_t mb_row_len(const mb200_seqs* s, int64_t n) { return s->ragged ? s->hlens[(size_t)n] : s->Lb; }
+
+// Effective table entry of the scan: what column j of pwm (comp = 0) or of reverse(pwm) (comp = 1: rc[b][j] = pwm[3-b][len-1-j])
+// adds for base b.  greedy_search! adds pwm * onehot over all four bases, so a non-finite entry of another base turns into
+// Inf * 0 = NaN (0x7E00).  pw(a, j) returns the Float16 bits of pwm entry (base a, column j).
+template <class PW> static inline uint16_t mb_eff_entry(PW pw, int len, int b, int j, int comp) {
+    const int jj = comp ? len - 1 - j : j;
+    const uint16_t v = pw(comp ? 3 - b : b, jj);
+    int others = -(int)((v & 0x7C00u) == 0x7C00u);
+    for (int a = 0; a < 4; ++a) others += (pw(a, jj) & 0x7C00u) == 0x7C00u;
+    return others > 0 ? (uint16_t)0x7E00u : v;
+}
 
 #define MB_FAIL(ctx, code, ...) do { char _b[512]; snprintf(_b, sizeof _b, __VA_ARGS__); \
     if (ctx) (ctx)->err = _b; return (code); } while (0)

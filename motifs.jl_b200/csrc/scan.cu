@@ -1065,24 +1065,12 @@ static int build_plan(mb200_ctx* ctx, const uint16_t* pwms, const int64_t* lens,
                     // table layout [col][slot][base]
                     P.em[k].tab_off = mb.blob_off + toff + (int64_t)i * 16;
                     P.em[k].col_stride = COL_BYTES; P.em[k].base_stride = 2; P.em[k].strand_stride = 8;
-                    for (int j = 0; j < len; ++j) {
-                        int nf_f = 0;
-                        for (int a2 = 0; a2 < 4; ++a2) nf_f += h16_nonfinite(pw(k, a2, j));
+                    auto pwk = [&](int a, int ind) { return pw(k, a, ind); };
+                    for (int j = 0; j < len; ++j)
                         for (int b = 0; b < 4; ++b) {
-                            // forward table: column j, base b.  A non-selected non-finite entry times 0 is NaN
-                            // in the reference's sum (greedy_search! adds pwm*x for all four a).
-                            const uint16_t v = pw(k, b, j);
-                            const uint16_t ef = (nf_f - (int)h16_nonfinite(v)) > 0 ? (uint16_t)0x7E00u : v;
-                            T[((size_t)j * GROUP_SLOTS + i * 2 + 0) * 4 + b] = ef;
-                            // reverse(pwm): rc[a][j] = pwm[3-a][len-1-j]; its column j mirrors forward column len-1-j
-                            const int jr = len - 1 - j;
-                            const uint16_t vr = pw(k, 3 - b, jr);
-                            int nf_r = 0;
-                            for (int a2 = 0; a2 < 4; ++a2) nf_r += h16_nonfinite(pw(k, a2, jr));
-                            const uint16_t er = (nf_r - (int)h16_nonfinite(vr)) > 0 ? (uint16_t)0x7E00u : vr;
-                            T[((size_t)j * GROUP_SLOTS + i * 2 + 1) * 4 + b] = er;
+                            T[((size_t)j * GROUP_SLOTS + i * 2 + 0) * 4 + b] = mb_eff_entry(pwk, len, b, j, 0);
+                            T[((size_t)j * GROUP_SLOTS + i * 2 + 1) * 4 + b] = mb_eff_entry(pwk, len, b, j, 1);
                         }
-                    }
                 }
                 gm.thr[i * 2 + 0] = thr_f; gm.thr[i * 2 + 1] = thr_r;
             }

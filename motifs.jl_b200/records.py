@@ -491,3 +491,120 @@ def spacing_enrichment(sp: Spacing, secondary_lens) -> SpacingEnrichment:
             res.q[p, k], res.gap[p, k], res.count[p, k] = q, g, c
             res.p[p, k], res.p_adj[p, k] = pv, min(1.0, pv * B * K)
     return res
+
+
+# ---- exact p-values and q-values of scan hits and best sites (FIMO-style) ------------------------------------------------
+def base_background(rec: Records) -> np.ndarray:
+    """(4,) float64 A/C/G/T frequencies of the records' fragments, averaged with their reverse complement (A = T, C = G): the
+    default background of scan_fasta_pvalues and best_site_pvalues.  Both strands are scanned, so the null of either strand
+    should not depend on which strand the file happens to hold."""
+    code = np.full(256, 4, np.int64)
+    for i, c in enumerate(b"ACGT"):
+        code[c] = i
+    n = np.bincount(code[np.asarray(rec.bases, np.uint8)], minlength=5)[:4].astype(np.float64)
+    n = n + n[::-1]
+    if n.sum() == 0:
+        raise ValueError("the records hold no A/C/G/T bases: no background")
+    return n / n.sum()
+
+
+def _windows_per(frag_len, lens):
+    """(F, K) int64: windows of every motif on one strand of every fragment, max(0, L_f - m_k + 1)."""
+    return np.maximum(0, np.asarray(frag_len, np.int64)[:, None] - np.asarray(lens, np.int64)[None, :] + 1)
+
+
+def bh_qvalues(p, n_tests) -> np.ndarray:
+    """Benjamini-Hochberg q-values of hits with p-values p among n_tests >= len(p) tests whose other p-values are larger:
+    q_(i) = min(1, min_{j >= i} p_(j) n_tests / j) over the hits sorted by p (ties share the q of the last of them)."""
+    p = np.asarray(p, np.float64)
+    q = np.empty(len(p))
+    if len(p) == 0:
+        return q
+    o = np.argsort(p, kind="stable")
+    s = p[o] * float(n_tests) / np.arange(1, len(p) + 1)
+    q[o] = np.minimum(1.0, np.minimum.accumulate(s[::-1])[::-1])
+    return q
+
+
+def sidak(site_p, n) -> np.ndarray:
+    """1 - (1 - site_p)^n, evaluated as -expm1(n log1p(-site_p)) (stable for small site_p): the probability that the best of n
+    independent windows scores at least as high as a site of p-value site_p (CentriMo's and AME's correction)."""
+    site_p = np.asarray(site_p, np.float64)
+    with np.errstate(divide="ignore", invalid="ignore"):
+        return -np.expm1(np.asarray(n, np.float64) * np.log1p(-site_p))
+
+
+@dataclass
+class PValueScan:
+    """Hits of scan_fasta_pvalues: RECORD_HIT_DTYPE sorted by (record, motif, comp, pos) with p-value <= the requested one.
+    pvalue: exact P(score >= the hit's score) of one window of its strand under bg; qvalue: Benjamini-Hochberg per motif over
+    n_tests[k] windows (both strands of every fragment).  thresh: (K, 2) per-strand Float16 thresholds (score > thresh <=> p <=
+    the requested p); clamped: slots whose threshold is below 0, where the scan's score > 0 rule drops sites with p small
+    enough but score <= 0."""
+    hits: np.ndarray
+    pvalue: np.ndarray           # (n,) float64
+    qvalue: np.ndarray           # (n,) float64
+    n_tests: np.ndarray          # (K,) int64
+    thresh: np.ndarray           # (K, 2) float16
+    bg: np.ndarray               # (4,) float64
+    names: List[str]
+    clamped: np.ndarray          # (K, 2) bool
+
+
+def scan_fasta_pvalues(ctx, path_or_records, motifs_or_pwms, pvalue: float = 1e-4, *, bg=None,
+                       max_padding: float = 1.0 / 8) -> PValueScan:
+    """Scan a FASTA file (a path or a Records) "at p < pvalue": every window on either strand whose exact p-value under a
+    background of independent bases is at most pvalue, with Benjamini-Hochberg q-values per motif.
+
+    The null tables come from Context.score_null (exact for the scan's Float16 score).  The fragments are scanned as in
+    scan_fasta at the per-motif threshold min(fwd, rc) of the two strands' thresholds; each hit's p-value is looked up on its
+    own strand and hits with p > pvalue (the strand with the higher threshold) are dropped.  The q-values are exact from the
+    hits alone: every unreported window has a larger p-value and counts as p = 1.  The scan reports only score > 0, so on a
+    clamped slot (threshold < 0, i.e. pvalue above P(score > 0)) sites with p <= pvalue and score <= 0 are missing; their q
+    values then treat them as p = 1 (conservative).  bg: (4,) A/C/G/T frequencies, default base_background(records)."""
+    rec = path_or_records if isinstance(path_or_records, Records) else read_records(path_or_records)
+    pw, lens, _ = _pwm_args(motifs_or_pwms, None)
+    K = len(lens)
+    bg = base_background(rec) if bg is None else np.asarray(bg, np.float64)
+    null = ctx.score_null(pw, lens, bg)
+    try:
+        thresh = null.thresholds(float(pvalue))
+        res = _scan_records(ctx, rec, pw, lens, np.minimum(thresh[:, 0], thresh[:, 1]), True, max_padding)
+        hits = res.hits
+        p = null.pvalues(hits["motif"], hits["comp"], hits["score_f16"])
+    finally:
+        null.free()
+    keep = p <= pvalue
+    hits, p = hits[keep], p[keep]
+    n_tests = 2 * _windows_per(rec.frag_len, lens).sum(axis=0).astype(np.int64)
+    q = np.empty(len(p))
+    order = np.argsort(hits["motif"], kind="stable")          # the hits of each motif, as one slice of `order`
+    cut = np.searchsorted(hits["motif"][order], np.arange(K + 1))
+    for k in np.nonzero(np.diff(cut))[0]:
+        idx = order[cut[k]: cut[k + 1]]
+        q[idx] = bh_qvalues(p[idx], n_tests[k])
+    return PValueScan(hits, p, q, n_tests, thresh, bg, list(rec.names), thresh < np.float16(0))
+
+
+def best_site_pvalues(ctx, path_or_records, best: BestSites, motifs_or_pwms, *, bg=None):
+    """(site_p, seq_p), both (R, K) float64, NaN where the record has no site of the motif.  site_p: the exact p-value of the best
+    site's score on its strand; seq_p = -expm1(n log1p(-site_p)), the probability that the best of the record's n windows (both
+    strands of its fragments) scores at least as high, with the Sidak correction CentriMo and AME use.  best: best_sites of the
+    same records and motifs; bg: default base_background(records)."""
+    rec = path_or_records if isinstance(path_or_records, Records) else read_records(path_or_records)
+    pw, lens, _ = _pwm_args(motifs_or_pwms, None)
+    R, K = best.found.shape
+    bg = base_background(rec) if bg is None else np.asarray(bg, np.float64)
+    r, k = np.nonzero(best.found)
+    null = ctx.score_null(pw, lens, bg)
+    try:
+        p = null.pvalues(k, best.comp[r, k], best.score[r, k].view(np.uint16))
+    finally:
+        null.free()
+    site_p = np.full((R, K), np.nan)
+    site_p[r, k] = p
+    n = np.zeros((R, K), np.int64)
+    np.add.at(n, np.asarray(rec.frag_record, np.int64), 2 * _windows_per(rec.frag_len, lens))
+    seq_p = np.full((R, K), np.nan)
+    seq_p[r, k] = sidak(p, n[r, k])
+    return site_p, seq_p

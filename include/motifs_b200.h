@@ -204,6 +204,13 @@ int32_t mb200_scan_last_path(const mb200_ctx* ctx);
 int32_t mb200_scan_prefilter_bound(const uint16_t* cols_f16, int32_t len, uint16_t thresh_f16, double* E, double* t_prefilter,
                                    uint16_t* col0_f16, int32_t* possible);
 
+/* Diagnostic, host arithmetic only: the int8 B operand the tensor-core path multiplies for the same slot.  With f = the real-valued
+ * filter (col0_f16 above, then the remaining columns): q[j*4+b] = ceil(2^e f[j][b]) + k[j] (entries that cannot take part in a positive
+ * window may be raised further), sum_j k[j] = 0, q in [-128, 127], so the integer window sum is >= 2^e times the real-valued one
+ * (tests/test_scan_prefilter_int8_cpu.py).  k: len values, q: len x 4.  e, k and q are left unset when *possible = 0.              */
+int32_t mb200_scan_prefilter_int8(const uint16_t* cols_f16, int32_t len, uint16_t thresh_f16, int32_t* e, int32_t* k, int8_t* q,
+                                  int32_t* possible);
+
 /* Score histogram of the unthresholded scan (hits = score > 0): hist[k*32768 + b] = number of hits of motif k whose Float16
  * score has the 15-bit pattern b (positive halves order like their bit patterns).  Replaces the hit lists as the input of the
  * threshold sweep in get_best_thresh (inference/_s2_filter_pos_w_scores.jl:99-113) and of get_max_score / get_min_score

@@ -224,6 +224,19 @@ function pvalue2score(pwm::AbstractMatrix, pval::Real, eps::Real=1e-1; bg=[.25, 
     return found[] == 0 ? nothing : score[]
 end
 
+# Diagnostic: the int8 B operand of the tensor-core scan for one (motif, strand) slot. cols: (len, 4) Float16, row = PWM column in
+# scoring order. Returns (e, k, Q) with Q (len, 4) Int8, or `nothing` when no window can exceed the threshold.
+function scan_prefilter_int8(cols::AbstractMatrix{Float16}, thresh::Float16)
+    len = size(cols, 1)
+    rowmajor = collect(Float16, permutedims(cols))            # C side reads len x 4 row-major = Julia (4, len) column-major
+    e = Ref{Int32}(0); possible = Ref{Int32}(0); k = zeros(Int32, len); q = zeros(Int8, 4, len)
+    rc = GC.@preserve rowmajor k q ccall((:mb200_scan_prefilter_int8, lib), Int32,
+        (Ptr{Float16}, Int32, UInt16, Ref{Int32}, Ptr{Int32}, Ptr{Int8}, Ref{Int32}),
+        rowmajor, len, reinterpret(UInt16, thresh), e, k, q, possible)
+    rc == 0 || error("mb200_scan_prefilter_int8 failed ($rc)")
+    return possible[] == 0 ? nothing : (e[], k, permutedims(q))
+end
+
 # ------------------------------------------------------------------------------------------------------------------------------
 # multi-GPU: one Julia process per GPU (Distributed / MPI / plain `julia -p`), one NCCL communicator per ctx (csrc/comm.cu).
 # Rank 0 makes the id, the host ships the 128 bytes by its own means (e.g. `remotecall_fetch`), every rank calls comm_init.

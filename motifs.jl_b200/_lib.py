@@ -109,6 +109,7 @@ def load():
         "mb200_scan_take_hits": (i32, [p, p, i64, C.POINTER(i64)]),
         "mb200_scan_last_path": (i32, [p]),
         "mb200_scan_prefilter_bound": (i32, [p, i32, C.c_uint16, p, p, p, p]),
+        "mb200_scan_prefilter_int8": (i32, [p, i32, C.c_uint16, p, p, p, p]),
         "mb200_scan_hist": (i32, [p, p, p, p, i32, i32, C.c_uint32, p]),
         "mb200_scan_best": (i32, [p, p, p, p, i32, i32, C.c_uint32, p]),
         "mb200_scan_spacing": (i32, [p, p, p, i64, i32, i32, p, p, i32, i32, p, p, p]),
@@ -473,6 +474,18 @@ def scan_prefilter_bound(cols_f16, thresh_f16):
     if rc != 0:
         raise ValueError(f"mb200_scan_prefilter_bound failed ({rc})")
     return E.value, tp.value, col0.view(np.float16), bool(ok.value)
+
+
+def scan_prefilter_int8(cols_f16, thresh_f16):
+    """mb200_scan_prefilter_int8: (e, k int32[len], Q int8[len, 4]) of one slot's int8 B operand, None when the slot is disabled."""
+    c = np.ascontiguousarray(cols_f16, np.float16).view(np.uint16)
+    e, ok = C.c_int32(), C.c_int32()
+    k = np.zeros(c.shape[0], np.int32)
+    q = np.zeros((c.shape[0], 4), np.int8)
+    rc = load().mb200_scan_prefilter_int8(_ptr(c), c.shape[0], int(np.float16(thresh_f16).view(np.uint16)), C.byref(e), _ptr(k), _ptr(q), C.byref(ok))
+    if rc != 0:
+        raise ValueError(f"mb200_scan_prefilter_int8 failed ({rc})")
+    return (e.value, k, q) if ok.value else None
 
 
 def count_matrices(ctx: "Context", seqs: "Sequences", sites, lens):

@@ -854,6 +854,49 @@ static bool tc_prefilter_threshold(const std::vector<double>& w, int len, double
     return true;
 }
 
+// The exact integer form of a slot's filter, which the tensor core evaluates.  f: the real-valued filter [len][4] (Float16 values:
+// column 0 = w_0 - T' rounded up, then w_1 ..), D_real = sum_j f[j][x_j]; every true hit has D_real > eps32 > 0.
+//   Q[j][b] = ceil(2^e f[j][b]) + k[j],  sum_j k[j] = 0,  Q in [-128, 127]
+// 2^e f is exact (a power-of-two multiple of a Float16), so nothing is rounded down and sum_j Q[j][x_j] >= 2^e D_real for every
+// window: a true hit gives an integer >= 1 and the candidate test stays D > 0.  Int32 accumulation of |Q| <= 128 x 64 is exact.
+// An entry c with c + (the largest sum of the other columns) <= 0 never takes part in a positive window; it is raised to that bound
+// (raising keeps the inequality, and such windows stay <= 0), so that log-odds near -Inf do not force a small scale.  The offsets
+// k move column 0's large -T' term across the columns so that each fits the int8 range.  The largest e that fits has the finest
+// resolution and so the fewest candidates (the rounding up loosens the filter by < len / 2^e).  Returns e.
+static int tc_int8_filter(const std::vector<double>& f, int len, int8_t* Q, int32_t* k) {
+    std::vector<int64_t> c((size_t)len * 4), hi(len), lo(len);
+    for (int e = 24;; --e) {
+        const double s = std::ldexp(1.0, e);
+        int64_t H = 0;
+        for (int j = 0; j < len; ++j) {
+            hi[j] = INT64_MIN;
+            for (int b = 0; b < 4; ++b) { c[(size_t)j * 4 + b] = (int64_t)std::ceil(s * f[(size_t)j * 4 + b]); hi[j] = std::max(hi[j], c[(size_t)j * 4 + b]); }
+            H += hi[j];
+        }
+        bool fits = H <= 127ll * len;
+        int64_t L = 0;
+        for (int j = 0; j < len && fits; ++j) {
+            lo[j] = INT64_MAX;
+            for (int b = 0; b < 4; ++b) {
+                int64_t& x = c[(size_t)j * 4 + b];
+                x = std::max(x, std::min(hi[j], hi[j] - H));       // the other columns sum to at most H - hi[j]
+                lo[j] = std::min(lo[j], x);
+            }
+            fits = hi[j] - lo[j] <= 255;
+            L += lo[j];
+        }
+        if (!fits || L < -128ll * len) continue;                   // e = -24 always fits: every entry is then 0 or 1
+        // k[j] in [-128 - lo[j], 127 - hi[j]]: start at the lower ends (sum -128 len - L <= 0) and raise them to a zero sum
+        int64_t R = 128ll * len + L;
+        for (int j = 0; j < len; ++j) {
+            const int64_t d = std::min<int64_t>(255 - (hi[j] - lo[j]), R);
+            k[j] = (int32_t)(-128 - lo[j] + d); R -= d;
+            for (int b = 0; b < 4; ++b) Q[(size_t)j * 4 + b] = (int8_t)(c[(size_t)j * 4 + b] + k[j]);
+        }
+        return e;
+    }
+}
+
 struct TcPlan {
     std::vector<uint8_t> blob;
     std::vector<TcBlock> blocks;
@@ -872,7 +915,7 @@ static bool build_tc_plan(const ScanPlan& P, const uint16_t* pwms, const int64_t
     auto pw = [&](int k, int a, int ind) -> uint16_t { return pwms[(size_t)k + (size_t)K * ((size_t)a + 4 * (size_t)ind)]; };
     TcSlot off; memset(&off, 0, sizeof off); off.motif = -1; off.thr = 0x7C00u;
     T.slots.assign(nslots, off);
-    std::vector<std::vector<uint16_t>> col0(nslots);              // per slot: the B entries [len][4] (column 0 already holds w - T')
+    std::vector<std::vector<int8_t>> tab(nslots);                 // per slot: the B entries [len][4] (tc_int8_filter)
     std::vector<int> blen(nblocks, 0);
     for (int k = 0; k < K; ++k) {
         const int len = (int)lens[k];
@@ -907,42 +950,40 @@ static bool build_tc_plan(const ScanPlan& P, const uint16_t* pwms, const int64_t
             TcSlot sl; memset(&sl, 0, sizeof sl);
             sl.motif = k; sl.strand = strand; sl.len = len; sl.npos = (int32_t)std::max<int64_t>(0, Lb - len + 1); sl.thr = tb;
             T.slots[slot] = sl;
-            std::vector<uint16_t>& c = col0[slot];
-            c.resize((size_t)len * 4);
-            for (int j = 0; j < len; ++j)
-                for (int b = 0; b < 4; ++b) {
-                    const uint16_t v = strand ? pw(k, 3 - b, len - 1 - j) : pw(k, b, j);
-                    c[(size_t)j * 4 + b] = j == 0 ? h16_round_up(w[b] - Tp) : v;          // D > 0  <=>  real sum > T' (or a little less)
-                }
+            std::vector<double> f(w);
+            for (int b = 0; b < 4; ++b) f[b] = (double)h16_to_float(h16_round_up(w[b] - Tp));   // D_real > 0  <=>  real sum > T' (or a little less)
+            std::vector<int32_t> koff(len);
+            tab[slot].resize((size_t)len * 4);
+            tc_int8_filter(f, len, tab[slot].data(), koff.data());
             blen[slot / TCS_N] = std::max(blen[slot / TCS_N], len);
         }
     }
-    // B operands: [block][kchunk][256 slots][8 halves]; half e of chunk c = column 2c + e/4, base e%4
+    // B operands: [block][kchunk][256 slots][16 int8]; byte e of chunk c = column 4c + e/4, base e%4
     size_t total = 0;
     std::vector<int> kcs(nblocks);
     std::vector<int64_t> boff(nblocks);
     auto bbytes_of = [&](int kc) { return (size_t)kc * TCS_N * 16; };
     for (int bi = 0; bi < nblocks; ++bi) {
-        int kc = (std::max(blen[bi], 1) + 1) / 2;
+        int kc = (std::max(blen[bi], 1) + 3) / 4;
         kc = std::max(2, (kc + 1) & ~1);
         kcs[bi] = kc; boff[bi] = (int64_t)total;
         total += bbytes_of(kc);
     }
     T.blob.assign(total, 0);
     for (int bi = 0; bi < nblocks; ++bi) {
-        uint16_t* Bm = reinterpret_cast<uint16_t*>(T.blob.data() + boff[bi]);
+        int8_t* Bm = reinterpret_cast<int8_t*>(T.blob.data() + boff[bi]);
         for (int sidx = 0; sidx < TCS_N; ++sidx) {
             const int slot = bi * TCS_N + sidx;
-            const std::vector<uint16_t>& c = col0[slot];
-            auto at = [&](int ch, int e) -> size_t { return ((size_t)ch * TCS_N + sidx) * 8 + e; };     // half e of K chunk ch of this slot
+            const std::vector<int8_t>& c = tab[slot];
+            auto at = [&](int ch, int e) -> size_t { return ((size_t)ch * TCS_N + sidx) * 16 + e; };    // byte e of K chunk ch of this slot
             if (c.empty()) {                                       // disabled slot: D = -1 everywhere
-                for (int b = 0; b < 4; ++b) Bm[at(0, b)] = 0xBC00u;
+                for (int b = 0; b < 4; ++b) Bm[at(0, b)] = -1;
                 T.slots[slot].npos = 0;
                 continue;
             }
             const int len = (int)c.size() / 4;
             for (int j = 0; j < len; ++j)
-                for (int b = 0; b < 4; ++b) Bm[at(j >> 1, 4 * (j & 1) + b)] = c[(size_t)j * 4 + b];
+                for (int b = 0; b < 4; ++b) Bm[at(j >> 2, 4 * (j & 3) + b)] = c[(size_t)j * 4 + b];
         }
     }
     // Work entries: blocks sorted by length are paired with their neighbour while both B operands fit in shared memory.  Each block
@@ -965,12 +1006,12 @@ static bool build_tc_plan(const ScanPlan& P, const uint16_t* pwms, const int64_t
             const int S = ord[i + 1];
             e.b_off[1] = boff[S]; e.kchunks[1] = kcs[S]; e.slot0[1] = S * TCS_N; e.nsub = 2;
             bbytes += bbytes_of(kcs[S]);
-            // measured on config 4 (profiles/r01_scan_tc_role_clocks.txt): 1.19 x the MMA clocks when the MMAs bind, ~4 drains of
-            // ~1150 clocks when they do not
-            cost.push_back(std::max(1.19 * 2.0 * (kcs[L] + kcs[S]) * 64.0, 4.0 * drain + 700.0));
+            // per tile of 512 positions: 4 phases x kchunks / 2 MMAs of 128 clocks each per block; measured on config 4
+            // (profiles/r01_scan_tc_role_clocks.txt): 1.19 x the MMA clocks when the MMAs bind, ~8 drains of ~1150 clocks when they do not
+            cost.push_back(std::max(1.19 * 4.0 * (kcs[L] + kcs[S]) * 64.0, 8.0 * drain + 1400.0));
             i += 2;
         } else {
-            cost.push_back(std::max(1.19 * 2.0 * kcs[L] * 64.0, 2.0 * drain + 350.0));
+            cost.push_back(std::max(1.19 * 4.0 * kcs[L] * 64.0, 4.0 * drain + 700.0));
             i += 1;
         }
         // Tried and removed (git history: 59d1900, 004a558, 1f9ca7b; DESIGN.md 3.1b): four 128-column accumulators for short entries (25 %
@@ -1132,6 +1173,7 @@ struct ScanCall {
     uint8_t* d_tc = nullptr; const TcSlot* d_tc_slots = nullptr; size_t tc_smem = 0, tc_set_stride = 0, tc_uset_stride = 0;
     unsigned long long* d_tc_list = nullptr; unsigned long long* d_tc_ctr = nullptr; uint32_t* d_tc_ulist = nullptr; uint32_t* d_tc_ubits = nullptr;
     unsigned long long tc_stat_cand = 0, tc_stat_hits = 0;
+    double tc_stat_macs = 0;               // int8 multiply-adds the tensor core was given (every slot block over every position)
     uint32_t* d_unit_cnt = nullptr; unsigned long long* d_unit_off = nullptr; unsigned long long* d_bsum = nullptr;   // hit lists
     int64_t hits_written = 0, hits_needed = 0;
     unsigned int* d_hist = nullptr;                                                                                   // HIST
@@ -1385,7 +1427,9 @@ static int tc_launch(ScanCall& S, int64_t s0, int64_t ns, unsigned long long* li
     memset(ta.blocks, 0, sizeof ta.blocks); memcpy(ta.blocks, S.TP.blocks.data(), S.TP.blocks.size() * sizeof(TcBlock));
     ta.slots = S.d_tc_slots;
     ta.list = list; ta.cap = TC_CAP; ta.gcount = ctr; ta.overflow = (uint32_t*)(ctr + 1);
-    ta.ntiles = (int32_t)((ns * S.Lb + 255) / 256);
+    ta.ntiles = (int32_t)((ns * S.Lb + TCS_TILE - 1) / TCS_TILE);
+    for (const TcBlock& e : S.TP.blocks)
+        for (int sub = 0; sub < e.nsub; ++sub) S.tc_stat_macs += (double)ta.ntiles * TCS_TILE * TCS_N * e.kchunks[sub] * 16;
     ta.clocks = (long long*)(ctr + 8);
     ta.dbg = nullptr;
 #if TCS_PROFILE
@@ -1717,8 +1761,8 @@ static int scan_finish(ScanCall& S) {
     MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     S.tm.collect();
     if (S.d_tc_ctr && getenv("MB200_SCAN_TC_STATS")) {
-        fprintf(stderr, "[mb200] tensor-core scan: %s, candidates %llu, hits %llu, scan %.3f ms, count %.3f ms\n", S.use_tc ? "used" : "fell back", S.tc_stat_cand,
-                S.tc_stat_hits, ctx->ms[T_SCAN], ctx->ms[T_COUNT]);
+        fprintf(stderr, "[mb200] tensor-core scan: %s, candidates %llu, hits %llu, scan %.3f ms, count %.3f ms, int8 MACs %.4e\n", S.use_tc ? "used" : "fell back",
+                S.tc_stat_cand, S.tc_stat_hits, ctx->ms[T_SCAN], ctx->ms[T_COUNT], S.tc_stat_macs);
     }
     if (S.seqs->pending) { rc = mb_seqs_finish(ctx, const_cast<mb200_seqs*>(S.seqs)); if (rc) return rc; }      // the upload has completed: report bad symbols
     if (o.n_hits) *o.n_hits = S.hits_needed;
@@ -1770,6 +1814,22 @@ extern "C" int32_t mb200_scan_prefilter_bound(const uint16_t* cols_f16, int32_t 
     *E = 0.0; *t_prefilter = 0.0;
     *possible = tc_prefilter_threshold(w, len, t, A, E, t_prefilter) ? 1 : 0;
     if (*possible && col0_f16) for (int b = 0; b < 4; ++b) col0_f16[b] = h16_round_up(w[b] - *t_prefilter);      // what column 0 of the B operand holds
+    return MB200_OK;
+}
+
+// Diagnostic (host arithmetic only, ctx-free): the int8 B operand of one slot, as k_scan_tc multiplies it.  Same arguments as
+// mb200_scan_prefilter_bound; e: the scale 2^e, k: the len column offsets, q: len x 4 entries (tc_int8_filter).
+extern "C" int32_t mb200_scan_prefilter_int8(const uint16_t* cols_f16, int32_t len, uint16_t thresh_f16, int32_t* e, int32_t* k, int8_t* q,
+                                             int32_t* possible) {
+    if (!e || !k || !q) return MB200_E_INVALID;
+    double E = 0.0, tp = 0.0;
+    uint16_t col0[4];
+    const int32_t rc = mb200_scan_prefilter_bound(cols_f16, len, thresh_f16, &E, &tp, col0, possible);
+    if (rc || !*possible) return rc;
+    std::vector<double> f((size_t)len * 4);
+    for (int j = 0; j < len; ++j)
+        for (int b = 0; b < 4; ++b) f[(size_t)j * 4 + b] = (double)h16_to_float(j ? cols_f16[j * 4 + b] : col0[b]);
+    *e = tc_int8_filter(f, len, q, k);
     return MB200_OK;
 }
 

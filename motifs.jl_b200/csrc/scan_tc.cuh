@@ -1,41 +1,44 @@
-// Tensor-core pre-filter for the thresholded PWM scan (tcgen05.mma kind::f16, accumulators in TMEM) + exact verification.
+// Tensor-core pre-filter for the thresholded PWM scan (tcgen05.mma kind::i8, exact int32 accumulators in TMEM) + exact verification.
 //
 // What it replaces: the same reference functions as scan_kernel (greedy_search! _h3_1_alignment.jl:18-36 followed by
 // filter_position_by_best_thresh! _s2_filter_pos_w_scores.jl:116-125), for the case the fused-threshold callers use
 // (thresh given).  The reference's score is a LEFT-TO-RIGHT Float16 running sum; a GEMM cannot reproduce its rounding, so the
 // GEMM is only a FILTER and every position it lets through is re-scored with the sequential Float16 adds:
 //
-//   1. k_scan_tc: D[v, s] = sum_{j,b} onehot(base[v+j])[b] * W_s[j][b]   (FP16 operands, exact products, FP32 accumulation)
-//      for every start position v of the batch and every (motif, strand) slot s, with the slot's pre-filter threshold T'_s
-//      folded into column 0 of W_s (rounded up), so that "D > 0" is the candidate test.  T'_s = t_s - E_s - eps32 where E_s bounds
-//      |Float16 running sum - real sum| over all paths whose Float16 score exceeds t_s (tc_error_bound below: U_j = the Float16
-//      running sum of column maxima bounds every partial sum from above by monotonicity of rounding, a backward recursion bounds
-//      the partial sums of hit paths from below, each add errs by at most 2^-11 |partial sum|).  Hence every true hit is a
-//      candidate; candidates (a few 1e-4 of all cells at the usual thresholds) go to a list in HBM.
+//   1. k_scan_tc: D[v, s] = sum_{j,b} onehot(base[v+j])[b] * Q_s[j][b]   (int8 operands, int32 accumulation: no rounding at all)
+//      for every start position v of the batch and every (motif, strand) slot s.  Q_s is the exact integer form of the real-valued
+//      filter D_real = col0[x0] + sum_{j>=1} w_j[x_j], col0 = w_0 - T'_s rounded up to Float16: Q_s[j][b] = ceil(2^e * entry) + k_j
+//      with sum_j k_j = 0, so that D >= 2^e * D_real and "D > 0" is the candidate test (tc_int8_filter in scan.cu).  T'_s = t_s - E_s
+//      - eps32 where E_s bounds |Float16 running sum - real sum| over all paths whose Float16 score exceeds t_s (tc_error_bound below:
+//      U_j = the Float16 running sum of column maxima bounds every partial sum from above by monotonicity of rounding, a backward
+//      recursion bounds the partial sums of hit paths from below, each add errs by at most 2^-11 |partial sum|).  Hence every true
+//      hit has D_real > eps32 > 0 and D >= 1; candidates (a few 1e-4 of all cells at the usual thresholds) go to a list in HBM.
 //   2. k_scan_tc_verify: one thread per candidate re-computes the sequential Float16 score (same table, same adds as
 //      emit_kernel) and sets the bit of the hit mask when score > thresh.  The masks then feed count / emit / hist unchanged, so
 //      hit sets are bit-identical to scan_kernel's (tests/test_scan_gpu.py runs both paths on the same inputs).
 //
-// Operand layout (the im2col matrix is never materialised): a tile is 128 start positions of one parity, v = v0 + par + 2m.
-// Its one-hot stream in shared memory holds one 16-byte chunk per base PAIR (2 bases x {A,C,G,T} halves); row m of the A operand
-// is the stream from chunk m on, so in the canonical K-major no-swizzle UMMA layout (core matrix = 8 rows x 16 B, rows 16 B
+// Operand layout (the im2col matrix is never materialised): a tile is 128 start positions of one phase, v = v0 + ph + 4m, ph < 4.
+// Its one-hot stream in shared memory holds one 16-byte chunk per 4 bases (one byte per base and class {A,C,G,T}); row m of the A
+// operand is the stream from chunk m on, so in the canonical K-major no-swizzle UMMA layout (core matrix = 8 rows x 16 B, rows 16 B
 // apart) the operand of K-chunk c is the same stream advanced by c*16 B.  Two copies ("planes", the second shifted by one chunk)
-// give the two K-chunks of one K=16 MMA at LBO = plane stride; SBO = 128 B.  B = W'[K chunk][256 slots][8 halves] stays resident.
+// give the two K-chunks of one K=32 MMA at LBO = plane stride; SBO = 128 B.  B = Q[K chunk][256 slots][16 bytes] stays resident.
 // One CTA per SM owns one or two blocks of 256 slots; warps 0 and 18 build streams (from the 2-bit words in L2), warp 1 (converged, one
-// elected lane per instruction) issues kchunks/2 MMAs of 128x256x16 per tile, block and parity, warps 2-17 drain every accumulator use:
+// elected lane per instruction) issues kchunks/2 MMAs of 128x256x32 per tile, block and phase, warps 2-17 drain every accumulator use:
 // two tcgen05.ld of 32 lanes x 32 columns each, accumulator handed back, then a 3-input max tree; individual columns are looked at only
 // when some lane saw a positive value.  "tc_error_bound below" = tc_error_bound() in scan.cu (host).
 #pragma once
 
 #define TCS_M 128
 #define TCS_N 256                          // slots per block = accumulator columns
-#define TCS_STREAM 160                     // 16-byte chunks per stream plane: 128 rows + up to 32 K-chunks
+#define TCS_PHASES 4                       // start positions v0 + ph + 4m of one tile: 4 phases x 128 rows
+#define TCS_TILE (TCS_PHASES * TCS_M)      // start positions per tile
+#define TCS_STREAM 160                     // 16-byte chunks per stream plane: 128 rows + up to 16 K-chunks, in the producers' steps of 32
 #define TCS_PLANE_BYTES (TCS_STREAM * 16)
-#define TCS_STAGE_BYTES (4 * TCS_PLANE_BYTES)   // one tile: {even, odd} x {plane 0, plane 1}
+#define TCS_STAGE_BYTES (TCS_PHASES * 2 * TCS_PLANE_BYTES)   // one tile: 4 phases x {plane 0, plane 1}
 #define TCS_STAGES 4
 #define TCS_THREADS 608                    // warps: 0 and 18 producers, 1 MMA issue, 2-17 epilogue
 #define TCS_RESERVE 256                    // candidate records reserved per global atomic
-#define TCS_MAX_KCHUNKS 32                 // 64 columns x 4 bases / 8
+#define TCS_MAX_KCHUNKS 16                 // 64 columns x 4 bases / 16
 #define TCS_MAX_ENTRIES 16                 // work entries (single or paired slot blocks) per launch: up to 4096 motifs
 #ifndef TCS_PROFILE
 #define TCS_PROFILE 0                      // 1: per-role wait clocks in TcArgs::dbg (printed with MB200_SCAN_TC_DEBUG=1)
@@ -48,7 +51,7 @@
 
 struct TcBlock {                           // what one CTA works on: one block of 256 slots, or a long and a short block paired
     int64_t b_off[2];                      // byte offsets of the B operands in the TC blob
-    int32_t kchunks[2];                    // 16-byte K chunks (8 halves = 2 PWM columns), even
+    int32_t kchunks[2];                    // 16-byte K chunks (16 int8 = 4 PWM columns), even
     int32_t slot0[2];                      // first global slot
     int32_t nsub;                          // 1, or 2: sub-block 0 (the longer one) accumulates in TMEM columns [0,256), sub-block 1 in [256,512)
     int32_t cta0, nctas;                   // CTAs [cta0, cta0 + nctas) work on this entry
@@ -70,7 +73,7 @@ struct TcArgs {
     const TcSlot* slots;
     unsigned long long* list; unsigned long long cap; unsigned long long* gcount;   // candidate list, its capacity, reserved records
     uint32_t* overflow;
-    int32_t ntiles;                        // tiles of 256 positions (2 units each)
+    int32_t ntiles;                        // tiles of TCS_TILE positions (TCS_PHASES units each)
     long long* clocks;                     // [grid][2]: clocks the MMA lane spent on its tiles, tiles done (feeds the host's re-balancing of CTAs over blocks)
     long long* dbg;                        // TCS_PROFILE builds: [grid][8] wait clocks per role
 };
@@ -82,7 +85,7 @@ __device__ __forceinline__ uint64_t tcs_desc(uint32_t smem_addr, uint32_t lbo_by
 // Issued by the whole (converged) MMA warp: one elected lane executes the instruction.  Keeping the warp converged lets the compiler
 // hold descriptors, TMEM address and instruction descriptor in uniform registers (no per-MMA R2UR/ELECT sequences).
 __device__ __forceinline__ void tcs_mma(uint32_t tmem_d, uint64_t da, uint64_t db, uint32_t idesc, uint32_t accumulate) {
-    asm volatile("{\n\t.reg .pred p, q;\n\tsetp.ne.b32 p, %4, 0;\n\telect.sync _|q, 0xFFFFFFFF;\n\t@q tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}\n"
+    asm volatile("{\n\t.reg .pred p, q;\n\tsetp.ne.b32 p, %4, 0;\n\telect.sync _|q, 0xFFFFFFFF;\n\t@q tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n\t}\n"
                  :: "r"(tmem_d), "l"(da), "l"(db), "r"(idesc), "r"(accumulate) : "memory");
 }
 __device__ __forceinline__ void tcs_commit(uint32_t bar) {
@@ -96,20 +99,8 @@ __device__ __forceinline__ void tcs_wait(uint32_t bar, uint32_t parity) {
         if (!done && ++spins > (1u << 26)) __trap();             // never hang the device on a lost completion
     } while (!done);
 }
-__device__ __forceinline__ float tcs_max3(float a, float b, float c) {
-    float d;
-    asm("max.f32 %0, %1, %2, %3;" : "=f"(d) : "f"(a), "f"(b), "f"(c));
-    return d;
-}
-// 16-byte one-hot chunk of a base pair: halves {A,C,G,T} of b0 then of b1, 1.0 = 0x3C00
-__device__ __forceinline__ uint4 tcs_onehot(uint32_t b0, uint32_t b1) {
-    uint4 r;
-    r.x = b0 < 2 ? 0x3C00u << (16 * b0) : 0u;
-    r.y = b0 >= 2 ? 0x3C00u << (16 * (b0 - 2)) : 0u;
-    r.z = b1 < 2 ? 0x3C00u << (16 * b1) : 0u;
-    r.w = b1 >= 2 ? 0x3C00u << (16 * (b1 - 2)) : 0u;
-    return r;
-}
+// one-hot bytes {A,C,G,T} of one base: 4 bases make a 16-byte chunk
+__device__ __forceinline__ uint32_t tcs_onehot(uint32_t b) { return 1u << (8 * b); }
 __device__ __forceinline__ uint32_t tcs_base(const TcArgs& a, uint32_t v) {
     if (v >= a.vtotal) return 0u;
     const uint32_t n = v / a.Lb, p = v - n * a.Lb;
@@ -139,18 +130,19 @@ __device__ __noinline__ unsigned long long tcs_reserve(unsigned long long* list,
                    "=r"(U[21]), "=r"(U[22]), "=r"(U[23]), "=r"(U[24]), "=r"(U[25]), "=r"(U[26]), "=r"(U[27]), "=r"(U[28]), "=r"(U[29]), "=r"(U[30]), "=r"(U[31]) \
                  : "r"(TADDR) : "memory")
 
-// max of 32 accumulator values as four independent chains (latency, not issue, bounds the epilogue)
-__device__ __forceinline__ float tcs_max32(const uint32_t (&u)[32]) {
-    float m[4];
+// max of 32 int32 accumulator values as four independent chains (latency, not issue, bounds the epilogue).  Integer max: read as
+// floats, bit patterns >= 0x7F800001 would be NaN and be dropped by max.f32.
+__device__ __forceinline__ int tcs_max32(const uint32_t (&u)[32]) {
+    int m[4];
     #pragma unroll
     for (int k = 0; k < 4; ++k) {
-        m[k] = tcs_max3(__uint_as_float(u[8 * k]), __uint_as_float(u[8 * k + 1]), __uint_as_float(u[8 * k + 2]));
-        m[k] = tcs_max3(m[k], __uint_as_float(u[8 * k + 3]), __uint_as_float(u[8 * k + 4]));
-        m[k] = tcs_max3(m[k], __uint_as_float(u[8 * k + 5]), __uint_as_float(u[8 * k + 6]));
+        m[k] = __vimax3_s32((int)u[8 * k], (int)u[8 * k + 1], (int)u[8 * k + 2]);
+        m[k] = __vimax3_s32(m[k], (int)u[8 * k + 3], (int)u[8 * k + 4]);
+        m[k] = __vimax3_s32(m[k], (int)u[8 * k + 5], (int)u[8 * k + 6]);
     }
-    return fmaxf(tcs_max3(m[0], m[1], m[2]), tcs_max3(m[3], __uint_as_float(u[7]), tcs_max3(__uint_as_float(u[15]), __uint_as_float(u[23]), __uint_as_float(u[31]))));
+    return max(__vimax3_s32(m[0], m[1], m[2]), __vimax3_s32(m[3], (int)u[7], __vimax3_s32((int)u[15], (int)u[23], (int)u[31])));
 }
-// bit c set when column c is positive (D > 0  <=>  its bits as a signed integer are > 0)
+// bit c set when column c is positive
 __device__ __forceinline__ uint32_t tcs_posbits(const uint32_t (&u)[32]) {
     uint32_t b = 0;
     #pragma unroll
@@ -187,7 +179,7 @@ __device__ __noinline__ void tcs_append(unsigned long long* list, unsigned long 
 }
 
 // The K loop of one accumulator use, fully unrolled per trip count: with compile-time t the descriptors of step t are the first
-// ones plus constants (one uniform 64-bit add each).  A run-time loop costs ~26 dependent instructions per MMA in the single issuing
+// ones plus constants (one uniform 64-bit add each); KP = ceil(len / 8) <= 8.  A run-time loop costs ~26 dependent instructions per MMA in the single issuing
 // thread (ELECT + seven R2UR per MMA): ~180 clocks per 128-clock MMA, i.e. the issuing thread, not the tensor pipe, set the pace.
 template <int KP>
 __device__ __forceinline__ void tcs_issue_n(uint32_t tmem_d, uint64_t da0, uint64_t db0, uint32_t idesc) {
@@ -196,28 +188,24 @@ __device__ __forceinline__ void tcs_issue_n(uint32_t tmem_d, uint64_t da0, uint6
 }
 __device__ __forceinline__ void tcs_issue(int kp, uint32_t tmem_d, uint64_t da0, uint64_t db0, uint32_t idesc) {
     switch (kp) {
-        case 1: tcs_issue_n<1>(tmem_d, da0, db0, idesc); break;   case 2: tcs_issue_n<2>(tmem_d, da0, db0, idesc); break;
-        case 3: tcs_issue_n<3>(tmem_d, da0, db0, idesc); break;   case 4: tcs_issue_n<4>(tmem_d, da0, db0, idesc); break;
-        case 5: tcs_issue_n<5>(tmem_d, da0, db0, idesc); break;   case 6: tcs_issue_n<6>(tmem_d, da0, db0, idesc); break;
-        case 7: tcs_issue_n<7>(tmem_d, da0, db0, idesc); break;   case 8: tcs_issue_n<8>(tmem_d, da0, db0, idesc); break;
-        case 9: tcs_issue_n<9>(tmem_d, da0, db0, idesc); break;   case 10: tcs_issue_n<10>(tmem_d, da0, db0, idesc); break;
-        case 11: tcs_issue_n<11>(tmem_d, da0, db0, idesc); break; case 12: tcs_issue_n<12>(tmem_d, da0, db0, idesc); break;
-        case 13: tcs_issue_n<13>(tmem_d, da0, db0, idesc); break; case 14: tcs_issue_n<14>(tmem_d, da0, db0, idesc); break;
-        case 15: tcs_issue_n<15>(tmem_d, da0, db0, idesc); break; default: tcs_issue_n<16>(tmem_d, da0, db0, idesc); break;
+        case 1: tcs_issue_n<1>(tmem_d, da0, db0, idesc); break; case 2: tcs_issue_n<2>(tmem_d, da0, db0, idesc); break;
+        case 3: tcs_issue_n<3>(tmem_d, da0, db0, idesc); break; case 4: tcs_issue_n<4>(tmem_d, da0, db0, idesc); break;
+        case 5: tcs_issue_n<5>(tmem_d, da0, db0, idesc); break; case 6: tcs_issue_n<6>(tmem_d, da0, db0, idesc); break;
+        case 7: tcs_issue_n<7>(tmem_d, da0, db0, idesc); break; default: tcs_issue_n<8>(tmem_d, da0, db0, idesc); break;
     }
 }
 
-// Work item = one tile of 256 consecutive virtual start positions = two parities (even / odd offsets) of 128 rows.
-// Single block: parity 0 accumulates in TMEM columns [0,256), parity 1 in [256,512).
-// Paired blocks (nsub = 2): draining 128 x 256 FP32 accumulators costs >= 512 clocks of TMEM read bandwidth, more than the MMA
-// time of a short block (K = 64: 512 clocks) and far less than that of a long one, so a long and a short block share the CTA
-// and the one-hot streams: unit order (long, p0) (short, p0) (long, p1) (short, p1), long -> accumulator 0, short -> accumulator 1;
-// the long block's accumulator drains under the short block's MMAs and vice versa.
+// Work item = one tile of 512 consecutive virtual start positions = four phases (offsets mod 4) of 128 rows.
+// Single block: even phases accumulate in TMEM columns [0,256), odd phases in [256,512).
+// Paired blocks (nsub = 2): draining 128 x 256 int32 accumulators costs >= 512 clocks of TMEM read bandwidth, more than the MMA
+// time of a short block (16 columns: 256 clocks) and far less than that of a long one, so a long and a short block share the CTA
+// and the one-hot streams: unit order (long, ph0) (short, ph0) (long, ph1) (short, ph1) ..., long -> accumulator 0, short ->
+// accumulator 1; the long block's accumulator drains under the short block's MMAs and vice versa.
 // Warps: 0 and 18 build the one-hot streams of alternate tiles, one lane of warp 1 issues the MMAs, warps 2-17 drain the
 // accumulators (8 warps each: 4 TMEM lane quarters x 2 column halves).
 __global__ void __launch_bounds__(TCS_THREADS, 1) k_scan_tc(const TcArgs a) {
     extern __shared__ __align__(1024) uint8_t tcs_smem[];
-    uint8_t* sA = tcs_smem;                                              // [TCS_STAGES][2 parities][2 planes][TCS_STREAM][16 B]
+    uint8_t* sA = tcs_smem;                                              // [TCS_STAGES][TCS_PHASES][2 planes][TCS_STREAM][16 B]
     uint8_t* sB = tcs_smem + TCS_STAGES * TCS_STAGE_BYTES;               // per sub-block [kchunks][256][16 B]
     __shared__ __align__(8) uint64_t s_bars[2 * TCS_STAGES + 5];         // full[S], empty[S], accfull[2], accempty[2], B landed
     __shared__ uint32_t s_tmem;
@@ -242,7 +230,7 @@ __global__ void __launch_bounds__(TCS_THREADS, 1) k_scan_tc(const TcArgs a) {
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
     }
     // the last chunk of every shifted plane is never written by the producers (and never needed): keep it zero
-    for (int i = tid; i < TCS_STAGES * 2; i += blockDim.x)
+    for (int i = tid; i < TCS_STAGES * TCS_PHASES; i += blockDim.x)
         *reinterpret_cast<uint4*>(sA + (size_t)i * (2 * TCS_PLANE_BYTES) + TCS_PLANE_BYTES + (TCS_STREAM - 1) * 16) = make_uint4(0, 0, 0, 0);
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
@@ -250,53 +238,55 @@ __global__ void __launch_bounds__(TCS_THREADS, 1) k_scan_tc(const TcArgs a) {
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     const uint32_t tmem = s_tmem;
     const uint32_t sA_addr = (uint32_t)__cvta_generic_to_shared(sA), sB_addr = (uint32_t)__cvta_generic_to_shared(sB);
-    // instruction descriptor: D = F32 (1<<4), A = B = F16 (format 0), both K-major, N>>3 at bit 17, M>>4 at bit 24
-    const uint32_t idesc = (1u << 4) | ((uint32_t)(TCS_N >> 3) << 17) | ((uint32_t)(TCS_M >> 4) << 24);
+    // instruction descriptor: D = S32 (2<<4), A and B signed 8-bit (1<<7, 1<<10), both K-major, N>>3 at bit 17, M>>4 at bit 24
+    const uint32_t idesc = (2u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(TCS_N >> 3) << 17) | ((uint32_t)(TCS_M >> 4) << 24);
 
     if (warp == 0 || warp == TCS_THREADS / 32 - 1) {
-        // ---- producers: bases v0 .. v0+319 of the tile -> even stream E[m] = (b[2m], b[2m+1]), odd stream O[m] = (b[2m+1], b[2m+2]),
-        //      each stored twice (plane 1 = plane 0 shifted by one chunk) ----
+        // ---- producers: bases v0 .. v0+642 of the tile -> the stream of phase f, S_f[m] = (b[4m+f], .., b[4m+f+3]), stored twice
+        //      (plane 1 = plane 0 shifted by one chunk) ----
         const int pw = warp == 0 ? 0 : 1;
         TCS_PROF(long long w_prod = 0;)
         int it = 0;
         for (int tile = rank; tile < a.ntiles; tile += blk.nctas, ++it) {
             if ((it & 1) != pw) continue;
             const int st = it % TCS_STAGES; const uint32_t ph = (it / TCS_STAGES) & 1;
-            uint32_t v = (uint32_t)tile * 256u + 2u * lane;
+            uint32_t v = (uint32_t)tile * TCS_TILE + 4u * lane;
             uint32_t n = v / a.Lb, p = v - n * a.Lb;
             const uint32_t* row = a.seqw + (a.seq0 + n) * a.rowwords;
-            uint32_t b0[TCS_STREAM / 32], b1[TCS_STREAM / 32];
+            uint32_t bb[TCS_STREAM / 32];                                                // bases 4m .. 4m+3 of chunk m = lane + 32 i, 2 bits each
             #pragma unroll
             for (int i = 0; i < TCS_STREAM / 32; ++i) {
-                uint32_t w0 = 0, w1 = 0;
-                const bool second_in_row = p + 1 < a.Lb;
-                const uint32_t p1 = second_in_row ? p + 1 : 0u;
-                const uint32_t* row1 = second_in_row ? row : row + a.rowwords;
-                if (v < a.vtotal) w0 = __ldg(row + (p >> 4));
-                if (v + 1 < a.vtotal) w1 = __ldg(row1 + (p1 >> 4));
-                b0[i] = (w0 >> ((p & 15) * 2)) & 3u;
-                b1[i] = (w1 >> ((p1 & 15) * 2)) & 3u;
-                v += 64; p += 64;
+                bb[i] = 0;
+                #pragma unroll
+                for (int k = 0; k < 4; ++k) {
+                    uint32_t pk = p + k; const uint32_t* rk = row;
+                    while (pk >= a.Lb) { pk -= a.Lb; rk += a.rowwords; }
+                    const uint32_t w = v + k < a.vtotal ? __ldg(rk + (pk >> 4)) : 0u;
+                    bb[i] |= ((w >> ((pk & 15) * 2)) & 3u) << (2 * k);
+                }
+                v += 128; p += 128;
                 while (p >= a.Lb) { p -= a.Lb; row += a.rowwords; }
             }
             TCS_PROF(const long long t0 = clock64();)
             tcs_wait(bar(TCS_STAGES + st), ph ^ 1);                                      // stage free
             TCS_PROF(w_prod += clock64() - t0;)
-            uint8_t* e0 = sA + (size_t)st * TCS_STAGE_BYTES;                             // even: plane 0, plane 1; odd: plane 0, plane 1
-            uint8_t* o0 = e0 + 2 * TCS_PLANE_BYTES;
+            uint8_t* s0 = sA + (size_t)st * TCS_STAGE_BYTES;                             // phase f: plane 0 at s0 + 2f planes, plane 1 after it
             #pragma unroll
             for (int i = 0; i < TCS_STREAM / 32; ++i) {
                 const uint32_t m = lane + 32 * i;
-                uint32_t b2 = __shfl_down_sync(0xffffffffu, b0[i], 1);
-                const uint32_t nxt = __shfl_sync(0xffffffffu, i + 1 < TCS_STREAM / 32 ? b0[(i + 1) % (TCS_STREAM / 32)] : 0u, 0);
-                if (lane == 31) b2 = nxt;
-                const uint4 ev = tcs_onehot(b0[i], b1[i]);
-                const uint4 od = tcs_onehot(b1[i], b2);
-                *reinterpret_cast<uint4*>(e0 + m * 16) = ev;
-                *reinterpret_cast<uint4*>(o0 + m * 16) = od;
-                if (m > 0) {
-                    *reinterpret_cast<uint4*>(e0 + TCS_PLANE_BYTES + (m - 1) * 16) = ev;
-                    *reinterpret_cast<uint4*>(o0 + TCS_PLANE_BYTES + (m - 1) * 16) = od;
+                uint32_t nb = __shfl_down_sync(0xffffffffu, bb[i], 1);                    // bases 4m+4 .. 4m+7: the next chunk's
+                const uint32_t nxt = __shfl_sync(0xffffffffu, i + 1 < TCS_STREAM / 32 ? bb[(i + 1) % (TCS_STREAM / 32)] : 0u, 0);
+                if (lane == 31) nb = nxt;
+                const uint32_t b7 = bb[i] | (nb << 8);
+                uint32_t o[7];                                                           // one-hot of bases 4m .. 4m+6
+                #pragma unroll
+                for (int k = 0; k < 7; ++k) o[k] = tcs_onehot((b7 >> (2 * k)) & 3u);
+                #pragma unroll
+                for (int f = 0; f < TCS_PHASES; ++f) {
+                    const uint4 c = make_uint4(o[f], o[f + 1], o[f + 2], o[f + 3]);
+                    uint8_t* pl = s0 + (size_t)f * 2 * TCS_PLANE_BYTES;
+                    *reinterpret_cast<uint4*>(pl + m * 16) = c;
+                    if (m > 0) *reinterpret_cast<uint4*>(pl + TCS_PLANE_BYTES + (m - 1) * 16) = c;
                 }
             }
             asm volatile("fence.proxy.async.shared::cta;" ::: "memory");                 // generic-proxy writes -> visible to the tensor core
@@ -321,11 +311,7 @@ __global__ void __launch_bounds__(TCS_THREADS, 1) k_scan_tc(const TcArgs a) {
             }
             tcs_wait(bar(2 * TCS_STAGES + 4), 0);
             const uint64_t dbA = tcs_desc(sB_addr, TCS_N * 16, 128), dbB = tcs_desc(sB_addr + b_bytes0, TCS_N * 16, 128);
-#ifdef TCS_EMULATE_HALF_K      // timing experiment only (results are wrong): half the MMAs per accumulator use = the MMA time an FP8 operand format would leave
-            const int kpA = max(1, blk.kchunks[0] >> 2), kpB = max(1, blk.kchunks[1] >> 2);
-#else
             const int kpA = blk.kchunks[0] >> 1, kpB = blk.kchunks[1] >> 1;
-#endif
             TCS_PROF(long long w_full = 0; long long w_acc = 0;)
             const long long t_start = clock64();
             uint32_t use0 = 0, use1 = 0;                                                 // completed uses of each accumulator
@@ -336,15 +322,15 @@ __global__ void __launch_bounds__(TCS_THREADS, 1) k_scan_tc(const TcArgs a) {
                 tcs_wait(bar(st), ph);                                                   // streams built
                 TCS_PROF(w_full += clock64() - t0;)
                 #pragma unroll
-                for (int par = 0; par < 2; ++par) {
+                for (int f = 0; f < TCS_PHASES; ++f) {
                     for (int sub = 0; sub < blk.nsub; ++sub) {
-                        const int ac = blk.nsub > 1 ? sub : par;
+                        const int ac = blk.nsub > 1 ? sub : (f & 1);
                         const uint32_t uses = ac ? use1 : use0;
                         TCS_PROF(t0 = clock64();)
                         tcs_wait(bar(2 * TCS_STAGES + 2 + ac), (uses & 1) ^ 1);          // accumulator drained
                         TCS_PROF(w_acc += clock64() - t0;)
                         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                        const uint64_t da0 = tcs_desc(sA_addr + st * TCS_STAGE_BYTES + par * 2 * TCS_PLANE_BYTES, TCS_PLANE_BYTES, 128);
+                        const uint64_t da0 = tcs_desc(sA_addr + st * TCS_STAGE_BYTES + f * 2 * TCS_PLANE_BYTES, TCS_PLANE_BYTES, 128);
                         const uint64_t dbs = sub ? dbB : dbA;
                         const int kp = sub ? kpB : kpA;
                         tcs_issue(kp, tmem + ac * TCS_N, da0, dbs, idesc);
@@ -370,12 +356,13 @@ __global__ void __launch_bounds__(TCS_THREADS, 1) k_scan_tc(const TcArgs a) {
         uint32_t use0 = 0, use1 = 0;                                                     // completed uses of each accumulator
         int it = 0;
         for (int tile = rank; tile < a.ntiles; tile += blk.nctas, ++it)
-        for (int par = 0; par < 2; ++par)
+        #pragma unroll 1
+        for (int f = 0; f < TCS_PHASES; ++f)
         for (int sub = 0; sub < blk.nsub; ++sub) {
-            const int ac = blk.nsub > 1 ? sub : par;
+            const int ac = blk.nsub > 1 ? sub : (f & 1);
             const uint32_t uses = ac ? use1 : use0;
             if (ac) ++use1; else ++use0;
-            const uint32_t v = (uint32_t)tile * 256u + (uint32_t)par + 2u * (uint32_t)(q * 32 + lane);
+            const uint32_t v = (uint32_t)tile * TCS_TILE + (uint32_t)f + 4u * (uint32_t)(q * 32 + lane);
             const bool inb = v < a.vtotal;
             TCS_PROF(const long long t0 = clock64();)
             tcs_wait(bar(2 * TCS_STAGES + ac), uses & 1);
@@ -399,8 +386,8 @@ __global__ void __launch_bounds__(TCS_THREADS, 1) k_scan_tc(const TcArgs a) {
             asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
             __syncwarp();
             if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" :: "r"(bar(2 * TCS_STAGES + 2 + ac)) : "memory");    // the values are in registers: the accumulator may be overwritten
-            const float ma = tcs_max32(ua), mb = tcs_max32(ub);
-            bool pos = inb && fmaxf(ma, mb) > 0.f;
+            const int ma = tcs_max32(ua), mb = tcs_max32(ub);
+            bool pos = inb && max(ma, mb) > 0;
             if (__any_sync(0xffffffffu, pos)) {          /* about one use in ten at the usual thresholds */
                 // ragged store: a start position in the row's zero padding (poly-A) is no candidate, or an A-rich PWM would fill the
                 // list with padding.  Windows that start inside the row and run into the padding are left to the verifier.
@@ -412,8 +399,8 @@ __global__ void __launch_bounds__(TCS_THREADS, 1) k_scan_tc(const TcArgs a) {
                 }
                 if (!a.lens || __any_sync(0xffffffffu, pos)) {
                     uint32_t cb0 = 0u, cb1 = 0u;             // bit masks of the positive columns, only for the chunk(s) that have any
-                    if (__any_sync(0xffffffffu, live && ma > 0.f)) cb0 = pos ? tcs_posbits(ua) : 0u;
-                    if (__any_sync(0xffffffffu, live && mb > 0.f)) cb1 = pos ? tcs_posbits(ub) : 0u;
+                    if (__any_sync(0xffffffffu, live && ma > 0)) cb0 = pos ? tcs_posbits(ua) : 0u;
+                    if (__any_sync(0xffffffffu, live && mb > 0)) cb1 = pos ? tcs_posbits(ub) : 0u;
                     tcs_append(a.list, a.gcount, a.cap, a.overflow, lane, cb0, cb1, (uint32_t)(blk.slot0[sub] + cg * 64), v, cur_end, &dead);
                 }
             }
